@@ -16,7 +16,6 @@
 
 #include "simt_kernels.cuh"
 #include "tc_kernels.cuh"
-#include "tc_gcnp.cuh"
 #include "tc_gcnt.cuh"
 #ifdef COSK_WITH_AGCNT  // k_tc_agcnt has never run on hardware: compiled in only on request (lib.py: COSK_WITH_AGCNT=1)
 #include "tc_agcnt.cuh"
@@ -32,6 +31,8 @@ typedef CUresult (*EncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t
                                   CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 
 inline int round_up(int x, int m) { return (x + m - 1) / m * m; }
+// q | k | v columns of the unfused tensor-core qkv conv (C = 64: 96 columns), padded to a temporal-conv kernel width
+constexpr int kSaQkvCols = 128;
 // ring slot of frame n (frames before the start of the stream, n < 0, map to slots that are still zero)
 inline int mod_slot(long long n, int slots) { return (int)(((n % slots) + slots) % slots); }
 
@@ -62,21 +63,17 @@ struct BlockW {
   CUtensorMap map_sa_w, map_sa_w_half;
   bool tc_sa_out = false, sa_res_kblock = false;
   ActBuf sa;  // attention output rows of the frame in flight (1 slot), operand of the output conv
-  // tensor-core qkv conv: normalised input rows, q | k | v rows (zero-padded to nq_pad columns), and the conv split into
-  // column chunks of a width the single-tap temporal-conv kernel is instantiated for
+  // tensor-core qkv conv: normalised input rows; unfused (C = 64), the conv runs on the single-tap temporal-conv kernel
+  // into q | k | v rows zero-padded to kSaQkvCols columns
   bool tc_sa_qkv = false;
   bool tc_sa_fused = false;  // qkv conv + attention in one kernel (k_tc_sa): q, k, v never leave the SM
   __nv_bfloat16 *d_sa_fw16 = nullptr;  // qkv weights regrouped per head group: [items][hi: q, k, v | lo: same][cin]
   float *d_sa_fbias = nullptr;         // [items][96]
   CUtensorMap map_sa_fw;
   ActBuf sa_x, sa_q;
-  int nq_pad = 0, n_qchunks = 0;
-  struct QChunk {
-    int width = 0, col0 = 0;
-    __nv_bfloat16 *w16 = nullptr;
-    float *bias = nullptr;
-    CUtensorMap map, map_half;
-  } qchunk[2];
+  __nv_bfloat16 *d_sa_qw16 = nullptr;  // unfused qkv conv: [2*kSaQkvCols rows (hi, lo)][cin]
+  float *d_sa_qbias = nullptr;
+  CUtensorMap map_sa_q;
   int mix_max_nz = 0;
   int gcn_parts = 4;  // accumulator column groups of the tensor-core graph conv (3 or 4)
   bool gcn_folded = false;  // gcn_residual folded into W_0 on the host (every self link exactly 1): no residual rows, three groups
@@ -86,9 +83,9 @@ struct BlockW {
   __nv_bfloat16 *d_gcn_w16 = nullptr, *d_tcn_w16 = nullptr, *d_att_w16 = nullptr;
   CUtensorMap map_gcn_w, map_tcn_w, map_tcn_w_half, map_att_w;  // _half: box of cout/2 rows for the CTA-pair kernel
   bool tc_gcn = false, tc_tcn = false;
-  // pre-mix graph conv (k_tc_gcnp): weights [2*cout rows (hi, lo)][gcnp_parts*cin], partition-major K
-  bool tc_gcnp = false, gcnp_stacked = false, gcnp_unit_diag = false;
-  bool gcnp_ready = false;  // weights of the pre-mix form are uploaded (k_tc_gcnp and the fused block kernel use them)
+  // pre-mix graph conv weights of the fused block kernel: [2*cout rows (hi, lo)][gcnp_parts*cin], partition-major K
+  bool gcnp_unit_diag = false;
+  bool gcnp_ready = false;  // weights of the pre-mix form are uploaded
   bool fuse = false;        // this block's step runs as ONE kernel (k_tc_block64)
   CUtensorMap map_tcn_w_full;  // temporal-conv weights with a 2*cout-row box: hi and lo rows in one stacked slab
 
@@ -103,13 +100,10 @@ struct BlockW {
   CUtensorMap map_gcnt_w;
   float gcnt_coef[3][32];
   bool tc_attn = false;  // adaptive graph conv: attention half on the tcgen05 kernel
-  bool gcn_res_in_mix = false;  // P = 3 plain graph conv: identity residual added by the mix warps (else by the drain warps)
   bool tcn_res_kblock = false;  // tensor-core temporal conv: the residual enters as extra K-blocks of the GEMM (folded
                                 // strided conv, or identity weights for the narrow layers) instead of epilogue loads
   long long n_in = 0, n_out = 0;
   ActBuf ring, out;
-  unsigned int *d_tile_cnt = nullptr;  // per-tile completion counters of this block's temporal conv (merged launches)
-  long long merge_ticket = 0;
 };
 
 struct ProfRec {
@@ -122,35 +116,12 @@ struct ProfRec {
 struct cosk_model {
   cosk_config cfg;
   int num_sms = 148;
-  int gcn_identity_mma = 3;  // COSK_GCN_IDENTITY_MMA: 1 = identity gcn_residual as a 4th GEMM column group everywhere, 0 = the drain
-                             // warps add the input rows instead, 2 = the mix warps do, 3 = per width (see prepare)
-  int tcn_reverse = 1;  // temporal convs walk tiles last-to-first so producer->consumer hand-offs hit L2 (COSK_TCN_REVERSE=0 disables)
-  int gcn_single_stage = 1;  // cin = 64 graph convs: 1 operand stage + 4 exchange buffers (COSK_GCN_SINGLE_STAGE=0: 2 stages + 1 buffer)
-  int merge = 0;           // temporal conv of block L + graph conv of block L+1 in one cooperative launch (COSK_MERGE=1);
-                           // off: both roles turned out to be limited per SM, so splitting the SMs between them loses
-  int merge_min_tiles = 4 * 148;  // below this the two CTA groups are not worth splitting (COSK_MERGE_MIN_TILES)
-  int merge_split64 = 100;  // CTAs given to the temporal-conv role (64-channel layers)
-  int merge_split128 = 92;  // same for the 128-channel layers (CTA pairs)
-  int sa_fused = 1;   // self-attention unit: qkv conv and attention fused in one tcgen05 kernel for C >= 128 (COSK_SA_FUSED=0: separate
-                      // launches everywhere, 2: fused everywhere)
-  int sa_qkv_tc = 1;  // qkv conv of the self-attention unit on the tcgen05 single-tap kernel (COSK_SA_QKV_TC=0: fp32 CUDA-core GEMM)
-  int attn_tc = 1;  // attention half of the adaptive graph conv on tcgen05 (COSK_ATTN_TC=0: fp32 CUDA-core kernel)
-  int agcn_tc = 1;  // adaptive graph conv on the tcgen05 kernels (COSK_AGCN_TC=0: fp32 CUDA-core kernels)
-  int tcn_identity_mma = 1;  // narrow temporal convs: identity residual as a K-block of the GEMM (COSK_TCN_IDENTITY_MMA=0: epilogue add)
-  int pdl = 1;  // programmatic dependent launch between the kernels of a step: +16 % at 256 streams, +4 % at 1024, neutral at 4096 (COSK_PDL=0 disables)
-  int gcn_premix = 0;  // which plain graph-conv widths run on the standalone pre-mix / A-in-TMEM kernel k_tc_gcnp (bit 0: 64, bit 1: 128,
-                       // bit 2: 256 output channels); the rest stays on k_tc_gcn (COSK_GCN_PREMIX).  Off: measured slower standalone
-                       // (profiles/r2a_gcnp_ab.txt) -- its CUDA-core mix only pays off hidden under the temporal conv's HBM stream
-  int gcn_fold_unit = 1;  // k_tc_gcn: fold the gcn_residual branch into W_0 when every self link is exactly 1 (COSK_GCN_FOLD_UNIT=0 disables)
   int gcn_transposed = 1;  // plain graph convs with cout in {128, 256}, cin in {64, 128} on a skeleton tree the kernel is compiled for run on
                            // k_tc_gcnt (channels on the TMEM lanes, adjacency contraction in registers); COSK_GCN_T=0: k_tc_gcn
   int agcn_transposed = 0;  // adaptive graph convs with cout in {128, 256}, cin in {64, 128}: dense mix on k_tc_agcnt.  OFF and not in the
                             // default build: the kernel was written after the round's GPU budget was spent and has never run on hardware
                             // (build with COSK_WITH_AGCNT=1, enable with COSK_AGCN_T=1, test with COSK_TEST_UNVERIFIED=1)
-  int gcnt_pack = 1;  // k_tc_gcnt: lane pairs trade tokens before the store (32-bit stores of two channels); COSK_GCNT_PACK=0: 16-bit stores
   int fuse_block = 1;  // 64 -> 64 identity-residual blocks: graph conv + temporal conv in one kernel per step (COSK_FUSE_BLOCK=0: two kernels)
-  int gcnp_stacked = 1;       // widths (bit 0: 64, bit 1: 128) using the stacked-B product form in k_tc_gcnp
-  int pair_mask = 6;  // which temporal-conv widths run on CTA pairs (bit 0: 64, bit 1: 128, bit 2: 256); COSK_TCN_PAIR
   EncodeTiledFn encode = nullptr;
   std::vector<BlockW> blk;
   std::vector<float> h_bn_scale, h_bn_shift, h_fc_w, h_fc_b;
@@ -227,7 +198,6 @@ void free_state(cosk_model *m) {
   for (auto &b : m->blk) {
     dfree(b.ring.ptr);
     dfree(b.out.ptr);
-    dfree(b.d_tile_cnt);
     dfree(b.sa.ptr);
     dfree(b.sa_x.ptr);
     dfree(b.sa_q.ptr);
@@ -414,29 +384,25 @@ int prepare(cosk_model *m) {
     if (attention)
       b.tc_gcn = false;  // qkv + attention run on CUDA cores this round; the output conv below is the tensor-core part
     else if (adaptive)  // dense-mix kernel: instantiated for the two skeleton sizes the reference ships
-      b.tc_gcn = want_tc && m->agcn_tc && bc.cout % 64 == 0 && bc.cout <= 256 && bc.cin % kBK == 0 && (V == 25 || V == 18);
+      b.tc_gcn = want_tc && bc.cout % 64 == 0 && bc.cout <= 256 && bc.cin % kBK == 0 && (V == 25 || V == 18);
     else
       b.tc_gcn = want_tc && bc.cout % 64 == 0 && bc.cout <= 256 && bc.cin % kBK == 0 && b.mix_max_row12 <= kMixSlots && b.mix_diag0;
     b.tc_tcn = want_tc && tc_width(bc.cout) && (bc.res_kind != COSK_RES_CONV || bc.cin % kBK == 0);
     if (b.tc_gcn) {
       // Rows regrouped per pass of 64 output channels: row = pass*(P*64) + part*64 + c, K = cin.
       // Part 3 is the gcn_residual branch: the folded 1x1 conv when cin != cout, else the identity
-      // matrix (x = hi + lo passes through the split-precision products exactly).  The P = 3 variant of
-      // the kernel (identity added from the input rows by the drain warps) exists but measured slower:
-      // its row-per-thread global loads cost more load/store-unit cycles than the extra MMA columns.
+      // matrix (x = hi + lo passes through the split-precision products exactly).  The identity rides in the GEMM
+      // except for the 256-channel layers, where the mix warps have the slack to add the input rows and the narrower
+      // accumulator saves MMA columns and TMEM reads (measured -8 %).
       // (adaptive: 4 parts need the single-stage layout, so the identity rides along only when one K-block is all there is)
-      // mode 3 (default): the identity rides in the GEMM except for the 256-channel layers, where the mix warps have the
-      // slack to add the input rows and the narrower accumulator saves MMA columns and TMEM reads (measured -8 %)
-      const bool ident_mma = m->gcn_identity_mma == 1 || (m->gcn_identity_mma == 3 && bc.cin < 256);
-      b.gcn_res_in_mix = m->gcn_identity_mma >= 2;
+      const bool ident_mma = bc.cin < 256;
       // Every self link exactly 1 (A_0 = I with graph_attn's diagonal at 1, the reference initialisation): the own-row term of
       // partition 0 and the gcn_residual branch act on the same rows, x W_0^T + x R^T = x (W_0 + R)^T, so the residual (identity
       // or folded conv) is added into W_0 on the host and the accumulator shrinks to three column groups: a quarter fewer MMAs
       // and TMEM reads, no residual rows fetched.  Trained self-link coefficients keep the four-group form.
-      bool unit_diag = !adaptive && b.mix_diag0 && m->gcn_fold_unit;
+      bool unit_diag = !adaptive && b.mix_diag0;
       for (int w0 = 0; unit_diag && w0 < V; ++w0) unit_diag = (ptr[w0 + 1] - ptr[w0] == 1 && val[ptr[w0]] == 1.0f);
       b.gcn_folded = unit_diag;
-      if (unit_diag) b.gcn_res_in_mix = false;
       const int P = b.gcn_parts = adaptive ? ((res_conv || bc.cin == kBK) ? 4 : 3) : (unit_diag ? 3 : ((res_conv || ident_mma) ? 4 : 3));
       std::vector<float> re((size_t)P * bc.cout * bc.cin, 0.f);
       for (int o = 0; o < bc.cout; ++o)
@@ -526,13 +492,11 @@ int prepare(cosk_model *m) {
       b.tc_agcnt = true;
     }
     {
-      // pre-mix kernel: sources per (partition >= 1, output vertex) must fit its register CSR
+      // pre-mix form of the fused block kernel: sources per (partition >= 1, output vertex) must fit its register CSR
       int part_max = 0;
       for (int p = 1; p < 3; ++p)
         for (int w = 0; w < V; ++w) part_max = std::max(part_max, ptr[p * V + w + 1] - ptr[p * V + w]);
-      const int wbit = bc.cout == 64 ? 1 : bc.cout == 128 ? 2 : 4;
       b.gcnp_ready = b.tc_gcn && !adaptive && !attention && tc_width(bc.cout) && part_max <= kPartSrcMax;
-      b.tc_gcnp = b.gcnp_ready && (m->gcn_premix & wbit);
       if (b.gcnp_ready) {
         b.gcnp_unit_diag = true;
         for (int w0 = 0; w0 < V; ++w0) b.gcnp_unit_diag &= (ptr[w0 + 1] - ptr[w0] == 1 && val[ptr[w0]] == 1.0f);
@@ -556,7 +520,6 @@ int prepare(cosk_model *m) {
         std::vector<uint16_t> s = split_rows(w, bc.cout, K);
         if ((rc = upload(m, reinterpret_cast<uint16_t *&>(b.d_gcnp_w16), s.data(), s.size()))) return rc;
         if ((rc = make_map(m, &b.map_gcnp_w, b.d_gcnp_w16, (uint64_t)K, (uint64_t)2 * bc.cout, (uint32_t)std::min(2 * bc.cout, 256)))) return rc;
-        b.gcnp_stacked = bc.cout <= 128 && (m->gcnp_stacked & wbit);
       }
     }
     if (attention) {
@@ -565,34 +528,20 @@ int prepare(cosk_model *m) {
       if ((rc = upload(m, b.d_sa_qkv_b, b.sa_qkv_b.data(), b.sa_qkv_b.size()))) return rc;
       if ((rc = upload(m, b.d_sa_scale, b.sa_scale.data(), b.sa_scale.size()))) return rc;
       if ((rc = upload(m, b.d_sa_shift, b.sa_shift.data(), b.sa_shift.size()))) return rc;
-      b.tc_sa_qkv = want_tc && m->sa_qkv_tc && bc.cin % kBK == 0 && tc_width(bc.cout);
-      if (b.tc_sa_qkv) {
-        const int nq = 2 * (bc.cout / 4) + bc.cout;
-        b.n_qchunks = bc.cout == 256 ? 2 : 1;
-        b.qchunk[0].width = bc.cout == 64 ? 128 : 256;
-        b.qchunk[0].col0 = 0;
-        b.qchunk[1].width = 128;
-        b.qchunk[1].col0 = 256;
-        b.nq_pad = bc.cout == 64 ? 128 : bc.cout == 128 ? 256 : 384;
-        for (int q = 0; q < b.n_qchunks; ++q) {
-          BlockW::QChunk &qc = b.qchunk[q];
-          std::vector<float> w((size_t)qc.width * bc.cin, 0.f), bb((size_t)qc.width, 0.f);
-          for (int r = 0; r < qc.width; ++r) {
-            const int src = qc.col0 + r;
-            if (src >= nq) continue;  // zero padding
-            memcpy(&w[(size_t)r * bc.cin], &b.sa_qkv_w[(size_t)src * bc.cin], sizeof(float) * bc.cin);
-            bb[r] = b.sa_qkv_b[src];
-          }
-          std::vector<uint16_t> s16 = split_rows(w, qc.width, bc.cin);
-          if ((rc = upload(m, reinterpret_cast<uint16_t *&>(qc.w16), s16.data(), s16.size()))) return rc;
-          if ((rc = upload(m, qc.bias, bb.data(), bb.size()))) return rc;
-          if ((rc = make_map(m, &qc.map, qc.w16, (uint64_t)bc.cin, (uint64_t)2 * qc.width, (uint32_t)qc.width))) return rc;
-          if ((rc = make_map(m, &qc.map_half, qc.w16, (uint64_t)bc.cin, (uint64_t)2 * qc.width, (uint32_t)qc.width / 2))) return rc;
-        }
-      }
+      b.tc_sa_qkv = want_tc && bc.cin % kBK == 0 && tc_width(bc.cout);
       // the fused kernel has eight epilogue warps per SM for the attention math: a win where the q | k | v round trip
       // dominates (C >= 128), a loss for the 64-channel unit, whose eight tiny heads want the separate kernel's occupancy
-      b.tc_sa_fused = b.tc_sa_qkv && (m->sa_fused == 2 || (m->sa_fused == 1 && bc.cout >= 128));
+      b.tc_sa_fused = b.tc_sa_qkv && bc.cout >= 128;
+      if (b.tc_sa_qkv && !b.tc_sa_fused) {
+        const int nq = 2 * (bc.cout / 4) + bc.cout;
+        std::vector<float> w((size_t)kSaQkvCols * bc.cin, 0.f), bb((size_t)kSaQkvCols, 0.f);  // rows nq.. stay zero
+        memcpy(w.data(), b.sa_qkv_w.data(), sizeof(float) * nq * bc.cin);
+        memcpy(bb.data(), b.sa_qkv_b.data(), sizeof(float) * nq);
+        std::vector<uint16_t> s16 = split_rows(w, kSaQkvCols, bc.cin);
+        if ((rc = upload(m, reinterpret_cast<uint16_t *&>(b.d_sa_qw16), s16.data(), s16.size()))) return rc;
+        if ((rc = upload(m, b.d_sa_qbias, bb.data(), bb.size()))) return rc;
+        if ((rc = make_map(m, &b.map_sa_q, b.d_sa_qw16, (uint64_t)bc.cin, (uint64_t)2 * kSaQkvCols, (uint32_t)kSaQkvCols))) return rc;
+      }
       if (b.tc_sa_fused) {
         const int dk = bc.cout / 4, dvh = bc.cout / 8, dkh = dk / 8, G = 64 / dvh, items = 8 / G;
         std::vector<float> w((size_t)items * 96 * bc.cin), bb((size_t)items * 96);
@@ -640,7 +589,7 @@ int prepare(cosk_model *m) {
         if ((rc = make_map(m, &b.map_sa_w_half, b.d_sa_w16, (uint64_t)(K0 + Kr), (uint64_t)2 * bc.cout, (uint32_t)bc.cout / 2))) return rc;
       }
     }
-    b.tc_attn = adaptive && b.tc_gcn && m->attn_tc && tc_width(bc.cout);
+    b.tc_attn = adaptive && b.tc_gcn && tc_width(bc.cout);
     if (b.tc_attn) {
       // per partition: hi rows of (theta, phi), then their lo rows -- one stacked operand of 4*IC rows
       const int ic = bc.cout / 4;
@@ -661,7 +610,7 @@ int prepare(cosk_model *m) {
       // strided 1x1 conv as its weights (layers 5 and 8), or -- for the identity residual of the HBM-bound
       // narrow layers -- with identity weights (exact under the split products), which removes every
       // latency-bound load from the epilogue.  The 256-channel layers are tensor-bound and keep the add.
-      const bool ident_k = bc.res_kind == COSK_RES_IDENTITY && bc.cout <= 128 && m->tcn_identity_mma;
+      const bool ident_k = bc.res_kind == COSK_RES_IDENTITY && bc.cout <= 128;
       b.tcn_res_kblock = bc.res_kind == COSK_RES_CONV || ident_k;
       const int Kr = b.tcn_res_kblock ? bc.cin : 0;
       std::vector<float> cat((size_t)bc.cout * (Kt + Kr));
@@ -694,9 +643,7 @@ int zero_state(cosk_model *m, cudaStream_t s) {
   for (auto &b : m->blk) {
     CK(cudaMemsetAsync(b.ring.ptr, 0, b.ring.bytes(), s));
     CK(cudaMemsetAsync(b.out.ptr, 0, b.out.bytes(), s));
-    CK(cudaMemsetAsync(b.d_tile_cnt, 0, sizeof(unsigned int) * (size_t)(m->n_tiles + 2), s));
     b.n_in = b.n_out = 0;
-    b.merge_ticket = 0;
   }
   if (m->cfg.classes > 0) {
     const size_t cl = (size_t)m->cfg.blocks[m->cfg.n_blocks - 1].cout;
@@ -712,10 +659,10 @@ int zero_state(cosk_model *m, cudaStream_t s) {
   return COSK_OK;
 }
 
-// Every kernel goes through here: with PDL the launch carries the programmatic-stream-serialization
-// attribute (the kernels call griddepcontrol.wait before touching their predecessor's output).
+// Every kernel goes through here: the launch carries the programmatic-stream-serialization attribute (PDL; the kernels
+// call griddepcontrol.wait before touching their predecessor's output): +16 % at 256 streams, +4 % at 1024, neutral at 4096.
 template <typename... KArgs, typename... Args>
-cudaError_t launch_k(cosk_model *m, void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t s, Args &&...args) {
+cudaError_t launch_k(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t s, Args &&...args) {
   cudaLaunchConfig_t cfg = {};
   cfg.gridDim = grid;
   cfg.blockDim = block;
@@ -725,7 +672,7 @@ cudaError_t launch_k(cosk_model *m, void (*kernel)(KArgs...), dim3 grid, dim3 bl
   attr[0].id = cudaLaunchAttributeProgrammaticStreamSerialization;
   attr[0].val.programmaticStreamSerializationAllowed = 1;
   cfg.attrs = attr;
-  cfg.numAttrs = m->pdl ? 1 : 0;
+  cfg.numAttrs = 1;
   return cudaLaunchKernelEx(&cfg, kernel, std::forward<Args>(args)...);
 }
 
@@ -742,46 +689,48 @@ int prof_mark(cosk_model *m, int kind, int block, cudaStream_t s) {
   return COSK_OK;
 }
 
+// The launchers size their grids for the (frame, tile) work items of `args`: n_tiles * n_frames, at most one CTA per SM.
 template <int COUT>
 int launch_tc_tcn(cosk_model *m, const TcTcnArgs &args, cudaStream_t s) {
-  const int grid = m->n_tiles < m->num_sms ? m->n_tiles : m->num_sms;
-  CK(launch_k(m, k_tc_tcn<COUT>, dim3(grid), dim3(256), TcTcnCfg<COUT>::kSmemBytes, s, args));
+  const int items = m->n_tiles * args.n_frames;
+  const int grid = items < m->num_sms ? items : m->num_sms;
+  CK(launch_k(k_tc_tcn<COUT>, dim3(grid), dim3(256), TcTcnCfg<COUT>::kSmemBytes, s, args));
   return COSK_OK;
 }
 template <int COUT>
 int launch_tc_tcn2(cosk_model *m, const TcTcnArgs &args, cudaStream_t s) {
   // CTA pairs: one cluster of 2 per pair of adjacent token tiles, at most one CTA per SM
-  const int n_pairs = (m->n_tiles + 1) / 2;
+  const int n_pairs = (m->n_tiles + 1) / 2 * args.n_frames;
   const int max_clusters = m->num_sms / 2;
   const int grid = 2 * (n_pairs < max_clusters ? n_pairs : max_clusters);
-  CK(launch_k(m, k_tc_tcn2<COUT>, dim3(grid), dim3(256), TcTcn2Cfg<COUT>::kSmemBytes, s, args));
+  CK(launch_k(k_tc_tcn2<COUT>, dim3(grid), dim3(256), TcTcn2Cfg<COUT>::kSmemBytes, s, args));
   return COSK_OK;
 }
 template <int P, int STAGES>
 int launch_tc_gcn(cosk_model *m, const TcGcnArgs &args, cudaStream_t s) {
-  const int grid = m->n_tiles < m->num_sms ? m->n_tiles : m->num_sms;
-  if (m->d_trace) CK(launch_k(m, k_tc_gcn<P, STAGES, true>, dim3(grid), dim3(512), TcGcnCfg<P, STAGES>::kSmemBytes, s, args));
-  else CK(launch_k(m, k_tc_gcn<P, STAGES, false>, dim3(grid), dim3(512), TcGcnCfg<P, STAGES>::kSmemBytes, s, args));
+  const int items = m->n_tiles * args.n_frames;
+  const int grid = items < m->num_sms ? items : m->num_sms;
+  if (m->d_trace) CK(launch_k(k_tc_gcn<P, STAGES, true>, dim3(grid), dim3(512), TcGcnCfg<P, STAGES>::kSmemBytes, s, args));
+  else CK(launch_k(k_tc_gcn<P, STAGES, false>, dim3(grid), dim3(512), TcGcnCfg<P, STAGES>::kSmemBytes, s, args));
   return COSK_OK;
 }
 
 template <int P, int STAGES, int V>
 int launch_tc_agcn(cosk_model *m, const TcGcnArgs &args, cudaStream_t s) {
   const int grid = m->n_tiles < m->num_sms ? m->n_tiles : m->num_sms;
-  CK(launch_k(m, k_tc_agcn<P, STAGES, V>, dim3(grid), dim3(512), TcAgcnCfg<P, STAGES>::kSmemBytes, s, args));
+  CK(launch_k(k_tc_agcn<P, STAGES, V>, dim3(grid), dim3(512), TcAgcnCfg<P, STAGES>::kSmemBytes, s, args));
   return COSK_OK;
 }
 
 template <int IC, int V>
 int launch_tc_attn(cosk_model *m, const TcAttnArgs &args, cudaStream_t s) {
   const int grid = m->n_tiles < m->num_sms ? m->n_tiles : m->num_sms;
-  CK(launch_k(m, k_tc_attn<IC, V>, dim3(grid), dim3(384), TcAttnCfg<IC, V>::kSmemBytes, s, args));
+  CK(launch_k(k_tc_attn<IC, V>, dim3(grid), dim3(384), TcAttnCfg<IC, V>::kSmemBytes, s, args));
   return COSK_OK;
 }
 
 int set_smem_attrs(cosk_model *m) {
   CK(cudaFuncSetAttribute(k_agcn_attn, cudaFuncAttributeMaxDynamicSharedMemorySize, kAttnMaxSmem));
-  CK(cudaFuncSetAttribute(k_tc_sa<8>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcSaCfg<8>::kSmemBytes));
   CK(cudaFuncSetAttribute(k_tc_sa<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcSaCfg<16>::kSmemBytes));
   CK(cudaFuncSetAttribute(k_tc_sa<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcSaCfg<32>::kSmemBytes));
   CK(cudaFuncSetAttribute(k_tc_attn<16, 25>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcAttnCfg<16, 25>::kSmemBytes));
@@ -797,7 +746,6 @@ int set_smem_attrs(cosk_model *m) {
   CK(cudaFuncSetAttribute(k_tc_tcn<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcTcnCfg<64>::kSmemBytes));
   CK(cudaFuncSetAttribute(k_tc_tcn<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcTcnCfg<128>::kSmemBytes));
   CK(cudaFuncSetAttribute(k_tc_tcn<256>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcTcnCfg<256>::kSmemBytes));
-  CK(cudaFuncSetAttribute(k_tc_tcn2<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcTcn2Cfg<64>::kSmemBytes));
   CK(cudaFuncSetAttribute(k_tc_tcn2<128>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcTcn2Cfg<128>::kSmemBytes));
   CK(cudaFuncSetAttribute(k_tc_tcn2<256>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcTcn2Cfg<256>::kSmemBytes));
   CK(cudaFuncSetAttribute(k_tc_gcn<3, 1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcGcnCfg<3, 1>::kSmemBytes));
@@ -808,11 +756,6 @@ int set_smem_attrs(cosk_model *m) {
   CK(cudaFuncSetAttribute(k_tc_gcn<4, 1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcGcnCfg<4, 1>::kSmemBytes));
   CK(cudaFuncSetAttribute(k_tc_gcn<4, 2, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcGcnCfg<4, 2>::kSmemBytes));
   CK(cudaFuncSetAttribute(k_tc_gcn<4, 2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcGcnCfg<4, 2>::kSmemBytes));
-  CK(cudaFuncSetAttribute(k_tc_gcnp<64, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcGcnpCfg<64, true>::kSmemBytes));
-  CK(cudaFuncSetAttribute(k_tc_gcnp<64, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcGcnpCfg<64, false>::kSmemBytes));
-  CK(cudaFuncSetAttribute(k_tc_gcnp<128, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcGcnpCfg<128, true>::kSmemBytes));
-  CK(cudaFuncSetAttribute(k_tc_gcnp<128, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcGcnpCfg<128, false>::kSmemBytes));
-  CK(cudaFuncSetAttribute(k_tc_gcnp<256, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcGcnpCfg<256, false>::kSmemBytes));
   CK(cudaFuncSetAttribute(k_tc_block64, cudaFuncAttributeMaxDynamicSharedMemorySize, TcBlockCfg::kSmemBytes));
 #ifdef COSK_WITH_AGCNT
   CK(cudaFuncSetAttribute(k_tc_agcnt<25, 1, 128>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcAgcntCfg<25, 1>::kSmemBytes));
@@ -828,10 +771,6 @@ int set_smem_attrs(cosk_model *m) {
   CK(cudaFuncSetAttribute(k_tc_gcnt<18, 1, 128>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcGcntCfg<18, 1>::kSmemBytes));
   CK(cudaFuncSetAttribute(k_tc_gcnt<18, 2, 128>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcGcntCfg<18, 2>::kSmemBytes));
   CK(cudaFuncSetAttribute(k_tc_gcnt<18, 2, 256>, cudaFuncAttributeMaxDynamicSharedMemorySize, TcGcntCfg<18, 2>::kSmemBytes));
-  CK(cudaFuncSetAttribute(k_tc_tcn_gcn<64, 4, 1>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                          std::max(TcTcnCfg<64>::kSmemBytes, TcGcnCfg<4, 1>::kSmemBytes)));
-  CK(cudaFuncSetAttribute(k_tc_tcn2_gcn<128, 4, 2>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                          std::max(TcTcn2Cfg<128>::kSmemBytes, TcGcnCfg<4, 2>::kSmemBytes)));
   return COSK_OK;
 }
 
@@ -853,10 +792,8 @@ TcGcnArgs make_gcn_args(cosk_model *m, int i, const ActBuf &in, int in_slot, int
   a.mix_src = b.d_mix_src;
   a.mix_val = b.d_mix_val;
   a.trace = m->d_trace;
-  a.wait_cnt = nullptr;
-  a.wait_need = 0;
   a.epi.bias = b.d_gcn_b;
-  const bool epi_res = b.gcn_parts == 3 && !b.gcn_folded;  // identity gcn_residual added from the input rows by the drain / mix warps
+  const bool epi_res = b.gcn_parts == 3 && !b.gcn_folded;  // identity gcn_residual added from the input rows by the epilogue
   a.epi.r_hi = epi_res ? in.hi(in_slot) : nullptr;
   a.epi.r_lo = epi_res ? in.lo(in_slot) : nullptr;
   a.epi.cs_r = in.cs;
@@ -867,7 +804,6 @@ TcGcnArgs make_gcn_args(cosk_model *m, int i, const ActBuf &in, int in_slot, int
   a.dense = m->d_dense;
   a.dense_ld = 3 * m->dense_vp;
   a.dense_vp = m->dense_vp;
-  a.res_in_mix = b.gcn_res_in_mix ? 1 : 0;
   return a;
 }
 
@@ -881,19 +817,18 @@ int launch_tc_gcnt(cosk_model *m, int i, TcGcnArgs a, cudaStream_t s) {
   t.g.epi.r_hi = t.g.epi.r_lo = nullptr;  // gcn_residual always rides in the GEMM here
   memcpy(t.coef, b.gcnt_coef, sizeof t.coef);
   t.n_parts = b.gcnt_parts;
-  t.pack = m->gcnt_pack;
   const int items = ((m->n_tiles + 1) / 2) * a.n_frames;
   const dim3 grid(items < m->num_sms ? items : m->num_sms), block(384);
   const bool v25 = m->cfg.vertices == 25;
   if (bc.cout == 128 && bc.cin == 64) {
-    if (v25) CK(launch_k(m, k_tc_gcnt<25, 1, 128>, grid, block, TcGcntCfg<25, 1>::kSmemBytes, s, t));
-    else CK(launch_k(m, k_tc_gcnt<18, 1, 128>, grid, block, TcGcntCfg<18, 1>::kSmemBytes, s, t));
+    if (v25) CK(launch_k(k_tc_gcnt<25, 1, 128>, grid, block, TcGcntCfg<25, 1>::kSmemBytes, s, t));
+    else CK(launch_k(k_tc_gcnt<18, 1, 128>, grid, block, TcGcntCfg<18, 1>::kSmemBytes, s, t));
   } else if (bc.cout == 128) {
-    if (v25) CK(launch_k(m, k_tc_gcnt<25, 2, 128>, grid, block, TcGcntCfg<25, 2>::kSmemBytes, s, t));
-    else CK(launch_k(m, k_tc_gcnt<18, 2, 128>, grid, block, TcGcntCfg<18, 2>::kSmemBytes, s, t));
+    if (v25) CK(launch_k(k_tc_gcnt<25, 2, 128>, grid, block, TcGcntCfg<25, 2>::kSmemBytes, s, t));
+    else CK(launch_k(k_tc_gcnt<18, 2, 128>, grid, block, TcGcntCfg<18, 2>::kSmemBytes, s, t));
   } else {
-    if (v25) CK(launch_k(m, k_tc_gcnt<25, 2, 256>, grid, block, TcGcntCfg<25, 2>::kSmemBytes, s, t));
-    else CK(launch_k(m, k_tc_gcnt<18, 2, 256>, grid, block, TcGcntCfg<18, 2>::kSmemBytes, s, t));
+    if (v25) CK(launch_k(k_tc_gcnt<25, 2, 256>, grid, block, TcGcntCfg<25, 2>::kSmemBytes, s, t));
+    else CK(launch_k(k_tc_gcnt<18, 2, 256>, grid, block, TcGcntCfg<18, 2>::kSmemBytes, s, t));
   }
   return COSK_OK;
 }
@@ -912,58 +847,21 @@ int launch_tc_agcnt(cosk_model *m, int i, TcGcnArgs a, cudaStream_t s) {
   t.g.epi.r_hi = t.g.epi.r_lo = nullptr;  // gcn_residual rides in the GEMM as the fourth part
   memset(t.coef, 0, sizeof t.coef);
   t.n_parts = 4;
-  t.pack = 1;
   const int items = m->n_tiles * a.n_frames;
   const dim3 grid(items < m->num_sms ? items : m->num_sms), block(384);
   const bool v25 = m->cfg.vertices == 25;
   if (bc.cout == 128 && bc.cin == 64) {
-    if (v25) CK(launch_k(m, k_tc_agcnt<25, 1, 128>, grid, block, TcAgcntCfg<25, 1>::kSmemBytes, s, t));
-    else CK(launch_k(m, k_tc_agcnt<18, 1, 128>, grid, block, TcAgcntCfg<18, 1>::kSmemBytes, s, t));
+    if (v25) CK(launch_k(k_tc_agcnt<25, 1, 128>, grid, block, TcAgcntCfg<25, 1>::kSmemBytes, s, t));
+    else CK(launch_k(k_tc_agcnt<18, 1, 128>, grid, block, TcAgcntCfg<18, 1>::kSmemBytes, s, t));
   } else if (bc.cout == 128) {
-    if (v25) CK(launch_k(m, k_tc_agcnt<25, 2, 128>, grid, block, TcAgcntCfg<25, 2>::kSmemBytes, s, t));
-    else CK(launch_k(m, k_tc_agcnt<18, 2, 128>, grid, block, TcAgcntCfg<18, 2>::kSmemBytes, s, t));
+    if (v25) CK(launch_k(k_tc_agcnt<25, 2, 128>, grid, block, TcAgcntCfg<25, 2>::kSmemBytes, s, t));
+    else CK(launch_k(k_tc_agcnt<18, 2, 128>, grid, block, TcAgcntCfg<18, 2>::kSmemBytes, s, t));
   } else {
-    if (v25) CK(launch_k(m, k_tc_agcnt<25, 2, 256>, grid, block, TcAgcntCfg<25, 2>::kSmemBytes, s, t));
-    else CK(launch_k(m, k_tc_agcnt<18, 2, 256>, grid, block, TcAgcntCfg<18, 2>::kSmemBytes, s, t));
+    if (v25) CK(launch_k(k_tc_agcnt<25, 2, 256>, grid, block, TcAgcntCfg<25, 2>::kSmemBytes, s, t));
+    else CK(launch_k(k_tc_agcnt<18, 2, 256>, grid, block, TcAgcntCfg<18, 2>::kSmemBytes, s, t));
   }
   return COSK_OK;
 #endif
-}
-
-TcGcnpArgs make_gcnp_args(cosk_model *m, int i, const ActBuf &in, int in_slot, int ring_slot) {
-  const cosk_block_cfg &bc = m->cfg.blocks[i];
-  BlockW &b = m->blk[i];
-  TcGcnpArgs a;
-  a.tm_x = in.map;
-  a.tm_w = b.map_gcnp_w;
-  a.x_row = (int)in.row_hi(in_slot);
-  a.t_alloc = (int)m->t_alloc;
-  a.cin = bc.cin;
-  a.n_parts = b.gcnp_parts;
-  a.V = m->cfg.vertices;
-  a.n_tiles = m->n_tiles;
-  a.tile_tokens = m->tile_tokens;
-  a.n_tokens = m->n_tokens;
-  a.mix_ptr = b.d_mix_ptr;
-  a.mix_src = b.d_mix_src;
-  a.mix_val = b.d_mix_val;
-  a.trace = m->d_trace;
-  a.epi.bias = b.d_gcn_b;
-  a.epi.r_hi = nullptr;  // gcn_residual rides in the GEMM
-  a.epi.r_lo = nullptr;
-  a.epi.cs_r = in.cs;
-  a.epi.y_hi = b.ring.hi(ring_slot);
-  a.epi.y_lo = b.ring.lo(ring_slot);
-  a.epi.cs_out = b.ring.cs;
-  a.dbg = m->d_dbg;
-  return a;
-}
-
-template <int COUT, bool STACKED>
-int launch_tc_gcnp(cosk_model *m, const TcGcnpArgs &args, cudaStream_t s) {
-  const int grid = m->n_tiles < m->num_sms ? m->n_tiles : m->num_sms;
-  CK(launch_k(m, k_tc_gcnp<COUT, STACKED>, dim3(grid), dim3(512), TcGcnpCfg<COUT, STACKED>::kSmemBytes, s, args));
-  return COSK_OK;
 }
 
 TcTcnArgs make_tcn_args(cosk_model *m, int i, const ActBuf &in, int res_slot, long long n, int out_slot) {
@@ -981,7 +879,7 @@ TcTcnArgs make_tcn_args(cosk_model *m, int i, const ActBuf &in, int res_slot, lo
   a.kb_res = b.tcn_res_kblock ? bc.cin / kBK : 0;
   a.n_tiles = m->n_tiles;
   a.tile_tokens = m->tile_tokens;
-  a.reverse = m->tcn_reverse;
+  a.reverse = 1;
   a.n_tokens = m->n_tokens;
   a.epi.bias = b.d_tcn_b;
   const bool epi_res = bc.res_kind == COSK_RES_IDENTITY && !b.tcn_res_kblock;
@@ -991,75 +889,38 @@ TcTcnArgs make_tcn_args(cosk_model *m, int i, const ActBuf &in, int res_slot, lo
   a.epi.y_hi = b.out.hi(out_slot);
   a.epi.y_lo = b.out.lo(out_slot);
   a.epi.cs_out = b.out.cs;
-  a.tile_cnt = nullptr;
   a.trace = m->d_trace;
   a.dbg = m->d_dbg;
   return a;
 }
 
-// The temporal conv of block i and the graph conv of block i+1 in one cooperative launch (k_tc_tcn_gcn):
-// possible when both run on the tensor-core kernels, the temporal conv is one of the HBM-bound widths and
-// there are enough tiles to feed both CTA groups.
-bool can_merge(const cosk_model *m, int i) {
-  if (!m->merge || i + 1 >= m->cfg.n_blocks || m->d_trace || m->cfg.blocks[i + 1].gconv != COSK_GCONV_PLAIN) return false;
-  const BlockW &b = m->blk[i], &nb = m->blk[i + 1];
-  const int c = m->cfg.blocks[i].cout;
-  if (!b.tc_tcn || !nb.tc_gcn || nb.tc_gcnp || nb.tc_gcnt || nb.fuse || nb.gcn_parts != 4 || b.d_tile_cnt == nullptr) return false;
-  if (m->n_tiles < m->merge_min_tiles) return false;
-  if (c == 64) return m->gcn_single_stage && !(m->pair_mask & 1);
-  if (c == 128) return (m->pair_mask & 2) != 0;
-  return false;
-}
+// The 128- and 256-channel temporal convs run on CTA pairs (k_tc_tcn2) once there are two tiles to pair; the HBM-bound
+// 64-channel ones stay on single CTAs.
+bool tcn_on_pair(const cosk_model *m, int width) { return m->n_tiles >= 2 && (width == 128 || width == 256); }
 
-int run_tcn_gcn(cosk_model *m, int i, const ActBuf &in, int res_slot, long long n, int out_slot, cudaStream_t s) {
-  BlockW &b = m->blk[i], &nb = m->blk[i + 1];
-  const int c = m->cfg.blocks[i].cout;
-  int rc = prof_mark(m, 2, i, s);
-  if (rc) return rc;
-  TcTcnArgs ta = make_tcn_args(m, i, in, res_slot, n, out_slot);
-  // the graph conv of block i+1 reads the output slot written here and pushes into its own ring
-  const long long n_next = nb.n_in;
-  TcGcnArgs ga = make_gcn_args(m, i + 1, b.out, out_slot, (int)(n_next % m->R));
-  ta.reverse = 0;  // tiles are produced first to last, the order in which the other role consumes them
-  ta.tile_cnt = b.d_tile_cnt;
-  ga.wait_cnt = b.d_tile_cnt;
-  ga.wait_need = 4u * (unsigned)(++b.merge_ticket);  // four epilogue warps announce every tile of every launch
-  const int grid = m->num_sms & ~1;
-  int n_tcn = c == 64 ? m->merge_split64 : m->merge_split128;
-  n_tcn = (n_tcn < 2 ? 2 : (n_tcn > grid - 2 ? grid - 2 : n_tcn)) & ~1;
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(grid);
-  cfg.blockDim = dim3(512);
-  cfg.stream = s;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeCooperative;  // every CTA resident: the waiting role cannot starve the producer
-  attr[0].val.cooperative = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  if (c == 64) {
-    cfg.dynamicSmemBytes = std::max(TcTcnCfg<64>::kSmemBytes, TcGcnCfg<4, 1>::kSmemBytes);
-    CK(cudaLaunchKernelEx(&cfg, k_tc_tcn_gcn<64, 4, 1>, ta, ga, n_tcn));
-  } else {
-    cfg.dynamicSmemBytes = std::max(TcTcn2Cfg<128>::kSmemBytes, TcGcnCfg<4, 2>::kSmemBytes);
-    CK(cudaLaunchKernelEx(&cfg, k_tc_tcn2_gcn<128, 4, 2>, ta, ga, n_tcn));
-  }
-  m->launches++;
-  return COSK_OK;
-}
-
-// The temporal-conv kernel as a plain token-major GEMM of output width `width` (64 / 128 / 256), on CTA pairs where the
-// temporal convs of that width use them; `half` is the weight map with half-height boxes the 256-wide pair kernel wants.
-int launch_onetap(cosk_model *m, int width, TcTcnArgs &a, const CUtensorMap &half, cudaStream_t s) {
-  const bool pair = m->n_tiles >= 2 && (m->pair_mask & (width == 64 ? 1 : width == 128 ? 2 : 4));
-  if (pair) {
+// The temporal-conv kernel of output width `width` (64 / 128 / 256): the 9-tap conv of a block, or a plain token-major GEMM
+// with one tap.  `half` is the weight map with half-height boxes the 256-wide pair kernel wants.
+int launch_tcn(cosk_model *m, int width, TcTcnArgs &a, const CUtensorMap &half, cudaStream_t s) {
+  if (tcn_on_pair(m, width)) {
+    // stacked-B width (128): CTA 0 loads the whole hi plane, CTA 1 the whole lo plane (full-height box);
+    // C = 256: each CTA loads its half of the rows of both planes
     if (width > 128) a.tm_w = half;
-    if (width == 64) return launch_tc_tcn2<64>(m, a, s);
     if (width == 128) return launch_tc_tcn2<128>(m, a, s);
     return launch_tc_tcn2<256>(m, a, s);
   }
   if (width == 64) return launch_tc_tcn<64>(m, a, s);
   if (width == 128) return launch_tc_tcn<128>(m, a, s);
   return launch_tc_tcn<256>(m, a, s);
+}
+
+// Plain graph conv on the tensor cores: channel-major k_tc_gcnt where the skeleton tree allows, else token-major k_tc_gcn.
+int launch_gcn(cosk_model *m, int i, const TcGcnArgs &a, cudaStream_t s) {
+  const BlockW &b = m->blk[i];
+  if (b.tc_gcnt) return launch_tc_gcnt(m, i, a, s);
+  // one K-block per work item (cin = 64): single operand stage, four exchange buffers
+  const bool one_kb = m->cfg.blocks[i].cin == kBK;
+  if (b.gcn_parts == 4) return one_kb ? launch_tc_gcn<4, 1>(m, a, s) : launch_tc_gcn<4, 2>(m, a, s);
+  return one_kb ? launch_tc_gcn<3, 1>(m, a, s) : launch_tc_gcn<3, 2>(m, a, s);
 }
 
 // Self-attention unit of CoS-TR (GcnUnitAttention, only_attention): qkv conv on the data_bn-normalised frame, 8-head
@@ -1084,7 +945,7 @@ int run_attention_unit(cosk_model *m, int i, const ActBuf &in, int in_slot, int 
       a.shift = b.d_sa_shift;
       a.n_tokens = m->n_tokens;
       const long long n = m->n_tokens * (bc.cin / 8);
-      CK(launch_k(m, k_sa_affine, dim3((unsigned)((n + 255) / 256)), dim3(256), 0, s, a));
+      CK(launch_k(k_sa_affine, dim3((unsigned)((n + 255) / 256)), dim3(256), 0, s, a));
       m->launches++;
     }
     if (b.tc_sa_fused) {
@@ -1104,17 +965,14 @@ int run_attention_unit(cosk_model *m, int i, const ActBuf &in, int in_slot, int 
       a.cs_out = b.sa.cs;
       a.dbg = m->d_dbg;
       const int grid = m->n_tiles < m->num_sms ? m->n_tiles : m->num_sms;
-      if (bc.cout == 64) CK(launch_k(m, k_tc_sa<8>, dim3(grid), dim3(384), TcSaCfg<8>::kSmemBytes, s, a));
-      else if (bc.cout == 128) CK(launch_k(m, k_tc_sa<16>, dim3(grid), dim3(384), TcSaCfg<16>::kSmemBytes, s, a));
-      else CK(launch_k(m, k_tc_sa<32>, dim3(grid), dim3(384), TcSaCfg<32>::kSmemBytes, s, a));
+      if (bc.cout == 128) CK(launch_k(k_tc_sa<16>, dim3(grid), dim3(384), TcSaCfg<16>::kSmemBytes, s, a));
+      else CK(launch_k(k_tc_sa<32>, dim3(grid), dim3(384), TcSaCfg<32>::kSmemBytes, s, a));
       m->launches++;
-    }
-    for (int q = 0; !b.tc_sa_fused && q < b.n_qchunks; ++q) {  // qkv conv = single-tap temporal-conv kernel without ReLU, per column chunk
-      const BlockW::QChunk &qc = b.qchunk[q];
+    } else {  // qkv conv = single-tap temporal-conv kernel without ReLU
       TcTcnArgs a;
       a.tm_ring = b.sa_x.map;
       a.tm_res = b.sa_x.map;
-      a.tm_w = qc.map;
+      a.tm_w = b.map_sa_q;
       for (int k = 0; k < kTaps; ++k) a.tap_row[k] = (int)b.sa_x.row_hi(0);
       a.res_row = 0;
       a.t_alloc = (int)m->t_alloc;
@@ -1125,18 +983,17 @@ int run_attention_unit(cosk_model *m, int i, const ActBuf &in, int in_slot, int 
       a.tile_tokens = m->tile_tokens;
       a.reverse = 0;
       a.n_tokens = m->n_tokens;
-      a.epi.bias = qc.bias;
+      a.epi.bias = b.d_sa_qbias;
       a.epi.r_hi = nullptr;
       a.epi.r_lo = nullptr;
       a.epi.cs_r = 0;
-      a.epi.y_hi = b.sa_q.hi(0) + qc.col0;
-      a.epi.y_lo = b.sa_q.lo(0) + qc.col0;
+      a.epi.y_hi = b.sa_q.hi(0);
+      a.epi.y_lo = b.sa_q.lo(0);
       a.epi.cs_out = b.sa_q.cs;
       a.epi.floor = -INFINITY;
-      a.tile_cnt = nullptr;
       a.trace = nullptr;
       a.dbg = m->d_dbg;
-      if ((rc = launch_onetap(m, qc.width, a, qc.map_half, s))) return rc;
+      if ((rc = launch_tcn(m, kSaQkvCols, a, b.map_sa_q, s))) return rc;
       m->launches++;
     }
   } else {
@@ -1155,7 +1012,7 @@ int run_attention_unit(cosk_model *m, int i, const ActBuf &in, int in_slot, int 
     a.tile_tokens = m->tile_tokens;
     a.qkv = m->d_qkv;
     dim3 grid(m->n_tiles, (nq + kSimtN - 1) / kSimtN);
-    CK(launch_k(m, k_sa_qkv, grid, dim3(256), 0, s, a));
+    CK(launch_k(k_sa_qkv, grid, dim3(256), 0, s, a));
     m->launches++;
   }
   if (!b.tc_sa_fused) {
@@ -1173,10 +1030,10 @@ int run_attention_unit(cosk_model *m, int i, const ActBuf &in, int in_slot, int 
     a.y_lo = b.sa.lo(0);
     a.cs_out = b.sa.cs;
     const int dvh = dv / kSaHeads;
-    if (dvh == 8) CK(launch_k(m, k_sa_attn<8>, dim3(m->n_tiles), dim3(256), 0, s, a));
-    else if (dvh == 16) CK(launch_k(m, k_sa_attn<16>, dim3(m->n_tiles), dim3(256), 0, s, a));
-    else if (dvh == 32) CK(launch_k(m, k_sa_attn<32>, dim3(m->n_tiles), dim3(256), 0, s, a));
-    else CK(launch_k(m, k_sa_attn_any, dim3(m->n_tiles), dim3(128), 0, s, a));
+    if (dvh == 8) CK(launch_k(k_sa_attn<8>, dim3(m->n_tiles), dim3(256), 0, s, a));
+    else if (dvh == 16) CK(launch_k(k_sa_attn<16>, dim3(m->n_tiles), dim3(256), 0, s, a));
+    else if (dvh == 32) CK(launch_k(k_sa_attn<32>, dim3(m->n_tiles), dim3(256), 0, s, a));
+    else CK(launch_k(k_sa_attn_any, dim3(m->n_tiles), dim3(128), 0, s, a));
     m->launches++;
   }
   if ((rc = prof_mark(m, 1, i, s))) return rc;
@@ -1203,10 +1060,9 @@ int run_attention_unit(cosk_model *m, int i, const ActBuf &in, int in_slot, int 
     a.epi.y_hi = b.ring.hi(ring_slot);
     a.epi.y_lo = b.ring.lo(ring_slot);
     a.epi.cs_out = b.ring.cs;
-    a.tile_cnt = nullptr;
     a.trace = nullptr;
     a.dbg = m->d_dbg;
-    if ((rc = launch_onetap(m, bc.cout, a, b.map_sa_w_half, s))) return rc;
+    if ((rc = launch_tcn(m, bc.cout, a, b.map_sa_w_half, s))) return rc;
   } else {
     TcnArgs a;
     for (int k = 0; k < kTaps; ++k) {
@@ -1230,7 +1086,7 @@ int run_attention_unit(cosk_model *m, int i, const ActBuf &in, int in_slot, int 
     a.n_tokens = m->n_tokens;
     a.tile_tokens = m->tile_tokens;
     dim3 grid(m->n_tiles, (bc.cout + kSimtN - 1) / kSimtN);
-    CK(launch_k(m, k_tcn_simt, grid, dim3(256), 0, s, a));
+    CK(launch_k(k_tcn_simt, grid, dim3(256), 0, s, a));
   }
   m->launches++;
   return COSK_OK;
@@ -1281,8 +1137,8 @@ int run_gcn(cosk_model *m, int i, const ActBuf &in, int in_slot, int ring_slot, 
     t.tile_tokens = m->tile_tokens;
     t.dense = m->d_dense;
     t.dense_ld = 3 * m->dense_vp;
-    if (m->cfg.vertices == 25) CK(launch_k(m, k_attn_small<16, 25>, dim3(m->n_tiles), dim3(128), 0, s, t));
-    else CK(launch_k(m, k_attn_small<16, 18>, dim3(m->n_tiles), dim3(128), 0, s, t));
+    if (m->cfg.vertices == 25) CK(launch_k(k_attn_small<16, 25>, dim3(m->n_tiles), dim3(128), 0, s, t));
+    else CK(launch_k(k_attn_small<16, 18>, dim3(m->n_tiles), dim3(128), 0, s, t));
     m->launches++;
     if ((rc = prof_mark(m, 1, i, s))) return rc;
   } else if (adaptive) {
@@ -1302,7 +1158,7 @@ int run_gcn(cosk_model *m, int i, const ActBuf &in, int in_slot, int ring_slot, 
     t.dense = m->d_dense;
     t.dense_ld = 3 * m->dense_vp;
     t.dense_vp = m->dense_vp;
-    CK(launch_k(m, k_agcn_attn, dim3(m->n_tiles), dim3(256), (size_t)2 * t.inter_c * kTileRows * sizeof(float), s, t));
+    CK(launch_k(k_agcn_attn, dim3(m->n_tiles), dim3(256), (size_t)2 * t.inter_c * kTileRows * sizeof(float), s, t));
     m->launches++;
     if ((rc = prof_mark(m, 1, i, s))) return rc;
   }
@@ -1314,21 +1170,8 @@ int run_gcn(cosk_model *m, int i, const ActBuf &in, int in_slot, int ring_slot, 
     if (b.gcn_parts == 4) rc = v25 ? launch_tc_agcn<4, 1, 25>(m, a, s) : launch_tc_agcn<4, 1, 18>(m, a, s);
     else rc = v25 ? launch_tc_agcn<3, 2, 25>(m, a, s) : launch_tc_agcn<3, 2, 18>(m, a, s);
     if (rc) return rc;
-  } else if (b.tc_gcnt) {
-    if ((rc = launch_tc_gcnt(m, i, make_gcn_args(m, i, in, in_slot, ring_slot), s))) return rc;
-  } else if (b.tc_gcnp) {
-    TcGcnpArgs a = make_gcnp_args(m, i, in, in_slot, ring_slot);
-    if (bc.cout == 64) rc = b.gcnp_stacked ? launch_tc_gcnp<64, true>(m, a, s) : launch_tc_gcnp<64, false>(m, a, s);
-    else if (bc.cout == 128) rc = b.gcnp_stacked ? launch_tc_gcnp<128, true>(m, a, s) : launch_tc_gcnp<128, false>(m, a, s);
-    else rc = launch_tc_gcnp<256, false>(m, a, s);
-    if (rc) return rc;
   } else if (b.tc_gcn) {
-    TcGcnArgs a = make_gcn_args(m, i, in, in_slot, ring_slot);
-    // one K-block per work item (cin = 64): single operand stage, four exchange buffers
-    const bool one_kb = bc.cin == kBK && m->gcn_single_stage;
-    if (b.gcn_parts == 4) rc = one_kb ? launch_tc_gcn<4, 1>(m, a, s) : launch_tc_gcn<4, 2>(m, a, s);
-    else rc = one_kb ? launch_tc_gcn<3, 1>(m, a, s) : launch_tc_gcn<3, 2>(m, a, s);
-    if (rc) return rc;
+    if ((rc = launch_gcn(m, i, make_gcn_args(m, i, in, in_slot, ring_slot), s))) return rc;
   } else {
     GcnArgs a;
     a.x_hi = in.hi(in_slot);
@@ -1354,10 +1197,10 @@ int run_gcn(cosk_model *m, int i, const ActBuf &in, int in_slot, int ring_slot, 
     a.dense_vp = m->dense_vp;
     const int K = (3 + res_conv) * bc.cin;
     if (bc.cin <= 8 && res_conv && bc.cout % 32 == 0 && K <= kSmallKMax && m->cfg.path == COSK_PATH_AUTO) {
-      CK(launch_k(m, k_gcn_small, dim3(m->n_tiles), dim3(256), (size_t)(K + 1) * bc.cout * sizeof(float), s, a));
+      CK(launch_k(k_gcn_small, dim3(m->n_tiles), dim3(256), (size_t)(K + 1) * bc.cout * sizeof(float), s, a));
     } else {
       dim3 grid(m->n_tiles, (bc.cout + kSimtN - 1) / kSimtN);
-      CK(launch_k(m, k_gcn_simt, grid, dim3(256), 0, s, a));
+      CK(launch_k(k_gcn_simt, grid, dim3(256), 0, s, a));
     }
   }
   m->launches++;
@@ -1373,20 +1216,7 @@ int run_tcn(cosk_model *m, int i, const ActBuf &in, int res_slot, long long n, i
   for (int k = 0; k < kTaps; ++k) tap_slot[k] = mod_slot(n - (kTaps - 1) + k, m->R);  // frame n-8+k
   if (b.tc_tcn) {
     TcTcnArgs a = make_tcn_args(m, i, in, res_slot, n, out_slot);
-    const bool pair = m->n_tiles >= 2 && (m->pair_mask & (bc.cout == 64 ? 1 : bc.cout == 128 ? 2 : 4));
-    if (pair) {
-      // stacked-B widths (<= 128): CTA 0 loads the whole hi plane, CTA 1 the whole lo plane (full-height box);
-      // C = 256: each CTA loads its half of the rows of both planes
-      if (bc.cout > 128) a.tm_w = b.map_tcn_w_half;
-      if (bc.cout == 64) rc = launch_tc_tcn2<64>(m, a, s);
-      else if (bc.cout == 128) rc = launch_tc_tcn2<128>(m, a, s);
-      else rc = launch_tc_tcn2<256>(m, a, s);
-    } else {
-      if (bc.cout == 64) rc = launch_tc_tcn<64>(m, a, s);
-      else if (bc.cout == 128) rc = launch_tc_tcn<128>(m, a, s);
-      else rc = launch_tc_tcn<256>(m, a, s);
-    }
-    if (rc) return rc;
+    if ((rc = launch_tcn(m, bc.cout, a, b.map_tcn_w_half, s))) return rc;
   } else {
     TcnArgs a;
     for (int k = 0; k < kTaps; ++k) {
@@ -1410,7 +1240,7 @@ int run_tcn(cosk_model *m, int i, const ActBuf &in, int res_slot, long long n, i
     a.n_tokens = m->n_tokens;
     a.tile_tokens = m->tile_tokens;
     dim3 grid(m->n_tiles, (bc.cout + kSimtN - 1) / kSimtN);
-    CK(launch_k(m, k_tcn_simt, grid, dim3(256), 0, s, a));
+    CK(launch_k(k_tcn_simt, grid, dim3(256), 0, s, a));
   }
   m->launches++;
   return COSK_OK;
@@ -1454,7 +1284,7 @@ int run_block64(cosk_model *m, int i, const ActBuf &in, int in_slot, long long n
   a.trace = m->d_trace;
   a.dbg = m->d_dbg;
   const int grid = m->n_tiles < m->num_sms ? m->n_tiles : m->num_sms;
-  CK(launch_k(m, k_tc_block64, dim3(grid), dim3(512), TcBlockCfg::kSmemBytes, s, a));
+  CK(launch_k(k_tc_block64, dim3(grid), dim3(512), TcBlockCfg::kSmemBytes, s, a));
   m->launches++;
   return COSK_OK;
 }
@@ -1485,14 +1315,13 @@ int step_impl(cosk_model *m, const float *x, long long nc_stride, float *out, in
     const long long total = m->n_tokens * m->xin.cs;
     const int threads = 256;
     const long long blocks = (total + threads - 1) / threads;
-    CK(launch_k(m, k_input, dim3((unsigned)blocks), dim3(threads), 0, s, x, (long long)nc_stride, c.c_in, c.vertices, c.persons,
+    CK(launch_k(k_input, dim3((unsigned)blocks), dim3(threads), 0, s, x, (long long)nc_stride, c.c_in, c.vertices, c.persons,
                 (const float *)(c.data_bn ? m->d_bn_scale : nullptr), (const float *)(c.data_bn ? m->d_bn_shift : nullptr),
                 m->xin.hi(xslot), m->xin.lo(xslot), m->xin.cs, m->n_tokens, 0LL, RingWalk(), 0LL));
     m->launches++;
   }
   const ActBuf *in = &m->xin;
   bool alive = true;
-  bool gcn_done = false;  // the graph conv of the current block already ran inside the previous block's merged launch
   const bool head_flush = flush && enter >= c.n_blocks;
   for (int i = 0; i < c.n_blocks; ++i) {
     m->last_flags[i] = 0;
@@ -1507,7 +1336,7 @@ int step_impl(cosk_model *m, const float *x, long long nc_stride, float *out, in
     const int in_slot = (int)(n % m->Ro);
     const bool fire = tcn_fires(n, c.padding, bc.stride);
     const bool zero_in = flush && i == enter;  // a zero frame enters the temporal conv directly
-    const bool fused = b.fuse && !gcn_done && in->has_map && !zero_in;
+    const bool fused = b.fuse && in->has_map && !zero_in;
     if (zero_in) {
       const int rs = (int)(n % m->R);
       CK(cudaMemsetAsync(b.ring.hi(rs), 0, (size_t)2 * b.ring.t_alloc * b.ring.cs * sizeof(__nv_bfloat16), s));
@@ -1515,19 +1344,12 @@ int step_impl(cosk_model *m, const float *x, long long nc_stride, float *out, in
       const int res_slot = fire ? (int)((n - kResDelay) % m->Ro) : 0;
       if ((rc = run_block64(m, i, *in, in_slot, n, fire, res_slot, (int)(b.n_out % m->Ro), s))) return rc;
       if (fire) b.n_out++;
-    } else if (!gcn_done && (rc = run_gcn(m, i, *in, in_slot, (int)(n % m->R), s))) {
+    } else if ((rc = run_gcn(m, i, *in, in_slot, (int)(n % m->R), s))) {
       return rc;
     }
-    gcn_done = false;
     if (fire && !fused) {
       const int res_slot = (int)((n - kResDelay) % m->Ro);  // n >= first >= 4
-      const int out_slot = (int)(b.n_out % m->Ro);
-      if (can_merge(m, i)) {
-        if ((rc = run_tcn_gcn(m, i, *in, res_slot, n, out_slot, s))) return rc;
-        gcn_done = true;
-      } else if ((rc = run_tcn(m, i, *in, res_slot, n, out_slot, s))) {
-        return rc;
-      }
+      if ((rc = run_tcn(m, i, *in, res_slot, n, (int)(b.n_out % m->Ro), s))) return rc;
       b.n_out++;
     }
     b.n_in++;
@@ -1560,14 +1382,14 @@ int step_impl(cosk_model *m, const float *x, long long nc_stride, float *out, in
       h.b = m->d_fc_b;
       h.classes = c.classes;
       h.out = out;
-      CK(launch_k(m, k_head, dim3((unsigned)((m->n_streams + kHeadStreams - 1) / kHeadStreams)), dim3(256 * kHeadStreams),
+      CK(launch_k(k_head, dim3((unsigned)((m->n_streams + kHeadStreams - 1) / kHeadStreams)), dim3(256 * kHeadStreams),
                   (size_t)kHeadStreams * (2 * last.out.cs + last.out.c) * sizeof(float), s, h));
       m->launches++;
       m->pool_n++;
     } else {
       emit = 1;
       const long long total = m->n_tokens * last.out.c;
-      CK(launch_k(m, k_read_block, dim3((unsigned)((total + 255) / 256)), dim3(256), 0, s, (const __nv_bfloat16 *)last.out.hi(slot),
+      CK(launch_k(k_read_block, dim3((unsigned)((total + 255) / 256)), dim3(256), 0, s, (const __nv_bfloat16 *)last.out.hi(slot),
                   (const __nv_bfloat16 *)last.out.lo(slot), last.out.cs, last.out.c, c.vertices, m->n_tokens, out));
       m->launches++;
     }
@@ -1584,14 +1406,14 @@ int step_impl(cosk_model *m, const float *x, long long nc_stride, float *out, in
 // of a launch are (frame, tile) pairs and every frame's ring slots follow from a RingWalk.  Available when every block runs
 // on the tensor-core CoST-GCN kernels (k_tc_gcn, k_gcn_small for the first layer, k_tc_tcn / k_tc_tcn2).
 bool batched_ok(const cosk_model *m) {
-  if (m->tchunk <= 1 || m->cfg.path != COSK_PATH_AUTO || m->merge || m->d_trace) return false;
+  if (m->tchunk <= 1 || m->cfg.path != COSK_PATH_AUTO || m->d_trace) return false;
   for (int i = 0; i < m->cfg.n_blocks; ++i) {
     const cosk_block_cfg &bc = m->cfg.blocks[i];
     const BlockW &b = m->blk[i];
     if (bc.gconv != COSK_GCONV_PLAIN || !b.tc_tcn) return false;
     const int res_conv = bc.cin != bc.cout ? 1 : 0;
     const bool small = bc.cin <= 8 && res_conv && bc.cout % 32 == 0 && (3 + res_conv) * bc.cin <= kSmallKMax;
-    if (!((b.tc_gcn && !b.tc_gcnp) || small)) return false;
+    if (!(b.tc_gcn || small)) return false;
   }
   return true;
 }
@@ -1610,7 +1432,7 @@ int steps_chunk(cosk_model *m, const float *x, long long nc_stride, long long x_
     ow.slot0 = mod_slot(m->frame, m->Ro);
     ow.step = 1;
     ow.slots = m->Ro;
-    CK(launch_k(m, k_input, dim3((unsigned)blocks, (unsigned)F0), dim3(threads), 0, s, x, (long long)nc_stride, c.c_in, c.vertices, c.persons,
+    CK(launch_k(k_input, dim3((unsigned)blocks, (unsigned)F0), dim3(threads), 0, s, x, (long long)nc_stride, c.c_in, c.vertices, c.persons,
                 (const float *)(c.data_bn ? m->d_bn_scale : nullptr), (const float *)(c.data_bn ? m->d_bn_shift : nullptr),
                 m->xin.hi(0), m->xin.lo(0), m->xin.cs, m->n_tokens, x_frame_stride, ow, m->xin.slot_elems()));
     m->launches++;
@@ -1660,18 +1482,7 @@ int steps_chunk(cosk_model *m, const float *x, long long nc_stride, long long x_
             a.epi.r_lo = in->lo(0);
           }
         }
-        const bool one_kb = bc.cin == kBK && m->gcn_single_stage;
-        const int items = m->n_tiles * F;
-        const int grid = items < m->num_sms ? items : m->num_sms;
-        if (b.tc_gcnt) {
-          if ((rc = launch_tc_gcnt(m, i, a, s))) return rc;
-        } else if (b.gcn_parts == 4) {
-          if (one_kb) CK(launch_k(m, k_tc_gcn<4, 1, false>, dim3(grid), dim3(512), TcGcnCfg<4, 1>::kSmemBytes, s, a));
-          else CK(launch_k(m, k_tc_gcn<4, 2, false>, dim3(grid), dim3(512), TcGcnCfg<4, 2>::kSmemBytes, s, a));
-        } else {
-          if (one_kb) CK(launch_k(m, k_tc_gcn<3, 1, false>, dim3(grid), dim3(512), TcGcnCfg<3, 1>::kSmemBytes, s, a));
-          else CK(launch_k(m, k_tc_gcn<3, 2, false>, dim3(grid), dim3(512), TcGcnCfg<3, 2>::kSmemBytes, s, a));
-        }
+        if ((rc = launch_gcn(m, i, a, s))) return rc;
       } else {  // narrow first layer
         GcnArgs a;
         a.x_hi = in->hi(0);
@@ -1699,7 +1510,7 @@ int steps_chunk(cosk_model *m, const float *x, long long nc_stride, long long x_
         a.in_slot_elems = in->slot_elems();
         a.out_slot_elems = b.ring.slot_elems();
         const int K = 4 * bc.cin;
-        CK(launch_k(m, k_gcn_small, dim3(m->n_tiles, F), dim3(256), (size_t)(K + 1) * bc.cout * sizeof(float), s, a));
+        CK(launch_k(k_gcn_small, dim3(m->n_tiles, F), dim3(256), (size_t)(K + 1) * bc.cout * sizeof(float), s, a));
       }
       m->launches++;
       // temporal conv over the F_out firing executions
@@ -1721,22 +1532,7 @@ int steps_chunk(cosk_model *m, const float *x, long long nc_stride, long long x_
             a.epi.r_lo = in->lo(0);
           }
         }
-        const bool pair = m->n_tiles >= 2 && (m->pair_mask & (bc.cout == 64 ? 1 : bc.cout == 128 ? 2 : 4));
-        if (pair) {
-          if (bc.cout > 128) a.tm_w = b.map_tcn_w_half;
-          const int n_pairs = (m->n_tiles + 1) / 2 * F_out;
-          const int max_clusters = m->num_sms / 2;
-          const int grid = 2 * (n_pairs < max_clusters ? n_pairs : max_clusters);
-          if (bc.cout == 64) CK(launch_k(m, k_tc_tcn2<64>, dim3(grid), dim3(256), TcTcn2Cfg<64>::kSmemBytes, s, a));
-          else if (bc.cout == 128) CK(launch_k(m, k_tc_tcn2<128>, dim3(grid), dim3(256), TcTcn2Cfg<128>::kSmemBytes, s, a));
-          else CK(launch_k(m, k_tc_tcn2<256>, dim3(grid), dim3(256), TcTcn2Cfg<256>::kSmemBytes, s, a));
-        } else {
-          const int items = m->n_tiles * F_out;
-          const int grid = items < m->num_sms ? items : m->num_sms;
-          if (bc.cout == 64) CK(launch_k(m, k_tc_tcn<64>, dim3(grid), dim3(256), TcTcnCfg<64>::kSmemBytes, s, a));
-          else if (bc.cout == 128) CK(launch_k(m, k_tc_tcn<128>, dim3(grid), dim3(256), TcTcnCfg<128>::kSmemBytes, s, a));
-          else CK(launch_k(m, k_tc_tcn<256>, dim3(grid), dim3(256), TcTcnCfg<256>::kSmemBytes, s, a));
-        }
+        if ((rc = launch_tcn(m, bc.cout, a, b.map_tcn_w_half, s))) return rc;
         m->launches++;
       }
     }
@@ -1785,7 +1581,7 @@ int steps_chunk(cosk_model *m, const float *x, long long nc_stride, long long x_
         h.y_lo += (long long)h.in_walk.slot0 * h.in_slot_elems;
         h.emit = n_emit;
       }
-      CK(launch_k(m, k_head, dim3((unsigned)((m->n_streams + kHeadStreams - 1) / kHeadStreams)), dim3(256 * kHeadStreams),
+      CK(launch_k(k_head, dim3((unsigned)((m->n_streams + kHeadStreams - 1) / kHeadStreams)), dim3(256 * kHeadStreams),
                   (size_t)kHeadStreams * (2 * last.out.cs + last.out.c) * sizeof(float), s, h));
       m->launches++;
       m->pool_n += F;
@@ -1796,7 +1592,7 @@ int steps_chunk(cosk_model *m, const float *x, long long nc_stride, long long x_
         const int slot = mod_slot(o0 + f, m->Ro);
         const long long total = m->n_tokens * last.out.c;
         float *dst = out + (long long)(*cnt < max_out ? *cnt : max_out - 1) * out_stride;
-        CK(launch_k(m, k_read_block, dim3((unsigned)((total + 255) / 256)), dim3(256), 0, s, (const __nv_bfloat16 *)last.out.hi(slot),
+        CK(launch_k(k_read_block, dim3((unsigned)((total + 255) / 256)), dim3(256), 0, s, (const __nv_bfloat16 *)last.out.hi(slot),
                     (const __nv_bfloat16 *)last.out.lo(slot), last.out.cs, last.out.c, c.vertices, m->n_tokens, dst));
         m->launches++;
         *cnt += 1;
@@ -1854,27 +1650,9 @@ int cosk_create(const cosk_config *cfg, cosk_model **out) {
   cudaDeviceProp prop;
   cudaGetDeviceProperties(&prop, cfg->device);
   m->num_sms = prop.multiProcessorCount;
-  if (const char *e = getenv("COSK_TCN_PAIR")) m->pair_mask = atoi(e);
-  if (const char *e = getenv("COSK_PDL")) m->pdl = atoi(e);
-  if (const char *e = getenv("COSK_GCN_PREMIX")) m->gcn_premix = atoi(e);
   if (const char *e = getenv("COSK_FUSE_BLOCK")) m->fuse_block = atoi(e);
   if (const char *e = getenv("COSK_GCN_T")) m->gcn_transposed = atoi(e);
-  if (const char *e = getenv("COSK_GCNT_PACK")) m->gcnt_pack = atoi(e);
   if (const char *e = getenv("COSK_AGCN_T")) m->agcn_transposed = atoi(e);
-  if (const char *e = getenv("COSK_GCN_FOLD_UNIT")) m->gcn_fold_unit = atoi(e);
-  if (const char *e = getenv("COSK_GCNP_STACKED")) m->gcnp_stacked = atoi(e);
-  if (const char *e = getenv("COSK_AGCN_TC")) m->agcn_tc = atoi(e);
-  if (const char *e = getenv("COSK_ATTN_TC")) m->attn_tc = atoi(e);
-  if (const char *e = getenv("COSK_SA_QKV_TC")) m->sa_qkv_tc = atoi(e);
-  if (const char *e = getenv("COSK_SA_FUSED")) m->sa_fused = atoi(e);
-  if (const char *e = getenv("COSK_TCN_IDENTITY_MMA")) m->tcn_identity_mma = atoi(e);
-  if (const char *e = getenv("COSK_MERGE")) m->merge = atoi(e);
-  if (const char *e = getenv("COSK_MERGE_MIN_TILES")) m->merge_min_tiles = atoi(e);
-  if (const char *e = getenv("COSK_MERGE_SPLIT64")) m->merge_split64 = atoi(e);
-  if (const char *e = getenv("COSK_MERGE_SPLIT128")) m->merge_split128 = atoi(e);
-  if (const char *e = getenv("COSK_GCN_SINGLE_STAGE")) m->gcn_single_stage = atoi(e);
-  if (const char *e = getenv("COSK_TCN_REVERSE")) m->tcn_reverse = atoi(e);
-  if (const char *e = getenv("COSK_GCN_IDENTITY_MMA")) m->gcn_identity_mma = atoi(e);
   if (const char *e = getenv("COSK_TRACE")) {
     if (atoi(e) && cudaMalloc(&m->d_trace, 64 * sizeof(unsigned long long)) == cudaSuccess)
       cudaMemset(m->d_trace, 0, 64 * sizeof(unsigned long long));
@@ -1943,10 +1721,8 @@ void cosk_destroy(cosk_model *m) {
     dfree(b.d_res_w_sa);
     dfree(b.d_sa_fw16);
     dfree(b.d_sa_fbias);
-    for (auto &qc : b.qchunk) {
-      dfree(qc.w16);
-      dfree(qc.bias);
-    }
+    dfree(b.d_sa_qw16);
+    dfree(b.d_sa_qbias);
   }
   dfree(m->d_bn_scale);
   dfree(m->d_bn_shift);
@@ -2024,7 +1800,6 @@ int cosk_set_batch_ex(cosk_model *m, int64_t n_streams, int32_t time_chunk) {
   for (int i = 0; i < c.n_blocks; ++i) {
     if ((rc = alloc_act(m, m->blk[i].ring, m->R, c.blocks[i].cout))) return rc;
     if ((rc = alloc_act(m, m->blk[i].out, m->Ro, c.blocks[i].cout))) return rc;
-    CK(cudaMalloc(&m->blk[i].d_tile_cnt, sizeof(unsigned int) * (size_t)(m->n_tiles + 2)));
   }
   if (c.classes > 0) {
     const size_t cl = (size_t)c.blocks[c.n_blocks - 1].cout;
@@ -2044,7 +1819,7 @@ int cosk_set_batch_ex(cosk_model *m, int64_t n_streams, int32_t time_chunk) {
         if ((rc = alloc_act(m, m->blk[i].sa_x, 1, c.blocks[i].cin))) return rc;
         CK(cudaMemset(m->blk[i].sa_x.ptr, 0, m->blk[i].sa_x.bytes()));
         if (!m->blk[i].tc_sa_fused) {
-          if ((rc = alloc_act(m, m->blk[i].sa_q, 1, m->blk[i].nq_pad))) return rc;
+          if ((rc = alloc_act(m, m->blk[i].sa_q, 1, kSaQkvCols))) return rc;
           CK(cudaMemset(m->blk[i].sa_q.ptr, 0, m->blk[i].sa_q.bytes()));
         }
       }
@@ -2202,7 +1977,7 @@ int cosk_read_block(cosk_model *m, int32_t block, float *dst_dev, void *stream) 
   DeviceGuard guard_(m->cfg.device);
   const int slot = (int)((b.n_out - 1) % m->Ro);
   const long long total = m->n_tokens * b.out.c;
-  CK(launch_k(m, k_read_block, dim3((unsigned)((total + 255) / 256)), dim3(256), 0, (cudaStream_t)stream,
+  CK(launch_k(k_read_block, dim3((unsigned)((total + 255) / 256)), dim3(256), 0, (cudaStream_t)stream,
               (const __nv_bfloat16 *)b.out.hi(slot), (const __nv_bfloat16 *)b.out.lo(slot), b.out.cs, b.out.c, m->cfg.vertices,
               m->n_tokens, dst_dev));
   m->launches++;
@@ -2221,11 +1996,8 @@ int cosk_describe(const cosk_model *m, char *buf, size_t n) {
   std::string o = "{";
   char t[1024];
   snprintf(t, sizeof t,
-           "\"version\": \"%s\", \"path\": \"%s\", \"pdl\": %d, \"tcn_pair_mask\": %d, \"tcn_reverse\": %d, \"tcn_identity_mma\": %d, "
-           "\"fuse_block\": %d, \"gcn_transposed\": %d, \"gcnt_pack\": %d, \"agcn_transposed\": %d, \"gcn_fold_unit\": %d, \"gcn_premix\": %d, \"gcnp_stacked\": %d, \"gcn_identity_mma\": %d, \"merge\": %d, "
-           "\"sa_fused\": %d, \"attn_tc\": %d, \"agcn_tc\": %d, \"trace\": %d, ",
-           cosk_version(), m->cfg.path == COSK_PATH_AUTO ? "auto" : "simt", m->pdl, m->pair_mask, m->tcn_reverse, m->tcn_identity_mma,
-           m->fuse_block, m->gcn_transposed, m->gcnt_pack, m->agcn_transposed, m->gcn_fold_unit, m->gcn_premix, m->gcnp_stacked, m->gcn_identity_mma, m->merge, m->sa_fused, m->attn_tc, m->agcn_tc,
+           "\"version\": \"%s\", \"path\": \"%s\", \"fuse_block\": %d, \"gcn_transposed\": %d, \"agcn_transposed\": %d, \"trace\": %d, ",
+           cosk_version(), m->cfg.path == COSK_PATH_AUTO ? "auto" : "simt", m->fuse_block, m->gcn_transposed, m->agcn_transposed,
            m->d_trace ? 1 : 0);
   o += t;
   o += "\"blocks\": [";
@@ -2240,16 +2012,12 @@ int cosk_describe(const cosk_model *m, char *buf, size_t n) {
     else if (b.tc_gcnt) {
       snprintf(t, sizeof t, "k_tc_gcnt<%d> channel-major, mix in registers", b.gcnt_parts);
       g = t;
-    } else if (b.tc_gcnp) {
-      snprintf(t, sizeof t, "k_tc_gcnp<%d,%s> P=%d", bc.cout, b.gcnp_stacked ? "stacked" : "3-product", b.gcnp_parts);
-      g = t;
     } else if (b.tc_gcn) {
       snprintf(t, sizeof t, "k_tc_gcn<%d> GEMM-then-mix", b.gcn_parts);
       g = t;
     } else g = (m->cfg.path == COSK_PATH_AUTO && bc.cin <= 8) ? "k_gcn_small" : "k_gcn_simt";
     if (b.tc_tcn) {
-      const bool pair = m->pair_mask & (bc.cout == 64 ? 1 : bc.cout == 128 ? 2 : 4);
-      snprintf(t, sizeof t, "%s<%d>", pair ? "k_tc_tcn2" : "k_tc_tcn", bc.cout);
+      snprintf(t, sizeof t, "%s<%d>", tcn_on_pair(m, bc.cout) ? "k_tc_tcn2" : "k_tc_tcn", bc.cout);
       tc = t;
     } else tc = "k_tcn_simt";
     if (b.fuse) {
@@ -2265,7 +2033,7 @@ int cosk_describe(const cosk_model *m, char *buf, size_t n) {
   for (int w : {64, 128, 256})
     for (int i = 0; i < m->cfg.n_blocks; ++i)
       if (m->cfg.blocks[i].cout == w && m->cfg.blocks[i].cin >= 64 && m->cfg.blocks[i].gconv == COSK_GCONV_PLAIN) {
-        snprintf(t, sizeof t, "%s\"%d\": \"%s\"", firstw ? "" : ", ", w, m->blk[i].tc_gcnt ? "gcnt" : m->blk[i].tc_gcnp ? "gcnp" : m->blk[i].tc_gcn ? "gcn" : "simt");
+        snprintf(t, sizeof t, "%s\"%d\": \"%s\"", firstw ? "" : ", ", w, m->blk[i].tc_gcnt ? "gcnt" : m->blk[i].tc_gcn ? "gcn" : "simt");
         o += t;
         firstw = false;
         break;

@@ -282,14 +282,6 @@ __device__ __forceinline__ void umma_commit_pair(uint64_t *bar, uint16_t cta_mas
                : "memory");
 }
 
-__device__ __forceinline__ unsigned int ld_acquire_u32(const unsigned int *p) {
-  unsigned int v;
-  asm volatile("ld.acquire.gpu.global.u32 %0, [%1];" : "=r"(v) : "l"(p) : "memory");
-  return v;
-}
-// order prior generic-proxy accesses (here: the acquire above) before later async-proxy (TMA) accesses
-__device__ __forceinline__ void fence_proxy_async_all() { asm volatile("fence.proxy.async;" ::: "memory"); }
-
 // 128-bit global accesses for the epilogue
 __device__ __forceinline__ uint4 ldg_v4(const void *p) {
   uint4 r;

@@ -10,7 +10,7 @@
 //
 //   TMA: x_n tile (own 32 KB stage) | history ring (4 x 32 KB): g_{n-8} .. g_{n-1}, x_{n-4} | weight ring (3 x 16 KB slabs);
 //        three independent producer threads, so a full weight ring never holds up the history stream
-//   mix warps      x_n tile -> adjacency-mixed rows X'_i, re-split, tcgen05.st -> TMEM A slots        (as k_tc_gcnp)
+//   mix warps      x_n tile -> adjacency-mixed rows X'_i, re-split, tcgen05.st -> TMEM A slots
 //   MMA thread     G = [X'_0|X'_1|X'_2|x] [W_0|W_1|W_2|I]^T   (A from TMEM)                      -> TMEM accumulator G
 //   epilogue warps G -> +bias, ReLU, split -> ring slot n (the only state write of the graph conv)
 //                                             and -> TMEM "newest tap" slot (bf16 hi | lo, K-major)
@@ -36,11 +36,16 @@
 // link is exactly 1); (2) x = hi + lo is written back IN PLACE over the tile as fp32 rows, from which the partitions
 // gather with one FMA per adjacency entry and element.
 #pragma once
-#include "tc_gcnp.cuh"
+#include "tc_kernels.cuh"
 
 namespace cosk {
 
+constexpr int kPartSrcMax = 4;  // most sources of one output vertex inside partition 1 or 2
+
 enum : unsigned int {
+  kDbgMixXFull = 0x08000000u,
+  kDbgMixAEmpty = 0x09000000u,
+  kDbgMmaAFull = 0x0a000000u,
   kDbgBlkGFull = 0x0b000000u,
   kDbgBlkTapEmpty = 0x0c000000u,
   kDbgBlkTapFull = 0x0d000000u,
@@ -98,6 +103,19 @@ struct TcBlockCfg {
   static_assert(kMix + kMixSlots * 64 <= 512, "TMEM columns");
   static_assert(kSmemBytes <= kSmemLimit, "shared memory budget");
 };
+
+// 8 fp32 values -> 4 packed hi words + 4 packed lo words (even channel in the low half, as in memory)
+__device__ __forceinline__ void split8(const float (&v)[8], uint32_t *hi, uint32_t *lo) {
+#pragma unroll
+  for (int j = 0; j < 4; ++j) {
+    const uint32_t h = pack_bf16x2(v[2 * j], v[2 * j + 1]);
+    hi[j] = h;
+    lo[j] = pack_bf16x2(v[2 * j] - bf16_lo_as_float(h), v[2 * j + 1] - bf16_hi_as_float(h));
+  }
+}
+
+// byte offset of the 16-byte chunk `c` of row `r` inside a TMA SWIZZLE_128B tile with 128-byte rows
+__device__ __forceinline__ uint32_t sw128_off(int r, int c) { return (uint32_t)(r * 128 + ((c ^ (r & 7)) << 4)); }
 
 __global__ void __launch_bounds__(512, 1) k_tc_block64(const __grid_constant__ TcBlockArgs a) {
   using Cfg = TcBlockCfg;

@@ -86,7 +86,6 @@ struct TcGcntArgs {
   TcGcnArgs g;        // tm_w: weights [2 planes][chunk][part][128 channels] x cin, box {64, 128}
   float coef[3][32];  // d0[w], c1[w] (from the parent of w), c2[a] (child a into its parent)
   int n_parts;        // 3 (gcn_residual folded into W_0) or 4
-  int pack;           // 1: neighbouring lanes trade tokens so that every store carries two channels (half the store instructions)
 };
 
 template <int V, int NKB>
@@ -337,46 +336,33 @@ __global__ void __launch_bounds__(384, 1) k_tc_gcnt(const __grid_constant__ TcGc
         // ReLU, split, store: a warp writes 32 consecutive channels (64 bytes, two full sectors) per token and plane
         long long left = tile < a.n_tiles ? a.n_tokens - tok0 : 0;
         const int n_valid = left > NZ ? NZ : (left < 0 ? 0 : (int)left);  // tokens of this tile that exist
-        if (ta.pack) {
-          // lanes 2j and 2j+1 (channels c, c+1) trade: the even lane ends up with both channels of the even token, the odd lane
-          // with both of the odd token -> one 32-bit store per plane and token pair instead of two 16-bit ones
-          const uint32_t sel_keep = odd ? 0x7632u : 0x5410u, sel_send = odd ? 0x5410u : 0x7632u;
-          const uint32_t sel_hi = odd ? 0x1054u : 0x5410u, sel_lo = odd ? 0x3276u : 0x7632u;
-          __nv_bfloat16 *ph = epi.y_hi + (tok0 + (odd ? 1 : 0)) * COUT + (ch & ~1);
-          __nv_bfloat16 *pl = epi.y_lo + (tok0 + (odd ? 1 : 0)) * COUT + (ch & ~1);
-          static_for<NZ / 2>([&](auto t_) {
-            constexpr int t = 2 * decltype(t_)::value;
-            const float x0 = fmaxf(z[t], epi.floor), x1 = fmaxf(z[t + 1], epi.floor);
-            const uint32_t h2 = pack_bf16x2(x0, x1);
-            const uint32_t l2 = pack_bf16x2(x0 - bf16_lo_as_float(h2), x1 - bf16_hi_as_float(h2));
-            const uint32_t keep = __byte_perm(h2, l2, sel_keep);  // (hi, lo) of this lane's token
-            const uint32_t recv = __shfl_xor_sync(0xffffffffu, __byte_perm(h2, l2, sel_send), 1);
-            if (t + (odd ? 1 : 0) < n_valid) {
-              *reinterpret_cast<uint32_t *>(ph + t * COUT) = __byte_perm(keep, recv, sel_hi);
-              *reinterpret_cast<uint32_t *>(pl + t * COUT) = __byte_perm(keep, recv, sel_lo);
-            }
-          });
-          if constexpr (NZ % 2 == 1) {
-            if (NZ - 1 < n_valid) {
-              const float x = fmaxf(z[NZ - 1], epi.floor);
-              const __nv_bfloat16 h = __float2bfloat16_rn(x);
-              st_bf16(epi.y_hi + (tok0 + NZ - 1) * COUT + ch, h);
-              st_bf16(epi.y_lo + (tok0 + NZ - 1) * COUT + ch, __float2bfloat16_rn(x - __bfloat162float(h)));
-            }
+        if constexpr (NZ % 2 == 1) {  // odd token count: the last token on its own (stored first: in this order ptxas keeps
+                                      // every z[] of k_tc_gcnt<25, 2, 256> in registers)
+          if (NZ - 1 < n_valid) {
+            const float x = fmaxf(z[NZ - 1], epi.floor);
+            const __nv_bfloat16 h = __float2bfloat16_rn(x);
+            st_bf16(epi.y_hi + (tok0 + NZ - 1) * COUT + ch, h);
+            st_bf16(epi.y_lo + (tok0 + NZ - 1) * COUT + ch, __float2bfloat16_rn(x - __bfloat162float(h)));
           }
-        } else {
-          __nv_bfloat16 *ph = epi.y_hi + tok0 * COUT + ch;
-          __nv_bfloat16 *pl = epi.y_lo + tok0 * COUT + ch;
-          static_for<NZ>([&](auto t_) {
-            constexpr int t = decltype(t_)::value;
-            if (t < n_valid) {
-              const float x = fmaxf(z[t], epi.floor);
-              const __nv_bfloat16 h = __float2bfloat16_rn(x);
-              st_bf16(ph + t * COUT, h);
-              st_bf16(pl + t * COUT, __float2bfloat16_rn(x - __bfloat162float(h)));
-            }
-          });
         }
+        // lanes 2j and 2j+1 (channels c, c+1) trade: the even lane ends up with both channels of the even token, the odd lane
+        // with both of the odd token -> one 32-bit store per plane and token pair instead of two 16-bit ones
+        const uint32_t sel_keep = odd ? 0x7632u : 0x5410u, sel_send = odd ? 0x5410u : 0x7632u;
+        const uint32_t sel_hi = odd ? 0x1054u : 0x5410u, sel_lo = odd ? 0x3276u : 0x7632u;
+        __nv_bfloat16 *ph = epi.y_hi + (tok0 + (odd ? 1 : 0)) * COUT + (ch & ~1);
+        __nv_bfloat16 *pl = epi.y_lo + (tok0 + (odd ? 1 : 0)) * COUT + (ch & ~1);
+        static_for<NZ / 2>([&](auto t_) {
+          constexpr int t = 2 * decltype(t_)::value;
+          const float x0 = fmaxf(z[t], epi.floor), x1 = fmaxf(z[t + 1], epi.floor);
+          const uint32_t h2 = pack_bf16x2(x0, x1);
+          const uint32_t l2 = pack_bf16x2(x0 - bf16_lo_as_float(h2), x1 - bf16_hi_as_float(h2));
+          const uint32_t keep = __byte_perm(h2, l2, sel_keep);  // (hi, lo) of this lane's token
+          const uint32_t recv = __shfl_xor_sync(0xffffffffu, __byte_perm(h2, l2, sel_send), 1);
+          if (t + (odd ? 1 : 0) < n_valid) {
+            *reinterpret_cast<uint32_t *>(ph + t * COUT) = __byte_perm(keep, recv, sel_hi);
+            *reinterpret_cast<uint32_t *>(pl + t * COUT) = __byte_perm(keep, recv, sel_lo);
+          }
+        });
         if (tr) {
           trs[2] += clock64() - c2;
           trs[4] += 1;

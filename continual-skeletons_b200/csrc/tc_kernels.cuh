@@ -32,7 +32,6 @@ enum : unsigned int {
   kDbgEpiTmemFull = 0x04000000u,
   kDbgEpiExchEmpty = 0x05000000u,
   kDbgEpiExchFull = 0x06000000u,
-  kDbgTileFlag = 0x07000000u,
 };
 
 struct PipeState {
@@ -163,8 +162,6 @@ struct TcTcnArgs {
   EpiArgs epi;
   unsigned long long *trace;  // optional phase timers of CTA 0 (COSK_TRACE=1): [24] producer wait, [25] producer total,
                               // [26] MMA wait operands, [27] MMA wait accumulator, [28] MMA total
-  unsigned int *tile_cnt;  // optional [n_tiles] counters: each epilogue warp adds 1 once its rows of a tile are stored
-                           // (release), so a graph-conv role of the same launch can start on that tile
   unsigned int *dbg;
   // time-batched launch (n_frames > 1): frame f reads taps from slots (tap_walk.slot(f) + k) % tap_walk.slots of the temporal
   // ring, the delayed input from res_walk.slot(f) of the input ring, and writes out_walk.slot(f) of the output ring;
@@ -216,9 +213,6 @@ struct TcTcnCfg {
   static_assert(kTmemCols <= 512 && (kTmemCols & (kTmemCols - 1)) == 0, "TMEM columns");
 };
 
-// Role bodies are device functions so that one launch can run the temporal conv of block L on some CTAs
-// and the graph conv of block L+1 on the others (k_tc_tcn_gcn below).  `cta` / `ncta` = index of this CTA
-// among the CTAs running the role and their count.
 template <int COUT>
 __device__ __forceinline__ void tcn_body(const TcTcnArgs &a, uint8_t *smem_raw, const int cta, const int ncta) {
   using Cfg = TcTcnCfg<COUT>;
@@ -374,12 +368,8 @@ __device__ __forceinline__ void tcn_body(const TcTcnArgs &a, uint8_t *smem_raw, 
       const EpiArgs epi = tcn_epi(a, fr);
       epilogue_rows<COUT, Cfg::kStacked>(tmem_base + ((uint32_t)(q * 32) << 16) + acc * Cfg::kAccCols, bias_s, epi, tok, valid);
       ptx::tc_fence_before();
-      if (a.tile_cnt != nullptr) __threadfence();  // this lane's output rows are visible device-wide ...
       __syncwarp();
-      if (lane == 0) {
-        ptx::mbar_arrive(&tempty[acc]);
-        if (a.tile_cnt != nullptr) atomicAdd(a.tile_cnt + tile, 1u);  // ... before the tile is announced
-      }
+      if (lane == 0) ptx::mbar_arrive(&tempty[acc]);
     }
   }
   ptx::tc_fence_before();
@@ -585,12 +575,8 @@ __device__ __forceinline__ void tcn2_body(const TcTcnArgs &a, uint8_t *smem_raw,
       const EpiArgs epi = tcn_epi(a, fr);
       epilogue_rows<COUT, Cfg::kStacked>(tmem_base + ((uint32_t)(q * 32) << 16) + acc * Cfg::kAccCols, bias_s, epi, tok, valid);
       ptx::tc_fence_before();
-      if (a.tile_cnt != nullptr) __threadfence();
       __syncwarp();
-      if (lane == 0) {
-        ptx::mbar_arrive_cluster(ptx::mapa_u32(ptx::smem_u32(&tempty[acc]), 0));
-        if (a.tile_cnt != nullptr && tile < a.n_tiles) atomicAdd(a.tile_cnt + tile, 1u);
-      }
+      if (lane == 0) ptx::mbar_arrive_cluster(ptx::mapa_u32(ptx::smem_u32(&tempty[acc]), 0));
     }
   }
   ptx::tc_fence_before();
@@ -637,15 +623,12 @@ struct TcGcnArgs {
   const int *mix_src;
   const float *mix_val;
   unsigned long long *trace;  // optional phase timers written by CTA 0 (COSK_TRACE=1), else nullptr
-  const unsigned int *wait_cnt;  // optional [n_tiles] counters of the temporal conv that produces the input rows in
-  unsigned int wait_need;        // the same launch: tile t may be loaded once wait_cnt[t] >= wait_need
   EpiArgs epi;                // r_hi/r_lo = input rows when cin == cout (identity gcn_residual, P = 3), else nullptr
   unsigned int *dbg;
   // adaptive graph conv (k_tc_agcn): per-token dense mixing rows written by the attention kernel,
   // dense[token*dense_ld + partition*dense_vp + source vertex]
   const float *dense;
   int dense_ld, dense_vp;
-  int res_in_mix;  // P = 3 only: 1 = the mix warps add the identity residual rows (epi.r_hi / r_lo), 0 = the drain warps do
   // time-batched launch (n_frames > 1, plain graph conv only): frame f reads slot in_walk.slot(f) of the input ring and writes
   // slot out_walk.slot(f) of the temporal ring; epi.y_* / epi.r_* then point at slot 0 of their rings
   int n_frames = 1;
@@ -740,20 +723,6 @@ __device__ __forceinline__ void gcn_producer(const TcGcnArgs &a, uint64_t *full,
   for (int vt = cta; ok && vt < a.n_tiles * a.n_frames; vt += ncta) {
     const int fr = vt / a.n_tiles, tile = vt - fr * a.n_tiles;
     const int row = gcn_x_row(a, fr) + tile * a.tile_tokens;
-    if (a.wait_cnt != nullptr) {
-      // the input rows of this tile come from the temporal-conv role of the same launch
-      const long long t0 = clock64();
-      while (ptx::ld_acquire_u32(a.wait_cnt + tile) < a.wait_need) {
-        if (*(volatile unsigned int *)a.dbg != 0 || clock64() - t0 > ptx::kWaitLimitCycles) {
-          atomicCAS(a.dbg, 0u, kDbgTileFlag | (unsigned)(tile & 0xffffff));
-          ok = false;
-          break;
-        }
-        __nanosleep(200);
-      }
-      if (!ok) break;
-      ptx::fence_proxy_async_all();  // order the acquire (generic proxy) before the TMA reads (async proxy)
-    }
     for (int pass = 0; ok && pass < n_pass; ++pass) {
       for (int kc = 0; kc < nkb; ++kc) {
         ok = ptx::mbar_wait(&empty[ps.stage], ps.phase ^ 1, a.dbg, kDbgProdEmpty | (unsigned)(pass * 16 + kc));
@@ -915,28 +884,10 @@ __device__ __forceinline__ void gcn_body(const TcGcnArgs &a, uint8_t *smem_raw, 
     unsigned long long tr_t[4] = {0, 0, 0, 0};
     long long tr_c = 0;
     const long long tr_start = tr ? clock64() : 0;
-    const bool has_res = a.epi.r_hi != nullptr && !a.res_in_mix;  // identity gcn_residual (P == 3): own input row, prefetched one chunk ahead
     bool ok = true;
     int it = 0;
     uint32_t xc = 0;  // exchange chunks handed over so far
-    uint4 xr[4];      // next chunk's residual: 16 channels x {hi, lo} bf16
     const int n_items = a.n_tiles * a.n_frames;  // (frame, tile) work items of a time-batched launch
-    auto fetch_res = [&](int vt, int c0) {
-      const int fr = vt / a.n_tiles, tile = vt - fr * a.n_tiles;
-      const long long tok = (long long)tile * a.tile_tokens + row;
-      if (has_res && row < a.tile_tokens && tok < a.n_tokens) {
-        const long long fo = a.n_frames > 1 ? (long long)a.in_walk.slot(fr) * a.in_slot_elems : 0;
-        const uint4 *ph = reinterpret_cast<const uint4 *>(a.epi.r_hi + fo + tok * a.epi.cs_r + c0);
-        const uint4 *pl = reinterpret_cast<const uint4 *>(a.epi.r_lo + fo + tok * a.epi.cs_r + c0);
-        xr[0] = ptx::ldg_v4(ph);
-        xr[1] = ptx::ldg_v4(ph + 1);
-        xr[2] = ptx::ldg_v4(pl);
-        xr[3] = ptx::ldg_v4(pl + 1);
-      } else {
-        xr[0] = xr[1] = xr[2] = xr[3] = make_uint4(0, 0, 0, 0);
-      }
-    };
-    if (cta < n_items) fetch_res(cta, 0);
     for (int tile = cta; ok && tile < n_items; tile += ncta) {
       for (int pass = 0; ok && pass < n_pass; ++pass, ++it) {
         const int acc = it & 1;
@@ -950,23 +901,8 @@ __device__ __forceinline__ void gcn_body(const TcGcnArgs &a, uint8_t *smem_raw, 
         for (int c = 0; c < kChunks; ++c, ++xc) {
           const int c0 = pass * 64 + c * kGcnChunk;
           float t[16];
-          {  // own-row terms that do not come from TMEM: bias + identity residual (loaded a chunk ago)
-            const uint32_t hw[8] = {xr[0].x, xr[0].y, xr[0].z, xr[0].w, xr[1].x, xr[1].y, xr[1].z, xr[1].w};
-            const uint32_t lw[8] = {xr[2].x, xr[2].y, xr[2].z, xr[2].w, xr[3].x, xr[3].y, xr[3].z, xr[3].w};
 #pragma unroll
-            for (int w = 0; w < 8; ++w) {
-              t[2 * w] = bias_s[c0 + 2 * w] + (bf16_lo_as_float(hw[w]) + bf16_lo_as_float(lw[w]));
-              t[2 * w + 1] = bias_s[c0 + 2 * w + 1] + (bf16_hi_as_float(hw[w]) + bf16_hi_as_float(lw[w]));
-            }
-          }
-          {  // prefetch the residual of the next chunk / pass / tile
-            int nt = tile, nc0 = c0 + kGcnChunk;
-            if (nc0 >= a.cout) {
-              nc0 = 0;
-              nt = tile + ncta;
-            }
-            if (nt < n_items) fetch_res(nt, nc0);
-          }
+          for (int j = 0; j < 16; ++j) t[j] = bias_s[c0 + j];
           uint32_t y0[16], y1[16], y2[16];
           ptx::tmem_ld_32x16(taddr + 0 * 64 + c * kGcnChunk, y0);
           ptx::tmem_ld_32x16(taddr + 1 * 64 + c * kGcnChunk, y1);
@@ -1056,9 +992,9 @@ __device__ __forceinline__ void gcn_body(const TcGcnArgs &a, uint8_t *smem_raw, 
           const int c0 = pass * 64 + c * kGcnChunk + 4 * cq;
           const uint32_t b = xc % Cfg::kExchBufs;
           const uint32_t use = xc / Cfg::kExchBufs;
-          // identity gcn_residual added here (P == 3, res_in_mix): the two rows' 4 channels, issued before the wait
+          // identity gcn_residual added here (P == 3 and not folded into W_0): the two rows' 4 channels, issued before the wait
           uint2 rh[2] = {make_uint2(0, 0), make_uint2(0, 0)}, rl[2] = {make_uint2(0, 0), make_uint2(0, 0)};
-          if (P == 3 && a.res_in_mix) {
+          if (P == 3 && a.epi.r_hi != nullptr) {
 #pragma unroll
             for (int g = 0; g < 2; ++g) {
               const long long tok = tok0 + rows[g];
@@ -1085,7 +1021,7 @@ __device__ __forceinline__ void gcn_body(const TcGcnArgs &a, uint8_t *smem_raw, 
           }
           __syncwarp();
           if (lane == 0) ptx::mbar_arrive(&xempty[b]);  // planes consumed: the drain warps may refill them
-          if (P == 3 && a.res_in_mix) {
+          if (P == 3 && a.epi.r_hi != nullptr) {
 #pragma unroll
             for (int g = 0; g < 2; ++g) {
               z[g].x += bf16_lo_as_float(rh[g].x) + bf16_lo_as_float(rl[g].x);
@@ -1882,31 +1818,6 @@ __global__ void __launch_bounds__(384, 1) k_tc_sa(const __grid_constant__ TcSaAr
   ptx::tc_fence_before();
   __syncthreads();
   if (warp == 1) ptx::tmem_dealloc(tmem_base, Cfg::kTmemCols);
-}
-
-// =============================================================================================
-// One launch, two roles: CTAs [0, n_tcn) run the temporal conv of block L, the remaining CTAs the graph
-// conv of block L+1, which consumes the temporal conv's output tile by tile (per-tile release/acquire
-// counters in global memory).  The temporal convs of the 64- and 128-channel layers are bound by HBM and
-// leave the SMs' issue slots, tensor pipe and TMEM idle, while the graph conv is bound by its epilogue and
-// barely touches HBM: side by side the pair finishes in about the time of the temporal conv alone.
-// Launched cooperatively (all CTAs co-resident), so the waiting role cannot starve the producing one.
-// =============================================================================================
-template <int COUT, int P, int STAGES>
-__global__ void __launch_bounds__(512, 1) k_tc_tcn_gcn(const __grid_constant__ TcTcnArgs ta, const __grid_constant__ TcGcnArgs ga,
-                                                       const int n_tcn) {
-  extern __shared__ __align__(1024) uint8_t smem_raw[];
-  if ((int)blockIdx.x < n_tcn) tcn_body<COUT>(ta, smem_raw, (int)blockIdx.x, n_tcn);
-  else gcn_body<P, STAGES, false>(ga, smem_raw, (int)blockIdx.x - n_tcn, (int)gridDim.x - n_tcn);
-}
-
-// same with the temporal conv on CTA pairs: the role is chosen per cluster
-template <int COUT, int P, int STAGES>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(512, 1)
-    k_tc_tcn2_gcn(const __grid_constant__ TcTcnArgs ta, const __grid_constant__ TcGcnArgs ga, const int n_tcn) {
-  extern __shared__ __align__(1024) uint8_t smem_raw[];
-  if ((int)blockIdx.x < n_tcn) tcn2_body<COUT>(ta, smem_raw, (int)blockIdx.x / 2, n_tcn / 2);
-  else gcn_body<P, STAGES, false>(ga, smem_raw, (int)blockIdx.x - n_tcn, (int)gridDim.x - n_tcn);
 }
 
 }  // namespace cosk

@@ -303,26 +303,6 @@ def test_single_stream_and_step_vs_steps():
     assert m.device_error() == 0
 
 
-def test_merged_launch_matches_separate_kernels(monkeypatch):
-    """Temporal conv of block L + graph conv of block L+1 in one cooperative launch (two CTA roles handing
-    tiles over through release/acquire counters) must give bit-identical results to the separate kernels."""
-    base = weights.make_input((2, 3, 300, 25, 2), seed=11).to(DEV)
-    x = base.repeat(40, 1, 1, 1, 1)  # 80 streams -> 32 tiles
-    outs = {}
-    for merge in ("0", "1"):
-        monkeypatch.setenv("COSK_MERGE", merge)
-        monkeypatch.setenv("COSK_MERGE_MIN_TILES", "8")
-        monkeypatch.setenv("COSK_GCN_T", "0")  # the merged launch pairs the temporal conv with the token-major graph conv
-        arch, sd, m = _load_model(cs.CoStGcn, weights.cost_gcn_arch, True)
-        m._time_chunk = 1  # frame by frame: the merged launch is a per-step path
-        launches0 = m.launch_count()
-        outs[merge] = m.forward_steps(x).clone()
-        assert m.device_error() == 0, hex(m.device_error())
-        outs[merge + "n"] = m.launch_count() - launches0
-    assert outs["1n"] < outs["0n"], "the merged path did not run"
-    assert torch.equal(outs["0"], outs["1"])
-
-
 def test_benchmark_script_semantics():
     """scripts/benchmark_all_ntu60.py: warm-up then one prediction per stream on every timed call of `stride` frames."""
     import importlib.util

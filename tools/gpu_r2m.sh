@@ -4,7 +4,7 @@ cd "${GRAFT_REPO_ROOT:-/root/repo}"
 mkdir -p gpurun_out
 rm -f gpurun_out/summary.txt
 run() { name=$1; shift; timeout $1 "${@:2}" > gpurun_out/$name.log 2>&1; echo "$name rc=$?" >> gpurun_out/summary.txt; }
-run pytest_quick 400 python -m pytest tests/test_gpu_parity.py -x -q -m gpu --timeout 60 -k "${QUICK_K:-channel_major or forward_steps_vs_reference or kinetics or long_run or state_lifecycle or merged}"
+run pytest_quick 400 python -m pytest tests/test_gpu_parity.py -x -q -m gpu --timeout 60 -k "${QUICK_K:-channel_major or forward_steps_vs_reference or kinetics or long_run or state_lifecycle}"
 if ! grep -q "pytest_quick rc=0" gpurun_out/summary.txt; then tail -40 gpurun_out/pytest_quick.log | cut -c1-400; exit 1; fi
 run bench_a 300 python bench.py --steps 200 --warmup 8 --no-cpu-baseline ${BENCH_ARGS}
 run bench_b 300 python bench.py --steps 200 --warmup 8 --no-cpu-baseline ${BENCH_ARGS}
