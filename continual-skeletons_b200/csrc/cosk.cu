@@ -1092,6 +1092,18 @@ int run_attention_unit(cosk_model *m, int i, const ActBuf &in, int in_slot, int 
   return COSK_OK;
 }
 
+// Narrow first layer (cin <= 8): k_gcn_small keeps the weights and the mixed inputs of a tile in shared memory, and the
+// adaptive one computes its embeddings per thread (k_attn_small).  Shared by the launchers, the time-batched walk and
+// cosk_describe.
+bool gcn_small(const cosk_model *m, const cosk_block_cfg &bc) {
+  const int res_conv = bc.cin != bc.cout ? 1 : 0;
+  return m->cfg.path == COSK_PATH_AUTO && bc.cin <= 8 && res_conv && bc.cout % 32 == 0 && (3 + res_conv) * bc.cin <= kSmallKMax;
+}
+bool attn_small(const cosk_model *m, const cosk_block_cfg &bc) {
+  return bc.gconv == COSK_GCONV_ADAPTIVE && m->cfg.path == COSK_PATH_AUTO && bc.cin <= 8 && bc.cout == 64 &&
+         (m->cfg.vertices == 25 || m->cfg.vertices == 18);
+}
+
 int run_gcn(cosk_model *m, int i, const ActBuf &in, int in_slot, int ring_slot, cudaStream_t s) {
   const cosk_block_cfg &bc = m->cfg.blocks[i];
   BlockW &b = m->blk[i];
@@ -1123,7 +1135,7 @@ int run_gcn(cosk_model *m, int i, const ActBuf &in, int in_slot, int ring_slot, 
     if (rc) return rc;
     m->launches++;
     if ((rc = prof_mark(m, 1, i, s))) return rc;
-  } else if (adaptive && m->cfg.path == COSK_PATH_AUTO && bc.cin <= 8 && bc.cout == 64 && (m->cfg.vertices == 25 || m->cfg.vertices == 18)) {
+  } else if (attn_small(m, bc)) {
     // narrow first layer: embeddings computed per thread, same per-row softmax as the tensor-core kernel
     AttnSmallArgs t;
     t.x_hi = in.hi(in_slot);
@@ -1196,7 +1208,7 @@ int run_gcn(cosk_model *m, int i, const ActBuf &in, int in_slot, int ring_slot, 
     a.dense_ld = 3 * m->dense_vp;
     a.dense_vp = m->dense_vp;
     const int K = (3 + res_conv) * bc.cin;
-    if (bc.cin <= 8 && res_conv && bc.cout % 32 == 0 && K <= kSmallKMax && m->cfg.path == COSK_PATH_AUTO) {
+    if (gcn_small(m, bc)) {
       CK(launch_k(k_gcn_small, dim3(m->n_tiles), dim3(256), (size_t)(K + 1) * bc.cout * sizeof(float), s, a));
     } else {
       dim3 grid(m->n_tiles, (bc.cout + kSimtN - 1) / kSimtN);
@@ -1411,9 +1423,7 @@ bool batched_ok(const cosk_model *m) {
     const cosk_block_cfg &bc = m->cfg.blocks[i];
     const BlockW &b = m->blk[i];
     if (bc.gconv != COSK_GCONV_PLAIN || !b.tc_tcn) return false;
-    const int res_conv = bc.cin != bc.cout ? 1 : 0;
-    const bool small = bc.cin <= 8 && res_conv && bc.cout % 32 == 0 && (3 + res_conv) * bc.cin <= kSmallKMax;
-    if (!(b.tc_gcn || small)) return false;
+    if (!(b.tc_gcn || gcn_small(m, bc))) return false;
   }
   return true;
 }
@@ -2008,14 +2018,16 @@ int cosk_describe(const cosk_model *m, char *buf, size_t n) {
     std::string g, tc;
     if (bc.gconv == COSK_GCONV_ATTENTION) g = b.tc_sa_fused ? "k_tc_sa" : (b.tc_sa_qkv ? "k_tc_tcn(qkv)+k_sa_attn" : "k_sa_qkv+k_sa_attn");
     else if (bc.gconv == COSK_GCONV_ADAPTIVE && b.tc_agcnt) g = b.tc_attn ? "k_tc_attn+k_tc_agcnt" : "k_agcn_attn+k_tc_agcnt";
-    else if (bc.gconv == COSK_GCONV_ADAPTIVE) g = b.tc_gcn ? (b.tc_attn ? "k_tc_attn+k_tc_agcn" : "k_agcn_attn+k_tc_agcn") : "k_agcn_attn+k_gcn_simt";
+    else if (bc.gconv == COSK_GCONV_ADAPTIVE && b.tc_gcn) g = b.tc_attn ? "k_tc_attn+k_tc_agcn" : "k_agcn_attn+k_tc_agcn";
+    else if (bc.gconv == COSK_GCONV_ADAPTIVE)
+      g = std::string(attn_small(m, bc) ? "k_attn_small" : "k_agcn_attn") + (gcn_small(m, bc) ? "+k_gcn_small" : "+k_gcn_simt");
     else if (b.tc_gcnt) {
       snprintf(t, sizeof t, "k_tc_gcnt<%d> channel-major, mix in registers", b.gcnt_parts);
       g = t;
     } else if (b.tc_gcn) {
       snprintf(t, sizeof t, "k_tc_gcn<%d> GEMM-then-mix", b.gcn_parts);
       g = t;
-    } else g = (m->cfg.path == COSK_PATH_AUTO && bc.cin <= 8) ? "k_gcn_small" : "k_gcn_simt";
+    } else g = gcn_small(m, bc) ? "k_gcn_small" : "k_gcn_simt";
     if (b.tc_tcn) {
       snprintf(t, sizeof t, "%s<%d>", tcn_on_pair(m, bc.cout) ? "k_tc_tcn2" : "k_tc_tcn", bc.cout);
       tc = t;

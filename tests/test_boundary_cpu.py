@@ -336,3 +336,17 @@ def test_compiled_skeleton_trees_match_the_graph(V, graph_fn):
         while v != root:
             v, seen = parent[v], seen + 1
             assert seen <= V
+
+
+def test_every_launched_kernel_has_a_route_case():
+    """Every kernel (and template instantiation) csrc/cosk.cu passes to launch_k is declared covered by a case of the GPU
+    route table (tests/route_table.py), except the trace and opt-in variants listed in its EXCLUDED set."""
+    import route_table
+
+    launched = route_table.launched_kernels()
+    assert "k_tc_gcnt<25,1,128>" in launched and "k_tc_tcn2<256>" in launched, sorted(launched)
+    assert route_table.EXCLUDED <= launched, sorted(route_table.EXCLUDED - launched)
+    reachable = launched - route_table.EXCLUDED
+    covered = route_table.covered()
+    assert reachable == covered, {"without a route case": sorted(reachable - covered),
+                                  "declared but never launched": sorted(covered - reachable)}
