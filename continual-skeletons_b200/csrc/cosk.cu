@@ -30,6 +30,12 @@ typedef CUresult (*EncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t
                                   const cuuint64_t *, const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave,
                                   CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
 
+#ifdef COSK_WITH_AGCNT
+constexpr bool kAgcntBuilt = true;
+#else
+constexpr bool kAgcntBuilt = false;
+#endif
+
 inline int round_up(int x, int m) { return (x + m - 1) / m * m; }
 // q | k | v columns of the unfused tensor-core qkv conv (C = 64: 96 columns), padded to a temporal-conv kernel width
 constexpr int kSaQkvCols = 128;
@@ -49,9 +55,37 @@ struct ActBuf {  // token-major split-bf16 activation ring: [slots][plane hi/lo]
   long long slot_elems() const { return 2 * t_alloc * cs; }
 };
 
+// Which kernels serve a block.  prepare() decides it once per block; the launchers, the time-batched walk,
+// cosk_describe and cosk_block_uses_tensor_cores only read it.
+enum class GcnRoute : uint8_t {
+  kSimt,       // k_gcn_simt
+  kSmall,      // k_gcn_small: narrow first layer, weights and mixed inputs of a tile in shared memory
+  kTc,         // k_tc_gcn<gcn_parts, 1 or 2 operand stages>: token-major GEMM, then the mix
+  kTcT,        // k_tc_gcnt: channel-major, mix along the skeleton tree in registers
+  kTcAgcn,     // adaptive graph conv: dense mix on k_tc_agcn
+  kTcAgcnt,    // adaptive graph conv: dense mix on the channel-major k_tc_agcnt (COSK_WITH_AGCNT builds only)
+  kSaSimt,     // self-attention unit: k_sa_qkv + k_sa_attn
+  kSaTcQkv,    // self-attention unit: k_sa_affine + qkv conv on the single-tap k_tc_tcn + k_sa_attn
+  kSaTcFused,  // self-attention unit: k_sa_affine + k_tc_sa (qkv conv and attention in one kernel: q, k, v never leave the SM)
+};
+// attention half of an adaptive graph conv, run before its mix: k_agcn_attn, k_attn_small or k_tc_attn
+enum class AttnRoute : uint8_t { kNone, kSimt, kSmall, kTc };
+
+struct Route {
+  GcnRoute gcn = GcnRoute::kSimt;
+  AttnRoute attn = AttnRoute::kNone;
+  bool sa_out_tc = false;  // self-attention unit: output conv on the single-tap k_tc_tcn, else k_tcn_simt
+  bool tcn_tc = false;     // temporal conv on k_tc_tcn / k_tc_tcn2 (tcn_on_pair), else k_tcn_simt
+  bool block64 = false;    // the per-step walk runs graph conv + temporal conv as ONE kernel (k_tc_block64)
+  bool gcn_tc() const {
+    return gcn == GcnRoute::kTc || gcn == GcnRoute::kTcT || gcn == GcnRoute::kTcAgcn || gcn == GcnRoute::kTcAgcnt;
+  }
+};
+
 struct BlockW {
   // host copies as loaded (BN already folded by the caller)
   std::vector<float> mix, gcn_w, gcn_b, tcn_w, res_w, tcn_b, att_w, att_b, sa_scale, sa_shift, sa_qkv_w, sa_qkv_b, sa_skip;
+  Route route;
   // device, SIMT format (k-major fp32)
   float *d_gcn_w = nullptr, *d_gcn_b = nullptr, *d_tcn_w = nullptr, *d_res_w = nullptr, *d_tcn_b = nullptr;
   int *d_mix_ptr = nullptr, *d_mix_src = nullptr;
@@ -61,12 +95,9 @@ struct BlockW {
   float *d_sa_scale = nullptr, *d_sa_shift = nullptr, *d_sa_qkv_w = nullptr, *d_sa_qkv_b = nullptr, *d_res_w_sa = nullptr;
   __nv_bfloat16 *d_sa_w16 = nullptr;  // output conv (+ identity K-block) for the single-tap tcgen05 launch
   CUtensorMap map_sa_w, map_sa_w_half;
-  bool tc_sa_out = false, sa_res_kblock = false;
   ActBuf sa;  // attention output rows of the frame in flight (1 slot), operand of the output conv
   // tensor-core qkv conv: normalised input rows; unfused (C = 64), the conv runs on the single-tap temporal-conv kernel
   // into q | k | v rows zero-padded to kSaQkvCols columns
-  bool tc_sa_qkv = false;
-  bool tc_sa_fused = false;  // qkv conv + attention in one kernel (k_tc_sa): q, k, v never leave the SM
   __nv_bfloat16 *d_sa_fw16 = nullptr;  // qkv weights regrouped per head group: [items][hi: q, k, v | lo: same][cin]
   float *d_sa_fbias = nullptr;         // [items][96]
   CUtensorMap map_sa_fw;
@@ -74,34 +105,22 @@ struct BlockW {
   __nv_bfloat16 *d_sa_qw16 = nullptr;  // unfused qkv conv: [2*kSaQkvCols rows (hi, lo)][cin]
   float *d_sa_qbias = nullptr;
   CUtensorMap map_sa_q;
-  int mix_max_nz = 0;
   int gcn_parts = 4;  // accumulator column groups of the tensor-core graph conv (3 or 4)
   bool gcn_folded = false;  // gcn_residual folded into W_0 on the host (every self link exactly 1): no residual rows, three groups
-  int mix_max_row12 = 0;  // most non-zeros of partitions 1 and 2 together for one output vertex
-  bool mix_diag0 = true;  // partition 0 has only self links
   // device, tensor-core format: [2*cout rows (hi, lo)][K] bf16
   __nv_bfloat16 *d_gcn_w16 = nullptr, *d_tcn_w16 = nullptr, *d_att_w16 = nullptr;
   CUtensorMap map_gcn_w, map_tcn_w, map_tcn_w_half, map_att_w;  // _half: box of cout/2 rows for the CTA-pair kernel
-  bool tc_gcn = false, tc_tcn = false;
-  // pre-mix graph conv weights of the fused block kernel: [2*cout rows (hi, lo)][gcnp_parts*cin], partition-major K
-  bool gcnp_unit_diag = false;
-  bool gcnp_ready = false;  // weights of the pre-mix form are uploaded
-  bool fuse = false;        // this block's step runs as ONE kernel (k_tc_block64)
   CUtensorMap map_tcn_w_full;  // temporal-conv weights with a 2*cout-row box: hi and lo rows in one stacked slab
-
+  // pre-mix graph conv weights of the fused block kernel: [2*cout rows (hi, lo)][gcnp_parts*cin], partition-major K
   int gcnp_parts = 3;
   __nv_bfloat16 *d_gcnp_w16 = nullptr;
   CUtensorMap map_gcnp_w;
-  // channel-major graph conv (k_tc_gcnt): weights [2 planes][chunk of 128 channels][part][128] x cin, tree coefficients
-  bool tc_gcnt = false;
-  bool tc_agcnt = false;  // adaptive graph conv: dense mix on the channel-major kernel k_tc_agcnt (same weight layout, always 4 parts)
+  // channel-major graph conv (k_tc_gcnt, and k_tc_agcnt with always 4 parts): weights [2 planes][chunk of 128 channels][part][128]
+  // x cin, tree coefficients
   int gcnt_parts = 4;
   __nv_bfloat16 *d_gcnt_w16 = nullptr;
   CUtensorMap map_gcnt_w;
   float gcnt_coef[3][32];
-  bool tc_attn = false;  // adaptive graph conv: attention half on the tcgen05 kernel
-  bool tcn_res_kblock = false;  // tensor-core temporal conv: the residual enters as extra K-blocks of the GEMM (folded
-                                // strided conv, or identity weights for the narrow layers) instead of epilogue loads
   long long n_in = 0, n_out = 0;
   ActBuf ring, out;
 };
@@ -269,18 +288,90 @@ inline float bf2f(uint16_t h) {
   return f;
 }
 
-// [rows][K] fp32 -> [2*rows][K] bf16: hi rows then lo rows
-std::vector<uint16_t> split_rows(const std::vector<float> &w, int rows, int K) {
+// [rows][K] fp32 -> [2*rows][K] bf16, per group of `group` rows (rows % group == 0): its hi rows, then its lo rows
+std::vector<uint16_t> split_rows(const std::vector<float> &w, int rows, int K, int group) {
   std::vector<uint16_t> o((size_t)2 * rows * K);
+  const size_t gk = (size_t)group * K;
   for (size_t i = 0; i < (size_t)rows * K; ++i) {
+    const size_t hi = i + i / gk * gk;  // the rows of the groups before this one are stacked twice
     uint16_t h = f2bf(w[i]);
-    o[i] = h;
-    o[(size_t)rows * K + i] = f2bf(w[i] - bf2f(h));
+    o[hi] = h;
+    o[hi + gk] = f2bf(w[i] - bf2f(h));
   }
   return o;
 }
 
+// split_rows of a [rows][K] weight matrix uploaded to `dst`, with a TMA map of `box`-row boxes
+int upload_split(cosk_model *m, __nv_bfloat16 *&dst, CUtensorMap *map, const std::vector<float> &w, int rows, int K, uint32_t box,
+                 int group = 0) {
+  const std::vector<uint16_t> s = split_rows(w, rows, K, group ? group : rows);
+  int rc = upload(m, reinterpret_cast<uint16_t *&>(dst), s.data(), s.size());
+  return rc ? rc : make_map(m, map, dst, (uint64_t)K, (uint64_t)2 * rows, box);
+}
+
+// Graph-conv weights [cout][(3 + res_conv) * cin] regrouped per part for the tensor-core kernels: row
+// (o / group) * (P * group) + part * group + o % group holds W_part of output channel o, K = cin.  Part 3, when P = 4, is the
+// gcn_residual branch: the folded 1x1 conv when cin != cout, else the identity matrix.  `fold`: the residual is added into W_0
+// instead (every self link exactly 1).
+std::vector<float> regroup_parts(const std::vector<float> &gcn_w, int cin, int cout, int group, int P, bool fold) {
+  const bool res_conv = cin != cout;
+  const size_t Kg = (size_t)(3 + res_conv) * cin;
+  std::vector<float> re((size_t)P * cout * cin, 0.f);
+  for (int o = 0; o < cout; ++o)
+    for (int part = 0; part < P; ++part) {
+      float *row = &re[((size_t)(o / group) * (P * group) + (size_t)part * group + (o % group)) * cin];
+      if (part < 3 || res_conv) memcpy(row, &gcn_w[(size_t)o * Kg + (size_t)part * cin], sizeof(float) * cin);
+      else row[o] = 1.0f;
+      if (fold && part == 0) {
+        if (res_conv)
+          for (int k = 0; k < cin; ++k) row[k] += gcn_w[(size_t)o * Kg + (size_t)3 * cin + k];
+        else
+          row[o] += 1.0f;
+      }
+    }
+  return re;
+}
+
+// Does the mixing matrix have exactly the sparsity of the skeleton tree k_tc_gcnt is compiled for (partition 1 = one entry
+// per vertex, from its parent; partition 2 = entries from a vertex's children)?  Fills the kernel's coefficients.
+bool tree_coefs(const std::vector<float> &mix, int V, float coef[3][32]) {
+  auto parent = [&](int w) { return V == 25 ? skel_parent<25>(w) : skel_parent<18>(w); };
+  bool tree = true;
+  memset(coef, 0, sizeof(float) * 3 * 32);
+  for (int v = 0; v < V; ++v)
+    for (int w = 0; w < V; ++w) {
+      const float a0 = mix[((size_t)0 * V + v) * V + w], a1 = mix[((size_t)1 * V + v) * V + w], a2 = mix[((size_t)2 * V + v) * V + w];
+      if (v == w) coef[0][w] = a0;
+      if (a1 != 0.f) {
+        if (parent(w) == v) coef[1][w] = a1;
+        else tree = false;
+      }
+      if (a2 != 0.f) {
+        if (parent(v) == w) coef[2][v] = a2;
+        else tree = false;
+      }
+    }
+  return tree;
+}
+
 bool tc_width(int c) { return c == 64 || c == 128 || c == 256; }
+
+// Narrow first layer (cin <= 8): k_gcn_small keeps the weights and the mixed inputs of a tile in shared memory, and the
+// adaptive one computes its embeddings per thread (k_attn_small).
+bool gcn_small(const cosk_model *m, const cosk_block_cfg &bc) {
+  const int res_conv = bc.cin != bc.cout ? 1 : 0;
+  return m->cfg.path == COSK_PATH_AUTO && bc.cin <= 8 && res_conv && bc.cout % 32 == 0 && (3 + res_conv) * bc.cin <= kSmallKMax;
+}
+bool attn_small(const cosk_model *m, const cosk_block_cfg &bc) {
+  return bc.gconv == COSK_GCONV_ADAPTIVE && m->cfg.path == COSK_PATH_AUTO && bc.cin <= 8 && bc.cout == 64 &&
+         (m->cfg.vertices == 25 || m->cfg.vertices == 18);
+}
+
+// The tensor-core temporal conv takes the residual as extra K-blocks of its GEMM (folded strided conv, or identity weights
+// for the narrow layers) instead of epilogue loads.
+bool tcn_res_kblock(const cosk_block_cfg &bc) {
+  return bc.res_kind == COSK_RES_CONV || (bc.res_kind == COSK_RES_IDENTITY && bc.cout <= 128);
+}
 
 int prepare(cosk_model *m) {
   const cosk_config &c = m->cfg;
@@ -332,28 +423,32 @@ int prepare(cosk_model *m) {
     // CSR of A * graph_attn over (partition, output vertex)
     std::vector<int> ptr(3 * V + 1, 0), src;
     std::vector<float> val;
-    b.mix_max_nz = 0;
-    b.mix_diag0 = true;
+    bool mix_diag0 = true;  // partition 0 has only self links
     for (int p = 0; p < 3; ++p)
       for (int w = 0; w < V; ++w) {
-        int cnt = 0;
         for (int v = 0; v < V; ++v) {
           float a = b.mix[((size_t)p * V + v) * V + w];
           if (a != 0.f) {
             src.push_back(v);
             val.push_back(a);
-            ++cnt;
-            if (p == 0 && v != w) b.mix_diag0 = false;
+            if (p == 0 && v != w) mix_diag0 = false;
           }
         }
         ptr[p * V + w + 1] = (int)src.size();
-        if (cnt > b.mix_max_nz) b.mix_max_nz = cnt;
       }
-    b.mix_max_row12 = 0;
+    // most non-zeros of partitions 1 and 2 together, and of one of them, for one output vertex
+    int mix_max_row12 = 0, part_max = 0;
     for (int w = 0; w < V; ++w) {
-      const int n12 = ptr[2 * V + w + 1] - ptr[2 * V + w] + ptr[V + w + 1] - ptr[V + w];
-      if (n12 > b.mix_max_row12) b.mix_max_row12 = n12;
+      const int n1 = ptr[V + w + 1] - ptr[V + w], n2 = ptr[2 * V + w + 1] - ptr[2 * V + w];
+      mix_max_row12 = std::max(mix_max_row12, n1 + n2);
+      part_max = std::max({part_max, n1, n2});
     }
+    // Every self link exactly 1 (A_0 = I with graph_attn's diagonal at 1, the reference initialisation): the own-row term of
+    // partition 0 and the gcn_residual branch act on the same rows, x W_0^T + x R^T = x (W_0 + R)^T, so the plain tensor-core
+    // graph convs add the residual (identity or folded conv) into W_0 on the host and drop a part: a quarter fewer MMAs and
+    // TMEM reads, no residual rows fetched.  Trained self-link coefficients keep the four-part form.
+    bool unit_diag = !adaptive && mix_diag0;
+    for (int w0 = 0; unit_diag && w0 < V; ++w0) unit_diag = (ptr[w0 + 1] - ptr[w0] == 1 && val[ptr[w0]] == 1.0f);
     if (src.empty()) {
       src.push_back(0);
       val.push_back(0.f);
@@ -379,148 +474,79 @@ int prepare(cosk_model *m) {
       if ((rc = upload(m, b.d_att_b, b.att_b.data(), b.att_b.size()))) return rc;
       if ((rc = upload(m, b.d_adj, b.mix.data(), b.mix.size()))) return rc;
     }
-    // tensor-core eligibility + weights
+
+    // The route: which kernels serve this block.
+    Route &rt = b.route;
+    rt = Route();
     const bool want_tc = c.path == COSK_PATH_AUTO;
-    if (attention)
-      b.tc_gcn = false;  // qkv + attention run on CUDA cores this round; the output conv below is the tensor-core part
-    else if (adaptive)  // dense-mix kernel: instantiated for the two skeleton sizes the reference ships
-      b.tc_gcn = want_tc && bc.cout % 64 == 0 && bc.cout <= 256 && bc.cin % kBK == 0 && (V == 25 || V == 18);
-    else
-      b.tc_gcn = want_tc && bc.cout % 64 == 0 && bc.cout <= 256 && bc.cin % kBK == 0 && b.mix_max_row12 <= kMixSlots && b.mix_diag0;
-    b.tc_tcn = want_tc && tc_width(bc.cout) && (bc.res_kind != COSK_RES_CONV || bc.cin % kBK == 0);
-    if (b.tc_gcn) {
-      // Rows regrouped per pass of 64 output channels: row = pass*(P*64) + part*64 + c, K = cin.
-      // Part 3 is the gcn_residual branch: the folded 1x1 conv when cin != cout, else the identity
-      // matrix (x = hi + lo passes through the split-precision products exactly).  The identity rides in the GEMM
-      // except for the 256-channel layers, where the mix warps have the slack to add the input rows and the narrower
-      // accumulator saves MMA columns and TMEM reads (measured -8 %).
-      // (adaptive: 4 parts need the single-stage layout, so the identity rides along only when one K-block is all there is)
+    const bool skel_v = V == 25 || V == 18;  // the skeletons the dense-mix and channel-major kernels are instantiated for
+    const bool t_shape = (bc.cout == 128 || bc.cout == 256) && (bc.cin == 64 || bc.cin == 128) && skel_v;  // channel-major kernels
+    bool tc_gcn = false;  // graph conv (adaptive: its mix) on the tensor cores, with weights in the k_tc_gcn layout
+    if (adaptive)
+      tc_gcn = want_tc && bc.cout % 64 == 0 && bc.cout <= 256 && bc.cin % kBK == 0 && skel_v;
+    else if (!attention)
+      tc_gcn = want_tc && bc.cout % 64 == 0 && bc.cout <= 256 && bc.cin % kBK == 0 && mix_max_row12 <= kMixSlots && mix_diag0;
+    if (attention) {
+      // The fused kernel has eight epilogue warps per SM for the attention math: a win where the q | k | v round trip
+      // dominates (C >= 128), a loss for the 64-channel unit, whose eight tiny heads want the separate kernel's occupancy.
+      const bool tc_qkv = want_tc && bc.cin % kBK == 0 && tc_width(bc.cout);
+      rt.gcn = !tc_qkv ? GcnRoute::kSaSimt : bc.cout >= 128 ? GcnRoute::kSaTcFused : GcnRoute::kSaTcQkv;
+      rt.sa_out_tc = want_tc && tc_width(bc.cout);
+    } else if (adaptive) {
+      rt.attn = tc_gcn && tc_width(bc.cout) ? AttnRoute::kTc : attn_small(m, bc) ? AttnRoute::kSmall : AttnRoute::kSimt;
+      if (tc_gcn) rt.gcn = kAgcntBuilt && m->agcn_transposed && t_shape ? GcnRoute::kTcAgcnt : GcnRoute::kTcAgcn;
+      else rt.gcn = gcn_small(m, bc) ? GcnRoute::kSmall : GcnRoute::kSimt;
+    } else if (tc_gcn) {
+      rt.gcn = m->gcn_transposed && t_shape && tree_coefs(b.mix, V, b.gcnt_coef) ? GcnRoute::kTcT : GcnRoute::kTc;
+    } else {
+      rt.gcn = gcn_small(m, bc) ? GcnRoute::kSmall : GcnRoute::kSimt;
+    }
+    rt.tcn_tc = want_tc && tc_width(bc.cout) && (bc.res_kind != COSK_RES_CONV || bc.cin % kBK == 0);
+    // one kernel per block step: 64 -> 64 blocks with the identity residual riding in both GEMMs; the sources per
+    // (partition >= 1, output vertex) must fit the register CSR of its pre-mix graph conv
+    rt.block64 = m->fuse_block && tc_gcn && bc.gconv == COSK_GCONV_PLAIN && part_max <= kPartSrcMax && bc.cin == 64 &&
+                bc.cout == 64 && bc.stride == 1 && bc.res_kind == COSK_RES_IDENTITY && rt.tcn_tc && tcn_res_kblock(bc);
+
+    // Tensor-core weights of the route.
+    if (tc_gcn) {
+      // k_tc_gcn: 64-row groups.  The identity gcn_residual rides in the GEMM (fourth part) except for the 256-channel layers,
+      // where the mix warps have the slack to add the input rows and the narrower accumulator saves MMA columns and TMEM
+      // reads (measured -8 %).  (adaptive: 4 parts need the single-stage layout, so the identity rides along only when one
+      // K-block is all there is)
       const bool ident_mma = bc.cin < 256;
-      // Every self link exactly 1 (A_0 = I with graph_attn's diagonal at 1, the reference initialisation): the own-row term of
-      // partition 0 and the gcn_residual branch act on the same rows, x W_0^T + x R^T = x (W_0 + R)^T, so the residual (identity
-      // or folded conv) is added into W_0 on the host and the accumulator shrinks to three column groups: a quarter fewer MMAs
-      // and TMEM reads, no residual rows fetched.  Trained self-link coefficients keep the four-group form.
-      bool unit_diag = !adaptive && b.mix_diag0;
-      for (int w0 = 0; unit_diag && w0 < V; ++w0) unit_diag = (ptr[w0 + 1] - ptr[w0] == 1 && val[ptr[w0]] == 1.0f);
       b.gcn_folded = unit_diag;
       const int P = b.gcn_parts = adaptive ? ((res_conv || bc.cin == kBK) ? 4 : 3) : (unit_diag ? 3 : ((res_conv || ident_mma) ? 4 : 3));
-      std::vector<float> re((size_t)P * bc.cout * bc.cin, 0.f);
-      for (int o = 0; o < bc.cout; ++o)
-        for (int part = 0; part < P; ++part) {
-          const size_t r = (size_t)(o / 64) * (P * 64) + (size_t)part * 64 + (o % 64);
-          if (part < 3 || res_conv)
-            memcpy(&re[r * bc.cin], &b.gcn_w[(size_t)o * Kg + (size_t)part * bc.cin], sizeof(float) * bc.cin);
-          else
-            re[r * bc.cin + o] = 1.0f;
-          if (unit_diag && part == 0) {
-            if (res_conv)
-              for (int k = 0; k < bc.cin; ++k) re[r * bc.cin + k] += b.gcn_w[(size_t)o * Kg + (size_t)3 * bc.cin + k];
-            else
-              re[r * bc.cin + o] += 1.0f;
-          }
-        }
-      std::vector<uint16_t> s = split_rows(re, P * bc.cout, bc.cin);
-      if ((rc = upload(m, reinterpret_cast<uint16_t *&>(b.d_gcn_w16), s.data(), s.size()))) return rc;
-      if ((rc = make_map(m, &b.map_gcn_w, b.d_gcn_w16, (uint64_t)bc.cin, (uint64_t)2 * P * bc.cout, (uint32_t)(P * 64)))) return rc;
+      if ((rc = upload_split(m, b.d_gcn_w16, &b.map_gcn_w, regroup_parts(b.gcn_w, bc.cin, bc.cout, 64, P, unit_diag), P * bc.cout,
+                             bc.cin, (uint32_t)(P * 64))))
+        return rc;
     }
-    b.tc_gcnt = false;
-    if (b.tc_gcn && !adaptive && !attention && m->gcn_transposed && (bc.cout == 128 || bc.cout == 256) &&
-        (bc.cin == 64 || bc.cin == 128) && (V == 25 || V == 18) && b.mix_diag0) {
-      // The mixing matrix must have exactly the sparsity of the skeleton tree the kernel is compiled for: partition 1 = one
-      // entry per vertex, from its parent; partition 2 = entries from a vertex's children.
-      auto parent = [&](int w) { return V == 25 ? skel_parent<25>(w) : skel_parent<18>(w); };
-      bool tree = true;
-      memset(b.gcnt_coef, 0, sizeof b.gcnt_coef);
-      for (int v = 0; v < V; ++v)
-        for (int w = 0; w < V; ++w) {
-          const float a0 = b.mix[((size_t)0 * V + v) * V + w], a1 = b.mix[((size_t)1 * V + v) * V + w],
-                      a2 = b.mix[((size_t)2 * V + v) * V + w];
-          if (v == w) b.gcnt_coef[0][w] = a0;
-          if (a1 != 0.f) {
-            if (parent(w) == v) b.gcnt_coef[1][w] = a1;
-            else tree = false;
-          }
-          if (a2 != 0.f) {
-            if (parent(v) == w) b.gcnt_coef[2][v] = a2;
-            else tree = false;
-          }
+    if (rt.gcn == GcnRoute::kTcT || rt.gcn == GcnRoute::kTcAgcnt) {
+      // channel-major layout, 128-row groups, the residual folded as for k_tc_gcn (k_tc_agcnt: never, always four parts)
+      const int P = b.gcnt_parts = b.gcn_folded ? 3 : 4;
+      if ((rc = upload_split(m, b.d_gcnt_w16, &b.map_gcnt_w, regroup_parts(b.gcn_w, bc.cin, bc.cout, 128, P, b.gcn_folded),
+                             P * bc.cout, bc.cin, 128u)))
+        return rc;
+    }
+    if (rt.block64) {
+      // Pre-mix form.  K-blocks in the order the mix warps fill their A slots: the plain input rows (gcn_residual weights:
+      // folded 1x1 conv or identity; plus W_0 when every self link is exactly 1, so that x and 1*x share one part),
+      // [W_0 on a0*x], W_1, W_2
+      const int P = b.gcnp_parts = unit_diag ? 3 : 4;
+      const int K = P * bc.cin;
+      std::vector<float> w((size_t)bc.cout * K, 0.f);
+      for (int o = 0; o < bc.cout; ++o) {
+        float *row = &w[(size_t)o * K];
+        const float *src = &b.gcn_w[(size_t)o * Kg];
+        if (res_conv) memcpy(row, src + 3 * bc.cin, sizeof(float) * bc.cin);
+        else row[o] = 1.0f;
+        if (unit_diag) {
+          for (int k = 0; k < bc.cin; ++k) row[k] += src[k];
+          memcpy(row + bc.cin, src + bc.cin, sizeof(float) * 2 * bc.cin);
+        } else {
+          memcpy(row + bc.cin, src, sizeof(float) * 3 * bc.cin);
         }
-      if (tree) {
-        // as for k_tc_gcn: every self link exactly 1 -> gcn_residual folded into W_0, three parts; else the residual (folded
-        // 1x1 conv, or the identity matrix) is a fourth part
-        const int P = b.gcnt_parts = b.gcn_folded ? 3 : 4;
-        std::vector<float> re((size_t)P * bc.cout * bc.cin, 0.f);
-        for (int o = 0; o < bc.cout; ++o)
-          for (int part = 0; part < P; ++part) {
-            float *row = &re[(((size_t)(o / 128) * P + part) * 128 + (o % 128)) * bc.cin];
-            if (part < 3 || res_conv) memcpy(row, &b.gcn_w[(size_t)o * Kg + (size_t)part * bc.cin], sizeof(float) * bc.cin);
-            else row[o] = 1.0f;
-            if (b.gcn_folded && part == 0) {
-              if (res_conv)
-                for (int k = 0; k < bc.cin; ++k) row[k] += b.gcn_w[(size_t)o * Kg + (size_t)3 * bc.cin + k];
-              else
-                row[o] += 1.0f;
-            }
-          }
-        std::vector<uint16_t> s = split_rows(re, P * bc.cout, bc.cin);
-        if ((rc = upload(m, reinterpret_cast<uint16_t *&>(b.d_gcnt_w16), s.data(), s.size()))) return rc;
-        if ((rc = make_map(m, &b.map_gcnt_w, b.d_gcnt_w16, (uint64_t)bc.cin, (uint64_t)2 * P * bc.cout, 128u))) return rc;
-        b.tc_gcnt = true;
       }
-    }
-    b.tc_agcnt = false;
-#ifdef COSK_WITH_AGCNT
-    const bool agcnt_built = true;
-#else
-    const bool agcnt_built = false;
-#endif
-    if (agcnt_built && b.tc_gcn && adaptive && m->agcn_transposed && (bc.cout == 128 || bc.cout == 256) && (bc.cin == 64 || bc.cin == 128) &&
-        (V == 25 || V == 18)) {
-      // channel-major layout, always four parts: W_0, W_1, W_2, gcn_residual (folded 1x1 conv, or the identity matrix)
-      const int P = 4;
-      std::vector<float> re((size_t)P * bc.cout * bc.cin, 0.f);
-      for (int o = 0; o < bc.cout; ++o)
-        for (int part = 0; part < P; ++part) {
-          float *row = &re[(((size_t)(o / 128) * P + part) * 128 + (o % 128)) * bc.cin];
-          if (part < 3 || res_conv) memcpy(row, &b.gcn_w[(size_t)o * Kg + (size_t)part * bc.cin], sizeof(float) * bc.cin);
-          else row[o] = 1.0f;
-        }
-      std::vector<uint16_t> s = split_rows(re, P * bc.cout, bc.cin);
-      if ((rc = upload(m, reinterpret_cast<uint16_t *&>(b.d_gcnt_w16), s.data(), s.size()))) return rc;
-      if ((rc = make_map(m, &b.map_gcnt_w, b.d_gcnt_w16, (uint64_t)bc.cin, (uint64_t)2 * P * bc.cout, 128u))) return rc;
-      b.gcnt_parts = P;
-      b.tc_agcnt = true;
-    }
-    {
-      // pre-mix form of the fused block kernel: sources per (partition >= 1, output vertex) must fit its register CSR
-      int part_max = 0;
-      for (int p = 1; p < 3; ++p)
-        for (int w = 0; w < V; ++w) part_max = std::max(part_max, ptr[p * V + w + 1] - ptr[p * V + w]);
-      b.gcnp_ready = b.tc_gcn && !adaptive && !attention && tc_width(bc.cout) && part_max <= kPartSrcMax;
-      if (b.gcnp_ready) {
-        b.gcnp_unit_diag = true;
-        for (int w0 = 0; w0 < V; ++w0) b.gcnp_unit_diag &= (ptr[w0 + 1] - ptr[w0] == 1 && val[ptr[w0]] == 1.0f);
-        // K-blocks in the order the mix warps fill their A slots: the plain input rows (gcn_residual weights: folded 1x1 conv
-        // or identity; plus W_0 when every self link is exactly 1, so that x and 1*x share one part), [W_0 on a0*x], W_1, W_2
-        const int P = b.gcnp_parts = b.gcnp_unit_diag ? 3 : 4;
-        const int K = P * bc.cin;
-        std::vector<float> w((size_t)bc.cout * K, 0.f);
-        for (int o = 0; o < bc.cout; ++o) {
-          float *row = &w[(size_t)o * K];
-          const float *src = &b.gcn_w[(size_t)o * Kg];
-          if (res_conv) memcpy(row, src + 3 * bc.cin, sizeof(float) * bc.cin);
-          else row[o] = 1.0f;
-          if (b.gcnp_unit_diag) {
-            for (int k = 0; k < bc.cin; ++k) row[k] += src[k];
-            memcpy(row + bc.cin, src + bc.cin, sizeof(float) * 2 * bc.cin);
-          } else {
-            memcpy(row + bc.cin, src, sizeof(float) * 3 * bc.cin);
-          }
-        }
-        std::vector<uint16_t> s = split_rows(w, bc.cout, K);
-        if ((rc = upload(m, reinterpret_cast<uint16_t *&>(b.d_gcnp_w16), s.data(), s.size()))) return rc;
-        if ((rc = make_map(m, &b.map_gcnp_w, b.d_gcnp_w16, (uint64_t)K, (uint64_t)2 * bc.cout, (uint32_t)std::min(2 * bc.cout, 256)))) return rc;
-      }
+      if ((rc = upload_split(m, b.d_gcnp_w16, &b.map_gcnp_w, w, bc.cout, K, (uint32_t)std::min(2 * bc.cout, 256)))) return rc;
     }
     if (attention) {
       std::vector<float> tq = transpose(b.sa_qkv_w.data(), 2 * (bc.cout / 4) + bc.cout, bc.cin);
@@ -528,21 +554,15 @@ int prepare(cosk_model *m) {
       if ((rc = upload(m, b.d_sa_qkv_b, b.sa_qkv_b.data(), b.sa_qkv_b.size()))) return rc;
       if ((rc = upload(m, b.d_sa_scale, b.sa_scale.data(), b.sa_scale.size()))) return rc;
       if ((rc = upload(m, b.d_sa_shift, b.sa_shift.data(), b.sa_shift.size()))) return rc;
-      b.tc_sa_qkv = want_tc && bc.cin % kBK == 0 && tc_width(bc.cout);
-      // the fused kernel has eight epilogue warps per SM for the attention math: a win where the q | k | v round trip
-      // dominates (C >= 128), a loss for the 64-channel unit, whose eight tiny heads want the separate kernel's occupancy
-      b.tc_sa_fused = b.tc_sa_qkv && bc.cout >= 128;
-      if (b.tc_sa_qkv && !b.tc_sa_fused) {
+      if (rt.gcn == GcnRoute::kSaTcQkv) {
         const int nq = 2 * (bc.cout / 4) + bc.cout;
         std::vector<float> w((size_t)kSaQkvCols * bc.cin, 0.f), bb((size_t)kSaQkvCols, 0.f);  // rows nq.. stay zero
         memcpy(w.data(), b.sa_qkv_w.data(), sizeof(float) * nq * bc.cin);
         memcpy(bb.data(), b.sa_qkv_b.data(), sizeof(float) * nq);
-        std::vector<uint16_t> s16 = split_rows(w, kSaQkvCols, bc.cin);
-        if ((rc = upload(m, reinterpret_cast<uint16_t *&>(b.d_sa_qw16), s16.data(), s16.size()))) return rc;
+        if ((rc = upload_split(m, b.d_sa_qw16, &b.map_sa_q, w, kSaQkvCols, bc.cin, (uint32_t)kSaQkvCols))) return rc;
         if ((rc = upload(m, b.d_sa_qbias, bb.data(), bb.size()))) return rc;
-        if ((rc = make_map(m, &b.map_sa_q, b.d_sa_qw16, (uint64_t)bc.cin, (uint64_t)2 * kSaQkvCols, (uint32_t)kSaQkvCols))) return rc;
       }
-      if (b.tc_sa_fused) {
+      if (rt.gcn == GcnRoute::kSaTcFused) {
         const int dk = bc.cout / 4, dvh = bc.cout / 8, dkh = dk / 8, G = 64 / dvh, items = 8 / G;
         std::vector<float> w((size_t)items * 96 * bc.cin), bb((size_t)items * 96);
         for (int it = 0; it < items; ++it)
@@ -554,18 +574,8 @@ int prepare(cosk_model *m) {
             memcpy(&w[((size_t)it * 96 + r) * bc.cin], &b.sa_qkv_w[(size_t)src * bc.cin], sizeof(float) * bc.cin);
             bb[(size_t)it * 96 + r] = b.sa_qkv_b[src];
           }
-        std::vector<uint16_t> st((size_t)items * 192 * bc.cin);
-        for (int it = 0; it < items; ++it)
-          for (int r = 0; r < 96; ++r)
-            for (int k = 0; k < bc.cin; ++k) {
-              const float x = w[((size_t)it * 96 + r) * bc.cin + k];
-              const uint16_t h = f2bf(x);
-              st[((size_t)it * 192 + r) * bc.cin + k] = h;
-              st[((size_t)it * 192 + 96 + r) * bc.cin + k] = f2bf(x - bf2f(h));
-            }
-        if ((rc = upload(m, reinterpret_cast<uint16_t *&>(b.d_sa_fw16), st.data(), st.size()))) return rc;
+        if ((rc = upload_split(m, b.d_sa_fw16, &b.map_sa_fw, w, items * 96, bc.cin, 192u, 96))) return rc;  // hi | lo per item
         if ((rc = upload(m, b.d_sa_fbias, bb.data(), bb.size()))) return rc;
-        if ((rc = make_map(m, &b.map_sa_fw, b.d_sa_fw16, (uint64_t)bc.cin, (uint64_t)items * 192, 192u))) return rc;
       }
       // The skip connection is added before the unit's bn, so it enters scaled per channel: a diagonal "residual conv".
       if (!res_conv) {
@@ -574,65 +584,42 @@ int prepare(cosk_model *m) {
         if ((rc = upload(m, b.d_res_w_sa, diag.data(), diag.size()))) return rc;
       }
       // output conv on the temporal-conv kernel with a single tap: [W0 | diag(skip scale) K-block on the input rows]
-      b.tc_sa_out = want_tc && tc_width(bc.cout);
-      if (b.tc_sa_out) {
-        b.sa_res_kblock = !res_conv;
-        const int Kr = b.sa_res_kblock ? bc.cin : 0, K0 = bc.cout;
+      if (rt.sa_out_tc) {
+        const int Kr = res_conv ? 0 : bc.cin, K0 = bc.cout;
         std::vector<float> cat((size_t)bc.cout * (K0 + Kr), 0.f);
         for (int r = 0; r < bc.cout; ++r) {
           memcpy(&cat[(size_t)r * (K0 + Kr)], &b.gcn_w[(size_t)r * K0], sizeof(float) * K0);
-          if (b.sa_res_kblock) cat[(size_t)r * (K0 + Kr) + K0 + r] = b.sa_skip[r];
+          if (Kr) cat[(size_t)r * (K0 + Kr) + K0 + r] = b.sa_skip[r];
         }
-        std::vector<uint16_t> s16 = split_rows(cat, bc.cout, K0 + Kr);
-        if ((rc = upload(m, reinterpret_cast<uint16_t *&>(b.d_sa_w16), s16.data(), s16.size()))) return rc;
-        if ((rc = make_map(m, &b.map_sa_w, b.d_sa_w16, (uint64_t)(K0 + Kr), (uint64_t)2 * bc.cout, (uint32_t)bc.cout))) return rc;
+        if ((rc = upload_split(m, b.d_sa_w16, &b.map_sa_w, cat, bc.cout, K0 + Kr, (uint32_t)bc.cout))) return rc;
         if ((rc = make_map(m, &b.map_sa_w_half, b.d_sa_w16, (uint64_t)(K0 + Kr), (uint64_t)2 * bc.cout, (uint32_t)bc.cout / 2))) return rc;
       }
     }
-    b.tc_attn = adaptive && b.tc_gcn && tc_width(bc.cout);
-    if (b.tc_attn) {
+    if (rt.attn == AttnRoute::kTc) {
       // per partition: hi rows of (theta, phi), then their lo rows -- one stacked operand of 4*IC rows
       const int ic = bc.cout / 4;
-      std::vector<uint16_t> st((size_t)12 * ic * bc.cin);
-      for (int part = 0; part < 3; ++part)
-        for (int r = 0; r < 2 * ic; ++r)
-          for (int k = 0; k < bc.cin; ++k) {
-            const float w = b.att_w[((size_t)part * 2 * ic + r) * bc.cin + k];
-            const uint16_t h = f2bf(w);
-            st[((size_t)part * 4 * ic + r) * bc.cin + k] = h;
-            st[((size_t)part * 4 * ic + 2 * ic + r) * bc.cin + k] = f2bf(w - bf2f(h));
-          }
-      if ((rc = upload(m, reinterpret_cast<uint16_t *&>(b.d_att_w16), st.data(), st.size()))) return rc;
-      if ((rc = make_map(m, &b.map_att_w, b.d_att_w16, (uint64_t)bc.cin, (uint64_t)12 * ic, (uint32_t)(4 * ic)))) return rc;
+      if ((rc = upload_split(m, b.d_att_w16, &b.map_att_w, b.att_w, 6 * ic, bc.cin, (uint32_t)(4 * ic), 2 * ic))) return rc;
     }
-    if (b.tc_tcn) {
+    if (rt.tcn_tc) {
       // The delayed residual x_{n-4} is streamed through the operand ring like a tenth tap: with the folded
       // strided 1x1 conv as its weights (layers 5 and 8), or -- for the identity residual of the HBM-bound
       // narrow layers -- with identity weights (exact under the split products), which removes every
       // latency-bound load from the epilogue.  The 256-channel layers are tensor-bound and keep the add.
-      const bool ident_k = bc.res_kind == COSK_RES_IDENTITY && bc.cout <= 128;
-      b.tcn_res_kblock = bc.res_kind == COSK_RES_CONV || ident_k;
-      const int Kr = b.tcn_res_kblock ? bc.cin : 0;
+      const int Kr = tcn_res_kblock(bc) ? bc.cin : 0;
       std::vector<float> cat((size_t)bc.cout * (Kt + Kr));
       for (int r = 0; r < bc.cout; ++r) {
         memcpy(&cat[(size_t)r * (Kt + Kr)], &b.tcn_w[(size_t)r * Kt], sizeof(float) * Kt);
         if (bc.res_kind == COSK_RES_CONV) memcpy(&cat[(size_t)r * (Kt + Kr) + Kt], &b.res_w[(size_t)r * Kr], sizeof(float) * Kr);
-        else if (ident_k)
+        else
           for (int k = 0; k < Kr; ++k) cat[(size_t)r * (Kt + Kr) + Kt + k] = k == r ? 1.0f : 0.0f;
       }
-      std::vector<uint16_t> s = split_rows(cat, bc.cout, Kt + Kr);
-      if ((rc = upload(m, reinterpret_cast<uint16_t *&>(b.d_tcn_w16), s.data(), s.size()))) return rc;
-      if ((rc = make_map(m, &b.map_tcn_w, b.d_tcn_w16, (uint64_t)(Kt + Kr), (uint64_t)2 * bc.cout, (uint32_t)bc.cout)))
-        return rc;
+      if ((rc = upload_split(m, b.d_tcn_w16, &b.map_tcn_w, cat, bc.cout, Kt + Kr, (uint32_t)bc.cout))) return rc;
       if ((rc = make_map(m, &b.map_tcn_w_half, b.d_tcn_w16, (uint64_t)(Kt + Kr), (uint64_t)2 * bc.cout, (uint32_t)bc.cout / 2)))
         return rc;
       if (bc.cout <= 128 &&
           (rc = make_map(m, &b.map_tcn_w_full, b.d_tcn_w16, (uint64_t)(Kt + Kr), (uint64_t)2 * bc.cout, (uint32_t)(2 * bc.cout))))
         return rc;
     }
-    // one kernel per block step: 64 -> 64 blocks with the identity residual riding in both GEMMs
-    b.fuse = m->fuse_block && b.gcnp_ready && bc.cin == 64 && bc.cout == 64 && bc.stride == 1 &&
-             bc.res_kind == COSK_RES_IDENTITY && b.tc_tcn && b.tcn_res_kblock && bc.gconv == COSK_GCONV_PLAIN;
   }
   m->prepared = true;
   return COSK_OK;
@@ -689,12 +676,14 @@ int prof_mark(cosk_model *m, int kind, int block, cudaStream_t s) {
   return COSK_OK;
 }
 
-// The launchers size their grids for the (frame, tile) work items of `args`: n_tiles * n_frames, at most one CTA per SM.
+// Persistent kernels: one CTA per work item, at most one per SM.
+int persistent_grid(const cosk_model *m, int items) { return std::min(items, m->num_sms); }
+
+// The launchers size their grids for the (frame, tile) work items of `args`: n_tiles * n_frames.
 template <int COUT>
 int launch_tc_tcn(cosk_model *m, const TcTcnArgs &args, cudaStream_t s) {
-  const int items = m->n_tiles * args.n_frames;
-  const int grid = items < m->num_sms ? items : m->num_sms;
-  CK(launch_k(k_tc_tcn<COUT>, dim3(grid), dim3(256), TcTcnCfg<COUT>::kSmemBytes, s, args));
+  const dim3 grid(persistent_grid(m, m->n_tiles * args.n_frames));
+  CK(launch_k(k_tc_tcn<COUT>, grid, dim3(256), TcTcnCfg<COUT>::kSmemBytes, s, args));
   return COSK_OK;
 }
 template <int COUT>
@@ -708,24 +697,21 @@ int launch_tc_tcn2(cosk_model *m, const TcTcnArgs &args, cudaStream_t s) {
 }
 template <int P, int STAGES>
 int launch_tc_gcn(cosk_model *m, const TcGcnArgs &args, cudaStream_t s) {
-  const int items = m->n_tiles * args.n_frames;
-  const int grid = items < m->num_sms ? items : m->num_sms;
-  if (m->d_trace) CK(launch_k(k_tc_gcn<P, STAGES, true>, dim3(grid), dim3(512), TcGcnCfg<P, STAGES>::kSmemBytes, s, args));
-  else CK(launch_k(k_tc_gcn<P, STAGES, false>, dim3(grid), dim3(512), TcGcnCfg<P, STAGES>::kSmemBytes, s, args));
+  const dim3 grid(persistent_grid(m, m->n_tiles * args.n_frames));
+  if (m->d_trace) CK(launch_k(k_tc_gcn<P, STAGES, true>, grid, dim3(512), TcGcnCfg<P, STAGES>::kSmemBytes, s, args));
+  else CK(launch_k(k_tc_gcn<P, STAGES, false>, grid, dim3(512), TcGcnCfg<P, STAGES>::kSmemBytes, s, args));
   return COSK_OK;
 }
 
 template <int P, int STAGES, int V>
 int launch_tc_agcn(cosk_model *m, const TcGcnArgs &args, cudaStream_t s) {
-  const int grid = m->n_tiles < m->num_sms ? m->n_tiles : m->num_sms;
-  CK(launch_k(k_tc_agcn<P, STAGES, V>, dim3(grid), dim3(512), TcAgcnCfg<P, STAGES>::kSmemBytes, s, args));
+  CK(launch_k(k_tc_agcn<P, STAGES, V>, dim3(persistent_grid(m, m->n_tiles)), dim3(512), TcAgcnCfg<P, STAGES>::kSmemBytes, s, args));
   return COSK_OK;
 }
 
 template <int IC, int V>
 int launch_tc_attn(cosk_model *m, const TcAttnArgs &args, cudaStream_t s) {
-  const int grid = m->n_tiles < m->num_sms ? m->n_tiles : m->num_sms;
-  CK(launch_k(k_tc_attn<IC, V>, dim3(grid), dim3(384), TcAttnCfg<IC, V>::kSmemBytes, s, args));
+  CK(launch_k(k_tc_attn<IC, V>, dim3(persistent_grid(m, m->n_tiles)), dim3(384), TcAttnCfg<IC, V>::kSmemBytes, s, args));
   return COSK_OK;
 }
 
@@ -774,9 +760,20 @@ int set_smem_attrs(cosk_model *m) {
   return COSK_OK;
 }
 
-TcGcnArgs make_gcn_args(cosk_model *m, int i, const ActBuf &in, int in_slot, int ring_slot) {
+// Ring slots of a launch over consecutive executions: frame f of the launch is frame n + f * step of the stream.
+RingWalk ring_walk(long long n, int step, int slots) {
+  RingWalk w;
+  w.slot0 = mod_slot(n, slots), w.step = step, w.slots = slots;
+  return w;
+}
+
+// Arguments of the tensor-core graph convs for n_frames executions of block i: frame f reads slot in_walk.slot(f) of `in` and
+// writes slot ring_walk.slot(f) of the block's temporal ring.
+TcGcnArgs make_gcn_args(cosk_model *m, int i, const ActBuf &in, int n_frames, RingWalk in_walk, RingWalk ring_walk) {
   const cosk_block_cfg &bc = m->cfg.blocks[i];
   BlockW &b = m->blk[i];
+  const bool batched = n_frames > 1;  // pointers at slot 0 of their rings, the slots from the walks
+  const int in_slot = batched ? 0 : in_walk.slot0, ring_slot = batched ? 0 : ring_walk.slot0;
   TcGcnArgs a;
   a.tm_x = in.map;
   a.tm_w = b.map_gcn_w;
@@ -804,6 +801,14 @@ TcGcnArgs make_gcn_args(cosk_model *m, int i, const ActBuf &in, int in_slot, int
   a.dense = m->d_dense;
   a.dense_ld = 3 * m->dense_vp;
   a.dense_vp = m->dense_vp;
+  if (batched) {
+    a.n_frames = n_frames;
+    a.slot_rows = (int)(2 * m->t_alloc);
+    a.in_walk = in_walk;
+    a.out_walk = ring_walk;
+    a.in_slot_elems = in.slot_elems();
+    a.out_slot_elems = b.ring.slot_elems();
+  }
   return a;
 }
 
@@ -817,8 +822,7 @@ int launch_tc_gcnt(cosk_model *m, int i, TcGcnArgs a, cudaStream_t s) {
   t.g.epi.r_hi = t.g.epi.r_lo = nullptr;  // gcn_residual always rides in the GEMM here
   memcpy(t.coef, b.gcnt_coef, sizeof t.coef);
   t.n_parts = b.gcnt_parts;
-  const int items = ((m->n_tiles + 1) / 2) * a.n_frames;
-  const dim3 grid(items < m->num_sms ? items : m->num_sms), block(384);
+  const dim3 grid(persistent_grid(m, ((m->n_tiles + 1) / 2) * a.n_frames)), block(384);
   const bool v25 = m->cfg.vertices == 25;
   if (bc.cout == 128 && bc.cin == 64) {
     if (v25) CK(launch_k(k_tc_gcnt<25, 1, 128>, grid, block, TcGcntCfg<25, 1>::kSmemBytes, s, t));
@@ -847,8 +851,7 @@ int launch_tc_agcnt(cosk_model *m, int i, TcGcnArgs a, cudaStream_t s) {
   t.g.epi.r_hi = t.g.epi.r_lo = nullptr;  // gcn_residual rides in the GEMM as the fourth part
   memset(t.coef, 0, sizeof t.coef);
   t.n_parts = 4;
-  const int items = m->n_tiles * a.n_frames;
-  const dim3 grid(items < m->num_sms ? items : m->num_sms), block(384);
+  const dim3 grid(persistent_grid(m, m->n_tiles * a.n_frames)), block(384);
   const bool v25 = m->cfg.vertices == 25;
   if (bc.cout == 128 && bc.cin == 64) {
     if (v25) CK(launch_k(k_tc_agcnt<25, 1, 128>, grid, block, TcAgcntCfg<25, 1>::kSmemBytes, s, t));
@@ -864,32 +867,33 @@ int launch_tc_agcnt(cosk_model *m, int i, TcGcnArgs a, cudaStream_t s) {
 #endif
 }
 
-TcTcnArgs make_tcn_args(cosk_model *m, int i, const ActBuf &in, int res_slot, long long n, int out_slot) {
-  const cosk_block_cfg &bc = m->cfg.blocks[i];
-  BlockW &b = m->blk[i];
+// Arguments of k_tc_tcn / k_tc_tcn2 for one frame.  n_taps = kTaps: the temporal conv of input n over the slots of frames
+// n-8 .. n of the ring `x` (with phase timers); n_taps = 1: a token-major GEMM on slot 0 of `x`.  The residual rows are slot
+// res_slot of `res` (nullptr: none), taken as kb_res extra K-blocks of the GEMM, or, with `res_epi`, added by the epilogue.
+TcTcnArgs make_tc_tcn_args(const cosk_model *m, const ActBuf &x, int n_taps, long long n, int kb_per_tap, const CUtensorMap &w,
+                           const float *bias, const ActBuf *res, int res_slot, int kb_res, bool res_epi, const ActBuf &y, int y_slot) {
   TcTcnArgs a;
-  a.tm_ring = b.ring.map;
-  a.tm_res = b.tcn_res_kblock ? in.map : b.ring.map;
-  a.tm_w = b.map_tcn_w;
-  for (int k = 0; k < kTaps; ++k) a.tap_row[k] = (int)b.ring.row_hi(mod_slot(n - (kTaps - 1) + k, m->R));  // frame n-8+k
-  a.res_row = (int)in.row_hi(res_slot);
+  a.tm_ring = x.map;
+  a.tm_res = kb_res ? res->map : x.map;
+  a.tm_w = w;
+  for (int k = 0; k < kTaps; ++k) a.tap_row[k] = (int)x.row_hi(n_taps == 1 ? 0 : mod_slot(n - (kTaps - 1) + k, x.slots));
+  a.res_row = res ? (int)res->row_hi(res_slot) : 0;
   a.t_alloc = (int)m->t_alloc;
-  a.n_taps = kTaps;
-  a.kb_per_tap = bc.cout / kBK;
-  a.kb_res = b.tcn_res_kblock ? bc.cin / kBK : 0;
+  a.n_taps = n_taps;
+  a.kb_per_tap = kb_per_tap;
+  a.kb_res = kb_res;
   a.n_tiles = m->n_tiles;
   a.tile_tokens = m->tile_tokens;
-  a.reverse = 1;
+  a.reverse = n_taps == kTaps ? 1 : 0;
   a.n_tokens = m->n_tokens;
-  a.epi.bias = b.d_tcn_b;
-  const bool epi_res = bc.res_kind == COSK_RES_IDENTITY && !b.tcn_res_kblock;
-  a.epi.r_hi = epi_res ? in.hi(res_slot) : nullptr;
-  a.epi.r_lo = epi_res ? in.lo(res_slot) : nullptr;
-  a.epi.cs_r = in.cs;
-  a.epi.y_hi = b.out.hi(out_slot);
-  a.epi.y_lo = b.out.lo(out_slot);
-  a.epi.cs_out = b.out.cs;
-  a.trace = m->d_trace;
+  a.epi.bias = bias;
+  a.epi.r_hi = res_epi ? res->hi(res_slot) : nullptr;
+  a.epi.r_lo = res_epi ? res->lo(res_slot) : nullptr;
+  a.epi.cs_r = res ? res->cs : 0;
+  a.epi.y_hi = y.hi(y_slot);
+  a.epi.y_lo = y.lo(y_slot);
+  a.epi.cs_out = y.cs;
+  a.trace = n_taps == kTaps ? m->d_trace : nullptr;
   a.dbg = m->d_dbg;
   return a;
 }
@@ -913,25 +917,16 @@ int launch_tcn(cosk_model *m, int width, TcTcnArgs &a, const CUtensorMap &half, 
   return launch_tc_tcn<256>(m, a, s);
 }
 
-// Plain graph conv on the tensor cores: channel-major k_tc_gcnt where the skeleton tree allows, else token-major k_tc_gcn.
-int launch_gcn(cosk_model *m, int i, const TcGcnArgs &a, cudaStream_t s) {
-  const BlockW &b = m->blk[i];
-  if (b.tc_gcnt) return launch_tc_gcnt(m, i, a, s);
-  // one K-block per work item (cin = 64): single operand stage, four exchange buffers
-  const bool one_kb = m->cfg.blocks[i].cin == kBK;
-  if (b.gcn_parts == 4) return one_kb ? launch_tc_gcn<4, 1>(m, a, s) : launch_tc_gcn<4, 2>(m, a, s);
-  return one_kb ? launch_tc_gcn<3, 1>(m, a, s) : launch_tc_gcn<3, 2>(m, a, s);
-}
-
 // Self-attention unit of CoS-TR (GcnUnitAttention, only_attention): qkv conv on the data_bn-normalised frame, 8-head
 // attention over the vertices of each skeleton, then the output conv + bn + skip + ReLU -- the last one is the
 // temporal-conv kernel run with a single tap on the attention rows.
 int run_attention_unit(cosk_model *m, int i, const ActBuf &in, int in_slot, int ring_slot, cudaStream_t s) {
   const cosk_block_cfg &bc = m->cfg.blocks[i];
   BlockW &b = m->blk[i];
+  const GcnRoute g = b.route.gcn;
   const int dk = bc.cout / 4, dv = bc.cout, nq = 2 * dk + dv;
   int rc;
-  if (b.tc_sa_qkv) {
+  if (g != GcnRoute::kSaSimt) {
     {  // data_bn of the unit as a pre-pass: the GEMM operand must exist in memory for TMA
       SaAffineArgs a;
       a.x_hi = in.hi(in_slot);
@@ -948,7 +943,7 @@ int run_attention_unit(cosk_model *m, int i, const ActBuf &in, int in_slot, int 
       CK(launch_k(k_sa_affine, dim3((unsigned)((n + 255) / 256)), dim3(256), 0, s, a));
       m->launches++;
     }
-    if (b.tc_sa_fused) {
+    if (g == GcnRoute::kSaTcFused) {
       TcSaArgs a;
       a.tm_x = b.sa_x.map;
       a.tm_w = b.map_sa_fw;
@@ -964,35 +959,13 @@ int run_attention_unit(cosk_model *m, int i, const ActBuf &in, int in_slot, int 
       a.y_lo = b.sa.lo(0);
       a.cs_out = b.sa.cs;
       a.dbg = m->d_dbg;
-      const int grid = m->n_tiles < m->num_sms ? m->n_tiles : m->num_sms;
-      if (bc.cout == 128) CK(launch_k(k_tc_sa<16>, dim3(grid), dim3(384), TcSaCfg<16>::kSmemBytes, s, a));
-      else CK(launch_k(k_tc_sa<32>, dim3(grid), dim3(384), TcSaCfg<32>::kSmemBytes, s, a));
+      const dim3 grid(persistent_grid(m, m->n_tiles));
+      if (bc.cout == 128) CK(launch_k(k_tc_sa<16>, grid, dim3(384), TcSaCfg<16>::kSmemBytes, s, a));
+      else CK(launch_k(k_tc_sa<32>, grid, dim3(384), TcSaCfg<32>::kSmemBytes, s, a));
       m->launches++;
     } else {  // qkv conv = single-tap temporal-conv kernel without ReLU
-      TcTcnArgs a;
-      a.tm_ring = b.sa_x.map;
-      a.tm_res = b.sa_x.map;
-      a.tm_w = b.map_sa_q;
-      for (int k = 0; k < kTaps; ++k) a.tap_row[k] = (int)b.sa_x.row_hi(0);
-      a.res_row = 0;
-      a.t_alloc = (int)m->t_alloc;
-      a.n_taps = 1;
-      a.kb_per_tap = bc.cin / kBK;
-      a.kb_res = 0;
-      a.n_tiles = m->n_tiles;
-      a.tile_tokens = m->tile_tokens;
-      a.reverse = 0;
-      a.n_tokens = m->n_tokens;
-      a.epi.bias = b.d_sa_qbias;
-      a.epi.r_hi = nullptr;
-      a.epi.r_lo = nullptr;
-      a.epi.cs_r = 0;
-      a.epi.y_hi = b.sa_q.hi(0);
-      a.epi.y_lo = b.sa_q.lo(0);
-      a.epi.cs_out = b.sa_q.cs;
+      TcTcnArgs a = make_tc_tcn_args(m, b.sa_x, 1, 0, bc.cin / kBK, b.map_sa_q, b.d_sa_qbias, nullptr, 0, 0, false, b.sa_q, 0);
       a.epi.floor = -INFINITY;
-      a.trace = nullptr;
-      a.dbg = m->d_dbg;
       if ((rc = launch_tcn(m, kSaQkvCols, a, b.map_sa_q, s))) return rc;
       m->launches++;
     }
@@ -1015,11 +988,11 @@ int run_attention_unit(cosk_model *m, int i, const ActBuf &in, int in_slot, int 
     CK(launch_k(k_sa_qkv, grid, dim3(256), 0, s, a));
     m->launches++;
   }
-  if (!b.tc_sa_fused) {
+  if (g != GcnRoute::kSaTcFused) {
     SaAttnArgs a;
     a.qkv = m->d_qkv;
-    a.q_hi = b.tc_sa_qkv ? b.sa_q.hi(0) : nullptr;
-    a.q_lo = b.tc_sa_qkv ? b.sa_q.lo(0) : nullptr;
+    a.q_hi = g == GcnRoute::kSaTcQkv ? b.sa_q.hi(0) : nullptr;
+    a.q_lo = g == GcnRoute::kSaTcQkv ? b.sa_q.lo(0) : nullptr;
     a.cs_q = b.sa_q.cs;
     a.dk = dk;
     a.dv = dv;
@@ -1038,30 +1011,10 @@ int run_attention_unit(cosk_model *m, int i, const ActBuf &in, int in_slot, int 
   }
   if ((rc = prof_mark(m, 1, i, s))) return rc;
   const bool skip = bc.cin == bc.cout;  // skip_conn and in_channels == out_channels (s_tr.py:464-467)
-  if (b.tc_sa_out) {
-    TcTcnArgs a;
-    a.tm_ring = b.sa.map;
-    a.tm_res = b.sa_res_kblock ? in.map : b.sa.map;
-    a.tm_w = b.map_sa_w;
-    for (int k = 0; k < kTaps; ++k) a.tap_row[k] = (int)b.sa.row_hi(0);
-    a.res_row = (int)in.row_hi(in_slot);
-    a.t_alloc = (int)m->t_alloc;
-    a.n_taps = 1;
-    a.kb_per_tap = bc.cout / kBK;
-    a.kb_res = b.sa_res_kblock ? bc.cin / kBK : 0;
-    a.n_tiles = m->n_tiles;
-    a.tile_tokens = m->tile_tokens;
-    a.reverse = 0;
-    a.n_tokens = m->n_tokens;
-    a.epi.bias = b.d_gcn_b;
-    a.epi.r_hi = nullptr;  // the scaled skip connection is the K-block above
-    a.epi.r_lo = nullptr;
-    a.epi.cs_r = in.cs;
-    a.epi.y_hi = b.ring.hi(ring_slot);
-    a.epi.y_lo = b.ring.lo(ring_slot);
-    a.epi.cs_out = b.ring.cs;
-    a.trace = nullptr;
-    a.dbg = m->d_dbg;
+  if (b.route.sa_out_tc) {
+    // the scaled skip connection is a K-block of the GEMM
+    TcTcnArgs a = make_tc_tcn_args(m, b.sa, 1, 0, bc.cout / kBK, b.map_sa_w, b.d_gcn_b, &in, in_slot, skip ? bc.cin / kBK : 0, false,
+                                   b.ring, ring_slot);
     if ((rc = launch_tcn(m, bc.cout, a, b.map_sa_w_half, s))) return rc;
   } else {
     TcnArgs a;
@@ -1092,27 +1045,17 @@ int run_attention_unit(cosk_model *m, int i, const ActBuf &in, int in_slot, int 
   return COSK_OK;
 }
 
-// Narrow first layer (cin <= 8): k_gcn_small keeps the weights and the mixed inputs of a tile in shared memory, and the
-// adaptive one computes its embeddings per thread (k_attn_small).  Shared by the launchers, the time-batched walk and
-// cosk_describe.
-bool gcn_small(const cosk_model *m, const cosk_block_cfg &bc) {
-  const int res_conv = bc.cin != bc.cout ? 1 : 0;
-  return m->cfg.path == COSK_PATH_AUTO && bc.cin <= 8 && res_conv && bc.cout % 32 == 0 && (3 + res_conv) * bc.cin <= kSmallKMax;
-}
-bool attn_small(const cosk_model *m, const cosk_block_cfg &bc) {
-  return bc.gconv == COSK_GCONV_ADAPTIVE && m->cfg.path == COSK_PATH_AUTO && bc.cin <= 8 && bc.cout == 64 &&
-         (m->cfg.vertices == 25 || m->cfg.vertices == 18);
-}
-
-int run_gcn(cosk_model *m, int i, const ActBuf &in, int in_slot, int ring_slot, cudaStream_t s) {
+// Graph conv of block i for n_frames executions: frame f reads slot in_walk.slot(f) of `in` and writes slot ring_walk.slot(f)
+// of the block's temporal ring.  Time-batched (n_frames > 1) only on the routes batched_ok admits.
+int run_gcn(cosk_model *m, int i, const ActBuf &in, int n_frames, RingWalk in_walk, RingWalk ring_walk, cudaStream_t s) {
   const cosk_block_cfg &bc = m->cfg.blocks[i];
   BlockW &b = m->blk[i];
-  const int res_conv = bc.cin != bc.cout ? 1 : 0;
-  const bool adaptive = bc.gconv == COSK_GCONV_ADAPTIVE;
+  const Route &r = b.route;
+  const int in_slot = in_walk.slot0, ring_slot = ring_walk.slot0;  // of the single-frame launches
   int rc = prof_mark(m, bc.gconv != COSK_GCONV_PLAIN ? 4 : 1, i, s);
   if (rc) return rc;
   if (bc.gconv == COSK_GCONV_ATTENTION) return run_attention_unit(m, i, in, in_slot, ring_slot, s);
-  if (adaptive && b.tc_attn) {
+  if (r.attn == AttnRoute::kTc) {
     TcAttnArgs t;
     t.tm_x = in.map;
     t.tm_w = b.map_att_w;
@@ -1133,9 +1076,7 @@ int run_gcn(cosk_model *m, int i, const ActBuf &in, int in_slot, int ring_slot, 
     else
       rc = ic == 16 ? launch_tc_attn<16, 18>(m, t, s) : ic == 32 ? launch_tc_attn<32, 18>(m, t, s) : launch_tc_attn<64, 18>(m, t, s);
     if (rc) return rc;
-    m->launches++;
-    if ((rc = prof_mark(m, 1, i, s))) return rc;
-  } else if (attn_small(m, bc)) {
+  } else if (r.attn == AttnRoute::kSmall) {
     // narrow first layer: embeddings computed per thread, same per-row softmax as the tensor-core kernel
     AttnSmallArgs t;
     t.x_hi = in.hi(in_slot);
@@ -1151,9 +1092,7 @@ int run_gcn(cosk_model *m, int i, const ActBuf &in, int in_slot, int ring_slot, 
     t.dense_ld = 3 * m->dense_vp;
     if (m->cfg.vertices == 25) CK(launch_k(k_attn_small<16, 25>, dim3(m->n_tiles), dim3(128), 0, s, t));
     else CK(launch_k(k_attn_small<16, 18>, dim3(m->n_tiles), dim3(128), 0, s, t));
-    m->launches++;
-    if ((rc = prof_mark(m, 1, i, s))) return rc;
-  } else if (adaptive) {
+  } else if (r.attn == AttnRoute::kSimt) {
     // attention half: the per-token mixing rows of this frame go to the dense scratch
     AttnArgs t;
     t.x_hi = in.hi(in_slot);
@@ -1171,83 +1110,118 @@ int run_gcn(cosk_model *m, int i, const ActBuf &in, int in_slot, int ring_slot, 
     t.dense_ld = 3 * m->dense_vp;
     t.dense_vp = m->dense_vp;
     CK(launch_k(k_agcn_attn, dim3(m->n_tiles), dim3(256), (size_t)2 * t.inter_c * kTileRows * sizeof(float), s, t));
+  }
+  if (r.attn != AttnRoute::kNone) {
     m->launches++;
     if ((rc = prof_mark(m, 1, i, s))) return rc;
   }
-  if (b.tc_agcnt) {
-    if ((rc = launch_tc_agcnt(m, i, make_gcn_args(m, i, in, in_slot, ring_slot), s))) return rc;
-  } else if (b.tc_gcn && adaptive) {
-    TcGcnArgs a = make_gcn_args(m, i, in, in_slot, ring_slot);
-    const bool v25 = m->cfg.vertices == 25;
-    if (b.gcn_parts == 4) rc = v25 ? launch_tc_agcn<4, 1, 25>(m, a, s) : launch_tc_agcn<4, 1, 18>(m, a, s);
-    else rc = v25 ? launch_tc_agcn<3, 2, 25>(m, a, s) : launch_tc_agcn<3, 2, 18>(m, a, s);
-    if (rc) return rc;
-  } else if (b.tc_gcn) {
-    if ((rc = launch_gcn(m, i, make_gcn_args(m, i, in, in_slot, ring_slot), s))) return rc;
-  } else {
-    GcnArgs a;
-    a.x_hi = in.hi(in_slot);
-    a.x_lo = in.lo(in_slot);
-    a.cs_in = in.cs;
-    a.cin = bc.cin;
-    a.y_hi = b.ring.hi(ring_slot);
-    a.y_lo = b.ring.lo(ring_slot);
-    a.cs_out = b.ring.cs;
-    a.cout = bc.cout;
-    a.w = b.d_gcn_w;
-    a.bias = b.d_gcn_b;
-    a.res_conv = res_conv;
-    a.res_identity = !res_conv;
-    a.mix_ptr = b.d_mix_ptr;
-    a.mix_src = b.d_mix_src;
-    a.mix_val = b.d_mix_val;
-    a.V = m->cfg.vertices;
-    a.n_tokens = m->n_tokens;
-    a.tile_tokens = m->tile_tokens;
-    a.dense = adaptive ? m->d_dense : nullptr;
-    a.dense_ld = 3 * m->dense_vp;
-    a.dense_vp = m->dense_vp;
-    const int K = (3 + res_conv) * bc.cin;
-    if (gcn_small(m, bc)) {
-      CK(launch_k(k_gcn_small, dim3(m->n_tiles), dim3(256), (size_t)(K + 1) * bc.cout * sizeof(float), s, a));
-    } else {
-      dim3 grid(m->n_tiles, (bc.cout + kSimtN - 1) / kSimtN);
-      CK(launch_k(k_gcn_simt, grid, dim3(256), 0, s, a));
+  const bool v25 = m->cfg.vertices == 25;
+  const bool one_kb = bc.cin == kBK;  // one K-block per work item: single operand stage
+  switch (r.gcn) {
+    case GcnRoute::kTcAgcnt:
+      rc = launch_tc_agcnt(m, i, make_gcn_args(m, i, in, n_frames, in_walk, ring_walk), s);
+      break;
+    case GcnRoute::kTcAgcn: {
+      const TcGcnArgs a = make_gcn_args(m, i, in, n_frames, in_walk, ring_walk);
+      if (b.gcn_parts == 4) rc = v25 ? launch_tc_agcn<4, 1, 25>(m, a, s) : launch_tc_agcn<4, 1, 18>(m, a, s);
+      else rc = v25 ? launch_tc_agcn<3, 2, 25>(m, a, s) : launch_tc_agcn<3, 2, 18>(m, a, s);
+      break;
+    }
+    case GcnRoute::kTcT:
+      rc = launch_tc_gcnt(m, i, make_gcn_args(m, i, in, n_frames, in_walk, ring_walk), s);
+      break;
+    case GcnRoute::kTc: {
+      const TcGcnArgs a = make_gcn_args(m, i, in, n_frames, in_walk, ring_walk);
+      if (b.gcn_parts == 4) rc = one_kb ? launch_tc_gcn<4, 1>(m, a, s) : launch_tc_gcn<4, 2>(m, a, s);
+      else rc = one_kb ? launch_tc_gcn<3, 1>(m, a, s) : launch_tc_gcn<3, 2>(m, a, s);
+      break;
+    }
+    default: {  // kSimt, kSmall (time-batched: blockIdx.y = frame, pointers at slot 0 of their rings)
+      const bool batched = n_frames > 1;
+      const int res_conv = bc.cin != bc.cout ? 1 : 0;
+      GcnArgs a;
+      a.x_hi = in.hi(batched ? 0 : in_slot);
+      a.x_lo = in.lo(batched ? 0 : in_slot);
+      a.cs_in = in.cs;
+      a.cin = bc.cin;
+      a.y_hi = b.ring.hi(batched ? 0 : ring_slot);
+      a.y_lo = b.ring.lo(batched ? 0 : ring_slot);
+      a.cs_out = b.ring.cs;
+      a.cout = bc.cout;
+      a.w = b.d_gcn_w;
+      a.bias = b.d_gcn_b;
+      a.res_conv = res_conv;
+      a.res_identity = !res_conv;
+      a.mix_ptr = b.d_mix_ptr;
+      a.mix_src = b.d_mix_src;
+      a.mix_val = b.d_mix_val;
+      a.V = m->cfg.vertices;
+      a.n_tokens = m->n_tokens;
+      a.tile_tokens = m->tile_tokens;
+      a.dense = bc.gconv == COSK_GCONV_ADAPTIVE ? m->d_dense : nullptr;
+      a.dense_ld = 3 * m->dense_vp;
+      a.dense_vp = m->dense_vp;
+      if (batched) {
+        a.in_walk = in_walk;
+        a.out_walk = ring_walk;
+        a.in_slot_elems = in.slot_elems();
+        a.out_slot_elems = b.ring.slot_elems();
+      }
+      const int K = (3 + res_conv) * bc.cin;
+      if (r.gcn == GcnRoute::kSmall)
+        CK(launch_k(k_gcn_small, dim3(m->n_tiles, n_frames), dim3(256), (size_t)(K + 1) * bc.cout * sizeof(float), s, a));
+      else
+        CK(launch_k(k_gcn_simt, dim3(m->n_tiles, (bc.cout + kSimtN - 1) / kSimtN), dim3(256), 0, s, a));
     }
   }
+  if (rc) return rc;
   m->launches++;
   return COSK_OK;
 }
 
-int run_tcn(cosk_model *m, int i, const ActBuf &in, int res_slot, long long n, int out_slot, cudaStream_t s) {
+// Temporal conv of block i for n_frames firing executions, the first on input n: frame f adds the delayed residual from slot
+// res_walk.slot(f) of `in` and writes slot out_walk.slot(f) of the block's output ring (time-batched: tensor cores only).
+int run_tcn(cosk_model *m, int i, const ActBuf &in, long long n, int n_frames, RingWalk res_walk, RingWalk out_walk, cudaStream_t s) {
   const cosk_block_cfg &bc = m->cfg.blocks[i];
   BlockW &b = m->blk[i];
   int rc = prof_mark(m, 2, i, s);
   if (rc) return rc;
-  int tap_slot[kTaps];
-  for (int k = 0; k < kTaps; ++k) tap_slot[k] = mod_slot(n - (kTaps - 1) + k, m->R);  // frame n-8+k
-  if (b.tc_tcn) {
-    TcTcnArgs a = make_tcn_args(m, i, in, res_slot, n, out_slot);
+  if (b.route.tcn_tc) {
+    const bool batched = n_frames > 1;  // pointers at slot 0 of their rings, the slots from the walks
+    const bool kblock = tcn_res_kblock(bc);
+    TcTcnArgs a = make_tc_tcn_args(m, b.ring, kTaps, n, bc.cout / kBK, b.map_tcn_w, b.d_tcn_b, &in, batched ? 0 : res_walk.slot0,
+                                   kblock ? bc.cin / kBK : 0, bc.res_kind == COSK_RES_IDENTITY && !kblock, b.out,
+                                   batched ? 0 : out_walk.slot0);
+    if (batched) {
+      a.n_frames = n_frames;
+      a.slot_rows = (int)(2 * m->t_alloc);
+      a.tap_walk = ring_walk(n - (kTaps - 1), bc.stride, m->R);
+      a.res_walk = res_walk;
+      a.out_walk = out_walk;
+      a.out_slot_elems = b.out.slot_elems();
+      a.res_slot_elems = in.slot_elems();
+    }
     if ((rc = launch_tcn(m, bc.cout, a, b.map_tcn_w_half, s))) return rc;
   } else {
     TcnArgs a;
     for (int k = 0; k < kTaps; ++k) {
-      a.tap_hi[k] = b.ring.hi(tap_slot[k]);
-      a.tap_lo[k] = b.ring.lo(tap_slot[k]);
+      const int slot = mod_slot(n - (kTaps - 1) + k, m->R);  // frame n-8+k
+      a.tap_hi[k] = b.ring.hi(slot);
+      a.tap_lo[k] = b.ring.lo(slot);
     }
     a.n_taps = kTaps;
     a.cs = b.ring.cs;
     a.c = bc.cout;
     a.w = b.d_tcn_w;
-    a.r_hi = in.hi(res_slot);
-    a.r_lo = in.lo(res_slot);
+    a.r_hi = in.hi(res_walk.slot0);
+    a.r_lo = in.lo(res_walk.slot0);
     a.cs_r = in.cs;
     a.cr = bc.cin;
     a.res_kind = bc.res_kind;
     a.w_r = b.d_res_w;
     a.bias = b.d_tcn_b;
-    a.y_hi = b.out.hi(out_slot);
-    a.y_lo = b.out.lo(out_slot);
+    a.y_hi = b.out.hi(out_walk.slot0);
+    a.y_lo = b.out.lo(out_walk.slot0);
     a.cs_out = b.out.cs;
     a.n_tokens = m->n_tokens;
     a.tile_tokens = m->tile_tokens;
@@ -1295,8 +1269,70 @@ int run_block64(cosk_model *m, int i, const ActBuf &in, int in_slot, long long n
   a.tepi.cs_out = b.out.cs;
   a.trace = m->d_trace;
   a.dbg = m->d_dbg;
-  const int grid = m->n_tiles < m->num_sms ? m->n_tiles : m->num_sms;
-  CK(launch_k(k_tc_block64, dim3(grid), dim3(512), TcBlockCfg::kSmemBytes, s, a));
+  CK(launch_k(k_tc_block64, dim3(persistent_grid(m, m->n_tiles)), dim3(512), TcBlockCfg::kSmemBytes, s, a));
+  m->launches++;
+  return COSK_OK;
+}
+
+// k_input: n_frames input frames (frame f at x + f * x_frame_stride) -> slots walk.slot(f) of the input ring, data_bn folded in
+int run_input(cosk_model *m, const float *x, long long nc_stride, long long x_frame_stride, int n_frames, RingWalk walk, cudaStream_t s) {
+  const cosk_config &c = m->cfg;
+  const long long total = m->n_tokens * m->xin.cs;
+  const int threads = 256;
+  const long long blocks = (total + threads - 1) / threads;
+  CK(launch_k(k_input, dim3((unsigned)blocks, (unsigned)n_frames), dim3(threads), 0, s, x, nc_stride, c.c_in, c.vertices, c.persons,
+              (const float *)(c.data_bn ? m->d_bn_scale : nullptr), (const float *)(c.data_bn ? m->d_bn_shift : nullptr), m->xin.hi(0),
+              m->xin.lo(0), m->xin.cs, m->n_tokens, x_frame_stride, walk, m->xin.slot_elems()));
+  m->launches++;
+  return COSK_OK;
+}
+
+// k_head over n_frames emissions of the last block, frame f from slot in_walk.slot(f) of its output ring (`zero`: one zero
+// vector enters the pooling window instead).  One frame emits logits iff `emit`; more emit from frame first_emit on,
+// emission j at out + j * out_stride.
+int run_head(cosk_model *m, int n_frames, RingWalk in_walk, bool zero, int emit, int first_emit, float *out, long long out_stride,
+             cudaStream_t s) {
+  const cosk_config &c = m->cfg;
+  const ActBuf &y = m->blk[c.n_blocks - 1].out;
+  const bool batched = n_frames > 1;  // y_* at slot 0 of the ring, the slots from the walk
+  int rc = prof_mark(m, 3, -1, s);
+  if (rc) return rc;
+  HeadArgs h;
+  h.y_hi = zero ? nullptr : y.hi(batched ? 0 : in_walk.slot0);
+  h.y_lo = zero ? nullptr : y.lo(batched ? 0 : in_walk.slot0);
+  h.cs = y.cs;
+  h.c = y.c;
+  h.V = c.vertices;
+  h.S = c.persons;
+  h.ring = m->d_pool_ring;
+  h.sum = m->d_pool_sum;
+  h.slot = (int)(m->pool_n % c.pool_size);
+  h.P = c.pool_size;
+  h.n_streams = m->n_streams;
+  h.emit = emit;
+  h.w = m->d_fc_w;
+  h.b = m->d_fc_b;
+  h.classes = c.classes;
+  h.out = out;
+  h.first_emit = first_emit;
+  h.out_stride = out_stride;
+  if (batched) {
+    h.n_frames = n_frames;
+    h.in_walk = in_walk;
+    h.in_slot_elems = y.slot_elems();
+  }
+  CK(launch_k(k_head, dim3((unsigned)((m->n_streams + kHeadStreams - 1) / kHeadStreams)), dim3(256 * kHeadStreams),
+              (size_t)kHeadStreams * (2 * y.cs + y.c) * sizeof(float), s, h));
+  m->launches++;
+  m->pool_n += n_frames;
+  return COSK_OK;
+}
+
+// k_read_block: slot `slot` of a block's output ring -> fp32 at dst
+int read_block(cosk_model *m, const ActBuf &o, int slot, float *dst, cudaStream_t s) {
+  const long long total = m->n_tokens * o.c;
+  CK(launch_k(k_read_block, dim3((unsigned)((total + 255) / 256)), dim3(256), 0, s, (const __nv_bfloat16 *)o.hi(slot),
+              (const __nv_bfloat16 *)o.lo(slot), o.cs, o.c, m->cfg.vertices, m->n_tokens, dst));
   m->launches++;
   return COSK_OK;
 }
@@ -1321,17 +1357,8 @@ int step_impl(cosk_model *m, const float *x, long long nc_stride, float *out, in
   const cosk_config &c = m->cfg;
   int rc;
   // input frame -> token rows (data_bn folded in)
-  const int xslot = (int)(m->frame % m->Ro);
   if ((rc = prof_mark(m, 0, -1, s))) return rc;
-  if (!flush) {
-    const long long total = m->n_tokens * m->xin.cs;
-    const int threads = 256;
-    const long long blocks = (total + threads - 1) / threads;
-    CK(launch_k(k_input, dim3((unsigned)blocks), dim3(threads), 0, s, x, (long long)nc_stride, c.c_in, c.vertices, c.persons,
-                (const float *)(c.data_bn ? m->d_bn_scale : nullptr), (const float *)(c.data_bn ? m->d_bn_shift : nullptr),
-                m->xin.hi(xslot), m->xin.lo(xslot), m->xin.cs, m->n_tokens, 0LL, RingWalk(), 0LL));
-    m->launches++;
-  }
+  if (!flush && (rc = run_input(m, x, nc_stride, 0, 1, ring_walk(m->frame, 1, m->Ro), s))) return rc;
   const ActBuf *in = &m->xin;
   bool alive = true;
   const bool head_flush = flush && enter >= c.n_blocks;
@@ -1348,7 +1375,7 @@ int step_impl(cosk_model *m, const float *x, long long nc_stride, float *out, in
     const int in_slot = (int)(n % m->Ro);
     const bool fire = tcn_fires(n, c.padding, bc.stride);
     const bool zero_in = flush && i == enter;  // a zero frame enters the temporal conv directly
-    const bool fused = b.fuse && in->has_map && !zero_in;
+    const bool fused = b.route.block64 && in->has_map && !zero_in;
     if (zero_in) {
       const int rs = (int)(n % m->R);
       CK(cudaMemsetAsync(b.ring.hi(rs), 0, (size_t)2 * b.ring.t_alloc * b.ring.cs * sizeof(__nv_bfloat16), s));
@@ -1356,12 +1383,11 @@ int step_impl(cosk_model *m, const float *x, long long nc_stride, float *out, in
       const int res_slot = fire ? (int)((n - kResDelay) % m->Ro) : 0;
       if ((rc = run_block64(m, i, *in, in_slot, n, fire, res_slot, (int)(b.n_out % m->Ro), s))) return rc;
       if (fire) b.n_out++;
-    } else if ((rc = run_gcn(m, i, *in, in_slot, (int)(n % m->R), s))) {
+    } else if ((rc = run_gcn(m, i, *in, 1, ring_walk(n, 1, m->Ro), ring_walk(n, 1, m->R), s))) {
       return rc;
     }
-    if (fire && !fused) {
-      const int res_slot = (int)((n - kResDelay) % m->Ro);  // n >= first >= 4
-      if ((rc = run_tcn(m, i, *in, res_slot, n, (int)(b.n_out % m->Ro), s))) return rc;
+    if (fire && !fused) {  // n >= first >= 4
+      if ((rc = run_tcn(m, i, *in, n, 1, ring_walk(n - kResDelay, 1, m->Ro), ring_walk(b.n_out, 1, m->Ro), s))) return rc;
       b.n_out++;
     }
     b.n_in++;
@@ -1376,34 +1402,10 @@ int step_impl(cosk_model *m, const float *x, long long nc_stride, float *out, in
     const int slot = (int)(((last.n_out > 0 ? last.n_out : 1) - 1) % m->Ro);
     if (c.classes > 0) {
       emit = head_fires(m->pool_n, c.pool_size, c.pool_padding) ? 1 : 0;
-      if ((rc = prof_mark(m, 3, -1, s))) return rc;
-      HeadArgs h;
-      h.y_hi = head_flush ? nullptr : last.out.hi(slot);  // nullptr: a zero vector enters the window
-      h.y_lo = head_flush ? nullptr : last.out.lo(slot);
-      h.cs = last.out.cs;
-      h.c = last.out.c;
-      h.V = c.vertices;
-      h.S = c.persons;
-      h.ring = m->d_pool_ring;
-      h.sum = m->d_pool_sum;
-      h.slot = (int)(m->pool_n % c.pool_size);
-      h.P = c.pool_size;
-      h.n_streams = m->n_streams;
-      h.emit = emit;
-      h.w = m->d_fc_w;
-      h.b = m->d_fc_b;
-      h.classes = c.classes;
-      h.out = out;
-      CK(launch_k(k_head, dim3((unsigned)((m->n_streams + kHeadStreams - 1) / kHeadStreams)), dim3(256 * kHeadStreams),
-                  (size_t)kHeadStreams * (2 * last.out.cs + last.out.c) * sizeof(float), s, h));
-      m->launches++;
-      m->pool_n++;
+      if ((rc = run_head(m, 1, ring_walk(slot, 1, m->Ro), head_flush, emit, 0, out, 0, s))) return rc;
     } else {
       emit = 1;
-      const long long total = m->n_tokens * last.out.c;
-      CK(launch_k(k_read_block, dim3((unsigned)((total + 255) / 256)), dim3(256), 0, s, (const __nv_bfloat16 *)last.out.hi(slot),
-                  (const __nv_bfloat16 *)last.out.lo(slot), last.out.cs, last.out.c, c.vertices, m->n_tokens, out));
-      m->launches++;
+      if ((rc = read_block(m, last.out, slot, out, s))) return rc;
     }
   }
   if ((rc = prof_mark(m, -1, -1, s))) return rc;  // closes the last interval of this step
@@ -1416,14 +1418,13 @@ int step_impl(cosk_model *m, const float *x, long long nc_stride, float *out, in
 // ---- time-batched stepping (cosk_steps with a time chunk > 1) ------------------------------------------------------
 // The stack is walked module by module over a chunk of F0 <= tchunk frames, one launch per kernel and chunk; the work items
 // of a launch are (frame, tile) pairs and every frame's ring slots follow from a RingWalk.  Available when every block runs
-// on the tensor-core CoST-GCN kernels (k_tc_gcn, k_gcn_small for the first layer, k_tc_tcn / k_tc_tcn2).
+// on the tensor-core CoST-GCN kernels (k_tc_gcn or k_tc_gcnt, k_gcn_small for the first layer, k_tc_tcn / k_tc_tcn2).
 bool batched_ok(const cosk_model *m) {
-  if (m->tchunk <= 1 || m->cfg.path != COSK_PATH_AUTO || m->d_trace) return false;
-  for (int i = 0; i < m->cfg.n_blocks; ++i) {
-    const cosk_block_cfg &bc = m->cfg.blocks[i];
-    const BlockW &b = m->blk[i];
-    if (bc.gconv != COSK_GCONV_PLAIN || !b.tc_tcn) return false;
-    if (!(b.tc_gcn || gcn_small(m, bc))) return false;
+  if (m->tchunk <= 1 || m->d_trace) return false;
+  for (const BlockW &b : m->blk) {
+    const Route &r = b.route;
+    if (r.attn != AttnRoute::kNone || !r.tcn_tc) return false;
+    if (r.gcn != GcnRoute::kTc && r.gcn != GcnRoute::kTcT && r.gcn != GcnRoute::kSmall) return false;
   }
   return true;
 }
@@ -1431,22 +1432,9 @@ bool batched_ok(const cosk_model *m) {
 int steps_chunk(cosk_model *m, const float *x, long long nc_stride, long long x_frame_stride, int F0, float *out, long long out_stride,
                 int32_t max_out, int32_t *cnt, cudaStream_t s) {
   const cosk_config &c = m->cfg;
-  const int slot_rows = (int)(2 * m->t_alloc);
   int rc;
   if ((rc = prof_mark(m, 0, -1, s))) return rc;
-  {
-    const long long total = m->n_tokens * m->xin.cs;
-    const int threads = 256;
-    const long long blocks = (total + threads - 1) / threads;
-    RingWalk ow;
-    ow.slot0 = mod_slot(m->frame, m->Ro);
-    ow.step = 1;
-    ow.slots = m->Ro;
-    CK(launch_k(k_input, dim3((unsigned)blocks, (unsigned)F0), dim3(threads), 0, s, x, (long long)nc_stride, c.c_in, c.vertices, c.persons,
-                (const float *)(c.data_bn ? m->d_bn_scale : nullptr), (const float *)(c.data_bn ? m->d_bn_shift : nullptr),
-                m->xin.hi(0), m->xin.lo(0), m->xin.cs, m->n_tokens, x_frame_stride, ow, m->xin.slot_elems()));
-    m->launches++;
-  }
+  if ((rc = run_input(m, x, nc_stride, x_frame_stride, F0, ring_walk(m->frame, 1, m->Ro), s))) return rc;
   const ActBuf *in = &m->xin;
   int F = F0;  // executions of the current block in this chunk == emissions of its predecessor
   for (int i = 0; i < c.n_blocks; ++i) {
@@ -1462,90 +1450,13 @@ int steps_chunk(cosk_model *m, const float *x, long long nc_stride, long long x_
     // firing executions among n0 .. n0+F-1: n >= first and (n - first) % stride == 0
     long long nf = n0 < first ? first : n0 + ((first - n0) % bc.stride + bc.stride) % bc.stride;
     const int F_out = nf <= n0 + F - 1 ? (int)((n0 + F - 1 - nf) / bc.stride) + 1 : 0;
-    const long long out0 = b.n_out;
-    RingWalk in_walk, ring_walk, tap_walk, res_walk, out_walk;
-    in_walk.slot0 = mod_slot(n0, m->Ro), in_walk.step = 1, in_walk.slots = m->Ro;
-    ring_walk.slot0 = mod_slot(n0, m->R), ring_walk.step = 1, ring_walk.slots = m->R;
-    tap_walk.slot0 = mod_slot(nf - (kTaps - 1), m->R), tap_walk.step = bc.stride, tap_walk.slots = m->R;
-    res_walk.slot0 = mod_slot(nf - kResDelay, m->Ro), res_walk.step = bc.stride, res_walk.slots = m->Ro;
-    out_walk.slot0 = mod_slot(out0, m->Ro), out_walk.step = 1, out_walk.slots = m->Ro;
     // (The fused block kernel is not used here: frame n's temporal conv reads the graph-conv outputs of frames n-8 .. n-1,
     // which a launch covering many frames would produce concurrently.  The chunk runs graph conv and temporal conv of such a
     // block as two launches -- module by module, every frame of the first complete before the second starts.)
-    {
-      // graph conv over the F executions
-      if ((rc = prof_mark(m, 1, i, s))) return rc;
-      if (b.tc_gcn) {
-        TcGcnArgs a = make_gcn_args(m, i, *in, in_walk.slot0, ring_walk.slot0);
-        if (F > 1) {
-          a.n_frames = F;
-          a.slot_rows = slot_rows;
-          a.in_walk = in_walk;
-          a.out_walk = ring_walk;
-          a.in_slot_elems = in->slot_elems();
-          a.out_slot_elems = b.ring.slot_elems();
-          a.x_row = 0;
-          a.epi.y_hi = b.ring.hi(0);
-          a.epi.y_lo = b.ring.lo(0);
-          if (a.epi.r_hi != nullptr) {
-            a.epi.r_hi = in->hi(0);
-            a.epi.r_lo = in->lo(0);
-          }
-        }
-        if ((rc = launch_gcn(m, i, a, s))) return rc;
-      } else {  // narrow first layer
-        GcnArgs a;
-        a.x_hi = in->hi(0);
-        a.x_lo = in->lo(0);
-        a.cs_in = in->cs;
-        a.cin = bc.cin;
-        a.y_hi = b.ring.hi(0);
-        a.y_lo = b.ring.lo(0);
-        a.cs_out = b.ring.cs;
-        a.cout = bc.cout;
-        a.w = b.d_gcn_w;
-        a.bias = b.d_gcn_b;
-        a.res_conv = 1;
-        a.res_identity = 0;
-        a.mix_ptr = b.d_mix_ptr;
-        a.mix_src = b.d_mix_src;
-        a.mix_val = b.d_mix_val;
-        a.V = c.vertices;
-        a.n_tokens = m->n_tokens;
-        a.tile_tokens = m->tile_tokens;
-        a.dense = nullptr;
-        a.dense_ld = a.dense_vp = 0;
-        a.in_walk = in_walk;
-        a.out_walk = ring_walk;
-        a.in_slot_elems = in->slot_elems();
-        a.out_slot_elems = b.ring.slot_elems();
-        const int K = 4 * bc.cin;
-        CK(launch_k(k_gcn_small, dim3(m->n_tiles, F), dim3(256), (size_t)(K + 1) * bc.cout * sizeof(float), s, a));
-      }
-      m->launches++;
-      // temporal conv over the F_out firing executions
-      if (F_out > 0) {
-        if ((rc = prof_mark(m, 2, i, s))) return rc;
-        TcTcnArgs a = make_tcn_args(m, i, *in, res_walk.slot0, nf, out_walk.slot0);
-        if (F_out > 1) {
-          a.n_frames = F_out;
-          a.slot_rows = slot_rows;
-          a.tap_walk = tap_walk;
-          a.res_walk = res_walk;
-          a.out_walk = out_walk;
-          a.out_slot_elems = b.out.slot_elems();
-          a.res_slot_elems = in->slot_elems();
-          a.epi.y_hi = b.out.hi(0);
-          a.epi.y_lo = b.out.lo(0);
-          if (a.epi.r_hi != nullptr) {
-            a.epi.r_hi = in->hi(0);
-            a.epi.r_lo = in->lo(0);
-          }
-        }
-        if ((rc = launch_tcn(m, bc.cout, a, b.map_tcn_w_half, s))) return rc;
-        m->launches++;
-      }
-    }
+    if ((rc = run_gcn(m, i, *in, F, ring_walk(n0, 1, m->Ro), ring_walk(n0, 1, m->R), s))) return rc;
+    if (F_out > 0 &&
+        (rc = run_tcn(m, i, *in, nf, F_out, ring_walk(nf - kResDelay, bc.stride, m->Ro), ring_walk(b.n_out, 1, m->Ro), s)))
+      return rc;
     // did the block fire on the LAST frame of the chunk?  (schedule parity is defined per frame)
     m->last_flags[i] = (F_out > 0 && nf + (long long)(F_out - 1) * bc.stride == n0 + F - 1) ? 1 : 0;
     b.n_in += F;
@@ -1559,52 +1470,20 @@ int steps_chunk(cosk_model *m, const float *x, long long nc_stride, long long x_
     const BlockW &last = m->blk[c.n_blocks - 1];
     const long long o0 = last.n_out - F;  // index of the first of these emissions
     if (c.classes > 0) {
-      if ((rc = prof_mark(m, 3, -1, s))) return rc;
       const long long first_emit_n = (long long)c.pool_size - 1 - c.pool_padding;
       const int skip = (int)std::min<long long>(std::max<long long>(first_emit_n - m->pool_n, 0), F);  // frames before the first logits
       const int n_emit = F - skip;
       const int32_t room = *cnt < max_out ? max_out - *cnt : 0;
-      HeadArgs h;
-      h.y_hi = last.out.hi(0);
-      h.y_lo = last.out.lo(0);
-      h.cs = last.out.cs;
-      h.c = last.out.c;
-      h.V = c.vertices;
-      h.S = c.persons;
-      h.ring = m->d_pool_ring;
-      h.sum = m->d_pool_sum;
-      h.slot = (int)(m->pool_n % c.pool_size);
-      h.P = c.pool_size;
-      h.n_streams = m->n_streams;
-      h.emit = 0;
-      h.w = m->d_fc_w;
-      h.b = m->d_fc_b;
-      h.classes = c.classes;
-      h.out = out + (long long)(*cnt < max_out ? *cnt : max_out - 1) * out_stride;
-      h.n_frames = F;
-      h.in_walk.slot0 = mod_slot(o0, m->Ro), h.in_walk.step = 1, h.in_walk.slots = m->Ro;
-      h.in_slot_elems = last.out.slot_elems();
-      h.first_emit = skip;
-      h.out_stride = n_emit <= room ? out_stride : 0;  // more emissions than room: they all land in the last slot
-      if (F == 1) {  // single frame: plain per-step arguments
-        h.y_hi += (long long)h.in_walk.slot0 * h.in_slot_elems;
-        h.y_lo += (long long)h.in_walk.slot0 * h.in_slot_elems;
-        h.emit = n_emit;
-      }
-      CK(launch_k(k_head, dim3((unsigned)((m->n_streams + kHeadStreams - 1) / kHeadStreams)), dim3(256 * kHeadStreams),
-                  (size_t)kHeadStreams * (2 * last.out.cs + last.out.c) * sizeof(float), s, h));
-      m->launches++;
-      m->pool_n += F;
+      float *dst = out + (long long)(*cnt < max_out ? *cnt : max_out - 1) * out_stride;
+      // more emissions than room: they all land in the last slot
+      if ((rc = run_head(m, F, ring_walk(o0, 1, m->Ro), false, F == 1 ? n_emit : 0, skip, dst, n_emit <= room ? out_stride : 0, s)))
+        return rc;
       *cnt += n_emit;
       emit_last = n_emit > 0 ? 1 : 0;
     } else {
       for (int f = 0; f < F; ++f) {
-        const int slot = mod_slot(o0 + f, m->Ro);
-        const long long total = m->n_tokens * last.out.c;
         float *dst = out + (long long)(*cnt < max_out ? *cnt : max_out - 1) * out_stride;
-        CK(launch_k(k_read_block, dim3((unsigned)((total + 255) / 256)), dim3(256), 0, s, (const __nv_bfloat16 *)last.out.hi(slot),
-                    (const __nv_bfloat16 *)last.out.lo(slot), last.out.cs, last.out.c, c.vertices, m->n_tokens, dst));
-        m->launches++;
+        if ((rc = read_block(m, last.out, mod_slot(o0 + f, m->Ro), dst, s))) return rc;
         *cnt += 1;
       }
       emit_last = 1;
@@ -1614,6 +1493,24 @@ int steps_chunk(cosk_model *m, const float *x, long long nc_stride, long long x_
   m->last_flags[c.n_blocks] = (emit_last && m->last_flags[c.n_blocks - 1]) ? 1 : 0;
   m->frame += F0;
   return COSK_OK;
+}
+
+// cosk_describe's name of the kernels that serve a block's graph conv (the adaptive one: attention half + mix)
+std::string gcn_name(const BlockW &b) {
+  static const char *const attn[] = {"", "k_agcn_attn+", "k_attn_small+", "k_tc_attn+"};  // by AttnRoute
+  char t[64] = "";
+  switch (b.route.gcn) {
+    case GcnRoute::kSimt: snprintf(t, sizeof t, "k_gcn_simt"); break;
+    case GcnRoute::kSmall: snprintf(t, sizeof t, "k_gcn_small"); break;
+    case GcnRoute::kTc: snprintf(t, sizeof t, "k_tc_gcn<%d> GEMM-then-mix", b.gcn_parts); break;
+    case GcnRoute::kTcT: snprintf(t, sizeof t, "k_tc_gcnt<%d> channel-major, mix in registers", b.gcnt_parts); break;
+    case GcnRoute::kTcAgcn: snprintf(t, sizeof t, "k_tc_agcn"); break;
+    case GcnRoute::kTcAgcnt: snprintf(t, sizeof t, "k_tc_agcnt"); break;
+    case GcnRoute::kSaSimt: snprintf(t, sizeof t, "k_sa_qkv+k_sa_attn"); break;
+    case GcnRoute::kSaTcQkv: snprintf(t, sizeof t, "k_tc_tcn(qkv)+k_sa_attn"); break;
+    case GcnRoute::kSaTcFused: snprintf(t, sizeof t, "k_tc_sa"); break;
+  }
+  return std::string(attn[(int)b.route.attn]) + t;
 }
 
 }  // namespace
@@ -1825,10 +1722,11 @@ int cosk_set_batch_ex(cosk_model *m, int64_t n_streams, int32_t time_chunk) {
       max_nq = std::max(max_nq, 2 * (c.blocks[i].cout / 4) + c.blocks[i].cout);
       if ((rc = alloc_act(m, m->blk[i].sa, 1, c.blocks[i].cout))) return rc;
       CK(cudaMemset(m->blk[i].sa.ptr, 0, m->blk[i].sa.bytes()));
-      if (m->blk[i].tc_sa_qkv) {
+      const GcnRoute g = m->blk[i].route.gcn;
+      if (g != GcnRoute::kSaSimt) {
         if ((rc = alloc_act(m, m->blk[i].sa_x, 1, c.blocks[i].cin))) return rc;
         CK(cudaMemset(m->blk[i].sa_x.ptr, 0, m->blk[i].sa_x.bytes()));
-        if (!m->blk[i].tc_sa_fused) {
+        if (g == GcnRoute::kSaTcQkv) {
           if ((rc = alloc_act(m, m->blk[i].sa_q, 1, kSaQkvCols))) return rc;
           CK(cudaMemset(m->blk[i].sa_q.ptr, 0, m->blk[i].sa_q.bytes()));
         }
@@ -1985,20 +1883,15 @@ int cosk_read_block(cosk_model *m, int32_t block, float *dst_dev, void *stream) 
   const BlockW &b = m->blk[block];
   if (b.n_out == 0) return fail(m, COSK_ERR_STATE, "block %d has not emitted yet", block);
   DeviceGuard guard_(m->cfg.device);
-  const int slot = (int)((b.n_out - 1) % m->Ro);
-  const long long total = m->n_tokens * b.out.c;
-  CK(launch_k(k_read_block, dim3((unsigned)((total + 255) / 256)), dim3(256), 0, (cudaStream_t)stream,
-              (const __nv_bfloat16 *)b.out.hi(slot), (const __nv_bfloat16 *)b.out.lo(slot), b.out.cs, b.out.c, m->cfg.vertices,
-              m->n_tokens, dst_dev));
-  m->launches++;
-  return COSK_OK;
+  return read_block(m, b.out, (int)((b.n_out - 1) % m->Ro), dst_dev, (cudaStream_t)stream);
 }
 
 int64_t cosk_launch_count(const cosk_model *m) { return m ? m->launches : 0; }
 
 int cosk_block_uses_tensor_cores(const cosk_model *m, int32_t block) {
   if (!m || block < 0 || block >= m->cfg.n_blocks) return COSK_ERR_ARG;
-  return ((m->blk[block].tc_gcn || m->blk[block].tc_sa_out) ? 1 : 0) | (m->blk[block].tc_tcn ? 2 : 0);
+  const Route &r = m->blk[block].route;
+  return ((r.gcn_tc() || r.sa_out_tc) ? 1 : 0) | (r.tcn_tc ? 2 : 0);
 }
 
 int cosk_describe(const cosk_model *m, char *buf, size_t n) {
@@ -2011,33 +1904,17 @@ int cosk_describe(const cosk_model *m, char *buf, size_t n) {
            m->d_trace ? 1 : 0);
   o += t;
   o += "\"blocks\": [";
-  std::string by_width = "";
   for (int i = 0; i < m->cfg.n_blocks; ++i) {
     const cosk_block_cfg &bc = m->cfg.blocks[i];
-    const BlockW &b = m->blk[i];
-    std::string g, tc;
-    if (bc.gconv == COSK_GCONV_ATTENTION) g = b.tc_sa_fused ? "k_tc_sa" : (b.tc_sa_qkv ? "k_tc_tcn(qkv)+k_sa_attn" : "k_sa_qkv+k_sa_attn");
-    else if (bc.gconv == COSK_GCONV_ADAPTIVE && b.tc_agcnt) g = b.tc_attn ? "k_tc_attn+k_tc_agcnt" : "k_agcn_attn+k_tc_agcnt";
-    else if (bc.gconv == COSK_GCONV_ADAPTIVE && b.tc_gcn) g = b.tc_attn ? "k_tc_attn+k_tc_agcn" : "k_agcn_attn+k_tc_agcn";
-    else if (bc.gconv == COSK_GCONV_ADAPTIVE)
-      g = std::string(attn_small(m, bc) ? "k_attn_small" : "k_agcn_attn") + (gcn_small(m, bc) ? "+k_gcn_small" : "+k_gcn_simt");
-    else if (b.tc_gcnt) {
-      snprintf(t, sizeof t, "k_tc_gcnt<%d> channel-major, mix in registers", b.gcnt_parts);
-      g = t;
-    } else if (b.tc_gcn) {
-      snprintf(t, sizeof t, "k_tc_gcn<%d> GEMM-then-mix", b.gcn_parts);
-      g = t;
-    } else g = gcn_small(m, bc) ? "k_gcn_small" : "k_gcn_simt";
-    if (b.tc_tcn) {
-      snprintf(t, sizeof t, "%s<%d>", tcn_on_pair(m, bc.cout) ? "k_tc_tcn2" : "k_tc_tcn", bc.cout);
-      tc = t;
-    } else tc = "k_tcn_simt";
-    if (b.fuse) {
+    const Route &r = m->blk[i].route;
+    if (r.block64) {
       snprintf(t, sizeof t, "%s{\"block\": \"k_tc_block64 (graph conv + temporal conv in one kernel)\"}", i ? ", " : "");
       o += t;
       continue;
     }
-    snprintf(t, sizeof t, "%s{\"gcn\": \"%s\", \"tcn\": \"%s\"}", i ? ", " : "", g.c_str(), tc.c_str());
+    if (r.tcn_tc) snprintf(t, sizeof t, "%s<%d>", tcn_on_pair(m, bc.cout) ? "k_tc_tcn2" : "k_tc_tcn", bc.cout);
+    const std::string tc = r.tcn_tc ? t : "k_tcn_simt";
+    snprintf(t, sizeof t, "%s{\"gcn\": \"%s\", \"tcn\": \"%s\"}", i ? ", " : "", gcn_name(m->blk[i]).c_str(), tc.c_str());
     o += t;
   }
   o += "], \"graph_conv\": {";
@@ -2045,7 +1922,8 @@ int cosk_describe(const cosk_model *m, char *buf, size_t n) {
   for (int w : {64, 128, 256})
     for (int i = 0; i < m->cfg.n_blocks; ++i)
       if (m->cfg.blocks[i].cout == w && m->cfg.blocks[i].cin >= 64 && m->cfg.blocks[i].gconv == COSK_GCONV_PLAIN) {
-        snprintf(t, sizeof t, "%s\"%d\": \"%s\"", firstw ? "" : ", ", w, m->blk[i].tc_gcnt ? "gcnt" : m->blk[i].tc_gcn ? "gcn" : "simt");
+        const GcnRoute g = m->blk[i].route.gcn;
+        snprintf(t, sizeof t, "%s\"%d\": \"%s\"", firstw ? "" : ", ", w, g == GcnRoute::kTcT ? "gcnt" : g == GcnRoute::kTc ? "gcn" : "simt");
         o += t;
         firstw = false;
         break;
