@@ -49,8 +49,9 @@ What the bound cannot see
   (1 + SOFTMAX_REL) factor and the cancellation inside the softmax-weighted sum S @ v.  No emulation shows that a
   dropped product in k_tc_sa or k_sa_attn would exceed it.  For attention units the bound is a coarse check: it
   catches wrong rows, heads or tokens, not last-bit arithmetic.
-* Chained through a whole stack (tests/test_gpu_routes.py::test_whole_model_signed_input), the magnitudes compound
-  from block to block, so that check is coarse as well.
+* Chained through a whole stack (``model``), the magnitudes compound from block to block, so that check is coarse as
+  well.  A whole model is held tightly by checking each block on the previous block's actual output (``block``) and
+  the logits on the last block's actual outputs (``head``), as tests/test_gpu_models.py does.
 """
 import torch
 import torch.nn.functional as F
@@ -173,6 +174,58 @@ def block(x, sd, key, spec, pad, xm=None):
         w, b, _ = _folded(sd, key + "residual.t_conv.", key + "residual.bn.")
         mag = mag + _mconv(xms, w, b, spec.stride)
     return value, mag
+
+
+def data_bn(x, sd):
+    """Raw frames (N, C, T, V, M) -> data_bn-normalised (value, mag), both float64 (N*M, C, T, V).  The affine map on
+    magnitudes is |scale| * |x| + |shift|."""
+    x = x.double()
+    N, C, T, V, M = x.shape
+    s = sd["data_bn.weight"].double() / torch.sqrt(sd["data_bn.running_var"].double() + regular.BN_EPS)
+    t = sd["data_bn.bias"].double() - sd["data_bn.running_mean"].double() * s
+    y = x.permute(0, 4, 3, 1, 2).reshape(N, M * V * C, T)
+    m = (s.abs()[:, None] * y.abs() + t.abs()[:, None]).view(N, M, V, C, T).permute(0, 1, 3, 4, 2).reshape(N * M, C, T, V)
+    return regular.normalise_input(x, sd), m
+
+
+def head(y_seq, sd, arch, ym=None):
+    """Last-block outputs (N*M, C, n, V) in emission order -> fp64 (value, mag) of the logits (N, classes, n_emit), the way
+    the continual head computes them: spatial and person mean, the sliding window of ``arch.pool_size`` entries whose
+    first ``arch.pool_padding`` positions start as zeros (the sum is always divided by ``pool_size``), then fc.
+    ``ym``: magnitude of the input (|y| by default).  The magnitudes go through |fc|."""
+    y = y_seq.double()
+    ym = y.abs() if ym is None else ym.double()
+    P, pp, M = arch.pool_size, arch.pool_padding, arch.persons
+    first = P - 1 - pp  # pool inputs before the first emission
+    w, b = sd["fc.weight"].double(), sd["fc.bias"].double()
+    out = []
+    for seq, wt, bt in ((y, w, b), (ym, w.abs(), b.abs())):
+        NM, C, n, V = seq.shape
+        p = seq.view(NM // M, M, C, n, V).mean(4).mean(1)  # (N, C, n)
+        p = F.pad(p, (P - 1, 0))  # the window's zero entries before the first input
+        win = p.unfold(2, P, 1)[:, :, first:].sum(3) / P  # (N, C, n_emit): window ending at input first + e
+        out.append(torch.einsum("kc,nce->nke", wt, win) + bt[None, :, None])
+    return out[0], out[1]
+
+
+def model(x, sd, arch):
+    """Raw frames (N, C, T, V, M) -> fp64 (value, mag) of the logits of every emission (N, classes, n_emit) of a whole
+    continual model.  The block bound is chained: each block's ``mag`` is built from its predecessor's, starting from
+    ``data_bn`` on |x|, and the head averages and pools the last ``mag`` and passes it through |fc|.  Each block adds at
+    most EPS * its own ``mag``, and later blocks carry it no further than their magnitudes do, so the logits are held to
+    n_blocks * EPS * mag, a coarse figure next to the single-block bound."""
+    h, hm = data_bn(x, sd)
+    for name, spec in zip(arch.block_names, arch.blocks):
+        h, hm = block(h, sd, name, spec, arch.padding, xm=hm)
+    # the regular clip math pads the end of every block: keep the outputs the continual walk has emitted
+    n = emitted(x.shape[2], arch)
+    return head(h[:, :, :n], sd, arch, ym=hm[:, :, :n])
+
+
+def emitted(frames, arch):
+    """Outputs the last block of a continual stack has emitted after ``frames`` steps from a fresh state."""
+    first = arch.receptive_field - 1 - arch.stack_padding
+    return max(0, (frames - 1 - first) // arch.stack_stride + 1)
 
 
 def headroom(got, value, mag):

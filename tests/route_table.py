@@ -82,6 +82,30 @@ def skeletons(n, skel, sms):
     return tiles * SPT[skel] - 2
 
 
+# --- what the GPU tests check ----------------------------------------------------------------------------------------
+def picked(B, skel, sms):
+    """Skeletons the oracle checks: all of them at small counts, else the first and last and both sides of every wave
+    boundary of the launchers' grids (work items of one tile or of a tile pair, one or two CTAs each)."""
+    if B <= 64:
+        return list(range(B))
+    spt = SPT[skel]
+    pick = {0, 1, B - 2, B - 1}
+    for tiles in {j * (sms // 2) for j in range(1, 9)} | {j * sms for j in range(1, 5)}:
+        for s in (tiles * spt - 1, tiles * spt):
+            if 0 <= s < B:
+                pick.add(s)
+    return sorted(pick)
+
+
+def signed_coordinates(rng, shape, skel, channel_dim=1):
+    """Skeleton coordinates in metres: signed x, y, z in [-2, 4); on Kinetics (x, y, confidence in [0, 1))."""
+    x = torch.from_numpy(rng.uniform(-2.0, 4.0, size=shape).astype(np.float32))
+    if skel == "kinetics":
+        conf = x.narrow(channel_dim, 2, 1)
+        conf.copy_(torch.from_numpy(rng.uniform(0.0, 1.0, size=tuple(conf.shape)).astype(np.float32)))
+    return x
+
+
 # --- the table -----------------------------------------------------------------------------------------------------
 # shape: (cin, cout, stride, residual, gconv); route: the knobs() entry of the block ({"block": prefix} for the one-kernel
 # block step, else {"gcn": prefix, "tcn": exact name}); batched: forward_steps walks the stack time-batched; covers: the
@@ -217,7 +241,7 @@ ROUTES = {
                      ("k_sa_qkv", "k_sa_attn_any", "k_tcn_simt")),
 }
 
-# test_gpu_routes.py::test_whole_model_signed_input: CoStGcn stepped frame by frame (64 -> 64 blocks as one kernel) and
+# test_gpu_routes.py::test_whole_model_signed_input, CoStGcn on NTU among its cases: stepped frame by frame (64 -> 64 blocks as one kernel) and
 # time-batched (every block as graph conv + temporal conv), with data_bn, pooling and fc
 WHOLE_MODEL_COVERS = ("k_input", "k_gcn_small", "k_tc_tcn<64>", "k_tc_block64", "k_tc_gcn<4,1,false>", "k_tc_gcnt<25,1,128>",
                       "k_tc_gcnt<25,2,128>", "k_tc_gcnt<25,2,256>", "k_tc_tcn<128>", "k_tc_tcn<256>", "k_head")

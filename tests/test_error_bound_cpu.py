@@ -6,12 +6,16 @@ fp32 mix over the vertices, the identity residual as an exact K-block, and every
 The correct emulation must sit at least 4x inside ``EPS * mag``; each arithmetic fault a kernel could plausibly have
 must break the bound on some element (by 4x, except as noted at MUTATIONS).  That is what makes the bound a trustworthy tolerance for the
 GPU route tests (tests/test_gpu_routes.py) before any of them runs.
+
+For whole models, ``bound.model`` and ``bound.head`` must compute what the step oracle computes, for all four
+architectures, and each plausible fault of the continual head (window length, padding, person mean, rows of two streams
+swapped) must break the head's bound by 4x.
 """
 import numpy as np
 import pytest
 import torch
 
-from oracle import bound, regular, weights
+from oracle import bound, regular, step, weights
 
 SKEL_PER_TILE = {"ntu": 5, "kinetics": 7}  # 128 token rows per tile / V
 
@@ -144,3 +148,90 @@ def test_each_fault_breaks_bound(case, mut):
     h = bound.headroom(got, value, mag)
     print(f"\n[bound] {tag} {mut}: max err/(EPS*mag) = {h:.2f}")
     assert h >= MUTATIONS[mut], (mut, h)
+
+
+# --- whole models: bound.model and bound.head against the step oracle ---------------------------------------------------
+ARCHS = {"cost_gcn": weights.cost_gcn_arch, "cost_gcn_mod": weights.cost_gcn_mod_arch, "coa_gcn": weights.coa_gcn_arch,
+         "cos_tr": weights.cos_tr_arch}
+# A short window with padding: the first two emissions still hold zero entries, and the window moves on for seven more.
+POOL_SIZE, POOL_PADDING, EMISSIONS = 6, 2, 9
+
+
+def _stepped(tag):
+    """Two streams of one model stepped by the oracle in float64: frames, state dict, arch, logits (N, classes, n_emit)
+    and the last block's outputs (N*M, C, n, V) in emission order."""
+    arch = ARCHS[tag](pool_size=POOL_SIZE, pool_padding=POOL_PADDING)
+    sd = weights.make_state_dict(arch, seed=sum(map(ord, tag)), randomize=True)
+    first = arch.receptive_field - 1 - arch.stack_padding + (POOL_SIZE - 1 - POOL_PADDING) * arch.stack_stride
+    x = weights.make_input((2, 3, first + 1 + (EMISSIONS - 1) * arch.stack_stride, arch.vertices, 2), seed=73).double()
+    model = step.StepModel(sd, arch)
+    last, seq = model.blocks[-1], []
+    last_step = last.step
+
+    def record(h):
+        y = last_step(h)
+        if y is not None:
+            seq.append(y)
+        return y
+
+    last.step = record
+    with torch.no_grad():
+        logits = model.forward_steps(x)
+    assert logits.shape[2] == EMISSIONS
+    return x, sd, arch, logits, torch.stack(seq, dim=2)
+
+
+@pytest.fixture(scope="module", params=list(ARCHS))
+def stepped(request):
+    return (request.param,) + _stepped(request.param)
+
+
+def _rel(a, b):
+    return float((a - b).abs().max()) / float(b.abs().max())
+
+
+def test_model_oracle_is_the_step_model(stepped):
+    tag, x, sd, arch, want, y_seq = stepped
+    value, mag = bound.model(x, sd, arch)
+    assert value.shape == want.shape
+    assert _rel(value, want) <= 1e-12, (tag, _rel(value, want))
+    assert bool((mag >= value.abs() - 1e-12).all())
+
+
+def test_head_oracle_is_the_step_head(stepped):
+    tag, x, sd, arch, want, y_seq = stepped
+    value, mag = bound.head(y_seq, sd, arch)
+    assert value.shape == want.shape
+    assert _rel(value, want) <= 1e-12, (tag, _rel(value, want))
+    assert bool((mag >= value.abs() - 1e-12).all())
+
+
+def faulty_head(y, sd, arch, fault):
+    """The continual head with one fault, in float64: (N*M, C, n, V) -> (N, classes, n_emit)."""
+    P, pp, M = arch.pool_size, arch.pool_padding, arch.persons
+    if fault == "rows_swapped":  # stream 0 person 1 and stream 1 person 0: one 128-row token tile holds both
+        y = y.clone()
+        y[[1, 2]] = y[[2, 1]]
+    per_person = y.view(y.shape[0] // M, M, *y.shape[1:]).mean(4)  # (N, M, C, n)
+    p = per_person[:, 0] if fault == "one_person" else per_person.mean(1)
+    size = {"window_short": P - 1, "window_long": P + 1}.get(fault, P)
+    out = []
+    for e in range(y.shape[2] - (P - 1 - pp)):
+        newest = e + P - 1 - pp
+        real = p[:, :, max(0, newest - size + 1): newest + 1]  # entries before input 0 are the window's zeros
+        div = real.shape[2] if fault == "padding_dropped" else P
+        out.append(torch.nn.functional.linear(real.sum(2) / div, sd["fc.weight"].double(), sd["fc.bias"].double()))
+    return torch.stack(out, dim=2)
+
+
+HEAD_FAULTS = ["window_short", "window_long", "padding_dropped", "one_person", "rows_swapped"]
+
+
+@pytest.mark.parametrize("fault", HEAD_FAULTS)
+def test_each_head_fault_breaks_bound(stepped, fault):
+    tag, x, sd, arch, want, y_seq = stepped
+    value, mag = bound.head(y_seq, sd, arch)
+    assert bound.headroom(faulty_head(y_seq, sd, arch, None), value, mag) <= 1e-6
+    h = bound.headroom(faulty_head(y_seq, sd, arch, fault), value, mag)
+    print(f"\n[bound] head {tag} {fault}: max err/(EPS*mag) = {h:.3g}")
+    assert h >= 4.0, (tag, fault, h)

@@ -17,7 +17,8 @@ wraps the rings -- and checks
 
 The table, with the kernels each case launches, lives in tests/route_table.py; tests/test_boundary_cpu.py checks that
 it declares every kernel csrc/cosk.cu can launch.  test_whole_model_signed_input runs the first-layer path with data_bn
-and the head (k_input, k_gcn_small, k_head) on signed skeleton coordinates through a whole CoStGcn.
+and the head (k_input, k_gcn_small, k_head) on signed skeleton coordinates through each of the four whole models, on
+both skeletons.
 
 The printed figure per case is max |got - value| / (EPS * mag), the headroom observed on the GPU.
 """
@@ -27,8 +28,8 @@ import torch
 
 import continual_skeletons_b200 as cs
 import route_table
-from oracle import bound, regular, step, weights
-from route_table import ROUTES, SPT
+from oracle import bound, weights
+from route_table import ROUTES
 
 pytestmark = pytest.mark.gpu
 
@@ -38,29 +39,6 @@ T = 12  # frames per clip: the first emission is at frame 4 (padding 4), the rin
 
 def _sms():
     return torch.cuda.get_device_properties(0).multi_processor_count
-
-
-def _picked(B, skel):
-    """Streams the oracle checks: all of them at small counts, else the first and last and both sides of every wave
-    boundary of the launchers' grids (work items of one tile or of a tile pair, one or two CTAs each)."""
-    if B <= 64:
-        return list(range(B))
-    spt, sms = SPT[skel], _sms()
-    pick = {0, 1, B - 2, B - 1}
-    for tiles in {j * (sms // 2) for j in range(1, 9)} | {j * sms for j in range(1, 5)}:
-        for s in (tiles * spt - 1, tiles * spt):
-            if 0 <= s < B:
-                pick.add(s)
-    return sorted(pick)
-
-
-def _signed_coordinates(rng, shape, skel, channel_dim=1):
-    """Skeleton coordinates in metres: signed x, y, z in [-2, 4); on Kinetics (x, y, confidence in [0, 1))."""
-    x = torch.from_numpy(rng.uniform(-2.0, 4.0, size=shape).astype(np.float32))
-    if skel == "kinetics":
-        conf = x.narrow(channel_dim, 2, 1)
-        conf.copy_(torch.from_numpy(rng.uniform(0.0, 1.0, size=tuple(conf.shape)).astype(np.float32)))
-    return x
 
 
 def _state(tag):
@@ -85,7 +63,7 @@ def _state(tag):
     B = route_table.skeletons(case.n, case.skel, _sms())
     V = arch.vertices
     if cin == 3:
-        x = _signed_coordinates(rng, (B, 3, T, V), case.skel)
+        x = route_table.signed_coordinates(rng, (B, 3, T, V), case.skel)
     else:
         x = torch.from_numpy(rng.uniform(-1.0, 1.0, size=(B, cin, T, V)).astype(np.float32))
     return spec, sd, mapped, x
@@ -113,7 +91,7 @@ def test_route(tag):
     case = ROUTES[tag]
     spec, sd, mapped, x = _state(tag)
     B = x.shape[0]
-    pick = _picked(B, case.skel)
+    pick = route_table.picked(B, case.skel, _sms())
     value, mag = bound.block(x[pick].double(), sd, "0.", spec, 4)
     xd = x.to(DEV)
     # frame by frame
@@ -160,50 +138,37 @@ def test_route(tag):
     assert h <= 1.0, (tag, h_step, h_whole, h_full)
 
 
+WHOLE_MODELS = {"cost_gcn": (cs.CoStGcn, weights.cost_gcn_arch), "cost_gcn_mod": (cs.CoStGcnMod, weights.cost_gcn_mod_arch),
+                "coa_gcn": (cs.CoAGcn, weights.coa_gcn_arch), "cos_tr": (cs.CoSTr, weights.cos_tr_arch)}
+
+
 @pytest.mark.parametrize("skel", ["ntu", "kinetics"])
-def test_whole_model_signed_input(skel):
-    """A whole CoStGcn on signed skeleton coordinates (data_bn folded into k_input, k_gcn_small, ten blocks, pooling and fc
-    in k_head), stepped frame by frame and time-batched, against the step oracle run in float64.  The error scale is the
-    block bound chained through the stack (each block's ``mag`` built from its predecessor's), averaged and pooled like
-    the logits, and passed through |fc|.  Each block adds at most EPS * its own ``mag`` and the later blocks carry it no
-    further than their magnitudes do, so the logits are held to n_blocks * EPS * mag."""
+@pytest.mark.parametrize("tag", list(WHOLE_MODELS))
+def test_whole_model_signed_input(tag, skel):
+    """A whole model on signed skeleton coordinates (data_bn folded into k_input, the first layer's graph conv, ten blocks,
+    pooling and fc in k_head), stepped frame by frame and time-batched, against ``bound.model``: the model in float64
+    with the block bound chained through the stack, which holds the logits to n_blocks * EPS * mag.  The window has two
+    entries of padding, so the first emissions average over its zeros."""
+    cls, arch_fn = WHOLE_MODELS[tag]
     classes = 60 if skel == "ntu" else 400
-    P, pp = 8, 0
-    arch = weights.cost_gcn_arch(skeleton=skel, classes=classes, pool_size=P, pool_padding=pp)
+    P, pp = 8, 2
+    arch = arch_fn(skeleton=skel, classes=classes, pool_size=P, pool_padding=pp)
     sd = weights.make_state_dict(arch, seed=91, randomize=True)
-    V = arch.vertices
     first = arch.receptive_field - 1 - arch.stack_padding + (P - 1 - pp) * arch.stack_stride
     Tm = first + 1 + 2 * arch.stack_stride  # three emissions
     rng = np.random.Generator(np.random.PCG64(92))
-    x = _signed_coordinates(rng, (2, 3, Tm, V, 2), skel)
-    xd64 = x.double()
+    x = route_table.signed_coordinates(rng, (2, 3, Tm, arch.vertices, 2), skel)
     with torch.no_grad():
-        want = step.StepModel(sd, arch).forward_steps(xd64)  # (N, classes, 3), float64
-        # chained error scale: data_bn as an affine map on |x|, then block by block
-        N, C, _, _, M = x.shape
-        s = sd["data_bn.weight"].double() / torch.sqrt(sd["data_bn.running_var"].double() + regular.BN_EPS)
-        t = sd["data_bn.bias"].double() - sd["data_bn.running_mean"].double() * s
-        y = xd64.permute(0, 4, 3, 1, 2).reshape(N, M * V * C, Tm)
-        hm = (s.abs()[:, None] * y.abs() + t.abs()[:, None]).view(N, M, V, C, Tm).permute(0, 1, 3, 4, 2).reshape(N * M, C, Tm, V)
-        h = regular.normalise_input(xd64, sd)
-        for name, spec in zip(arch.block_names, arch.blocks):
-            h, hm = bound.block(h, sd, name, spec, arch.padding, xm=hm)
-        pm = hm.view(N, M, hm.shape[1], hm.shape[2], V).mean(4).mean(1)  # (N, C, T_last)
-        mags = []
-        for e in range(want.shape[2]):
-            m = e + P - 1 - pp
-            win = pm[:, :, max(0, m - P + 1): m + 1].sum(2) / P
-            mags.append(win @ sd["fc.weight"].double().abs().T + sd["fc.bias"].double().abs())
-        mag = torch.stack(mags, dim=2)
+        want, mag = bound.model(x, sd, arch)  # (N, classes, 3)
     tol = len(arch.blocks) * bound.EPS
     for tc in (1, -1):
-        model = cs.CoStGcn({"dataset_name": "dummy_ntu" if skel == "ntu" else "dummy_kin", "pool_size": P, "pool_padding": pp,
-                            "time_chunk": tc})
+        model = cls({"dataset_name": "dummy_ntu" if skel == "ntu" else "dummy_kin", "pool_size": P, "pool_padding": pp,
+                     "time_chunk": tc})
         model.load_state_dict(model.map_state_dict(sd), strict=True)
         got = model.forward_steps(x.to(DEV))
         assert model.device_error() == 0, hex(model.device_error())
         assert tuple(got.shape) == tuple(want.shape), (got.shape, want.shape)
         r = float(((got.cpu().double() - want).abs() / (tol * mag + bound.TINY)).max())
-        print(f"\n[route] whole CoStGcn {skel} time_chunk={tc}: knobs={model.knobs()['blocks'][:2]} "
+        print(f"\n[route] whole {tag} {skel} time_chunk={tc}: knobs={model.knobs()['blocks'][:2]} "
               f"max err/({len(arch.blocks)}*EPS*mag) = {r:.4f}")
-        assert r <= 1.0, (skel, tc, r)
+        assert r <= 1.0, (tag, skel, tc, r)
