@@ -21,6 +21,7 @@
 #include "tc_agcnt.cuh"
 #endif
 #include "tc_block.cuh"
+#include "stream_state.cuh"
 
 using namespace cosk;
 
@@ -157,6 +158,9 @@ struct cosk_model {
   float *d_qkv = nullptr;    // self-attention unit: q | k | v rows [t_alloc][2*dk + dv] of the frame in flight (fp32)
   float *d_dense = nullptr;  // adaptive graph conv: per-token mixing rows [t_alloc][3][dense_vp] of the frame in flight
   int dense_vp = 0;
+  long long *d_idx = nullptr;      // [n_streams] stream indices of a per-stream state call (k_stream_state)
+  cudaEvent_t ev_idx = nullptr;    // recorded behind the last such call: the next one's index upload waits for it
+  std::vector<long long> h_idx;    // host copy the index upload reads
   long long pool_n = 0, frame = 0;
   std::vector<int32_t> last_flags;
   unsigned int *d_dbg = nullptr;
@@ -212,21 +216,83 @@ void dfree(T *&p) {
   p = nullptr;
 }
 
-void free_state(cosk_model *m) {
-  dfree(m->xin.ptr);
+// The per-stream buffers of one batch size and their geometry, detached from a handle (cosk_resize_batch keeps the old set
+// alive while the new one is filled).
+struct StateSet {
+  long long n_streams = 0, n_tokens = 0, t_alloc = 0;
+  int skel_per_tile = 0, tile_tokens = 0, n_tiles = 0, dense_vp = 0;
+  int64_t state_bytes = 0;
+  ActBuf xin;
+  std::vector<ActBuf> ring, out, sa, sa_x, sa_q;
+  float *d_qkv = nullptr, *d_pool_ring = nullptr, *d_dense = nullptr;
+  double *d_pool_sum = nullptr;
+  long long *d_idx = nullptr;
+};
+
+StateSet detach_state(cosk_model *m) {
+  StateSet s;
+  std::swap(s.n_streams, m->n_streams);
+  std::swap(s.n_tokens, m->n_tokens);
+  std::swap(s.t_alloc, m->t_alloc);
+  std::swap(s.skel_per_tile, m->skel_per_tile);
+  std::swap(s.tile_tokens, m->tile_tokens);
+  std::swap(s.n_tiles, m->n_tiles);
+  std::swap(s.dense_vp, m->dense_vp);
+  std::swap(s.state_bytes, m->state_bytes);
+  std::swap(s.xin, m->xin);
   for (auto &b : m->blk) {
-    dfree(b.ring.ptr);
-    dfree(b.out.ptr);
-    dfree(b.sa.ptr);
-    dfree(b.sa_x.ptr);
-    dfree(b.sa_q.ptr);
+    s.ring.push_back(b.ring);
+    s.out.push_back(b.out);
+    s.sa.push_back(b.sa);
+    s.sa_x.push_back(b.sa_x);
+    s.sa_q.push_back(b.sa_q);
+    b.ring = b.out = b.sa = b.sa_x = b.sa_q = ActBuf();
   }
-  dfree(m->d_qkv);
-  dfree(m->d_pool_ring);
-  dfree(m->d_pool_sum);
-  dfree(m->d_dense);
-  m->n_streams = 0;
-  m->state_bytes = 0;
+  std::swap(s.d_qkv, m->d_qkv);
+  std::swap(s.d_pool_ring, m->d_pool_ring);
+  std::swap(s.d_dense, m->d_dense);
+  std::swap(s.d_pool_sum, m->d_pool_sum);
+  std::swap(s.d_idx, m->d_idx);
+  return s;
+}
+
+// The inverse of detach_state, on a handle without buffers (after free_state).
+void attach_state(cosk_model *m, StateSet &s) {
+  std::swap(s.n_streams, m->n_streams);
+  std::swap(s.n_tokens, m->n_tokens);
+  std::swap(s.t_alloc, m->t_alloc);
+  std::swap(s.skel_per_tile, m->skel_per_tile);
+  std::swap(s.tile_tokens, m->tile_tokens);
+  std::swap(s.n_tiles, m->n_tiles);
+  std::swap(s.dense_vp, m->dense_vp);
+  std::swap(s.state_bytes, m->state_bytes);
+  std::swap(s.xin, m->xin);
+  for (size_t i = 0; i < m->blk.size(); ++i) {
+    BlockW &b = m->blk[i];
+    b.ring = s.ring[i], b.out = s.out[i], b.sa = s.sa[i], b.sa_x = s.sa_x[i], b.sa_q = s.sa_q[i];
+  }
+  s.ring.clear(), s.out.clear(), s.sa.clear(), s.sa_x.clear(), s.sa_q.clear();
+  std::swap(s.d_qkv, m->d_qkv);
+  std::swap(s.d_pool_ring, m->d_pool_ring);
+  std::swap(s.d_dense, m->d_dense);
+  std::swap(s.d_pool_sum, m->d_pool_sum);
+  std::swap(s.d_idx, m->d_idx);
+}
+
+void free_set(StateSet &s) {
+  dfree(s.xin.ptr);
+  for (auto *v : {&s.ring, &s.out, &s.sa, &s.sa_x, &s.sa_q})
+    for (ActBuf &b : *v) dfree(b.ptr);
+  dfree(s.d_qkv);
+  dfree(s.d_pool_ring);
+  dfree(s.d_pool_sum);
+  dfree(s.d_dense);
+  dfree(s.d_idx);
+}
+
+void free_state(cosk_model *m) {
+  StateSet s = detach_state(m);
+  free_set(s);
 }
 
 int make_map(cosk_model *m, CUtensorMap *map, void *base, uint64_t cols, uint64_t rows, uint32_t box_rows) {
@@ -625,18 +691,25 @@ int prepare(cosk_model *m) {
   return COSK_OK;
 }
 
-int zero_state(cosk_model *m, cudaStream_t s) {
+// Zeroes every state buffer (not the counters).
+int zero_buffers(cosk_model *m, cudaStream_t s) {
   CK(cudaMemsetAsync(m->xin.ptr, 0, m->xin.bytes(), s));
   for (auto &b : m->blk) {
     CK(cudaMemsetAsync(b.ring.ptr, 0, b.ring.bytes(), s));
     CK(cudaMemsetAsync(b.out.ptr, 0, b.out.bytes(), s));
-    b.n_in = b.n_out = 0;
   }
   if (m->cfg.classes > 0) {
     const size_t cl = (size_t)m->cfg.blocks[m->cfg.n_blocks - 1].cout;
     CK(cudaMemsetAsync(m->d_pool_ring, 0, (size_t)m->cfg.pool_size * m->n_streams * cl * sizeof(float), s));
     CK(cudaMemsetAsync(m->d_pool_sum, 0, (size_t)m->n_streams * cl * sizeof(double), s));
   }
+  return COSK_OK;
+}
+
+int zero_state(cosk_model *m, cudaStream_t s) {
+  int rc = zero_buffers(m, s);
+  if (rc) return rc;
+  for (auto &b : m->blk) b.n_in = b.n_out = 0;
   CK(cudaMemsetAsync(m->d_dbg, 0, 4 * sizeof(unsigned int), s));
   if (m->h_dbg) m->h_dbg[0] = 0;
   m->failed = false;
@@ -1347,6 +1420,44 @@ inline bool tcn_fires(long long n, int padding, int stride) {
 // co.AvgPool1d(P, stride 1, padding pp): the m-th pooled vector yields logits iff m >= P - 1 - pp.
 inline bool head_fires(long long m_, int pool_size, int pool_padding) { return m_ >= (long long)pool_size - 1 - pool_padding; }
 
+// One frame of the emission bookkeeping from counters n_in (per block) and pool_n: advances them, writes n_blocks + 1 flags
+// laid out like cosk_last_schedule.
+void schedule_frame(const cosk_config &c, long long *n_in, long long *pool_n, int32_t *flags) {
+  bool alive = true;
+  for (int i = 0; i < c.n_blocks; ++i) {
+    flags[i] = 0;
+    if (!alive) continue;
+    const bool fire = tcn_fires(n_in[i], c.padding, c.blocks[i].stride);
+    n_in[i]++;
+    alive = fire;
+    flags[i] = fire ? 1 : 0;
+  }
+  int emit = 0;
+  if (alive) {
+    if (c.classes > 0) emit = head_fires((*pool_n)++, c.pool_size, c.pool_padding) ? 1 : 0;
+    else emit = 1;
+  }
+  flags[c.n_blocks] = emit;
+}
+
+// The counters schedule_frame reaches after `frames` frames from zero, in closed form.
+void counters_at(const cosk_config &c, long long frames, long long *n_in, long long *pool_n) {
+  const int first = (kTaps - 1) - c.padding;
+  long long n = frames;
+  for (int i = 0; i < c.n_blocks; ++i) {
+    n_in[i] = n;
+    n = n > first ? (n - 1 - first) / c.blocks[i].stride + 1 : 0;  // firing inputs among 0 .. n-1
+  }
+  *pool_n = c.classes > 0 ? n : 0;
+}
+
+// Every block has reached its first firing input and the pooling window its first emission: the schedule is periodic.
+bool past_warmup(const cosk_config &c, const long long *n_in, long long pool_n) {
+  for (int i = 0; i < c.n_blocks; ++i)
+    if (n_in[i] < (kTaps - 1) - c.padding) return false;
+  return c.classes <= 0 || head_fires(pool_n, c.pool_size, c.pool_padding);
+}
+
 // One step of the stack.  `enter` = 0: a new input frame x enters at the first block (cosk_step).  End-of-sequence flush
 // (forward_steps(pad_end=True) of the library: every temporal module is fed its own end padding once the clip is over,
 // module by module): `enter` = i in [0, n_blocks) pushes one ZERO frame into the temporal conv of block i (not through its
@@ -1513,7 +1624,69 @@ std::string gcn_name(const BlockW &b) {
   return std::string(attn[(int)b.route.attn]) + t;
 }
 
+// Allocates the per-stream buffers of `n_streams` streams on a handle without buffers (contents undefined except the
+// scratch, which starts zeroed).
+int alloc_state(cosk_model *m, int64_t n_streams) {
+  const cosk_config &c = m->cfg;
+  m->n_streams = n_streams;
+  const long long skel = n_streams * c.persons;
+  m->n_tokens = skel * c.vertices;
+  m->skel_per_tile = kTileRows / c.vertices;
+  m->tile_tokens = m->skel_per_tile * c.vertices;
+  m->n_tiles = (int)((skel + m->skel_per_tile - 1) / m->skel_per_tile);
+  // +1 tile: with an odd tile count the second CTA of the last pair walks a phantom tile (loads only)
+  m->t_alloc = round_up((int)((long long)(m->n_tiles + 1) * m->tile_tokens + (kTileRows - m->tile_tokens)), 8);
+  if ((long long)m->R * 2 * m->t_alloc > 0x7fffffffLL) return fail(m, COSK_ERR_ARG, "too many streams (x time chunk) for 32-bit rows");
+  int rc = alloc_act(m, m->xin, m->Ro, c.c_in);
+  if (rc) return rc;
+  for (int i = 0; i < c.n_blocks; ++i) {
+    if ((rc = alloc_act(m, m->blk[i].ring, m->R, c.blocks[i].cout))) return rc;
+    if ((rc = alloc_act(m, m->blk[i].out, m->Ro, c.blocks[i].cout))) return rc;
+  }
+  if (c.classes > 0) {
+    const size_t cl = (size_t)c.blocks[c.n_blocks - 1].cout;
+    CK(cudaMalloc(&m->d_pool_ring, (size_t)c.pool_size * n_streams * cl * sizeof(float)));
+    CK(cudaMalloc(&m->d_pool_sum, (size_t)n_streams * cl * sizeof(double)));
+    m->state_bytes += (int64_t)((size_t)c.pool_size * n_streams * cl * sizeof(float) + (size_t)n_streams * cl * sizeof(double));
+  }
+  bool any_adaptive = false;
+  int max_nq = 0;
+  for (int i = 0; i < c.n_blocks; ++i) {
+    any_adaptive |= c.blocks[i].gconv == COSK_GCONV_ADAPTIVE;
+    if (c.blocks[i].gconv == COSK_GCONV_ATTENTION) {
+      max_nq = std::max(max_nq, 2 * (c.blocks[i].cout / 4) + c.blocks[i].cout);
+      if ((rc = alloc_act(m, m->blk[i].sa, 1, c.blocks[i].cout))) return rc;
+      CK(cudaMemset(m->blk[i].sa.ptr, 0, m->blk[i].sa.bytes()));
+      const GcnRoute g = m->blk[i].route.gcn;
+      if (g != GcnRoute::kSaSimt) {
+        if ((rc = alloc_act(m, m->blk[i].sa_x, 1, c.blocks[i].cin))) return rc;
+        CK(cudaMemset(m->blk[i].sa_x.ptr, 0, m->blk[i].sa_x.bytes()));
+        if (g == GcnRoute::kSaTcQkv) {
+          if ((rc = alloc_act(m, m->blk[i].sa_q, 1, kSaQkvCols))) return rc;
+          CK(cudaMemset(m->blk[i].sa_q.ptr, 0, m->blk[i].sa_q.bytes()));
+        }
+      }
+    }
+  }
+  if (max_nq) {
+    const size_t bytes = (size_t)m->t_alloc * max_nq * sizeof(float);
+    CK(cudaMalloc(&m->d_qkv, bytes));
+    m->state_bytes += (int64_t)bytes;  // scratch, counted in the footprint
+  }
+  if (any_adaptive) {
+    m->dense_vp = round_up(c.vertices, 4);
+    const size_t bytes = (size_t)m->t_alloc * 3 * m->dense_vp * sizeof(float);
+    CK(cudaMalloc(&m->d_dense, bytes));
+    CK(cudaMemset(m->d_dense, 0, bytes));
+    m->state_bytes += (int64_t)bytes;  // scratch, not state, but part of the per-stream footprint
+  }
+  CK(cudaMalloc(&m->d_idx, (size_t)n_streams * sizeof(long long)));  // index list of the per-stream calls, not counted
+  return COSK_OK;
+}
+
 }  // namespace
+
+#include "stream_state_host.cuh"
 
 extern "C" {
 
@@ -1639,6 +1812,7 @@ void cosk_destroy(cosk_model *m) {
   if (m->h_dbg) cudaFreeHost(m->h_dbg);
   dfree(m->d_trace);
   for (auto e : m->ev_pool) cudaEventDestroy(e);
+  if (m->ev_idx) cudaEventDestroy(m->ev_idx);
   delete m;
 }
 
@@ -1692,64 +1866,14 @@ int cosk_set_batch_ex(cosk_model *m, int64_t n_streams, int32_t time_chunk) {
   }
   CK(cudaDeviceSynchronize());
   free_state(m);
-  const cosk_config &c = m->cfg;
-  m->n_streams = n_streams;
-  const long long skel = n_streams * c.persons;
-  m->n_tokens = skel * c.vertices;
-  m->skel_per_tile = kTileRows / c.vertices;
-  m->tile_tokens = m->skel_per_tile * c.vertices;
-  m->n_tiles = (int)((skel + m->skel_per_tile - 1) / m->skel_per_tile);
-  // +1 tile: with an odd tile count the second CTA of the last pair walks a phantom tile (loads only)
-  m->t_alloc = round_up((int)((long long)(m->n_tiles + 1) * m->tile_tokens + (kTileRows - m->tile_tokens)), 8);
-  if ((long long)m->R * 2 * m->t_alloc > 0x7fffffffLL) return fail(m, COSK_ERR_ARG, "too many streams (x time chunk) for 32-bit rows");
-  int rc = alloc_act(m, m->xin, m->Ro, c.c_in);
+  int rc = alloc_state(m, n_streams);
   if (rc) return rc;
-  for (int i = 0; i < c.n_blocks; ++i) {
-    if ((rc = alloc_act(m, m->blk[i].ring, m->R, c.blocks[i].cout))) return rc;
-    if ((rc = alloc_act(m, m->blk[i].out, m->Ro, c.blocks[i].cout))) return rc;
-  }
-  if (c.classes > 0) {
-    const size_t cl = (size_t)c.blocks[c.n_blocks - 1].cout;
-    CK(cudaMalloc(&m->d_pool_ring, (size_t)c.pool_size * n_streams * cl * sizeof(float)));
-    CK(cudaMalloc(&m->d_pool_sum, (size_t)n_streams * cl * sizeof(double)));
-    m->state_bytes += (int64_t)((size_t)c.pool_size * n_streams * cl * sizeof(float) + (size_t)n_streams * cl * sizeof(double));
-  }
-  bool any_adaptive = false;
-  int max_nq = 0;
-  for (int i = 0; i < c.n_blocks; ++i) {
-    any_adaptive |= c.blocks[i].gconv == COSK_GCONV_ADAPTIVE;
-    if (c.blocks[i].gconv == COSK_GCONV_ATTENTION) {
-      max_nq = std::max(max_nq, 2 * (c.blocks[i].cout / 4) + c.blocks[i].cout);
-      if ((rc = alloc_act(m, m->blk[i].sa, 1, c.blocks[i].cout))) return rc;
-      CK(cudaMemset(m->blk[i].sa.ptr, 0, m->blk[i].sa.bytes()));
-      const GcnRoute g = m->blk[i].route.gcn;
-      if (g != GcnRoute::kSaSimt) {
-        if ((rc = alloc_act(m, m->blk[i].sa_x, 1, c.blocks[i].cin))) return rc;
-        CK(cudaMemset(m->blk[i].sa_x.ptr, 0, m->blk[i].sa_x.bytes()));
-        if (g == GcnRoute::kSaTcQkv) {
-          if ((rc = alloc_act(m, m->blk[i].sa_q, 1, kSaQkvCols))) return rc;
-          CK(cudaMemset(m->blk[i].sa_q.ptr, 0, m->blk[i].sa_q.bytes()));
-        }
-      }
-    }
-  }
-  if (max_nq) {
-    const size_t bytes = (size_t)m->t_alloc * max_nq * sizeof(float);
-    CK(cudaMalloc(&m->d_qkv, bytes));
-    m->state_bytes += (int64_t)bytes;  // scratch, counted in the footprint
-  }
-  if (any_adaptive) {
-    m->dense_vp = round_up(c.vertices, 4);
-    const size_t bytes = (size_t)m->t_alloc * 3 * m->dense_vp * sizeof(float);
-    CK(cudaMalloc(&m->d_dense, bytes));
-    CK(cudaMemset(m->d_dense, 0, bytes));
-    m->state_bytes += (int64_t)bytes;  // scratch, not state, but part of the per-stream footprint
-  }
   rc = zero_state(m, 0);
   if (rc) return rc;
   CK(cudaDeviceSynchronize());
   return COSK_OK;
 }
+
 
 int cosk_reset(cosk_model *m) {
   if (!m) return COSK_ERR_ARG;
@@ -1765,8 +1889,8 @@ int cosk_reset(cosk_model *m) {
 // Shared entry checks of cosk_step / cosk_steps: call order, and the failure latch.  A step that stopped half way
 // leaves the host counters ahead of the device state, and a fired pipeline watchdog (bounded mbarrier wait,
 // ptx.cuh) makes every later result garbage: both refuse further steps until cosk_reset / cosk_set_batch.
-static int step_entry(cosk_model *m) {
-  if (m->n_streams == 0) return fail(m, COSK_ERR_STATE, "step before cosk_set_batch");
+static int step_entry(cosk_model *m, const char *what = "step") {
+  if (m->n_streams == 0) return fail(m, COSK_ERR_STATE, "%s before cosk_set_batch", what);
   if (!m->prepared) return fail(m, COSK_ERR_STATE, "weights changed after cosk_set_batch: call cosk_set_batch again");
   if (m->h_dbg && m->h_dbg[0] != 0) m->failed = true;  // written by the async copy behind an earlier emitting step
   if (m->failed) {
@@ -1946,25 +2070,34 @@ int cosk_device_error(cosk_model *m, uint32_t *code) {
 int cosk_simulate_schedule(const cosk_config *cfg, int32_t T, int32_t *flags) {
   if (!cfg || !flags || T < 0 || cfg->n_blocks < 1 || cfg->n_blocks > COSK_MAX_BLOCKS) return COSK_ERR_ARG;
   long long n_in[COSK_MAX_BLOCKS] = {0}, pool_n = 0;
-  const int w = cfg->n_blocks + 1;
-  for (int t = 0; t < T; ++t) {
-    bool alive = true;
-    for (int i = 0; i < cfg->n_blocks; ++i) {
-      flags[t * w + i] = 0;
-      if (!alive) continue;
-      const bool fire = tcn_fires(n_in[i], cfg->padding, cfg->blocks[i].stride);
-      n_in[i]++;
-      alive = fire;
-      flags[t * w + i] = fire ? 1 : 0;
-    }
-    int emit = 0;
-    if (alive) {
-      if (cfg->classes > 0) emit = head_fires(pool_n++, cfg->pool_size, cfg->pool_padding) ? 1 : 0;
-      else emit = 1;
-    }
-    flags[t * w + cfg->n_blocks] = emit;
-  }
+  for (int t = 0; t < T; ++t) schedule_frame(*cfg, n_in, &pool_n, flags + (size_t)t * (cfg->n_blocks + 1));
   return COSK_OK;
+}
+
+int cosk_schedule_compatible(const cosk_config *cfg, int64_t frame_a, int64_t frame_b) {
+  if (!cfg || cfg->n_blocks < 1 || cfg->n_blocks > COSK_MAX_BLOCKS || frame_a < 0 || frame_b < 0) return COSK_ERR_ARG;
+  if (cfg->padding < 0 || cfg->padding > kTaps - 1 || (cfg->classes > 0 && cfg->pool_size < 1)) return COSK_ERR_ARG;
+  long long period = 1;
+  for (int i = 0; i < cfg->n_blocks; ++i) {
+    if (cfg->blocks[i].stride < 1) return COSK_ERR_ARG;
+    period *= cfg->blocks[i].stride;
+  }
+  if (frame_a == frame_b) return 1;
+  long long in_a[COSK_MAX_BLOCKS], in_b[COSK_MAX_BLOCKS], pool_a, pool_b;
+  counters_at(*cfg, frame_a, in_a, &pool_a);
+  counters_at(*cfg, frame_b, in_b, &pool_b);
+  // Compare the flags frame by frame until both counters are past the warm-up; from there on both schedules repeat with
+  // the period (the product of the strides), so one more period decides every later frame.
+  int32_t fa[COSK_MAX_BLOCKS + 1], fb[COSK_MAX_BLOCKS + 1];
+  long long left = -1;
+  while (left != 0) {
+    schedule_frame(*cfg, in_a, &pool_a, fa);
+    schedule_frame(*cfg, in_b, &pool_b, fb);
+    if (memcmp(fa, fb, sizeof(int32_t) * (cfg->n_blocks + 1)) != 0) return 0;
+    if (left > 0) --left;
+    else if (past_warmup(*cfg, in_a, pool_a) && past_warmup(*cfg, in_b, pool_b)) left = period;
+  }
+  return 1;
 }
 
 int cosk_trace_read(cosk_model *m, uint64_t *out, int32_t n) {
@@ -1999,6 +2132,75 @@ int cosk_profile_read(cosk_model *m, int32_t kind, int32_t block, double *ms, in
   }
   *ms = tot;
   *launches = cnt;
+  return COSK_OK;
+}
+
+int64_t cosk_stream_bytes(const cosk_model *m) {
+  if (!m) return 0;
+  return state_args(const_cast<cosk_model *>(m)).stream_bytes;
+}
+
+int cosk_reset_streams(cosk_model *m, const int64_t *idx, int64_t n, void *stream) {
+  if (!m) return COSK_ERR_ARG;
+  int rc = step_entry(m, "cosk_reset_streams");
+  if (rc || (rc = check_indices(m, idx, n, 0, m->n_streams, true))) return rc;
+  DeviceGuard guard_(m->cfg.device);
+  StateArgs a = state_args(m);
+  return launch_stream_state(m, a, kStateZero, nullptr, (cudaStream_t)stream);
+}
+
+int cosk_export_streams(cosk_model *m, const int64_t *idx, int64_t n, void *dst_dev, cosk_stream_meta *meta, void *stream) {
+  if (!m || !meta || (n > 0 && !dst_dev)) return COSK_ERR_ARG;
+  int rc = step_entry(m, "cosk_export_streams");
+  if (rc || (rc = check_indices(m, idx, n, 0, m->n_streams, true))) return rc;
+  DeviceGuard guard_(m->cfg.device);
+  meta->abi_version = COSK_ABI_VERSION;
+  meta->geometry = geometry_of(m->cfg);
+  meta->frame = m->frame;
+  StateArgs a = state_args(m);
+  return launch_stream_state(m, a, kStateGather, dst_dev, (cudaStream_t)stream);
+}
+
+int cosk_import_streams(cosk_model *m, const int64_t *idx, int64_t n, const void *src_dev, const cosk_stream_meta *meta,
+                        void *stream) {
+  if (!m || !meta || (n > 0 && !src_dev)) return COSK_ERR_ARG;
+  int rc = step_entry(m, "cosk_import_streams");
+  if (rc || (rc = check_indices(m, idx, n, 0, m->n_streams, true))) return rc;
+  if (meta->abi_version != COSK_ABI_VERSION || meta->geometry != geometry_of(m->cfg))
+    return fail(m, COSK_ERR_STATE, "stream payload of another model geometry or library version");
+  if (cosk_schedule_compatible(&m->cfg, meta->frame, m->frame) != 1)
+    return fail(m, COSK_ERR_STATE, "stream payload exported at frame %lld does not fit the schedule at frame %lld",
+                (long long)meta->frame, m->frame);
+  DeviceGuard guard_(m->cfg.device);
+  StateArgs a = state_args(m);
+  return launch_stream_state(m, a, kStateScatter, const_cast<void *>(src_dev), (cudaStream_t)stream);
+}
+
+int cosk_resize_batch(cosk_model *m, int64_t n_streams, const int64_t *src) {
+  if (!m) return COSK_ERR_ARG;
+  int rc = step_entry(m, "cosk_resize_batch");
+  if (rc) return rc;
+  if (n_streams < 1 || !src) return fail(m, COSK_ERR_ARG, "cosk_resize_batch: n_streams %lld", (long long)n_streams);
+  if ((rc = check_indices(m, src, n_streams, -1, m->n_streams, false))) return rc;
+  DeviceGuard guard_(m->cfg.device);
+  CK(cudaDeviceSynchronize());  // no step or state call is in flight on the old buffers
+  StateArgs a = state_args(m);
+  StateSet old = detach_state(m);
+  rc = alloc_state(m, n_streams);
+  if (!rc) rc = zero_buffers(m, 0);
+  if (!rc) {
+    StateArgs b = state_args(m);
+    memcpy(b.from, a.state, sizeof b.from);
+    rc = launch_stream_state(m, b, kStateMove, nullptr, 0);
+  }
+  if (!rc && cudaDeviceSynchronize() != cudaSuccess) rc = fail(m, COSK_ERR_CUDA, "cosk_resize_batch: state move failed");
+  if (rc) {  // the handle goes back to the old buffers, untouched
+    cudaGetLastError();
+    free_state(m);
+    attach_state(m, old);
+    return rc;
+  }
+  free_set(old);
   return COSK_OK;
 }
 

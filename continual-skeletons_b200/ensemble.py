@@ -43,6 +43,16 @@ class MultiStream:
         for m in self.models:
             m.clean_state()
 
+    def reset_streams(self, indices):
+        """``reset_streams`` on every member: the listed streams start over in all modalities."""
+        for m in self.models:
+            m.reset_streams(indices)
+
+    def resize_streams(self, keep):
+        """``resize_streams`` on every member, so the members stay in lock step on the same streams."""
+        for m in self.models:
+            m.resize_streams(keep)
+
     def forward_step(self, inputs):
         """inputs: one (N, C, V, S) CUDA tensor per member model.  Fused logits, or None when no prediction is due."""
         inputs = list(inputs)

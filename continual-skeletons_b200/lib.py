@@ -39,6 +39,11 @@ class Config(ctypes.Structure):
     ]
 
 
+class StreamMeta(ctypes.Structure):
+    """cosk_stream_meta: what an exported stream payload was taken from."""
+    _fields_ = [("abi_version", ctypes.c_int32), ("geometry", ctypes.c_uint64), ("frame", ctypes.c_int64)]
+
+
 def library_path():
     return os.path.join(CSRC, "libcosk.so")
 
@@ -107,7 +112,13 @@ SYMBOLS = {
     "cosk_state_bytes": (ctypes.c_int64, [_P]),
     "cosk_last_schedule": (ctypes.c_int, [_P, ctypes.POINTER(ctypes.c_int32), ctypes.c_int32]),
     "cosk_simulate_schedule": (ctypes.c_int, [ctypes.POINTER(Config), ctypes.c_int32, ctypes.POINTER(ctypes.c_int32)]),
+    "cosk_schedule_compatible": (ctypes.c_int, [ctypes.POINTER(Config), ctypes.c_int64, ctypes.c_int64]),
     "cosk_frame_count": (ctypes.c_int64, [_P]),
+    "cosk_stream_bytes": (ctypes.c_int64, [_P]),
+    "cosk_reset_streams": (ctypes.c_int, [_P, ctypes.POINTER(ctypes.c_int64), ctypes.c_int64, _P]),
+    "cosk_export_streams": (ctypes.c_int, [_P, ctypes.POINTER(ctypes.c_int64), ctypes.c_int64, _P, ctypes.POINTER(StreamMeta), _P]),
+    "cosk_import_streams": (ctypes.c_int, [_P, ctypes.POINTER(ctypes.c_int64), ctypes.c_int64, _P, ctypes.POINTER(StreamMeta), _P]),
+    "cosk_resize_batch": (ctypes.c_int, [_P, ctypes.c_int64, ctypes.POINTER(ctypes.c_int64)]),
     "cosk_read_block": (ctypes.c_int, [_P, ctypes.c_int32, _P, _P]),
     "cosk_launch_count": (ctypes.c_int64, [_P]),
     "cosk_block_uses_tensor_cores": (ctypes.c_int, [_P, ctypes.c_int32]),

@@ -43,6 +43,15 @@ class BlockSpec(namedtuple("BlockSpec", "cin cout stride residual gconv")):
         return 1 if (self.cin == self.cout and self.stride == 1) else 2
 
 
+StreamMeta = namedtuple("StreamMeta", "abi_version geometry frame")
+StreamMeta.__doc__ = """cosk_stream_meta: library ABI version, geometry fingerprint and frame count of an exported payload."""
+
+
+class StreamState(namedtuple("StreamState", "payload meta")):
+    """State of some streams taken by ``export_streams``: ``payload`` is a CUDA uint8 tensor (n, stream_bytes), row q the
+    q-th exported stream in the layout include/cosk.h documents; ``meta`` a ``StreamMeta``."""
+
+
 class AttributeDict(dict):
     __getattr__ = dict.__getitem__
     __setattr__ = dict.__setitem__
@@ -396,6 +405,81 @@ class _CoBase(nn.Module):
         """Zero every ring, delay line, pooling window and counter (models/base.py:150,175)."""
         if self._engine is not None and self._engine.n_streams is not None:
             self._engine.check(self._engine.lib.cosk_reset(self._engine.h), "cosk_reset")
+
+    # -- per-stream state (a serving extension: the reference only resets all streams at once) ---------------------
+    def _stream_engine(self, what):
+        e = self._engine
+        if e is None or e.n_streams is None or self._shape is None:
+            raise CoskError(f"{what}: the model holds no stream state yet (step it first)")
+        return e
+
+    @staticmethod
+    def _index_array(indices):
+        idx = np.ascontiguousarray(np.asarray(indices, dtype=np.int64).reshape(-1))
+        return idx, idx.ctypes.data_as(ctypes.POINTER(ctypes.c_int64))
+
+    @staticmethod
+    def _device_stream(e):
+        return ctypes.c_void_p(torch.cuda.current_stream(e.device).cuda_stream)
+
+    def schedule_compatible(self, frame_a, frame_b):
+        """True iff the emission schedule continues identically from frame counts ``frame_a`` and ``frame_b``
+        (cosk_schedule_compatible; host only): the frames between which ``import_streams`` accepts a payload."""
+        rc = _lib.load_library().cosk_schedule_compatible(ctypes.byref(self._config()), int(frame_a), int(frame_b))
+        if rc < 0:
+            raise CoskError(f"cosk_schedule_compatible failed ({rc})")
+        return rc == 1
+
+    def frame_count(self):
+        """Frames pushed since the state was last reset as a whole."""
+        return int(self._engine.lib.cosk_frame_count(self._engine.h)) if self._engine else 0
+
+    def stream_bytes(self):
+        """Bytes of one stream's exported state."""
+        e = self._sync(torch.device("cuda", torch.cuda.current_device()) if self._engine is None else self._engine.device)
+        return int(e.lib.cosk_stream_bytes(e.h))
+
+    def reset_streams(self, indices):
+        """Zero the state of the listed streams, as ``clean_state`` would, leaving every other stream and the shared
+        frame counter alone.  The streams predict on the shared schedule at once, from zero history."""
+        e = self._stream_engine("reset_streams")
+        idx, p = self._index_array(indices)
+        e.check(e.lib.cosk_reset_streams(e.h, p, idx.size, self._device_stream(e)), "cosk_reset_streams")
+
+    def export_streams(self, indices):
+        """The state of the listed streams as a ``StreamState`` (one payload row per index, in order)."""
+        e = self._stream_engine("export_streams")
+        idx, p = self._index_array(indices)
+        payload = torch.empty((idx.size, int(e.lib.cosk_stream_bytes(e.h))), dtype=torch.uint8, device=e.device)
+        meta = _lib.StreamMeta()
+        e.check(e.lib.cosk_export_streams(e.h, p, idx.size, ctypes.c_void_p(payload.data_ptr()), ctypes.byref(meta),
+                                          self._device_stream(e)), "cosk_export_streams")
+        return StreamState(payload, StreamMeta(int(meta.abi_version), int(meta.geometry), int(meta.frame)))
+
+    def import_streams(self, indices, state):
+        """Overwrite the state of the listed streams with the rows of ``state`` (from ``export_streams`` of a model with the
+        same geometry at a compatible frame count, see ``schedule_compatible``; any device).  Raises ``CoskError`` and
+        leaves the state untouched otherwise."""
+        e = self._stream_engine("import_streams")
+        idx, p = self._index_array(indices)
+        payload = state.payload
+        if payload.dtype != torch.uint8 or payload.dim() != 2 or payload.shape[0] != idx.size or \
+                payload.shape[1] != int(e.lib.cosk_stream_bytes(e.h)):
+            raise CoskError(f"import_streams: payload of shape {tuple(payload.shape)} for {idx.size} streams")
+        payload = payload.to(e.device).contiguous()
+        meta = _lib.StreamMeta(*state.meta)
+        e.check(e.lib.cosk_import_streams(e.h, p, idx.size, ctypes.c_void_p(payload.data_ptr()), ctypes.byref(meta),
+                                          self._device_stream(e)), "cosk_import_streams")
+
+    def resize_streams(self, keep):
+        """Change the number of streams to ``len(keep)`` without a reset: new stream j continues old stream ``keep[j]``,
+        or starts from zero state where ``keep[j]`` is -1.  The next ``forward_step`` / ``forward_steps`` with
+        ``len(keep)`` streams continues on the shared schedule.  Peak device memory: the state of both stream counts."""
+        e = self._stream_engine("resize_streams")
+        idx, p = self._index_array(keep)
+        e.check(e.lib.cosk_resize_batch(e.h, idx.size, p), "cosk_resize_batch")
+        e.n_streams = int(idx.size)
+        self._shape = (int(idx.size),) + tuple(self._shape[1:])
 
     def _pick_time_chunk(self, n_streams, frames):
         """Frames per launch of forward_steps (cosk_set_batch_ex).  ``time_chunk`` > 0 is taken as given; auto (-1): the whole

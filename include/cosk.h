@@ -150,8 +150,56 @@ int cosk_last_schedule(const cosk_model *m, int32_t *flags, int32_t n);
 /* Host-only: the emission schedule of T consecutive frames from a fresh state, without touching a device
  * (same integer bookkeeping cosk_step uses).  flags is [T][n_blocks + 1], laid out like cosk_last_schedule. */
 int cosk_simulate_schedule(const cosk_config *cfg, int32_t T, int32_t *flags);
+/* Host-only: 1 iff the emission bookkeeping started from frame count frame_a and from frame_b gives identical flags on
+ * every later frame, else 0 (negative: bad argument).  In practice: the counts are equal, or both are past the warm-up
+ * after which the schedule repeats and they are congruent modulo the product of the block strides (the model's stride:
+ * 4 for CoST-GCN, 1 for CoST-GCN*).  cosk_import_streams accepts a payload only between compatible frame counts. */
+int cosk_schedule_compatible(const cosk_config *cfg, int64_t frame_a, int64_t frame_b);
 /* frames pushed since the last reset */
 int64_t cosk_frame_count(const cosk_model *m);
+
+/* ---- per-stream state: a serving extension without counterpart in the reference ----------------------------------
+ * All streams of a handle share one frame counter and one emission schedule; these calls act on the state of chosen
+ * streams and never on the counters.  Index arrays are host memory of n int64 stream indices, checked on the host: an
+ * index out of range, or an index that repeats within one call, returns COSK_ERR_ARG and launches nothing.  n = 0 is a
+ * no-op.  Reset, export and import are one kernel launch each, asynchronous on `stream`, and never synchronise the host;
+ * the indices reach the device through a handle-owned buffer.  Every call returns COSK_ERR_STATE before cosk_set_batch
+ * and on a handle that has latched a failure (see cosk_step).
+ *
+ * Payload of one stream (cosk_stream_bytes bytes; rows of n streams are stored back to back).  Rings are stored in age
+ * order, newest entry first, and hold only the entries a later step can read, so the payload is the same for every
+ * time_chunk, stream count and tile position:
+ *   input ring        4 entries (the delayed residual x_{n-4} of block 0) if block 0 has a residual, else none
+ *   per block i:
+ *     temporal ring   the 8 history taps of its 9-tap conv
+ *     output ring     4 entries if block i+1 has a residual (its x_{n-4}), else 1 (the newest, cosk_read_block's rows)
+ *   pooling window    with a head: pool_size entries of [c_last] fp32, then the fp64 running window sum [c_last]
+ * A bf16 ring entry is its hi plane, then its lo plane, each [S*V tokens][round_up(c, 8)] bf16 (token s*V + v).  The
+ * values are the raw planes, so export followed by import is bit-exact. */
+typedef struct {
+  int32_t abi_version; /* COSK_ABI_VERSION of the exporting library */
+  uint64_t geometry;   /* fingerprint of every cosk_config field that shapes the payload or the meaning of its entries */
+  int64_t frame;       /* the exporter's cosk_frame_count */
+} cosk_stream_meta;
+/* payload bytes per stream (valid before cosk_set_batch) */
+int64_t cosk_stream_bytes(const cosk_model *m);
+/* The listed streams' state becomes what cosk_reset leaves: zero rings and pooling window.  The counters stay, so the
+ * streams predict on the handle's schedule at once, from zero history. */
+int cosk_reset_streams(cosk_model *m, const int64_t *idx, int64_t n, void *stream);
+/* Payload row q of dst_dev (device memory, n * cosk_stream_bytes bytes) := state of stream idx[q]; *meta describes it. */
+int cosk_export_streams(cosk_model *m, const int64_t *idx, int64_t n, void *dst_dev, cosk_stream_meta *meta, void *stream);
+/* State of stream idx[q] := payload row q of src_dev (device memory of this handle's device).  Refused with COSK_ERR_STATE,
+ * the handle untouched, when meta's abi_version or geometry differ from this handle's, or when
+ * cosk_schedule_compatible(cfg, meta->frame, cosk_frame_count) is 0.  Weights are not checked: a payload moved between
+ * handles with different weights continues with this handle's weights. */
+int cosk_import_streams(cosk_model *m, const int64_t *idx, int64_t n, const void *src_dev, const cosk_stream_meta *meta,
+                        void *stream);
+/* Changes the stream count to n_streams without cosk_set_batch's reset: new stream j takes old stream src[j]'s state
+ * (src[j] = -1: zero state, as cosk_reset_streams leaves it).  src is host memory of n_streams entries; sources may
+ * repeat.  The counters and the time chunk stay.  The new buffers are allocated and filled before the old ones are
+ * freed, so the peak device memory is the state of both stream counts (cosk_state_bytes before + after); if an
+ * allocation fails the handle stays exactly as it was.  Synchronises the device. */
+int cosk_resize_batch(cosk_model *m, int64_t n_streams, const int64_t *src);
 /* last emitted output of block i as fp32 (N*S, cout, V) into dst_dev (debug / feature taps) */
 int cosk_read_block(cosk_model *m, int32_t block, float *dst_dev, void *stream);
 /* kernels launched by this handle since creation */
