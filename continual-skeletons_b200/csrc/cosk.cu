@@ -56,7 +56,7 @@ struct ActBuf {  // token-major split-bf16 activation ring: [slots][plane hi/lo]
   long long slot_elems() const { return 2 * t_alloc * cs; }
 };
 
-// Which kernels serve a block.  prepare() decides it once per block; the launchers, the time-batched walk,
+// Which kernels serve a block.  prepare() decides it once per block; the launchers, the walk's batched_ok,
 // cosk_describe and cosk_block_uses_tensor_cores only read it.
 enum class GcnRoute : uint8_t {
   kSimt,       // k_gcn_simt
@@ -77,7 +77,7 @@ struct Route {
   AttnRoute attn = AttnRoute::kNone;
   bool sa_out_tc = false;  // self-attention unit: output conv on the single-tap k_tc_tcn, else k_tcn_simt
   bool tcn_tc = false;     // temporal conv on k_tc_tcn / k_tc_tcn2 (tcn_on_pair), else k_tcn_simt
-  bool block64 = false;    // the per-step walk runs graph conv + temporal conv as ONE kernel (k_tc_block64)
+  bool block64 = false;    // a frame-by-frame walk runs graph conv + temporal conv as ONE kernel (k_tc_block64)
   bool gcn_tc() const {
     return gcn == GcnRoute::kTc || gcn == GcnRoute::kTcT || gcn == GcnRoute::kTcAgcn || gcn == GcnRoute::kTcAgcnt;
   }
@@ -164,7 +164,7 @@ struct cosk_model {
   long long pool_n = 0, frame = 0;
   std::vector<int32_t> last_flags;
   unsigned int *d_dbg = nullptr;
-  unsigned int *h_dbg = nullptr;  // pinned copy of d_dbg, refreshed asynchronously after every emitting step
+  unsigned int *h_dbg = nullptr;  // pinned copy of d_dbg, refreshed asynchronously after every call that emitted
   bool failed = false;            // a step stopped half way or the device watchdog fired: only cosk_reset / cosk_set_batch clear it
   unsigned long long *d_trace = nullptr;  // phase timers of the graph-conv kernel (COSK_TRACE=1)
   int64_t launches = 0;
@@ -1410,15 +1410,23 @@ int read_block(cosk_model *m, const ActBuf &o, int slot, float *dst, cudaStream_
   return COSK_OK;
 }
 
-// ---- the integer schedule (shared by the device path and cosk_simulate_schedule) -------------------
-// co.Conv2d step semantics: the n-th input (0-based) of a 9-tap temporal conv with padding p and
-// stride s produces an output iff n >= 8 - p and (n - (8 - p)) % s == 0   (SURVEY.md section 3.3).
-inline bool tcn_fires(long long n, int padding, int stride) {
-  const int first = (kTaps - 1) - padding;
-  return n >= first && (n - first) % stride == 0;
+// ---- the integer schedule: one firing rule for the walk, cosk_simulate_schedule and cosk_schedule_compatible ----------
+// co.Conv2d step semantics: the n-th input (0-based) of a 9-tap temporal conv with padding p and stride s produces an output
+// iff n >= 8 - p and (n - (8 - p)) % s == 0   (SURVEY.md section 3.3).  Among the inputs n0 .. n0+F-1 of such a conv,
+// `first` is the first firing input at or after n0 (it may lie past the range) and `count` how many of them fire.
+struct Firing {
+  long long first, count;
+};
+Firing firing(int padding, int stride, long long n0, long long F) {
+  const int p0 = (kTaps - 1) - padding;  // first firing input of the stream
+  const long long nf = n0 < p0 ? p0 : n0 + ((p0 - n0) % stride + stride) % stride;
+  return {nf, nf <= n0 + F - 1 ? (n0 + F - 1 - nf) / stride + 1 : 0};
 }
-// co.AvgPool1d(P, stride 1, padding pp): the m-th pooled vector yields logits iff m >= P - 1 - pp.
-inline bool head_fires(long long m_, int pool_size, int pool_padding) { return m_ >= (long long)pool_size - 1 - pool_padding; }
+// co.AvgPool1d(P, stride 1, padding pp): the m-th pooled vector yields logits iff m >= P - 1 - pp.  Of F vectors entering the
+// window from the pool_n-th on, how many come before the first logits.
+long long head_skip(const cosk_config &c, long long pool_n, long long F) {
+  return std::min(std::max((long long)c.pool_size - 1 - c.pool_padding - pool_n, 0LL), F);
+}
 
 // One frame of the emission bookkeeping from counters n_in (per block) and pool_n: advances them, writes n_blocks + 1 flags
 // laid out like cosk_last_schedule.
@@ -1427,26 +1435,20 @@ void schedule_frame(const cosk_config &c, long long *n_in, long long *pool_n, in
   for (int i = 0; i < c.n_blocks; ++i) {
     flags[i] = 0;
     if (!alive) continue;
-    const bool fire = tcn_fires(n_in[i], c.padding, c.blocks[i].stride);
-    n_in[i]++;
-    alive = fire;
-    flags[i] = fire ? 1 : 0;
+    alive = firing(c.padding, c.blocks[i].stride, n_in[i]++, 1).count > 0;
+    flags[i] = alive ? 1 : 0;
   }
   int emit = 0;
-  if (alive) {
-    if (c.classes > 0) emit = head_fires((*pool_n)++, c.pool_size, c.pool_padding) ? 1 : 0;
-    else emit = 1;
-  }
+  if (alive) emit = c.classes > 0 ? head_skip(c, (*pool_n)++, 1) == 0 : 1;
   flags[c.n_blocks] = emit;
 }
 
-// The counters schedule_frame reaches after `frames` frames from zero, in closed form.
+// The counters schedule_frame reaches after `frames` frames from zero.
 void counters_at(const cosk_config &c, long long frames, long long *n_in, long long *pool_n) {
-  const int first = (kTaps - 1) - c.padding;
   long long n = frames;
   for (int i = 0; i < c.n_blocks; ++i) {
     n_in[i] = n;
-    n = n > first ? (n - 1 - first) / c.blocks[i].stride + 1 : 0;  // firing inputs among 0 .. n-1
+    n = firing(c.padding, c.blocks[i].stride, 0, n).count;
   }
   *pool_n = c.classes > 0 ? n : 0;
 }
@@ -1454,82 +1456,13 @@ void counters_at(const cosk_config &c, long long frames, long long *n_in, long l
 // Every block has reached its first firing input and the pooling window its first emission: the schedule is periodic.
 bool past_warmup(const cosk_config &c, const long long *n_in, long long pool_n) {
   for (int i = 0; i < c.n_blocks; ++i)
-    if (n_in[i] < (kTaps - 1) - c.padding) return false;
-  return c.classes <= 0 || head_fires(pool_n, c.pool_size, c.pool_padding);
+    if (n_in[i] < firing(c.padding, c.blocks[i].stride, 0, 0).first) return false;
+  return c.classes <= 0 || head_skip(c, pool_n, 1) == 0;
 }
 
-// One step of the stack.  `enter` = 0: a new input frame x enters at the first block (cosk_step).  End-of-sequence flush
-// (forward_steps(pad_end=True) of the library: every temporal module is fed its own end padding once the clip is over,
-// module by module): `enter` = i in [0, n_blocks) pushes one ZERO frame into the temporal conv of block i (not through its
-// graph conv: co.forward_stepping modules have no padding), `enter` = n_blocks pushes one zero vector into the pooling
-// window; whatever that emits propagates through the later stages exactly like a regular step.
-int step_impl(cosk_model *m, const float *x, long long nc_stride, float *out, int32_t *emitted, cudaStream_t s, int enter = 0,
-              bool flush = false) {
-  const cosk_config &c = m->cfg;
-  int rc;
-  // input frame -> token rows (data_bn folded in)
-  if ((rc = prof_mark(m, 0, -1, s))) return rc;
-  if (!flush && (rc = run_input(m, x, nc_stride, 0, 1, ring_walk(m->frame, 1, m->Ro), s))) return rc;
-  const ActBuf *in = &m->xin;
-  bool alive = true;
-  const bool head_flush = flush && enter >= c.n_blocks;
-  for (int i = 0; i < c.n_blocks; ++i) {
-    m->last_flags[i] = 0;
-    if (flush && (i < enter || head_flush)) {  // stages before the flushed one are over
-      in = &m->blk[i].out;
-      continue;
-    }
-    if (!alive) continue;
-    BlockW &b = m->blk[i];
-    const cosk_block_cfg &bc = c.blocks[i];
-    const long long n = b.n_in;  // index of this input == index of the predecessor's emission
-    const int in_slot = (int)(n % m->Ro);
-    const bool fire = tcn_fires(n, c.padding, bc.stride);
-    const bool zero_in = flush && i == enter;  // a zero frame enters the temporal conv directly
-    const bool fused = b.route.block64 && in->has_map && !zero_in;
-    if (zero_in) {
-      const int rs = (int)(n % m->R);
-      CK(cudaMemsetAsync(b.ring.hi(rs), 0, (size_t)2 * b.ring.t_alloc * b.ring.cs * sizeof(__nv_bfloat16), s));
-    } else if (fused) {
-      const int res_slot = fire ? (int)((n - kResDelay) % m->Ro) : 0;
-      if ((rc = run_block64(m, i, *in, in_slot, n, fire, res_slot, (int)(b.n_out % m->Ro), s))) return rc;
-      if (fire) b.n_out++;
-    } else if ((rc = run_gcn(m, i, *in, 1, ring_walk(n, 1, m->Ro), ring_walk(n, 1, m->R), s))) {
-      return rc;
-    }
-    if (fire && !fused) {  // n >= first >= 4
-      if ((rc = run_tcn(m, i, *in, n, 1, ring_walk(n - kResDelay, 1, m->Ro), ring_walk(b.n_out, 1, m->Ro), s))) return rc;
-      b.n_out++;
-    }
-    b.n_in++;
-    alive = fire;
-    m->last_flags[i] = fire ? 1 : 0;
-    in = &b.out;
-  }
-  int emit = 0;
-  if (head_flush && c.classes == 0) alive = false;  // nothing to flush without a pooling window
-  if (alive) {
-    const BlockW &last = m->blk[c.n_blocks - 1];
-    const int slot = (int)(((last.n_out > 0 ? last.n_out : 1) - 1) % m->Ro);
-    if (c.classes > 0) {
-      emit = head_fires(m->pool_n, c.pool_size, c.pool_padding) ? 1 : 0;
-      if ((rc = run_head(m, 1, ring_walk(slot, 1, m->Ro), head_flush, emit, 0, out, 0, s))) return rc;
-    } else {
-      emit = 1;
-      if ((rc = read_block(m, last.out, slot, out, s))) return rc;
-    }
-  }
-  if ((rc = prof_mark(m, -1, -1, s))) return rc;  // closes the last interval of this step
-  m->last_flags[c.n_blocks] = emit;
-  if (!flush) m->frame++;
-  if (emitted) *emitted = emit;
-  return COSK_OK;
-}
-
-// ---- time-batched stepping (cosk_steps with a time chunk > 1) ------------------------------------------------------
-// The stack is walked module by module over a chunk of F0 <= tchunk frames, one launch per kernel and chunk; the work items
-// of a launch are (frame, tile) pairs and every frame's ring slots follow from a RingWalk.  Available when every block runs
-// on the tensor-core CoST-GCN kernels (k_tc_gcn or k_tc_gcnt, k_gcn_small for the first layer, k_tc_tcn / k_tc_tcn2).
+// ---- the walk over the stack (cosk_step, cosk_steps) ---------------------------------------------------------------
+// Time-batched chunks (cosk_steps with a time chunk > 1) are available when every block runs on the tensor-core CoST-GCN
+// kernels (k_tc_gcn or k_tc_gcnt, k_gcn_small for the first layer, k_tc_tcn / k_tc_tcn2).
 bool batched_ok(const cosk_model *m) {
   if (m->tchunk <= 1 || m->d_trace) return false;
   for (const BlockW &b : m->blk) {
@@ -1540,54 +1473,78 @@ bool batched_ok(const cosk_model *m) {
   return true;
 }
 
-int steps_chunk(cosk_model *m, const float *x, long long nc_stride, long long x_frame_stride, int F0, float *out, long long out_stride,
-                int32_t max_out, int32_t *cnt, cudaStream_t s) {
+// F0 input frames (frame f at x + f * x_frame_stride) enter the stack, which is walked module by module: every block runs
+// over the F executions its predecessor emitted, one launch per kernel; the work items of a launch are (frame, tile) pairs
+// and every frame's ring slots follow from a RingWalk.  Emission j of the head (or of a headless stack's last block) is
+// written at out + (*cnt + j) * out_stride, and *cnt advances; once max_out are stored, later ones land in the last slot.
+//
+// `frame_by_frame` (F0 == 1): a block routed to k_tc_block64 runs as that one kernel.  Time-batched chunks run it as graph
+// conv + temporal conv launches, a chunk of one frame too: frame n's temporal conv reads the graph-conv outputs of frames
+// n-8 .. n-1, which a launch covering many frames would produce concurrently, and the one kernel rounds differently.
+//
+// End-of-sequence flush (`flush` >= 0; forward_steps(pad_end=True) of the library: every temporal module is fed its own end
+// padding once the clip is over, module by module): no input.  `flush` = i in [0, n_blocks) pushes one ZERO frame into the
+// temporal conv of block i (not through its graph conv: co.forward_stepping modules have no padding), `flush` = n_blocks
+// pushes one zero vector into the pooling window; whatever that emits propagates through the later stages like a regular
+// frame.  The frame counter does not advance.
+int walk(cosk_model *m, const float *x, long long nc_stride, long long x_frame_stride, int F0, bool frame_by_frame, float *out,
+         long long out_stride, int32_t max_out, int32_t *cnt, cudaStream_t s, int flush = -1) {
   const cosk_config &c = m->cfg;
   int rc;
   if ((rc = prof_mark(m, 0, -1, s))) return rc;
-  if ((rc = run_input(m, x, nc_stride, x_frame_stride, F0, ring_walk(m->frame, 1, m->Ro), s))) return rc;
+  if (flush < 0 && (rc = run_input(m, x, nc_stride, x_frame_stride, F0, ring_walk(m->frame, 1, m->Ro), s))) return rc;
   const ActBuf *in = &m->xin;
-  int F = F0;  // executions of the current block in this chunk == emissions of its predecessor
+  int F = flush < 0 ? F0 : 0;  // executions of the current block in this walk == emissions of its predecessor
   for (int i = 0; i < c.n_blocks; ++i) {
     BlockW &b = m->blk[i];
     const cosk_block_cfg &bc = c.blocks[i];
+    const bool zero_in = i == flush;  // the zero frame enters this block's temporal conv directly
+    if (zero_in) F = 1;
     m->last_flags[i] = 0;
     if (F == 0) {
       in = &b.out;
       continue;
     }
-    const long long n0 = b.n_in;
-    const int first = (kTaps - 1) - c.padding;
-    // firing executions among n0 .. n0+F-1: n >= first and (n - first) % stride == 0
-    long long nf = n0 < first ? first : n0 + ((first - n0) % bc.stride + bc.stride) % bc.stride;
-    const int F_out = nf <= n0 + F - 1 ? (int)((n0 + F - 1 - nf) / bc.stride) + 1 : 0;
-    // (The fused block kernel is not used here: frame n's temporal conv reads the graph-conv outputs of frames n-8 .. n-1,
-    // which a launch covering many frames would produce concurrently.  The chunk runs graph conv and temporal conv of such a
-    // block as two launches -- module by module, every frame of the first complete before the second starts.)
-    if ((rc = run_gcn(m, i, *in, F, ring_walk(n0, 1, m->Ro), ring_walk(n0, 1, m->R), s))) return rc;
-    if (F_out > 0 &&
-        (rc = run_tcn(m, i, *in, nf, F_out, ring_walk(nf - kResDelay, bc.stride, m->Ro), ring_walk(b.n_out, 1, m->Ro), s)))
+    const long long n0 = b.n_in;  // index of the first execution == index of the predecessor's emission
+    const Firing fire = firing(c.padding, bc.stride, n0, F);
+    const int F_out = (int)fire.count;
+    const bool fused = frame_by_frame && b.route.block64 && in->has_map && !zero_in;
+    if (zero_in) {
+      const int rs = (int)(n0 % m->R);
+      CK(cudaMemsetAsync(b.ring.hi(rs), 0, (size_t)2 * b.ring.t_alloc * b.ring.cs * sizeof(__nv_bfloat16), s));
+    } else if (fused) {
+      const int res_slot = F_out > 0 ? (int)((n0 - kResDelay) % m->Ro) : 0;
+      if ((rc = run_block64(m, i, *in, (int)(n0 % m->Ro), n0, F_out > 0, res_slot, (int)(b.n_out % m->Ro), s))) return rc;
+    } else if ((rc = run_gcn(m, i, *in, F, ring_walk(n0, 1, m->Ro), ring_walk(n0, 1, m->R), s))) {
       return rc;
-    // did the block fire on the LAST frame of the chunk?  (schedule parity is defined per frame)
-    m->last_flags[i] = (F_out > 0 && nf + (long long)(F_out - 1) * bc.stride == n0 + F - 1) ? 1 : 0;
+    }
+    if (F_out > 0 && !fused &&
+        (rc = run_tcn(m, i, *in, fire.first, F_out, ring_walk(fire.first - kResDelay, bc.stride, m->Ro), ring_walk(b.n_out, 1, m->Ro),
+                      s)))
+      return rc;
+    // did the block fire on its last execution?  (schedule parity is defined per frame)
+    m->last_flags[i] = (F_out > 0 && fire.first + (long long)(F_out - 1) * bc.stride == n0 + F - 1) ? 1 : 0;
     b.n_in += F;
     b.n_out += F_out;
     F = F_out;
     in = &b.out;
   }
-  // head over the F emissions of the last block
+  // head over the F emissions of the last block; a flushed zero vector enters the pooling window alone (a stack without a
+  // head has no window to flush)
+  const bool head_zero = flush == c.n_blocks;
+  if (head_zero) F = c.classes > 0 ? 1 : 0;
   int emit_last = 0;
   if (F > 0) {
     const BlockW &last = m->blk[c.n_blocks - 1];
     const long long o0 = last.n_out - F;  // index of the first of these emissions
     if (c.classes > 0) {
-      const long long first_emit_n = (long long)c.pool_size - 1 - c.pool_padding;
-      const int skip = (int)std::min<long long>(std::max<long long>(first_emit_n - m->pool_n, 0), F);  // frames before the first logits
+      const int skip = (int)head_skip(c, m->pool_n, F);  // frames before the first logits
       const int n_emit = F - skip;
       const int32_t room = *cnt < max_out ? max_out - *cnt : 0;
       float *dst = out + (long long)(*cnt < max_out ? *cnt : max_out - 1) * out_stride;
       // more emissions than room: they all land in the last slot
-      if ((rc = run_head(m, F, ring_walk(o0, 1, m->Ro), false, F == 1 ? n_emit : 0, skip, dst, n_emit <= room ? out_stride : 0, s)))
+      if ((rc = run_head(m, F, ring_walk(o0, 1, m->Ro), head_zero, F == 1 ? n_emit : 0, skip, dst, n_emit <= room ? out_stride : 0,
+                         s)))
         return rc;
       *cnt += n_emit;
       emit_last = n_emit > 0 ? 1 : 0;
@@ -1600,10 +1557,22 @@ int steps_chunk(cosk_model *m, const float *x, long long nc_stride, long long x_
       emit_last = 1;
     }
   }
-  if ((rc = prof_mark(m, -1, -1, s))) return rc;
+  if ((rc = prof_mark(m, -1, -1, s))) return rc;  // closes the last interval of this walk
   m->last_flags[c.n_blocks] = (emit_last && m->last_flags[c.n_blocks - 1]) ? 1 : 0;
-  m->frame += F0;
+  if (flush < 0) m->frame += F0;
   return COSK_OK;
+}
+
+// The end of a stepping call's walks.  A walk that stopped half way leaves the counters partly advanced: the failure latch
+// refuses further steps.  Otherwise, if anything emitted, the watchdog word is copied to pinned memory behind the call's
+// kernels, without a host sync, for step_entry of the next call to look at.  The device word only goes from 0 to a code
+// until a reset, so one copy per call sees what a copy behind every emitting frame would.
+int end_walks(cosk_model *m, int rc, int32_t cnt, cudaStream_t s) {
+  if (!rc && cnt > 0 && m->h_dbg &&
+      cudaMemcpyAsync(m->h_dbg, m->d_dbg, sizeof(unsigned int), cudaMemcpyDeviceToHost, s) != cudaSuccess)
+    rc = fail(m, COSK_ERR_CUDA, "cudaMemcpyAsync of the watchdog word failed");
+  if (rc) m->failed = true;
+  return rc;
 }
 
 // cosk_describe's name of the kernels that serve a block's graph conv (the adaptive one: attention half + mix)
@@ -1892,7 +1861,7 @@ int cosk_reset(cosk_model *m) {
 static int step_entry(cosk_model *m, const char *what = "step") {
   if (m->n_streams == 0) return fail(m, COSK_ERR_STATE, "%s before cosk_set_batch", what);
   if (!m->prepared) return fail(m, COSK_ERR_STATE, "weights changed after cosk_set_batch: call cosk_set_batch again");
-  if (m->h_dbg && m->h_dbg[0] != 0) m->failed = true;  // written by the async copy behind an earlier emitting step
+  if (m->h_dbg && m->h_dbg[0] != 0) m->failed = true;  // written by the async copy behind an earlier emitting call
   if (m->failed) {
     if (m->h_dbg && m->h_dbg[0] != 0)
       return fail(m, COSK_ERR_STATE, "device pipeline watchdog fired (code 0x%08x): results since then are invalid; cosk_reset to continue",
@@ -1902,32 +1871,16 @@ static int step_entry(cosk_model *m, const char *what = "step") {
   return COSK_OK;
 }
 
-static int step_guarded(cosk_model *m, const float *x, long long nc_stride, float *out, int32_t *emitted, cudaStream_t s, int enter = 0,
-                        bool flush = false) {
-  int32_t em = 0;
-  int rc = step_impl(m, x, nc_stride, out, &em, s, enter, flush);
-  if (rc) {
-    m->failed = true;  // counters may be partly advanced
-    return rc;
-  }
-  if (em && m->h_dbg) {
-    // surface the watchdog word without a host sync: it lands in pinned memory behind this step's kernels and is
-    // looked at on the next call
-    if (cudaMemcpyAsync(m->h_dbg, m->d_dbg, sizeof(unsigned int), cudaMemcpyDeviceToHost, s) != cudaSuccess) {
-      m->failed = true;
-      return fail(m, COSK_ERR_CUDA, "cudaMemcpyAsync of the watchdog word failed");
-    }
-  }
-  if (emitted) *emitted = em;
-  return COSK_OK;
-}
-
 int cosk_step(cosk_model *m, const float *x_dev, int64_t nc_stride, float *out_dev, int32_t *emitted, void *stream) {
   if (!m || !x_dev || !out_dev) return COSK_ERR_ARG;
   int rc = step_entry(m);
   if (rc) return rc;
   DeviceGuard guard_(m->cfg.device);
-  return step_guarded(m, x_dev, nc_stride, out_dev, emitted, (cudaStream_t)stream);
+  int32_t cnt = 0;
+  rc = walk(m, x_dev, nc_stride, 0, 1, true, out_dev, 0, 1, &cnt, (cudaStream_t)stream);
+  if ((rc = end_walks(m, rc, cnt, (cudaStream_t)stream))) return rc;
+  if (emitted) *emitted = cnt;
+  return COSK_OK;
 }
 
 int cosk_steps(cosk_model *m, const float *x_dev, int32_t T, float *out_dev, int64_t out_stride, int32_t max_out,
@@ -1941,52 +1894,30 @@ int cosk_steps_ex(cosk_model *m, const float *x_dev, int32_t T, float *out_dev, 
   int rc = step_entry(m);
   if (rc) return rc;
   DeviceGuard guard_(m->cfg.device);
+  const cudaStream_t s = (cudaStream_t)stream;
   const long long frame_elems = (long long)m->cfg.vertices * m->cfg.persons;
+  // chunks of up to tchunk frames, one launch per kernel and chunk; frame by frame on stacks the chunks cannot take
+  const bool batched = batched_ok(m);
+  const int chunk = batched ? m->tchunk : 1;
   int32_t cnt = 0;
-  int t_start = 0;
-  if (batched_ok(m)) {
-    // module by module over chunks of up to tchunk frames, one launch per kernel and chunk
-    for (int t0 = 0; t0 < T; t0 += m->tchunk) {
-      const int F0 = std::min(m->tchunk, T - t0);
-      rc = steps_chunk(m, x_dev + t0 * frame_elems, (long long)T * frame_elems, frame_elems, F0, out_dev, out_stride, max_out, &cnt,
-                       (cudaStream_t)stream);
-      if (rc) {
-        m->failed = true;
-        return rc;
-      }
-    }
-    if (cnt > 0 && m->h_dbg) cudaMemcpyAsync(m->h_dbg, m->d_dbg, sizeof(unsigned int), cudaMemcpyDeviceToHost, (cudaStream_t)stream);
-    t_start = T;
-  }
-  for (int t = t_start; t < T; ++t) {
-    int32_t em = 0;
-    // once max_out emissions are stored, later ones land in the last slot
-    const int32_t dst = cnt < max_out ? cnt : max_out - 1;
-    rc = step_guarded(m, x_dev + t * frame_elems, (long long)T * frame_elems, out_dev + (long long)dst * out_stride, &em,
-                      (cudaStream_t)stream);
-    if (rc) return rc;
-    cnt += em;
-  }
+  for (int t0 = 0; t0 < T && !rc; t0 += chunk)
+    rc = walk(m, x_dev + t0 * frame_elems, (long long)T * frame_elems, frame_elems, std::min(chunk, T - t0), !batched, out_dev,
+              out_stride, max_out, &cnt, s);
   if (pad_end) {
     // The clip is over: every temporal module flushes its end padding, module by module (first the blocks in order,
     // `padding` zero frames into each temporal conv, then `pool_padding` zero vectors into the pooling window).  What a
     // flush emits runs through the later stages at once (depth first), which yields the same output sequence as the
-    // library's module-by-module order because every stage is a causal sequential machine.
+    // library's module-by-module order because every stage is a causal sequential machine.  Each flush is one frame and
+    // walks frame by frame, whatever the time chunk.
     const int stages = m->cfg.n_blocks + 1;
-    for (int st = 0; st < stages; ++st) {
+    for (int st = 0; st < stages && !rc; ++st) {
       const int reps = st < m->cfg.n_blocks ? m->cfg.padding : (m->cfg.classes > 0 ? m->cfg.pool_padding : 0);
-      for (int z = 0; z < reps; ++z) {
-        int32_t em = 0;
-        const int32_t dst = cnt < max_out ? cnt : max_out - 1;
-        rc = step_guarded(m, nullptr, 0, out_dev + (long long)dst * out_stride, &em, (cudaStream_t)stream, st, true);
-        if (rc) return rc;
-        cnt += em;
-      }
+      for (int z = 0; z < reps && !rc; ++z) rc = walk(m, nullptr, 0, 0, 1, true, out_dev, out_stride, max_out, &cnt, s, st);
     }
-    // the padded frames are not part of the stream: the sequence ends here and the state starts over
-    rc = zero_state(m, (cudaStream_t)stream);
-    if (rc) return rc;
   }
+  if ((rc = end_walks(m, rc, cnt, s))) return rc;
+  // the padded frames are not part of the stream: the sequence ends here and the state starts over
+  if (pad_end && (rc = zero_state(m, s))) return rc;
   if (n_emitted) *n_emitted = cnt;
   return COSK_OK;
 }

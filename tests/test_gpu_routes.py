@@ -11,9 +11,9 @@ wraps the rings -- and checks
 * ``|got - value| <= EPS * mag`` on every emitted frame and element of the checked streams (all of them, or at large
   counts the first and last streams and those on both sides of every wave boundary of the grid);
 * ``forward_steps`` with ``time_chunk=1`` == ``forward_step`` bit for bit, and frame-by-frame == time-batched bit for bit
-  where both walks run the same kernels.  The one-kernel 64 -> 64 block step (k_tc_block64) is only compared within
-  the bound: the time-batched walk runs such a block as graph conv + temporal conv launches, which round differently.
-* a stack the time-batched walk cannot take falls back to stepping (same launch count as stepping).
+  where both run the same kernels.  The one-kernel 64 -> 64 block step (k_tc_block64) is only compared within the
+  bound: time-batched chunks run such a block as graph conv + temporal conv launches, which round differently.
+* a stack time-batched chunks cannot take falls back to stepping (same launch count as stepping).
 
 The table, with the kernels each case launches, lives in tests/route_table.py; tests/test_boundary_cpu.py checks that
 it declares every kernel csrc/cosk.cu can launch.  test_whole_model_signed_input runs the first-layer path with data_bn
