@@ -1575,6 +1575,19 @@ int end_walks(cosk_model *m, int rc, int32_t cnt, cudaStream_t s) {
   return rc;
 }
 
+// F frames of a (N, C, T, V, S) clip through the stack, the first at x (nc_stride = T*V*S): chunks of the time chunk where
+// batched_ok admits them, else frame by frame (cosk_steps, cosk_prime_streams).
+int walk_frames(cosk_model *m, const float *x, long long nc_stride, int F, float *out, long long out_stride, int32_t max_out,
+                int32_t *cnt, cudaStream_t s) {
+  const long long frame_elems = (long long)m->cfg.vertices * m->cfg.persons;
+  const bool batched = batched_ok(m);
+  const int chunk = batched ? m->tchunk : 1;
+  int rc = COSK_OK;
+  for (int t0 = 0; t0 < F && !rc; t0 += chunk)
+    rc = walk(m, x + t0 * frame_elems, nc_stride, frame_elems, std::min(chunk, F - t0), !batched, out, out_stride, max_out, cnt, s);
+  return rc;
+}
+
 // cosk_describe's name of the kernels that serve a block's graph conv (the adaptive one: attention half + mix)
 std::string gcn_name(const BlockW &b) {
   static const char *const attn[] = {"", "k_agcn_attn+", "k_attn_small+", "k_tc_attn+"};  // by AttnRoute
@@ -1895,14 +1908,8 @@ int cosk_steps_ex(cosk_model *m, const float *x_dev, int32_t T, float *out_dev, 
   if (rc) return rc;
   DeviceGuard guard_(m->cfg.device);
   const cudaStream_t s = (cudaStream_t)stream;
-  const long long frame_elems = (long long)m->cfg.vertices * m->cfg.persons;
-  // chunks of up to tchunk frames, one launch per kernel and chunk; frame by frame on stacks the chunks cannot take
-  const bool batched = batched_ok(m);
-  const int chunk = batched ? m->tchunk : 1;
   int32_t cnt = 0;
-  for (int t0 = 0; t0 < T && !rc; t0 += chunk)
-    rc = walk(m, x_dev + t0 * frame_elems, (long long)T * frame_elems, frame_elems, std::min(chunk, T - t0), !batched, out_dev,
-              out_stride, max_out, &cnt, s);
+  rc = walk_frames(m, x_dev, (long long)T * m->cfg.vertices * m->cfg.persons, T, out_dev, out_stride, max_out, &cnt, s);
   if (pad_end) {
     // The clip is over: every temporal module flushes its end padding, module by module (first the blocks in order,
     // `padding` zero frames into each temporal conv, then `pool_padding` zero vectors into the pooling window).  What a
@@ -2133,6 +2140,79 @@ int cosk_resize_batch(cosk_model *m, int64_t n_streams, const int64_t *src) {
   }
   free_set(old);
   return COSK_OK;
+}
+
+int cosk_prime_streams(cosk_model *m, const int64_t *idx, int64_t n, const float *x_dev, int32_t T, int32_t time_chunk,
+                       void *stream) {
+  if (!m) return COSK_ERR_ARG;
+  int rc = step_entry(m, "cosk_prime_streams");
+  if (rc || (rc = check_indices(m, idx, n, 0, m->n_streams, true))) return rc;
+  if (T < 0 || (n > 0 && T > 0 && !x_dev) || time_chunk < 1 || time_chunk > 4096)
+    return fail(m, COSK_ERR_ARG, "cosk_prime_streams: T %d, time_chunk %d", (int)T, (int)time_chunk);
+  if (n == 0) return COSK_OK;
+  DeviceGuard guard_(m->cfg.device);
+  const cudaStream_t s = (cudaStream_t)stream;
+  const int H = (int)std::min<long long>(T, m->frame);  // the handle's streams have not seen further back either
+  if (H == 0) {
+    StateArgs a = state_args(m);
+    if ((rc = launch_stream_state(m, a, kStateZero, nullptr, s))) return rc;
+    CK(cudaDeviceSynchronize());
+    return COSK_OK;
+  }
+  const cosk_config &c = m->cfg;
+  const std::vector<long long> dst = m->h_idx;
+  const HostSide saved = save_host_side(m);
+  const long long stream_bytes = state_args(m).stream_bytes;
+  const size_t out_elems = c.classes > 0 ? (size_t)n * c.classes : (size_t)n * c.persons * c.vertices * c.blocks[c.n_blocks - 1].cout;
+  void *payload = nullptr;
+  float *out = nullptr;
+  uint32_t watchdog = 0;
+  // The n streams walk on a scratch set of their own, rings sized for `time_chunk`, from the counters of frame F - H; the
+  // handle's set waits detached and untouched.
+  StateSet own = detach_state(m);
+  m->tchunk = time_chunk;
+  m->R = (kRingSlots - 1) + time_chunk;
+  m->Ro = (kOutSlots - 1) + time_chunk;
+  rc = alloc_state(m, n);
+  if (!rc) rc = zero_buffers(m, s);
+  if (!rc && (cudaMalloc(&payload, (size_t)n * stream_bytes) != cudaSuccess || cudaMalloc(&out, out_elems * sizeof(float)) != cudaSuccess))
+    rc = fail(m, COSK_ERR_CUDA, "cosk_prime_streams: out of device memory for %lld streams", (long long)n);
+  if (!rc) {
+    set_counters_at(m, saved.frame - H);
+    int32_t cnt = 0;  // emissions all land in the one scratch output row
+    rc = walk_frames(m, x_dev + (long long)(T - H) * c.vertices * c.persons, (long long)T * c.vertices * c.persons, H, out, 0, 1,
+                     &cnt, s);
+  }
+  // The counters are a function of the frame count alone, so the walk ends where the handle stands and the scratch
+  // streams' state fits the handle's schedule.
+  if (!rc && !counters_equal(m, saved)) rc = fail(m, COSK_ERR_STATE, "cosk_prime_streams: walk ended off the handle's counters");
+  if (!rc) {
+    m->h_idx.resize((size_t)n);
+    for (int64_t q = 0; q < n; ++q) m->h_idx[(size_t)q] = q;
+    StateArgs a = state_args(m);
+    rc = launch_stream_state(m, a, kStateGather, payload, s);
+  }
+  if (!rc && cudaMemcpyAsync(m->h_dbg, m->d_dbg, sizeof(unsigned int), cudaMemcpyDeviceToHost, s) != cudaSuccess)
+    rc = fail(m, COSK_ERR_CUDA, "cudaMemcpyAsync of the watchdog word failed");
+  if (!rc && cudaDeviceSynchronize() != cudaSuccess) rc = fail(m, COSK_ERR_CUDA, "cosk_prime_streams: priming walk failed");
+  if (!rc) watchdog = m->h_dbg[0];
+  if (rc) cudaGetLastError();
+  free_state(m);
+  attach_state(m, own);
+  restore_host_side(m, saved);
+  if (!rc && watchdog) {
+    m->failed = true;  // as after any walk: step_entry reports the code
+    rc = fail(m, COSK_ERR_STATE, "device pipeline watchdog fired (code 0x%08x) while priming streams; cosk_reset to continue", watchdog);
+  }
+  if (!rc) {
+    m->h_idx = dst;
+    StateArgs a = state_args(m);
+    rc = launch_stream_state(m, a, kStateScatter, payload, s);
+  }
+  if (!rc && cudaDeviceSynchronize() != cudaSuccess) rc = fail(m, COSK_ERR_CUDA, "cosk_prime_streams: scatter failed");
+  dfree(payload);
+  dfree(out);
+  return rc;
 }
 
 }  // extern "C"

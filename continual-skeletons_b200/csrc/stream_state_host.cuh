@@ -1,5 +1,6 @@
 // Host half of the per-stream state calls (cosk_reset_streams, cosk_export_streams, cosk_import_streams,
-// cosk_resize_batch): the payload layout as a StateArgs table, index checks, and the one k_stream_state launch per call.
+// cosk_resize_batch, cosk_prime_streams): the payload layout as a StateArgs table, index checks, the one k_stream_state
+// launch per call, and the host-side snapshot a priming walk saves and restores.
 // Part of cosk.cu (included after its helpers, whose names it uses); the kernel is in stream_state.cuh.  The step route
 // table of the GPU tests covers the step kernels; k_stream_state is checked by tests/test_gpu_streams.py.
 #pragma once
@@ -96,6 +97,49 @@ int launch_stream_state(cosk_model *m, StateArgs &a, int mode, void *payload, cu
   m->launches++;
   CK(cudaEventRecord(m->ev_idx, s));
   return COSK_OK;
+}
+
+// What of the handle's host side a priming walk (cosk_prime_streams) changes: the counters, the last step's flags and the
+// time chunk with the ring sizes it implies.  The walk runs on a scratch set whose rings are sized for its own chunk.
+struct HostSide {
+  long long frame = 0, pool_n = 0;
+  std::vector<long long> n_in, n_out;
+  std::vector<int32_t> last_flags;
+  int tchunk = 1, R = 0, Ro = 0;
+};
+
+HostSide save_host_side(const cosk_model *m) {
+  HostSide h;
+  h.frame = m->frame, h.pool_n = m->pool_n;
+  for (const BlockW &b : m->blk) h.n_in.push_back(b.n_in), h.n_out.push_back(b.n_out);
+  h.last_flags = m->last_flags;
+  h.tchunk = m->tchunk, h.R = m->R, h.Ro = m->Ro;
+  return h;
+}
+
+void restore_host_side(cosk_model *m, const HostSide &h) {
+  m->frame = h.frame, m->pool_n = h.pool_n;
+  for (size_t i = 0; i < m->blk.size(); ++i) m->blk[i].n_in = h.n_in[i], m->blk[i].n_out = h.n_out[i];
+  m->last_flags = h.last_flags;
+  m->tchunk = h.tchunk, m->R = h.R, m->Ro = h.Ro;
+}
+
+// The counters the walks reach after `frames` frames from zero: counters_at, plus each block's emission count.
+void set_counters_at(cosk_model *m, long long frames) {
+  const cosk_config &c = m->cfg;
+  long long n_in[COSK_MAX_BLOCKS];
+  counters_at(c, frames, n_in, &m->pool_n);
+  for (int i = 0; i < c.n_blocks; ++i) {
+    m->blk[i].n_in = n_in[i];
+    m->blk[i].n_out = firing(c.padding, c.blocks[i].stride, 0, n_in[i]).count;
+  }
+  m->frame = frames;
+}
+
+bool counters_equal(const cosk_model *m, const HostSide &h) {
+  for (size_t i = 0; i < m->blk.size(); ++i)
+    if (m->blk[i].n_in != h.n_in[i] || m->blk[i].n_out != h.n_out[i]) return false;
+  return m->frame == h.frame && m->pool_n == h.pool_n;
 }
 
 // Fingerprint of every config field that shapes the payload or the meaning of its entries (FNV-1a).

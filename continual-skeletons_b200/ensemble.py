@@ -53,6 +53,15 @@ class MultiStream:
         for m in self.models:
             m.resize_streams(keep)
 
+    def prime_streams(self, indices, clips):
+        """``prime_streams`` on every member, member i from ``clips[i]`` (its modality of the same frames), so the members
+        stay in lock step."""
+        clips = list(clips)
+        if len(clips) != len(self.models):
+            raise ValueError(f"expected {len(self.models)} clips, got {len(clips)}")
+        for m, clip in zip(self.models, clips):
+            m.prime_streams(indices, clip)
+
     def forward_step(self, inputs):
         """inputs: one (N, C, V, S) CUDA tensor per member model.  Fused logits, or None when no prediction is due."""
         inputs = list(inputs)

@@ -119,6 +119,7 @@ SYMBOLS = {
     "cosk_export_streams": (ctypes.c_int, [_P, ctypes.POINTER(ctypes.c_int64), ctypes.c_int64, _P, ctypes.POINTER(StreamMeta), _P]),
     "cosk_import_streams": (ctypes.c_int, [_P, ctypes.POINTER(ctypes.c_int64), ctypes.c_int64, _P, ctypes.POINTER(StreamMeta), _P]),
     "cosk_resize_batch": (ctypes.c_int, [_P, ctypes.c_int64, ctypes.POINTER(ctypes.c_int64)]),
+    "cosk_prime_streams": (ctypes.c_int, [_P, ctypes.POINTER(ctypes.c_int64), ctypes.c_int64, _P, ctypes.c_int32, ctypes.c_int32, _P]),
     "cosk_read_block": (ctypes.c_int, [_P, ctypes.c_int32, _P, _P]),
     "cosk_launch_count": (ctypes.c_int64, [_P]),
     "cosk_block_uses_tensor_cores": (ctypes.c_int, [_P, ctypes.c_int32]),

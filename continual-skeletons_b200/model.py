@@ -481,6 +481,29 @@ class _CoBase(nn.Module):
         e.n_streams = int(idx.size)
         self._shape = (int(idx.size),) + tuple(self._shape[1:])
 
+    def prime_streams(self, indices, clip):
+        """Give the listed streams the state their recent frames leave.  ``clip``: (k, C, H, V, S) -- (k, C, H, V) for
+        ``CoStack`` -- on the model's device, row j the history of stream ``indices[j]``, frame H - 1 the newest (the
+        frame the other streams received last).  With F = ``frame_count()`` and H' = min(H, F), each stream ends as if
+        ``reset_streams`` had been called at frame F - H' and it had then received the last H' frames of its row; older
+        frames are ignored.  With H' >= ``receptive_field`` the stream equals one that received those frames here all
+        along.  Every other stream, the frame count and the schedule stay as they were.  The frames are walked in chunks
+        of ``_pick_time_chunk(k, H)``.  Synchronises the device; peak memory: the state of k streams at that chunk plus
+        k * ``stream_bytes()`` on top of the model's own state."""
+        e = self._stream_engine("prime_streams")
+        idx, p = self._index_array(indices)
+        want = (idx.size, self._shape[1], None) + tuple(self._shape[2:])
+        if not isinstance(clip, torch.Tensor) or clip.dim() != len(want) or \
+                any(w is not None and g != w for g, w in zip(clip.shape, want)):
+            raise CoskError(f"prime_streams: clip of shape {tuple(getattr(clip, 'shape', ()))} for {idx.size} streams, "
+                            f"expected {tuple('H' if w is None else w for w in want)}")
+        if clip.device != e.device:
+            raise CoskError(f"prime_streams: clip on {clip.device}, the model steps on {e.device}")
+        x = self._check_input(clip, len(want))
+        H = int(x.shape[2])
+        e.check(e.lib.cosk_prime_streams(e.h, p, idx.size, ctypes.c_void_p(x.data_ptr()), H,
+                                         self._pick_time_chunk(idx.size, H), self._stream(x)), "cosk_prime_streams")
+
     def _pick_time_chunk(self, n_streams, frames):
         """Frames per launch of forward_steps (cosk_set_batch_ex).  ``time_chunk`` > 0 is taken as given; auto (-1): the whole
         call in one chunk when the extra ring slots fit a budget (a quarter of the free device memory, at most 8 GiB), else

@@ -200,6 +200,22 @@ int cosk_import_streams(cosk_model *m, const int64_t *idx, int64_t n, const void
  * freed, so the peak device memory is the state of both stream counts (cosk_state_bytes before + after); if an
  * allocation fails the handle stays exactly as it was.  Synchronises the device. */
 int cosk_resize_batch(cosk_model *m, int64_t n_streams, const int64_t *src);
+/* Primes joining streams from their recent frames.  x_dev: (n, C, T, V, S) contiguous fp32 device memory, row q the
+ * history of stream idx[q], frame T-1 the newest (the one the other streams received at cosk_frame_count - 1).  With
+ * F = cosk_frame_count and H = min(T, F), stream idx[q] ends with exactly the state it would have if cosk_reset_streams
+ * had been called at frame F - H and the stream had then received frames T-H .. T-1 of its row; the oldest T - H frames
+ * are ignored (the handle's streams have not seen further back either), and T = 0 is cosk_reset_streams.  With
+ * H >= the receptive field a primed stream equals a stream that received those frames in the handle all along.  The
+ * frames are walked as cosk_steps walks a clip on a handle of n streams with time chunk `time_chunk` (1: as cosk_step
+ * walks them), on scratch state of their own, which is then gathered into a payload and scattered into idx.  Every
+ * other stream's state, the counters, cosk_last_schedule's flags and the time chunk stay as they were; the primed
+ * streams emit on the handle's schedule.  Refused (COSK_ERR_ARG / COSK_ERR_STATE / COSK_ERR_CUDA) with the handle
+ * untouched on the index checks above, before cosk_set_batch, on a latched handle and when an allocation fails; a
+ * pipeline watchdog firing during the walk latches the handle as a step would.  Peak device memory: the handle's
+ * state, plus the state of n streams at time_chunk (as cosk_set_batch_ex(n, time_chunk) allocates), plus
+ * n * cosk_stream_bytes, plus one output row of n streams.  Synchronises the device. */
+int cosk_prime_streams(cosk_model *m, const int64_t *idx, int64_t n, const float *x_dev, int32_t T, int32_t time_chunk,
+                       void *stream);
 /* last emitted output of block i as fp32 (N*S, cout, V) into dst_dev (debug / feature taps) */
 int cosk_read_block(cosk_model *m, int32_t block, float *dst_dev, void *stream);
 /* kernels launched by this handle since creation */
