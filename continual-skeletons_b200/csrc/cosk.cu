@@ -96,13 +96,9 @@ struct BlockW {
   float *d_sa_scale = nullptr, *d_sa_shift = nullptr, *d_sa_qkv_w = nullptr, *d_sa_qkv_b = nullptr, *d_res_w_sa = nullptr;
   __nv_bfloat16 *d_sa_w16 = nullptr;  // output conv (+ identity K-block) for the single-tap tcgen05 launch
   CUtensorMap map_sa_w, map_sa_w_half;
-  ActBuf sa;  // attention output rows of the frame in flight (1 slot), operand of the output conv
-  // tensor-core qkv conv: normalised input rows; unfused (C = 64), the conv runs on the single-tap temporal-conv kernel
-  // into q | k | v rows zero-padded to kSaQkvCols columns
   __nv_bfloat16 *d_sa_fw16 = nullptr;  // qkv weights regrouped per head group: [items][hi: q, k, v | lo: same][cin]
   float *d_sa_fbias = nullptr;         // [items][96]
   CUtensorMap map_sa_fw;
-  ActBuf sa_x, sa_q;
   __nv_bfloat16 *d_sa_qw16 = nullptr;  // unfused qkv conv: [2*kSaQkvCols rows (hi, lo)][cin]
   float *d_sa_qbias = nullptr;
   CUtensorMap map_sa_q;
@@ -122,8 +118,44 @@ struct BlockW {
   __nv_bfloat16 *d_gcnt_w16 = nullptr;
   CUtensorMap map_gcnt_w;
   float gcnt_coef[3][32];
-  long long n_in = 0, n_out = 0;
-  ActBuf ring, out;
+};
+
+// The emission bookkeeping of a batch: frames entered, per block executions (n_in) and emissions (n_out), and vectors
+// entered into the pooling window.  A function of the frame count alone (counters_at).
+struct Counters {
+  long long frame = 0, pool_n = 0;
+  long long n_in[COSK_MAX_BLOCKS] = {}, n_out[COSK_MAX_BLOCKS] = {};
+};
+
+// A block's buffers in a batch (which of them are state and which scratch of the frame in flight: stream_state.cuh).
+struct BlockBufs {
+  ActBuf ring, out;  // temporal ring, block-output ring
+  ActBuf sa;         // self-attention unit: attention rows of the frame in flight (1 slot), operand of the output conv
+  // tensor-core qkv conv: normalised input rows; unfused (C = 64), the conv runs on the single-tap temporal-conv kernel
+  // into q | k | v rows zero-padded to kSaQkvCols columns
+  ActBuf sa_x, sa_q;
+};
+
+// The streams a handle steps: their geometry, ring sizes, buffers and counters.  alloc_batch builds one and free_batch
+// frees it; whatever runs on state is handed the batch it runs on.  n_streams == 0: no batch (geometry and counters zero,
+// ring sizes of time chunk 1, so the payload layout and the schedule can still be read from it).
+struct Batch {
+  long long n_streams = 0, n_tokens = 0, t_alloc = 0;
+  int skel_per_tile = 0, tile_tokens = 0, n_tiles = 0;
+  int dense_vp = 0;
+  int tchunk = 1;  // time chunk: frames of one block processed per launch by cosk_steps (cosk_set_batch_ex)
+  // slots of the temporal rings (8 + tchunk) and of the input / block-output rings (4 + tchunk)
+  int R = kRingSlots, Ro = kOutSlots;
+  ActBuf xin;
+  BlockBufs blk[COSK_MAX_BLOCKS];
+  float *d_pool_ring = nullptr;
+  double *d_pool_sum = nullptr;
+  float *d_qkv = nullptr;      // self-attention unit: q | k | v rows [t_alloc][2*dk + dv] of the frame in flight (fp32)
+  float *d_dense = nullptr;    // adaptive graph conv: per-token mixing rows [t_alloc][3][dense_vp] of the frame in flight
+  long long *d_idx = nullptr;  // [n_streams] stream indices of a per-stream state call (k_stream_state)
+  int64_t state_bytes = 0;
+  Counters cnt;
+  int32_t last_flags[COSK_MAX_BLOCKS + 1] = {};  // cosk_last_schedule
 };
 
 struct ProfRec {
@@ -147,28 +179,14 @@ struct cosk_model {
   std::vector<float> h_bn_scale, h_bn_shift, h_fc_w, h_fc_b;
   float *d_bn_scale = nullptr, *d_bn_shift = nullptr, *d_fc_w = nullptr, *d_fc_b = nullptr;
   bool prepared = false;
-  // state
-  long long n_streams = 0, n_tokens = 0, t_alloc = 0;
-  int tchunk = 1;                    // time chunk: frames of one block processed per launch by cosk_steps (cosk_set_batch_ex)
-  int R = kRingSlots, Ro = kOutSlots;  // slots of the temporal rings (8 + tchunk) and of the input / block-output rings (4 + tchunk)
-  int skel_per_tile = 0, tile_tokens = 0, n_tiles = 0;
-  ActBuf xin;
-  float *d_pool_ring = nullptr;
-  double *d_pool_sum = nullptr;
-  float *d_qkv = nullptr;    // self-attention unit: q | k | v rows [t_alloc][2*dk + dv] of the frame in flight (fp32)
-  float *d_dense = nullptr;  // adaptive graph conv: per-token mixing rows [t_alloc][3][dense_vp] of the frame in flight
-  int dense_vp = 0;
-  long long *d_idx = nullptr;      // [n_streams] stream indices of a per-stream state call (k_stream_state)
-  cudaEvent_t ev_idx = nullptr;    // recorded behind the last such call: the next one's index upload waits for it
+  Batch batch;
+  cudaEvent_t ev_idx = nullptr;    // recorded behind the last per-stream state call: the next one's index upload waits for it
   std::vector<long long> h_idx;    // host copy the index upload reads
-  long long pool_n = 0, frame = 0;
-  std::vector<int32_t> last_flags;
   unsigned int *d_dbg = nullptr;
   unsigned int *h_dbg = nullptr;  // pinned copy of d_dbg, refreshed asynchronously after every call that emitted
   bool failed = false;            // a step stopped half way or the device watchdog fired: only cosk_reset / cosk_set_batch clear it
   unsigned long long *d_trace = nullptr;  // phase timers of the graph-conv kernel (COSK_TRACE=1)
   int64_t launches = 0;
-  int64_t state_bytes = 0;
   // profiling
   bool prof_on = false;
   std::vector<ProfRec> prof;
@@ -216,83 +234,17 @@ void dfree(T *&p) {
   p = nullptr;
 }
 
-// The per-stream buffers of one batch size and their geometry, detached from a handle (cosk_resize_batch keeps the old set
-// alive while the new one is filled).
-struct StateSet {
-  long long n_streams = 0, n_tokens = 0, t_alloc = 0;
-  int skel_per_tile = 0, tile_tokens = 0, n_tiles = 0, dense_vp = 0;
-  int64_t state_bytes = 0;
-  ActBuf xin;
-  std::vector<ActBuf> ring, out, sa, sa_x, sa_q;
-  float *d_qkv = nullptr, *d_pool_ring = nullptr, *d_dense = nullptr;
-  double *d_pool_sum = nullptr;
-  long long *d_idx = nullptr;
-};
-
-StateSet detach_state(cosk_model *m) {
-  StateSet s;
-  std::swap(s.n_streams, m->n_streams);
-  std::swap(s.n_tokens, m->n_tokens);
-  std::swap(s.t_alloc, m->t_alloc);
-  std::swap(s.skel_per_tile, m->skel_per_tile);
-  std::swap(s.tile_tokens, m->tile_tokens);
-  std::swap(s.n_tiles, m->n_tiles);
-  std::swap(s.dense_vp, m->dense_vp);
-  std::swap(s.state_bytes, m->state_bytes);
-  std::swap(s.xin, m->xin);
-  for (auto &b : m->blk) {
-    s.ring.push_back(b.ring);
-    s.out.push_back(b.out);
-    s.sa.push_back(b.sa);
-    s.sa_x.push_back(b.sa_x);
-    s.sa_q.push_back(b.sa_q);
-    b.ring = b.out = b.sa = b.sa_x = b.sa_q = ActBuf();
-  }
-  std::swap(s.d_qkv, m->d_qkv);
-  std::swap(s.d_pool_ring, m->d_pool_ring);
-  std::swap(s.d_dense, m->d_dense);
-  std::swap(s.d_pool_sum, m->d_pool_sum);
-  std::swap(s.d_idx, m->d_idx);
-  return s;
-}
-
-// The inverse of detach_state, on a handle without buffers (after free_state).
-void attach_state(cosk_model *m, StateSet &s) {
-  std::swap(s.n_streams, m->n_streams);
-  std::swap(s.n_tokens, m->n_tokens);
-  std::swap(s.t_alloc, m->t_alloc);
-  std::swap(s.skel_per_tile, m->skel_per_tile);
-  std::swap(s.tile_tokens, m->tile_tokens);
-  std::swap(s.n_tiles, m->n_tiles);
-  std::swap(s.dense_vp, m->dense_vp);
-  std::swap(s.state_bytes, m->state_bytes);
-  std::swap(s.xin, m->xin);
-  for (size_t i = 0; i < m->blk.size(); ++i) {
-    BlockW &b = m->blk[i];
-    b.ring = s.ring[i], b.out = s.out[i], b.sa = s.sa[i], b.sa_x = s.sa_x[i], b.sa_q = s.sa_q[i];
-  }
-  s.ring.clear(), s.out.clear(), s.sa.clear(), s.sa_x.clear(), s.sa_q.clear();
-  std::swap(s.d_qkv, m->d_qkv);
-  std::swap(s.d_pool_ring, m->d_pool_ring);
-  std::swap(s.d_dense, m->d_dense);
-  std::swap(s.d_pool_sum, m->d_pool_sum);
-  std::swap(s.d_idx, m->d_idx);
-}
-
-void free_set(StateSet &s) {
-  dfree(s.xin.ptr);
-  for (auto *v : {&s.ring, &s.out, &s.sa, &s.sa_x, &s.sa_q})
-    for (ActBuf &b : *v) dfree(b.ptr);
-  dfree(s.d_qkv);
-  dfree(s.d_pool_ring);
-  dfree(s.d_pool_sum);
-  dfree(s.d_dense);
-  dfree(s.d_idx);
-}
-
-void free_state(cosk_model *m) {
-  StateSet s = detach_state(m);
-  free_set(s);
+// Frees what alloc_batch allocated, also when it stopped half way, and leaves `b` empty.
+void free_batch(Batch &b) {
+  dfree(b.xin.ptr);
+  for (BlockBufs &k : b.blk)
+    for (ActBuf *a : {&k.ring, &k.out, &k.sa, &k.sa_x, &k.sa_q}) dfree(a->ptr);
+  dfree(b.d_qkv);
+  dfree(b.d_pool_ring);
+  dfree(b.d_pool_sum);
+  dfree(b.d_dense);
+  dfree(b.d_idx);
+  b = Batch();
 }
 
 int make_map(cosk_model *m, CUtensorMap *map, void *base, uint64_t cols, uint64_t rows, uint32_t box_rows) {
@@ -308,13 +260,13 @@ int make_map(cosk_model *m, CUtensorMap *map, void *base, uint64_t cols, uint64_
   return COSK_OK;
 }
 
-int alloc_act(cosk_model *m, ActBuf &b, int slots, int c) {
+int alloc_act(cosk_model *m, Batch &bt, ActBuf &b, int slots, int c) {
   b.slots = slots;
   b.c = c;
   b.cs = round_up(c, 8);
-  b.t_alloc = m->t_alloc;
+  b.t_alloc = bt.t_alloc;
   CK(cudaMalloc(&b.ptr, b.bytes()));
-  m->state_bytes += (int64_t)b.bytes();
+  bt.state_bytes += (int64_t)b.bytes();
   b.has_map = false;
   if (b.cs % kBK == 0) {
     int rc = make_map(m, &b.map, b.ptr, (uint64_t)b.cs, (uint64_t)slots * 2 * b.t_alloc, kTileRows);
@@ -692,30 +644,29 @@ int prepare(cosk_model *m) {
 }
 
 // Zeroes every state buffer (not the counters).
-int zero_buffers(cosk_model *m, cudaStream_t s) {
-  CK(cudaMemsetAsync(m->xin.ptr, 0, m->xin.bytes(), s));
-  for (auto &b : m->blk) {
-    CK(cudaMemsetAsync(b.ring.ptr, 0, b.ring.bytes(), s));
-    CK(cudaMemsetAsync(b.out.ptr, 0, b.out.bytes(), s));
+int zero_buffers(cosk_model *m, const Batch &bt, cudaStream_t s) {
+  CK(cudaMemsetAsync(bt.xin.ptr, 0, bt.xin.bytes(), s));
+  for (int i = 0; i < m->cfg.n_blocks; ++i) {
+    CK(cudaMemsetAsync(bt.blk[i].ring.ptr, 0, bt.blk[i].ring.bytes(), s));
+    CK(cudaMemsetAsync(bt.blk[i].out.ptr, 0, bt.blk[i].out.bytes(), s));
   }
   if (m->cfg.classes > 0) {
     const size_t cl = (size_t)m->cfg.blocks[m->cfg.n_blocks - 1].cout;
-    CK(cudaMemsetAsync(m->d_pool_ring, 0, (size_t)m->cfg.pool_size * m->n_streams * cl * sizeof(float), s));
-    CK(cudaMemsetAsync(m->d_pool_sum, 0, (size_t)m->n_streams * cl * sizeof(double), s));
+    CK(cudaMemsetAsync(bt.d_pool_ring, 0, (size_t)m->cfg.pool_size * bt.n_streams * cl * sizeof(float), s));
+    CK(cudaMemsetAsync(bt.d_pool_sum, 0, (size_t)bt.n_streams * cl * sizeof(double), s));
   }
   return COSK_OK;
 }
 
-int zero_state(cosk_model *m, cudaStream_t s) {
-  int rc = zero_buffers(m, s);
+// Zeroes the batch's buffers and counters, and clears the handle's watchdog word and failure latch.
+int zero_state(cosk_model *m, Batch &bt, cudaStream_t s) {
+  int rc = zero_buffers(m, bt, s);
   if (rc) return rc;
-  for (auto &b : m->blk) b.n_in = b.n_out = 0;
   CK(cudaMemsetAsync(m->d_dbg, 0, 4 * sizeof(unsigned int), s));
   if (m->h_dbg) m->h_dbg[0] = 0;
   m->failed = false;
-  m->pool_n = 0;
-  m->frame = 0;
-  std::fill(m->last_flags.begin(), m->last_flags.end(), 0);
+  bt.cnt = Counters();
+  std::fill(std::begin(bt.last_flags), std::end(bt.last_flags), 0);
   return COSK_OK;
 }
 
@@ -754,37 +705,37 @@ int persistent_grid(const cosk_model *m, int items) { return std::min(items, m->
 
 // The launchers size their grids for the (frame, tile) work items of `args`: n_tiles * n_frames.
 template <int COUT>
-int launch_tc_tcn(cosk_model *m, const TcTcnArgs &args, cudaStream_t s) {
-  const dim3 grid(persistent_grid(m, m->n_tiles * args.n_frames));
+int launch_tc_tcn(cosk_model *m, const Batch &bt, const TcTcnArgs &args, cudaStream_t s) {
+  const dim3 grid(persistent_grid(m, bt.n_tiles * args.n_frames));
   CK(launch_k(k_tc_tcn<COUT>, grid, dim3(256), TcTcnCfg<COUT>::kSmemBytes, s, args));
   return COSK_OK;
 }
 template <int COUT>
-int launch_tc_tcn2(cosk_model *m, const TcTcnArgs &args, cudaStream_t s) {
+int launch_tc_tcn2(cosk_model *m, const Batch &bt, const TcTcnArgs &args, cudaStream_t s) {
   // CTA pairs: one cluster of 2 per pair of adjacent token tiles, at most one CTA per SM
-  const int n_pairs = (m->n_tiles + 1) / 2 * args.n_frames;
+  const int n_pairs = (bt.n_tiles + 1) / 2 * args.n_frames;
   const int max_clusters = m->num_sms / 2;
   const int grid = 2 * (n_pairs < max_clusters ? n_pairs : max_clusters);
   CK(launch_k(k_tc_tcn2<COUT>, dim3(grid), dim3(256), TcTcn2Cfg<COUT>::kSmemBytes, s, args));
   return COSK_OK;
 }
 template <int P, int STAGES>
-int launch_tc_gcn(cosk_model *m, const TcGcnArgs &args, cudaStream_t s) {
-  const dim3 grid(persistent_grid(m, m->n_tiles * args.n_frames));
+int launch_tc_gcn(cosk_model *m, const Batch &bt, const TcGcnArgs &args, cudaStream_t s) {
+  const dim3 grid(persistent_grid(m, bt.n_tiles * args.n_frames));
   if (m->d_trace) CK(launch_k(k_tc_gcn<P, STAGES, true>, grid, dim3(512), TcGcnCfg<P, STAGES>::kSmemBytes, s, args));
   else CK(launch_k(k_tc_gcn<P, STAGES, false>, grid, dim3(512), TcGcnCfg<P, STAGES>::kSmemBytes, s, args));
   return COSK_OK;
 }
 
 template <int P, int STAGES, int V>
-int launch_tc_agcn(cosk_model *m, const TcGcnArgs &args, cudaStream_t s) {
-  CK(launch_k(k_tc_agcn<P, STAGES, V>, dim3(persistent_grid(m, m->n_tiles)), dim3(512), TcAgcnCfg<P, STAGES>::kSmemBytes, s, args));
+int launch_tc_agcn(cosk_model *m, const Batch &bt, const TcGcnArgs &args, cudaStream_t s) {
+  CK(launch_k(k_tc_agcn<P, STAGES, V>, dim3(persistent_grid(m, bt.n_tiles)), dim3(512), TcAgcnCfg<P, STAGES>::kSmemBytes, s, args));
   return COSK_OK;
 }
 
 template <int IC, int V>
-int launch_tc_attn(cosk_model *m, const TcAttnArgs &args, cudaStream_t s) {
-  CK(launch_k(k_tc_attn<IC, V>, dim3(persistent_grid(m, m->n_tiles)), dim3(384), TcAttnCfg<IC, V>::kSmemBytes, s, args));
+int launch_tc_attn(cosk_model *m, const Batch &bt, const TcAttnArgs &args, cudaStream_t s) {
+  CK(launch_k(k_tc_attn<IC, V>, dim3(persistent_grid(m, bt.n_tiles)), dim3(384), TcAttnCfg<IC, V>::kSmemBytes, s, args));
   return COSK_OK;
 }
 
@@ -842,22 +793,23 @@ RingWalk ring_walk(long long n, int step, int slots) {
 
 // Arguments of the tensor-core graph convs for n_frames executions of block i: frame f reads slot in_walk.slot(f) of `in` and
 // writes slot ring_walk.slot(f) of the block's temporal ring.
-TcGcnArgs make_gcn_args(cosk_model *m, int i, const ActBuf &in, int n_frames, RingWalk in_walk, RingWalk ring_walk) {
+TcGcnArgs make_gcn_args(cosk_model *m, const Batch &bt, int i, const ActBuf &in, int n_frames, RingWalk in_walk, RingWalk ring_walk) {
   const cosk_block_cfg &bc = m->cfg.blocks[i];
   BlockW &b = m->blk[i];
+  const ActBuf &ring = bt.blk[i].ring;
   const bool batched = n_frames > 1;  // pointers at slot 0 of their rings, the slots from the walks
   const int in_slot = batched ? 0 : in_walk.slot0, ring_slot = batched ? 0 : ring_walk.slot0;
   TcGcnArgs a;
   a.tm_x = in.map;
   a.tm_w = b.map_gcn_w;
   a.x_row = (int)in.row_hi(in_slot);
-  a.t_alloc = (int)m->t_alloc;
+  a.t_alloc = (int)bt.t_alloc;
   a.cin = bc.cin;
   a.cout = bc.cout;
   a.V = m->cfg.vertices;
-  a.n_tiles = m->n_tiles;
-  a.tile_tokens = m->tile_tokens;
-  a.n_tokens = m->n_tokens;
+  a.n_tiles = bt.n_tiles;
+  a.tile_tokens = bt.tile_tokens;
+  a.n_tokens = bt.n_tokens;
   a.mix_ptr = b.d_mix_ptr;
   a.mix_src = b.d_mix_src;
   a.mix_val = b.d_mix_val;
@@ -867,26 +819,26 @@ TcGcnArgs make_gcn_args(cosk_model *m, int i, const ActBuf &in, int n_frames, Ri
   a.epi.r_hi = epi_res ? in.hi(in_slot) : nullptr;
   a.epi.r_lo = epi_res ? in.lo(in_slot) : nullptr;
   a.epi.cs_r = in.cs;
-  a.epi.y_hi = b.ring.hi(ring_slot);
-  a.epi.y_lo = b.ring.lo(ring_slot);
-  a.epi.cs_out = b.ring.cs;
+  a.epi.y_hi = ring.hi(ring_slot);
+  a.epi.y_lo = ring.lo(ring_slot);
+  a.epi.cs_out = ring.cs;
   a.dbg = m->d_dbg;
-  a.dense = m->d_dense;
-  a.dense_ld = 3 * m->dense_vp;
-  a.dense_vp = m->dense_vp;
+  a.dense = bt.d_dense;
+  a.dense_ld = 3 * bt.dense_vp;
+  a.dense_vp = bt.dense_vp;
   if (batched) {
     a.n_frames = n_frames;
-    a.slot_rows = (int)(2 * m->t_alloc);
+    a.slot_rows = (int)(2 * bt.t_alloc);
     a.in_walk = in_walk;
     a.out_walk = ring_walk;
     a.in_slot_elems = in.slot_elems();
-    a.out_slot_elems = b.ring.slot_elems();
+    a.out_slot_elems = ring.slot_elems();
   }
   return a;
 }
 
 // k_tc_gcnt: `a` as for k_tc_gcn (per-frame or time-batched); work items are pairs of adjacent tiles
-int launch_tc_gcnt(cosk_model *m, int i, TcGcnArgs a, cudaStream_t s) {
+int launch_tc_gcnt(cosk_model *m, const Batch &bt, int i, TcGcnArgs a, cudaStream_t s) {
   const cosk_block_cfg &bc = m->cfg.blocks[i];
   const BlockW &b = m->blk[i];
   TcGcntArgs t;
@@ -895,7 +847,7 @@ int launch_tc_gcnt(cosk_model *m, int i, TcGcnArgs a, cudaStream_t s) {
   t.g.epi.r_hi = t.g.epi.r_lo = nullptr;  // gcn_residual always rides in the GEMM here
   memcpy(t.coef, b.gcnt_coef, sizeof t.coef);
   t.n_parts = b.gcnt_parts;
-  const dim3 grid(persistent_grid(m, ((m->n_tiles + 1) / 2) * a.n_frames)), block(384);
+  const dim3 grid(persistent_grid(m, ((bt.n_tiles + 1) / 2) * a.n_frames)), block(384);
   const bool v25 = m->cfg.vertices == 25;
   if (bc.cout == 128 && bc.cin == 64) {
     if (v25) CK(launch_k(k_tc_gcnt<25, 1, 128>, grid, block, TcGcntCfg<25, 1>::kSmemBytes, s, t));
@@ -911,9 +863,9 @@ int launch_tc_gcnt(cosk_model *m, int i, TcGcnArgs a, cudaStream_t s) {
 }
 
 // k_tc_agcnt: dense mix of the adaptive graph conv, work items are single tiles
-int launch_tc_agcnt(cosk_model *m, int i, TcGcnArgs a, cudaStream_t s) {
+int launch_tc_agcnt(cosk_model *m, const Batch &bt, int i, TcGcnArgs a, cudaStream_t s) {
 #ifndef COSK_WITH_AGCNT
-  (void)i, (void)a, (void)s;
+  (void)bt, (void)i, (void)a, (void)s;
   return fail(m, COSK_ERR_STATE, "k_tc_agcnt is not compiled in (build with -DCOSK_WITH_AGCNT)");
 #else
   const cosk_block_cfg &bc = m->cfg.blocks[i];
@@ -924,7 +876,7 @@ int launch_tc_agcnt(cosk_model *m, int i, TcGcnArgs a, cudaStream_t s) {
   t.g.epi.r_hi = t.g.epi.r_lo = nullptr;  // gcn_residual rides in the GEMM as the fourth part
   memset(t.coef, 0, sizeof t.coef);
   t.n_parts = 4;
-  const dim3 grid(persistent_grid(m, m->n_tiles * a.n_frames)), block(384);
+  const dim3 grid(persistent_grid(m, bt.n_tiles * a.n_frames)), block(384);
   const bool v25 = m->cfg.vertices == 25;
   if (bc.cout == 128 && bc.cin == 64) {
     if (v25) CK(launch_k(k_tc_agcnt<25, 1, 128>, grid, block, TcAgcntCfg<25, 1>::kSmemBytes, s, t));
@@ -943,22 +895,23 @@ int launch_tc_agcnt(cosk_model *m, int i, TcGcnArgs a, cudaStream_t s) {
 // Arguments of k_tc_tcn / k_tc_tcn2 for one frame.  n_taps = kTaps: the temporal conv of input n over the slots of frames
 // n-8 .. n of the ring `x` (with phase timers); n_taps = 1: a token-major GEMM on slot 0 of `x`.  The residual rows are slot
 // res_slot of `res` (nullptr: none), taken as kb_res extra K-blocks of the GEMM, or, with `res_epi`, added by the epilogue.
-TcTcnArgs make_tc_tcn_args(const cosk_model *m, const ActBuf &x, int n_taps, long long n, int kb_per_tap, const CUtensorMap &w,
-                           const float *bias, const ActBuf *res, int res_slot, int kb_res, bool res_epi, const ActBuf &y, int y_slot) {
+TcTcnArgs make_tc_tcn_args(const cosk_model *m, const Batch &bt, const ActBuf &x, int n_taps, long long n, int kb_per_tap,
+                           const CUtensorMap &w, const float *bias, const ActBuf *res, int res_slot, int kb_res, bool res_epi,
+                           const ActBuf &y, int y_slot) {
   TcTcnArgs a;
   a.tm_ring = x.map;
   a.tm_res = kb_res ? res->map : x.map;
   a.tm_w = w;
   for (int k = 0; k < kTaps; ++k) a.tap_row[k] = (int)x.row_hi(n_taps == 1 ? 0 : mod_slot(n - (kTaps - 1) + k, x.slots));
   a.res_row = res ? (int)res->row_hi(res_slot) : 0;
-  a.t_alloc = (int)m->t_alloc;
+  a.t_alloc = (int)bt.t_alloc;
   a.n_taps = n_taps;
   a.kb_per_tap = kb_per_tap;
   a.kb_res = kb_res;
-  a.n_tiles = m->n_tiles;
-  a.tile_tokens = m->tile_tokens;
+  a.n_tiles = bt.n_tiles;
+  a.tile_tokens = bt.tile_tokens;
   a.reverse = n_taps == kTaps ? 1 : 0;
-  a.n_tokens = m->n_tokens;
+  a.n_tokens = bt.n_tokens;
   a.epi.bias = bias;
   a.epi.r_hi = res_epi ? res->hi(res_slot) : nullptr;
   a.epi.r_lo = res_epi ? res->lo(res_slot) : nullptr;
@@ -973,29 +926,30 @@ TcTcnArgs make_tc_tcn_args(const cosk_model *m, const ActBuf &x, int n_taps, lon
 
 // The 128- and 256-channel temporal convs run on CTA pairs (k_tc_tcn2) once there are two tiles to pair; the HBM-bound
 // 64-channel ones stay on single CTAs.
-bool tcn_on_pair(const cosk_model *m, int width) { return m->n_tiles >= 2 && (width == 128 || width == 256); }
+bool tcn_on_pair(const Batch &bt, int width) { return bt.n_tiles >= 2 && (width == 128 || width == 256); }
 
 // The temporal-conv kernel of output width `width` (64 / 128 / 256): the 9-tap conv of a block, or a plain token-major GEMM
 // with one tap.  `half` is the weight map with half-height boxes the 256-wide pair kernel wants.
-int launch_tcn(cosk_model *m, int width, TcTcnArgs &a, const CUtensorMap &half, cudaStream_t s) {
-  if (tcn_on_pair(m, width)) {
+int launch_tcn(cosk_model *m, const Batch &bt, int width, TcTcnArgs &a, const CUtensorMap &half, cudaStream_t s) {
+  if (tcn_on_pair(bt, width)) {
     // stacked-B width (128): CTA 0 loads the whole hi plane, CTA 1 the whole lo plane (full-height box);
     // C = 256: each CTA loads its half of the rows of both planes
     if (width > 128) a.tm_w = half;
-    if (width == 128) return launch_tc_tcn2<128>(m, a, s);
-    return launch_tc_tcn2<256>(m, a, s);
+    if (width == 128) return launch_tc_tcn2<128>(m, bt, a, s);
+    return launch_tc_tcn2<256>(m, bt, a, s);
   }
-  if (width == 64) return launch_tc_tcn<64>(m, a, s);
-  if (width == 128) return launch_tc_tcn<128>(m, a, s);
-  return launch_tc_tcn<256>(m, a, s);
+  if (width == 64) return launch_tc_tcn<64>(m, bt, a, s);
+  if (width == 128) return launch_tc_tcn<128>(m, bt, a, s);
+  return launch_tc_tcn<256>(m, bt, a, s);
 }
 
 // Self-attention unit of CoS-TR (GcnUnitAttention, only_attention): qkv conv on the data_bn-normalised frame, 8-head
 // attention over the vertices of each skeleton, then the output conv + bn + skip + ReLU -- the last one is the
 // temporal-conv kernel run with a single tap on the attention rows.
-int run_attention_unit(cosk_model *m, int i, const ActBuf &in, int in_slot, int ring_slot, cudaStream_t s) {
+int run_attention_unit(cosk_model *m, const Batch &bt, int i, const ActBuf &in, int in_slot, int ring_slot, cudaStream_t s) {
   const cosk_block_cfg &bc = m->cfg.blocks[i];
   BlockW &b = m->blk[i];
+  const BlockBufs &buf = bt.blk[i];
   const GcnRoute g = b.route.gcn;
   const int dk = bc.cout / 4, dv = bc.cout, nq = 2 * dk + dv;
   int rc;
@@ -1004,42 +958,42 @@ int run_attention_unit(cosk_model *m, int i, const ActBuf &in, int in_slot, int 
       SaAffineArgs a;
       a.x_hi = in.hi(in_slot);
       a.x_lo = in.lo(in_slot);
-      a.y_hi = b.sa_x.hi(0);
-      a.y_lo = b.sa_x.lo(0);
+      a.y_hi = buf.sa_x.hi(0);
+      a.y_lo = buf.sa_x.lo(0);
       a.cs = in.cs;
       a.c = bc.cin;
       a.V = m->cfg.vertices;
       a.scale = b.d_sa_scale;
       a.shift = b.d_sa_shift;
-      a.n_tokens = m->n_tokens;
-      const long long n = m->n_tokens * (bc.cin / 8);
+      a.n_tokens = bt.n_tokens;
+      const long long n = bt.n_tokens * (bc.cin / 8);
       CK(launch_k(k_sa_affine, dim3((unsigned)((n + 255) / 256)), dim3(256), 0, s, a));
       m->launches++;
     }
     if (g == GcnRoute::kSaTcFused) {
       TcSaArgs a;
-      a.tm_x = b.sa_x.map;
+      a.tm_x = buf.sa_x.map;
       a.tm_w = b.map_sa_fw;
-      a.x_row = (int)b.sa_x.row_hi(0);
-      a.t_alloc = (int)m->t_alloc;
+      a.x_row = (int)buf.sa_x.row_hi(0);
+      a.t_alloc = (int)bt.t_alloc;
       a.cin = bc.cin;
-      a.n_tiles = m->n_tiles;
-      a.tile_tokens = m->tile_tokens;
+      a.n_tiles = bt.n_tiles;
+      a.tile_tokens = bt.tile_tokens;
       a.V = m->cfg.vertices;
-      a.n_tokens = m->n_tokens;
+      a.n_tokens = bt.n_tokens;
       a.bias = b.d_sa_fbias;
-      a.y_hi = b.sa.hi(0);
-      a.y_lo = b.sa.lo(0);
-      a.cs_out = b.sa.cs;
+      a.y_hi = buf.sa.hi(0);
+      a.y_lo = buf.sa.lo(0);
+      a.cs_out = buf.sa.cs;
       a.dbg = m->d_dbg;
-      const dim3 grid(persistent_grid(m, m->n_tiles));
+      const dim3 grid(persistent_grid(m, bt.n_tiles));
       if (bc.cout == 128) CK(launch_k(k_tc_sa<16>, grid, dim3(384), TcSaCfg<16>::kSmemBytes, s, a));
       else CK(launch_k(k_tc_sa<32>, grid, dim3(384), TcSaCfg<32>::kSmemBytes, s, a));
       m->launches++;
     } else {  // qkv conv = single-tap temporal-conv kernel without ReLU
-      TcTcnArgs a = make_tc_tcn_args(m, b.sa_x, 1, 0, bc.cin / kBK, b.map_sa_q, b.d_sa_qbias, nullptr, 0, 0, false, b.sa_q, 0);
+      TcTcnArgs a = make_tc_tcn_args(m, bt, buf.sa_x, 1, 0, bc.cin / kBK, b.map_sa_q, b.d_sa_qbias, nullptr, 0, 0, false, buf.sa_q, 0);
       a.epi.floor = -INFINITY;
-      if ((rc = launch_tcn(m, kSaQkvCols, a, b.map_sa_q, s))) return rc;
+      if ((rc = launch_tcn(m, bt, kSaQkvCols, a, b.map_sa_q, s))) return rc;
       m->launches++;
     }
   } else {
@@ -1054,49 +1008,49 @@ int run_attention_unit(cosk_model *m, int i, const ActBuf &in, int in_slot, int 
     a.bias = b.d_sa_qkv_b;
     a.nq = nq;
     a.V = m->cfg.vertices;
-    a.n_tokens = m->n_tokens;
-    a.tile_tokens = m->tile_tokens;
-    a.qkv = m->d_qkv;
-    dim3 grid(m->n_tiles, (nq + kSimtN - 1) / kSimtN);
+    a.n_tokens = bt.n_tokens;
+    a.tile_tokens = bt.tile_tokens;
+    a.qkv = bt.d_qkv;
+    dim3 grid(bt.n_tiles, (nq + kSimtN - 1) / kSimtN);
     CK(launch_k(k_sa_qkv, grid, dim3(256), 0, s, a));
     m->launches++;
   }
   if (g != GcnRoute::kSaTcFused) {
     SaAttnArgs a;
-    a.qkv = m->d_qkv;
-    a.q_hi = g == GcnRoute::kSaTcQkv ? b.sa_q.hi(0) : nullptr;
-    a.q_lo = g == GcnRoute::kSaTcQkv ? b.sa_q.lo(0) : nullptr;
-    a.cs_q = b.sa_q.cs;
+    a.qkv = bt.d_qkv;
+    a.q_hi = g == GcnRoute::kSaTcQkv ? buf.sa_q.hi(0) : nullptr;
+    a.q_lo = g == GcnRoute::kSaTcQkv ? buf.sa_q.lo(0) : nullptr;
+    a.cs_q = buf.sa_q.cs;
     a.dk = dk;
     a.dv = dv;
     a.V = m->cfg.vertices;
-    a.n_tokens = m->n_tokens;
-    a.tile_tokens = m->tile_tokens;
-    a.y_hi = b.sa.hi(0);
-    a.y_lo = b.sa.lo(0);
-    a.cs_out = b.sa.cs;
+    a.n_tokens = bt.n_tokens;
+    a.tile_tokens = bt.tile_tokens;
+    a.y_hi = buf.sa.hi(0);
+    a.y_lo = buf.sa.lo(0);
+    a.cs_out = buf.sa.cs;
     const int dvh = dv / kSaHeads;
-    if (dvh == 8) CK(launch_k(k_sa_attn<8>, dim3(m->n_tiles), dim3(256), 0, s, a));
-    else if (dvh == 16) CK(launch_k(k_sa_attn<16>, dim3(m->n_tiles), dim3(256), 0, s, a));
-    else if (dvh == 32) CK(launch_k(k_sa_attn<32>, dim3(m->n_tiles), dim3(256), 0, s, a));
-    else CK(launch_k(k_sa_attn_any, dim3(m->n_tiles), dim3(128), 0, s, a));
+    if (dvh == 8) CK(launch_k(k_sa_attn<8>, dim3(bt.n_tiles), dim3(256), 0, s, a));
+    else if (dvh == 16) CK(launch_k(k_sa_attn<16>, dim3(bt.n_tiles), dim3(256), 0, s, a));
+    else if (dvh == 32) CK(launch_k(k_sa_attn<32>, dim3(bt.n_tiles), dim3(256), 0, s, a));
+    else CK(launch_k(k_sa_attn_any, dim3(bt.n_tiles), dim3(128), 0, s, a));
     m->launches++;
   }
   if ((rc = prof_mark(m, 1, i, s))) return rc;
   const bool skip = bc.cin == bc.cout;  // skip_conn and in_channels == out_channels (s_tr.py:464-467)
   if (b.route.sa_out_tc) {
     // the scaled skip connection is a K-block of the GEMM
-    TcTcnArgs a = make_tc_tcn_args(m, b.sa, 1, 0, bc.cout / kBK, b.map_sa_w, b.d_gcn_b, &in, in_slot, skip ? bc.cin / kBK : 0, false,
-                                   b.ring, ring_slot);
-    if ((rc = launch_tcn(m, bc.cout, a, b.map_sa_w_half, s))) return rc;
+    TcTcnArgs a = make_tc_tcn_args(m, bt, buf.sa, 1, 0, bc.cout / kBK, b.map_sa_w, b.d_gcn_b, &in, in_slot, skip ? bc.cin / kBK : 0, false,
+                                   buf.ring, ring_slot);
+    if ((rc = launch_tcn(m, bt, bc.cout, a, b.map_sa_w_half, s))) return rc;
   } else {
     TcnArgs a;
     for (int k = 0; k < kTaps; ++k) {
-      a.tap_hi[k] = b.sa.hi(0);
-      a.tap_lo[k] = b.sa.lo(0);
+      a.tap_hi[k] = buf.sa.hi(0);
+      a.tap_lo[k] = buf.sa.lo(0);
     }
     a.n_taps = 1;
-    a.cs = b.sa.cs;
+    a.cs = buf.sa.cs;
     a.c = bc.cout;
     a.w = b.d_gcn_w;
     a.r_hi = in.hi(in_slot);
@@ -1106,12 +1060,12 @@ int run_attention_unit(cosk_model *m, int i, const ActBuf &in, int in_slot, int 
     a.res_kind = skip ? COSK_RES_CONV : COSK_RES_NONE;  // diag(skip scale) as a 1x1 "conv" on the input rows
     a.w_r = b.d_res_w_sa;
     a.bias = b.d_gcn_b;
-    a.y_hi = b.ring.hi(ring_slot);
-    a.y_lo = b.ring.lo(ring_slot);
-    a.cs_out = b.ring.cs;
-    a.n_tokens = m->n_tokens;
-    a.tile_tokens = m->tile_tokens;
-    dim3 grid(m->n_tiles, (bc.cout + kSimtN - 1) / kSimtN);
+    a.y_hi = buf.ring.hi(ring_slot);
+    a.y_lo = buf.ring.lo(ring_slot);
+    a.cs_out = buf.ring.cs;
+    a.n_tokens = bt.n_tokens;
+    a.tile_tokens = bt.tile_tokens;
+    dim3 grid(bt.n_tiles, (bc.cout + kSimtN - 1) / kSimtN);
     CK(launch_k(k_tcn_simt, grid, dim3(256), 0, s, a));
   }
   m->launches++;
@@ -1120,34 +1074,40 @@ int run_attention_unit(cosk_model *m, int i, const ActBuf &in, int in_slot, int 
 
 // Graph conv of block i for n_frames executions: frame f reads slot in_walk.slot(f) of `in` and writes slot ring_walk.slot(f)
 // of the block's temporal ring.  Time-batched (n_frames > 1) only on the routes batched_ok admits.
-int run_gcn(cosk_model *m, int i, const ActBuf &in, int n_frames, RingWalk in_walk, RingWalk ring_walk, cudaStream_t s) {
+int run_gcn(cosk_model *m, const Batch &bt, int i, const ActBuf &in, int n_frames, RingWalk in_walk, RingWalk ring_walk,
+            cudaStream_t s) {
   const cosk_block_cfg &bc = m->cfg.blocks[i];
   BlockW &b = m->blk[i];
+  const BlockBufs &buf = bt.blk[i];
   const Route &r = b.route;
   const int in_slot = in_walk.slot0, ring_slot = ring_walk.slot0;  // of the single-frame launches
   int rc = prof_mark(m, bc.gconv != COSK_GCONV_PLAIN ? 4 : 1, i, s);
   if (rc) return rc;
-  if (bc.gconv == COSK_GCONV_ATTENTION) return run_attention_unit(m, i, in, in_slot, ring_slot, s);
+  if (bc.gconv == COSK_GCONV_ATTENTION) return run_attention_unit(m, bt, i, in, in_slot, ring_slot, s);
   if (r.attn == AttnRoute::kTc) {
     TcAttnArgs t;
     t.tm_x = in.map;
     t.tm_w = b.map_att_w;
     t.x_row = (int)in.row_hi(in_slot);
-    t.t_alloc = (int)m->t_alloc;
+    t.t_alloc = (int)bt.t_alloc;
     t.cin = bc.cin;
-    t.n_tiles = m->n_tiles;
-    t.tile_tokens = m->tile_tokens;
-    t.n_tokens = m->n_tokens;
+    t.n_tiles = bt.n_tiles;
+    t.tile_tokens = bt.tile_tokens;
+    t.n_tokens = bt.n_tokens;
     t.bias = b.d_att_b;
     t.adj = b.d_adj;
-    t.dense = m->d_dense;
-    t.dense_ld = 3 * m->dense_vp;
+    t.dense = bt.d_dense;
+    t.dense_ld = 3 * bt.dense_vp;
     t.dbg = m->d_dbg;
     const int ic = bc.cout / 4;
     if (m->cfg.vertices == 25)
-      rc = ic == 16 ? launch_tc_attn<16, 25>(m, t, s) : ic == 32 ? launch_tc_attn<32, 25>(m, t, s) : launch_tc_attn<64, 25>(m, t, s);
+      rc = ic == 16   ? launch_tc_attn<16, 25>(m, bt, t, s)
+           : ic == 32 ? launch_tc_attn<32, 25>(m, bt, t, s)
+                      : launch_tc_attn<64, 25>(m, bt, t, s);
     else
-      rc = ic == 16 ? launch_tc_attn<16, 18>(m, t, s) : ic == 32 ? launch_tc_attn<32, 18>(m, t, s) : launch_tc_attn<64, 18>(m, t, s);
+      rc = ic == 16   ? launch_tc_attn<16, 18>(m, bt, t, s)
+           : ic == 32 ? launch_tc_attn<32, 18>(m, bt, t, s)
+                      : launch_tc_attn<64, 18>(m, bt, t, s);
     if (rc) return rc;
   } else if (r.attn == AttnRoute::kSmall) {
     // narrow first layer: embeddings computed per thread, same per-row softmax as the tensor-core kernel
@@ -1159,12 +1119,12 @@ int run_gcn(cosk_model *m, int i, const ActBuf &in, int n_frames, RingWalk in_wa
     t.w = b.d_att_w;
     t.bias = b.d_att_b;
     t.adj = b.d_adj;
-    t.n_tokens = m->n_tokens;
-    t.tile_tokens = m->tile_tokens;
-    t.dense = m->d_dense;
-    t.dense_ld = 3 * m->dense_vp;
-    if (m->cfg.vertices == 25) CK(launch_k(k_attn_small<16, 25>, dim3(m->n_tiles), dim3(128), 0, s, t));
-    else CK(launch_k(k_attn_small<16, 18>, dim3(m->n_tiles), dim3(128), 0, s, t));
+    t.n_tokens = bt.n_tokens;
+    t.tile_tokens = bt.tile_tokens;
+    t.dense = bt.d_dense;
+    t.dense_ld = 3 * bt.dense_vp;
+    if (m->cfg.vertices == 25) CK(launch_k(k_attn_small<16, 25>, dim3(bt.n_tiles), dim3(128), 0, s, t));
+    else CK(launch_k(k_attn_small<16, 18>, dim3(bt.n_tiles), dim3(128), 0, s, t));
   } else if (r.attn == AttnRoute::kSimt) {
     // attention half: the per-token mixing rows of this frame go to the dense scratch
     AttnArgs t;
@@ -1177,12 +1137,12 @@ int run_gcn(cosk_model *m, int i, const ActBuf &in, int n_frames, RingWalk in_wa
     t.inter_c = bc.cout / 4;
     t.adj = b.d_adj;
     t.V = m->cfg.vertices;
-    t.n_tokens = m->n_tokens;
-    t.tile_tokens = m->tile_tokens;
-    t.dense = m->d_dense;
-    t.dense_ld = 3 * m->dense_vp;
-    t.dense_vp = m->dense_vp;
-    CK(launch_k(k_agcn_attn, dim3(m->n_tiles), dim3(256), (size_t)2 * t.inter_c * kTileRows * sizeof(float), s, t));
+    t.n_tokens = bt.n_tokens;
+    t.tile_tokens = bt.tile_tokens;
+    t.dense = bt.d_dense;
+    t.dense_ld = 3 * bt.dense_vp;
+    t.dense_vp = bt.dense_vp;
+    CK(launch_k(k_agcn_attn, dim3(bt.n_tiles), dim3(256), (size_t)2 * t.inter_c * kTileRows * sizeof(float), s, t));
   }
   if (r.attn != AttnRoute::kNone) {
     m->launches++;
@@ -1192,21 +1152,21 @@ int run_gcn(cosk_model *m, int i, const ActBuf &in, int n_frames, RingWalk in_wa
   const bool one_kb = bc.cin == kBK;  // one K-block per work item: single operand stage
   switch (r.gcn) {
     case GcnRoute::kTcAgcnt:
-      rc = launch_tc_agcnt(m, i, make_gcn_args(m, i, in, n_frames, in_walk, ring_walk), s);
+      rc = launch_tc_agcnt(m, bt, i, make_gcn_args(m, bt, i, in, n_frames, in_walk, ring_walk), s);
       break;
     case GcnRoute::kTcAgcn: {
-      const TcGcnArgs a = make_gcn_args(m, i, in, n_frames, in_walk, ring_walk);
-      if (b.gcn_parts == 4) rc = v25 ? launch_tc_agcn<4, 1, 25>(m, a, s) : launch_tc_agcn<4, 1, 18>(m, a, s);
-      else rc = v25 ? launch_tc_agcn<3, 2, 25>(m, a, s) : launch_tc_agcn<3, 2, 18>(m, a, s);
+      const TcGcnArgs a = make_gcn_args(m, bt, i, in, n_frames, in_walk, ring_walk);
+      if (b.gcn_parts == 4) rc = v25 ? launch_tc_agcn<4, 1, 25>(m, bt, a, s) : launch_tc_agcn<4, 1, 18>(m, bt, a, s);
+      else rc = v25 ? launch_tc_agcn<3, 2, 25>(m, bt, a, s) : launch_tc_agcn<3, 2, 18>(m, bt, a, s);
       break;
     }
     case GcnRoute::kTcT:
-      rc = launch_tc_gcnt(m, i, make_gcn_args(m, i, in, n_frames, in_walk, ring_walk), s);
+      rc = launch_tc_gcnt(m, bt, i, make_gcn_args(m, bt, i, in, n_frames, in_walk, ring_walk), s);
       break;
     case GcnRoute::kTc: {
-      const TcGcnArgs a = make_gcn_args(m, i, in, n_frames, in_walk, ring_walk);
-      if (b.gcn_parts == 4) rc = one_kb ? launch_tc_gcn<4, 1>(m, a, s) : launch_tc_gcn<4, 2>(m, a, s);
-      else rc = one_kb ? launch_tc_gcn<3, 1>(m, a, s) : launch_tc_gcn<3, 2>(m, a, s);
+      const TcGcnArgs a = make_gcn_args(m, bt, i, in, n_frames, in_walk, ring_walk);
+      if (b.gcn_parts == 4) rc = one_kb ? launch_tc_gcn<4, 1>(m, bt, a, s) : launch_tc_gcn<4, 2>(m, bt, a, s);
+      else rc = one_kb ? launch_tc_gcn<3, 1>(m, bt, a, s) : launch_tc_gcn<3, 2>(m, bt, a, s);
       break;
     }
     default: {  // kSimt, kSmall (time-batched: blockIdx.y = frame, pointers at slot 0 of their rings)
@@ -1217,9 +1177,9 @@ int run_gcn(cosk_model *m, int i, const ActBuf &in, int n_frames, RingWalk in_wa
       a.x_lo = in.lo(batched ? 0 : in_slot);
       a.cs_in = in.cs;
       a.cin = bc.cin;
-      a.y_hi = b.ring.hi(batched ? 0 : ring_slot);
-      a.y_lo = b.ring.lo(batched ? 0 : ring_slot);
-      a.cs_out = b.ring.cs;
+      a.y_hi = buf.ring.hi(batched ? 0 : ring_slot);
+      a.y_lo = buf.ring.lo(batched ? 0 : ring_slot);
+      a.cs_out = buf.ring.cs;
       a.cout = bc.cout;
       a.w = b.d_gcn_w;
       a.bias = b.d_gcn_b;
@@ -1229,22 +1189,22 @@ int run_gcn(cosk_model *m, int i, const ActBuf &in, int n_frames, RingWalk in_wa
       a.mix_src = b.d_mix_src;
       a.mix_val = b.d_mix_val;
       a.V = m->cfg.vertices;
-      a.n_tokens = m->n_tokens;
-      a.tile_tokens = m->tile_tokens;
-      a.dense = bc.gconv == COSK_GCONV_ADAPTIVE ? m->d_dense : nullptr;
-      a.dense_ld = 3 * m->dense_vp;
-      a.dense_vp = m->dense_vp;
+      a.n_tokens = bt.n_tokens;
+      a.tile_tokens = bt.tile_tokens;
+      a.dense = bc.gconv == COSK_GCONV_ADAPTIVE ? bt.d_dense : nullptr;
+      a.dense_ld = 3 * bt.dense_vp;
+      a.dense_vp = bt.dense_vp;
       if (batched) {
         a.in_walk = in_walk;
         a.out_walk = ring_walk;
         a.in_slot_elems = in.slot_elems();
-        a.out_slot_elems = b.ring.slot_elems();
+        a.out_slot_elems = buf.ring.slot_elems();
       }
       const int K = (3 + res_conv) * bc.cin;
       if (r.gcn == GcnRoute::kSmall)
-        CK(launch_k(k_gcn_small, dim3(m->n_tiles, n_frames), dim3(256), (size_t)(K + 1) * bc.cout * sizeof(float), s, a));
+        CK(launch_k(k_gcn_small, dim3(bt.n_tiles, n_frames), dim3(256), (size_t)(K + 1) * bc.cout * sizeof(float), s, a));
       else
-        CK(launch_k(k_gcn_simt, dim3(m->n_tiles, (bc.cout + kSimtN - 1) / kSimtN), dim3(256), 0, s, a));
+        CK(launch_k(k_gcn_simt, dim3(bt.n_tiles, (bc.cout + kSimtN - 1) / kSimtN), dim3(256), 0, s, a));
     }
   }
   if (rc) return rc;
@@ -1254,36 +1214,38 @@ int run_gcn(cosk_model *m, int i, const ActBuf &in, int n_frames, RingWalk in_wa
 
 // Temporal conv of block i for n_frames firing executions, the first on input n: frame f adds the delayed residual from slot
 // res_walk.slot(f) of `in` and writes slot out_walk.slot(f) of the block's output ring (time-batched: tensor cores only).
-int run_tcn(cosk_model *m, int i, const ActBuf &in, long long n, int n_frames, RingWalk res_walk, RingWalk out_walk, cudaStream_t s) {
+int run_tcn(cosk_model *m, const Batch &bt, int i, const ActBuf &in, long long n, int n_frames, RingWalk res_walk, RingWalk out_walk,
+            cudaStream_t s) {
   const cosk_block_cfg &bc = m->cfg.blocks[i];
   BlockW &b = m->blk[i];
+  const BlockBufs &buf = bt.blk[i];
   int rc = prof_mark(m, 2, i, s);
   if (rc) return rc;
   if (b.route.tcn_tc) {
     const bool batched = n_frames > 1;  // pointers at slot 0 of their rings, the slots from the walks
     const bool kblock = tcn_res_kblock(bc);
-    TcTcnArgs a = make_tc_tcn_args(m, b.ring, kTaps, n, bc.cout / kBK, b.map_tcn_w, b.d_tcn_b, &in, batched ? 0 : res_walk.slot0,
-                                   kblock ? bc.cin / kBK : 0, bc.res_kind == COSK_RES_IDENTITY && !kblock, b.out,
+    TcTcnArgs a = make_tc_tcn_args(m, bt, buf.ring, kTaps, n, bc.cout / kBK, b.map_tcn_w, b.d_tcn_b, &in, batched ? 0 : res_walk.slot0,
+                                   kblock ? bc.cin / kBK : 0, bc.res_kind == COSK_RES_IDENTITY && !kblock, buf.out,
                                    batched ? 0 : out_walk.slot0);
     if (batched) {
       a.n_frames = n_frames;
-      a.slot_rows = (int)(2 * m->t_alloc);
-      a.tap_walk = ring_walk(n - (kTaps - 1), bc.stride, m->R);
+      a.slot_rows = (int)(2 * bt.t_alloc);
+      a.tap_walk = ring_walk(n - (kTaps - 1), bc.stride, bt.R);
       a.res_walk = res_walk;
       a.out_walk = out_walk;
-      a.out_slot_elems = b.out.slot_elems();
+      a.out_slot_elems = buf.out.slot_elems();
       a.res_slot_elems = in.slot_elems();
     }
-    if ((rc = launch_tcn(m, bc.cout, a, b.map_tcn_w_half, s))) return rc;
+    if ((rc = launch_tcn(m, bt, bc.cout, a, b.map_tcn_w_half, s))) return rc;
   } else {
     TcnArgs a;
     for (int k = 0; k < kTaps; ++k) {
-      const int slot = mod_slot(n - (kTaps - 1) + k, m->R);  // frame n-8+k
-      a.tap_hi[k] = b.ring.hi(slot);
-      a.tap_lo[k] = b.ring.lo(slot);
+      const int slot = mod_slot(n - (kTaps - 1) + k, bt.R);  // frame n-8+k
+      a.tap_hi[k] = buf.ring.hi(slot);
+      a.tap_lo[k] = buf.ring.lo(slot);
     }
     a.n_taps = kTaps;
-    a.cs = b.ring.cs;
+    a.cs = buf.ring.cs;
     a.c = bc.cout;
     a.w = b.d_tcn_w;
     a.r_hi = in.hi(res_walk.slot0);
@@ -1293,12 +1255,12 @@ int run_tcn(cosk_model *m, int i, const ActBuf &in, long long n, int n_frames, R
     a.res_kind = bc.res_kind;
     a.w_r = b.d_res_w;
     a.bias = b.d_tcn_b;
-    a.y_hi = b.out.hi(out_walk.slot0);
-    a.y_lo = b.out.lo(out_walk.slot0);
-    a.cs_out = b.out.cs;
-    a.n_tokens = m->n_tokens;
-    a.tile_tokens = m->tile_tokens;
-    dim3 grid(m->n_tiles, (bc.cout + kSimtN - 1) / kSimtN);
+    a.y_hi = buf.out.hi(out_walk.slot0);
+    a.y_lo = buf.out.lo(out_walk.slot0);
+    a.cs_out = buf.out.cs;
+    a.n_tokens = bt.n_tokens;
+    a.tile_tokens = bt.tile_tokens;
+    dim3 grid(bt.n_tiles, (bc.cout + kSimtN - 1) / kSimtN);
     CK(launch_k(k_tcn_simt, grid, dim3(256), 0, s, a));
   }
   m->launches++;
@@ -1306,56 +1268,59 @@ int run_tcn(cosk_model *m, int i, const ActBuf &in, long long n, int n_frames, R
 }
 
 // Graph conv + temporal conv of a 64 -> 64 block as one launch (k_tc_block64).  `fire`: the temporal conv emits on this step.
-int run_block64(cosk_model *m, int i, const ActBuf &in, int in_slot, long long n, bool fire, int res_slot, int out_slot, cudaStream_t s) {
+int run_block64(cosk_model *m, const Batch &bt, int i, const ActBuf &in, int in_slot, long long n, bool fire, int res_slot, int out_slot,
+                cudaStream_t s) {
   BlockW &b = m->blk[i];
+  const BlockBufs &buf = bt.blk[i];
   int rc = prof_mark(m, 5, i, s);
   if (rc) return rc;
   TcBlockArgs a;
   a.tm_x = in.map;
-  a.tm_ring = b.ring.map;
+  a.tm_ring = buf.ring.map;
   a.tm_gw = b.map_gcnp_w;
   a.tm_tw = b.map_tcn_w_full;
   a.n_parts = b.gcnp_parts;
   a.x_row = (int)in.row_hi(in_slot);
   a.res_row = fire ? (int)in.row_hi(res_slot) : 0;
-  for (int k = 0; k < kTaps - 1; ++k) a.tap_row[k] = (int)b.ring.row_hi(mod_slot(n - (kTaps - 1) + k, m->R));  // frame n-8+k
-  a.t_alloc = (int)m->t_alloc;
+  for (int k = 0; k < kTaps - 1; ++k) a.tap_row[k] = (int)buf.ring.row_hi(mod_slot(n - (kTaps - 1) + k, bt.R));  // frame n-8+k
+  a.t_alloc = (int)bt.t_alloc;
   a.with_tcn = fire ? 1 : 0;
   a.V = m->cfg.vertices;
-  a.n_tiles = m->n_tiles;
-  a.tile_tokens = m->tile_tokens;
-  a.n_tokens = m->n_tokens;
+  a.n_tiles = bt.n_tiles;
+  a.tile_tokens = bt.tile_tokens;
+  a.n_tokens = bt.n_tokens;
   a.mix_ptr = b.d_mix_ptr;
   a.mix_src = b.d_mix_src;
   a.mix_val = b.d_mix_val;
   a.gbias = b.d_gcn_b;
-  const int ring_slot = (int)(n % m->R);
-  a.g_hi = b.ring.hi(ring_slot);
-  a.g_lo = b.ring.lo(ring_slot);
-  a.cs_g = b.ring.cs;
+  const int ring_slot = (int)(n % bt.R);
+  a.g_hi = buf.ring.hi(ring_slot);
+  a.g_lo = buf.ring.lo(ring_slot);
+  a.cs_g = buf.ring.cs;
   a.tepi.bias = b.d_tcn_b;
   a.tepi.r_hi = nullptr;  // the delayed identity residual is a K-block of the temporal GEMM
   a.tepi.r_lo = nullptr;
   a.tepi.cs_r = 0;
-  a.tepi.y_hi = b.out.hi(out_slot);
-  a.tepi.y_lo = b.out.lo(out_slot);
-  a.tepi.cs_out = b.out.cs;
+  a.tepi.y_hi = buf.out.hi(out_slot);
+  a.tepi.y_lo = buf.out.lo(out_slot);
+  a.tepi.cs_out = buf.out.cs;
   a.trace = m->d_trace;
   a.dbg = m->d_dbg;
-  CK(launch_k(k_tc_block64, dim3(persistent_grid(m, m->n_tiles)), dim3(512), TcBlockCfg::kSmemBytes, s, a));
+  CK(launch_k(k_tc_block64, dim3(persistent_grid(m, bt.n_tiles)), dim3(512), TcBlockCfg::kSmemBytes, s, a));
   m->launches++;
   return COSK_OK;
 }
 
 // k_input: n_frames input frames (frame f at x + f * x_frame_stride) -> slots walk.slot(f) of the input ring, data_bn folded in
-int run_input(cosk_model *m, const float *x, long long nc_stride, long long x_frame_stride, int n_frames, RingWalk walk, cudaStream_t s) {
+int run_input(cosk_model *m, const Batch &bt, const float *x, long long nc_stride, long long x_frame_stride, int n_frames,
+              RingWalk walk, cudaStream_t s) {
   const cosk_config &c = m->cfg;
-  const long long total = m->n_tokens * m->xin.cs;
+  const long long total = bt.n_tokens * bt.xin.cs;
   const int threads = 256;
   const long long blocks = (total + threads - 1) / threads;
   CK(launch_k(k_input, dim3((unsigned)blocks, (unsigned)n_frames), dim3(threads), 0, s, x, nc_stride, c.c_in, c.vertices, c.persons,
-              (const float *)(c.data_bn ? m->d_bn_scale : nullptr), (const float *)(c.data_bn ? m->d_bn_shift : nullptr), m->xin.hi(0),
-              m->xin.lo(0), m->xin.cs, m->n_tokens, x_frame_stride, walk, m->xin.slot_elems()));
+              (const float *)(c.data_bn ? m->d_bn_scale : nullptr), (const float *)(c.data_bn ? m->d_bn_shift : nullptr), bt.xin.hi(0),
+              bt.xin.lo(0), bt.xin.cs, bt.n_tokens, x_frame_stride, walk, bt.xin.slot_elems()));
   m->launches++;
   return COSK_OK;
 }
@@ -1363,10 +1328,10 @@ int run_input(cosk_model *m, const float *x, long long nc_stride, long long x_fr
 // k_head over n_frames emissions of the last block, frame f from slot in_walk.slot(f) of its output ring (`zero`: one zero
 // vector enters the pooling window instead).  One frame emits logits iff `emit`; more emit from frame first_emit on,
 // emission j at out + j * out_stride.
-int run_head(cosk_model *m, int n_frames, RingWalk in_walk, bool zero, int emit, int first_emit, float *out, long long out_stride,
-             cudaStream_t s) {
+int run_head(cosk_model *m, Batch &bt, int n_frames, RingWalk in_walk, bool zero, int emit, int first_emit, float *out,
+             long long out_stride, cudaStream_t s) {
   const cosk_config &c = m->cfg;
-  const ActBuf &y = m->blk[c.n_blocks - 1].out;
+  const ActBuf &y = bt.blk[c.n_blocks - 1].out;
   const bool batched = n_frames > 1;  // y_* at slot 0 of the ring, the slots from the walk
   int rc = prof_mark(m, 3, -1, s);
   if (rc) return rc;
@@ -1377,11 +1342,11 @@ int run_head(cosk_model *m, int n_frames, RingWalk in_walk, bool zero, int emit,
   h.c = y.c;
   h.V = c.vertices;
   h.S = c.persons;
-  h.ring = m->d_pool_ring;
-  h.sum = m->d_pool_sum;
-  h.slot = (int)(m->pool_n % c.pool_size);
+  h.ring = bt.d_pool_ring;
+  h.sum = bt.d_pool_sum;
+  h.slot = (int)(bt.cnt.pool_n % c.pool_size);
   h.P = c.pool_size;
-  h.n_streams = m->n_streams;
+  h.n_streams = bt.n_streams;
   h.emit = emit;
   h.w = m->d_fc_w;
   h.b = m->d_fc_b;
@@ -1394,18 +1359,18 @@ int run_head(cosk_model *m, int n_frames, RingWalk in_walk, bool zero, int emit,
     h.in_walk = in_walk;
     h.in_slot_elems = y.slot_elems();
   }
-  CK(launch_k(k_head, dim3((unsigned)((m->n_streams + kHeadStreams - 1) / kHeadStreams)), dim3(256 * kHeadStreams),
+  CK(launch_k(k_head, dim3((unsigned)((bt.n_streams + kHeadStreams - 1) / kHeadStreams)), dim3(256 * kHeadStreams),
               (size_t)kHeadStreams * (2 * y.cs + y.c) * sizeof(float), s, h));
   m->launches++;
-  m->pool_n += n_frames;
+  bt.cnt.pool_n += n_frames;
   return COSK_OK;
 }
 
 // k_read_block: slot `slot` of a block's output ring -> fp32 at dst
-int read_block(cosk_model *m, const ActBuf &o, int slot, float *dst, cudaStream_t s) {
-  const long long total = m->n_tokens * o.c;
+int read_block(cosk_model *m, const Batch &bt, const ActBuf &o, int slot, float *dst, cudaStream_t s) {
+  const long long total = bt.n_tokens * o.c;
   CK(launch_k(k_read_block, dim3((unsigned)((total + 255) / 256)), dim3(256), 0, s, (const __nv_bfloat16 *)o.hi(slot),
-              (const __nv_bfloat16 *)o.lo(slot), o.cs, o.c, m->cfg.vertices, m->n_tokens, dst));
+              (const __nv_bfloat16 *)o.lo(slot), o.cs, o.c, m->cfg.vertices, bt.n_tokens, dst));
   m->launches++;
   return COSK_OK;
 }
@@ -1428,43 +1393,46 @@ long long head_skip(const cosk_config &c, long long pool_n, long long F) {
   return std::min(std::max((long long)c.pool_size - 1 - c.pool_padding - pool_n, 0LL), F);
 }
 
-// One frame of the emission bookkeeping from counters n_in (per block) and pool_n: advances them, writes n_blocks + 1 flags
-// laid out like cosk_last_schedule.
-void schedule_frame(const cosk_config &c, long long *n_in, long long *pool_n, int32_t *flags) {
+// One frame of the emission bookkeeping: advances n_in and pool_n of `k`, writes n_blocks + 1 flags laid out like
+// cosk_last_schedule.
+void schedule_frame(const cosk_config &c, Counters &k, int32_t *flags) {
   bool alive = true;
   for (int i = 0; i < c.n_blocks; ++i) {
     flags[i] = 0;
     if (!alive) continue;
-    alive = firing(c.padding, c.blocks[i].stride, n_in[i]++, 1).count > 0;
+    alive = firing(c.padding, c.blocks[i].stride, k.n_in[i]++, 1).count > 0;
     flags[i] = alive ? 1 : 0;
   }
   int emit = 0;
-  if (alive) emit = c.classes > 0 ? head_skip(c, (*pool_n)++, 1) == 0 : 1;
+  if (alive) emit = c.classes > 0 ? head_skip(c, k.pool_n++, 1) == 0 : 1;
   flags[c.n_blocks] = emit;
 }
 
-// The counters schedule_frame reaches after `frames` frames from zero.
-void counters_at(const cosk_config &c, long long frames, long long *n_in, long long *pool_n) {
+// The counters the walk (and schedule_frame) reaches after `frames` frames from zero.
+Counters counters_at(const cosk_config &c, long long frames) {
+  Counters k;
+  k.frame = frames;
   long long n = frames;
   for (int i = 0; i < c.n_blocks; ++i) {
-    n_in[i] = n;
-    n = firing(c.padding, c.blocks[i].stride, 0, n).count;
+    k.n_in[i] = n;
+    n = k.n_out[i] = firing(c.padding, c.blocks[i].stride, 0, n).count;
   }
-  *pool_n = c.classes > 0 ? n : 0;
+  k.pool_n = c.classes > 0 ? n : 0;
+  return k;
 }
 
 // Every block has reached its first firing input and the pooling window its first emission: the schedule is periodic.
-bool past_warmup(const cosk_config &c, const long long *n_in, long long pool_n) {
+bool past_warmup(const cosk_config &c, const Counters &k) {
   for (int i = 0; i < c.n_blocks; ++i)
-    if (n_in[i] < firing(c.padding, c.blocks[i].stride, 0, 0).first) return false;
-  return c.classes <= 0 || head_skip(c, pool_n, 1) == 0;
+    if (k.n_in[i] < firing(c.padding, c.blocks[i].stride, 0, 0).first) return false;
+  return c.classes <= 0 || head_skip(c, k.pool_n, 1) == 0;
 }
 
 // ---- the walk over the stack (cosk_step, cosk_steps) ---------------------------------------------------------------
 // Time-batched chunks (cosk_steps with a time chunk > 1) are available when every block runs on the tensor-core CoST-GCN
 // kernels (k_tc_gcn or k_tc_gcnt, k_gcn_small for the first layer, k_tc_tcn / k_tc_tcn2).
-bool batched_ok(const cosk_model *m) {
-  if (m->tchunk <= 1 || m->d_trace) return false;
+bool batched_ok(const cosk_model *m, const Batch &bt) {
+  if (bt.tchunk <= 1 || m->d_trace) return false;
   for (const BlockW &b : m->blk) {
     const Route &r = b.route;
     if (r.attn != AttnRoute::kNone || !r.tcn_tc) return false;
@@ -1487,47 +1455,49 @@ bool batched_ok(const cosk_model *m) {
 // temporal conv of block i (not through its graph conv: co.forward_stepping modules have no padding), `flush` = n_blocks
 // pushes one zero vector into the pooling window; whatever that emits propagates through the later stages like a regular
 // frame.  The frame counter does not advance.
-int walk(cosk_model *m, const float *x, long long nc_stride, long long x_frame_stride, int F0, bool frame_by_frame, float *out,
-         long long out_stride, int32_t max_out, int32_t *cnt, cudaStream_t s, int flush = -1) {
+int walk(cosk_model *m, Batch &bt, const float *x, long long nc_stride, long long x_frame_stride, int F0, bool frame_by_frame,
+         float *out, long long out_stride, int32_t max_out, int32_t *cnt, cudaStream_t s, int flush = -1) {
   const cosk_config &c = m->cfg;
+  Counters &k = bt.cnt;
   int rc;
   if ((rc = prof_mark(m, 0, -1, s))) return rc;
-  if (flush < 0 && (rc = run_input(m, x, nc_stride, x_frame_stride, F0, ring_walk(m->frame, 1, m->Ro), s))) return rc;
-  const ActBuf *in = &m->xin;
+  if (flush < 0 && (rc = run_input(m, bt, x, nc_stride, x_frame_stride, F0, ring_walk(k.frame, 1, bt.Ro), s))) return rc;
+  const ActBuf *in = &bt.xin;
   int F = flush < 0 ? F0 : 0;  // executions of the current block in this walk == emissions of its predecessor
   for (int i = 0; i < c.n_blocks; ++i) {
-    BlockW &b = m->blk[i];
+    const Route &route = m->blk[i].route;
+    const BlockBufs &buf = bt.blk[i];
     const cosk_block_cfg &bc = c.blocks[i];
     const bool zero_in = i == flush;  // the zero frame enters this block's temporal conv directly
     if (zero_in) F = 1;
-    m->last_flags[i] = 0;
+    bt.last_flags[i] = 0;
     if (F == 0) {
-      in = &b.out;
+      in = &buf.out;
       continue;
     }
-    const long long n0 = b.n_in;  // index of the first execution == index of the predecessor's emission
+    const long long n0 = k.n_in[i];  // index of the first execution == index of the predecessor's emission
     const Firing fire = firing(c.padding, bc.stride, n0, F);
     const int F_out = (int)fire.count;
-    const bool fused = frame_by_frame && b.route.block64 && in->has_map && !zero_in;
+    const bool fused = frame_by_frame && route.block64 && in->has_map && !zero_in;
     if (zero_in) {
-      const int rs = (int)(n0 % m->R);
-      CK(cudaMemsetAsync(b.ring.hi(rs), 0, (size_t)2 * b.ring.t_alloc * b.ring.cs * sizeof(__nv_bfloat16), s));
+      const int rs = (int)(n0 % bt.R);
+      CK(cudaMemsetAsync(buf.ring.hi(rs), 0, (size_t)2 * buf.ring.t_alloc * buf.ring.cs * sizeof(__nv_bfloat16), s));
     } else if (fused) {
-      const int res_slot = F_out > 0 ? (int)((n0 - kResDelay) % m->Ro) : 0;
-      if ((rc = run_block64(m, i, *in, (int)(n0 % m->Ro), n0, F_out > 0, res_slot, (int)(b.n_out % m->Ro), s))) return rc;
-    } else if ((rc = run_gcn(m, i, *in, F, ring_walk(n0, 1, m->Ro), ring_walk(n0, 1, m->R), s))) {
+      const int res_slot = F_out > 0 ? (int)((n0 - kResDelay) % bt.Ro) : 0;
+      if ((rc = run_block64(m, bt, i, *in, (int)(n0 % bt.Ro), n0, F_out > 0, res_slot, (int)(k.n_out[i] % bt.Ro), s))) return rc;
+    } else if ((rc = run_gcn(m, bt, i, *in, F, ring_walk(n0, 1, bt.Ro), ring_walk(n0, 1, bt.R), s))) {
       return rc;
     }
     if (F_out > 0 && !fused &&
-        (rc = run_tcn(m, i, *in, fire.first, F_out, ring_walk(fire.first - kResDelay, bc.stride, m->Ro), ring_walk(b.n_out, 1, m->Ro),
-                      s)))
+        (rc = run_tcn(m, bt, i, *in, fire.first, F_out, ring_walk(fire.first - kResDelay, bc.stride, bt.Ro),
+                      ring_walk(k.n_out[i], 1, bt.Ro), s)))
       return rc;
     // did the block fire on its last execution?  (schedule parity is defined per frame)
-    m->last_flags[i] = (F_out > 0 && fire.first + (long long)(F_out - 1) * bc.stride == n0 + F - 1) ? 1 : 0;
-    b.n_in += F;
-    b.n_out += F_out;
+    bt.last_flags[i] = (F_out > 0 && fire.first + (long long)(F_out - 1) * bc.stride == n0 + F - 1) ? 1 : 0;
+    k.n_in[i] += F;
+    k.n_out[i] += F_out;
     F = F_out;
-    in = &b.out;
+    in = &buf.out;
   }
   // head over the F emissions of the last block; a flushed zero vector enters the pooling window alone (a stack without a
   // head has no window to flush)
@@ -1535,31 +1505,30 @@ int walk(cosk_model *m, const float *x, long long nc_stride, long long x_frame_s
   if (head_zero) F = c.classes > 0 ? 1 : 0;
   int emit_last = 0;
   if (F > 0) {
-    const BlockW &last = m->blk[c.n_blocks - 1];
-    const long long o0 = last.n_out - F;  // index of the first of these emissions
+    const long long o0 = k.n_out[c.n_blocks - 1] - F;  // index of the first of these emissions
     if (c.classes > 0) {
-      const int skip = (int)head_skip(c, m->pool_n, F);  // frames before the first logits
+      const int skip = (int)head_skip(c, k.pool_n, F);  // frames before the first logits
       const int n_emit = F - skip;
       const int32_t room = *cnt < max_out ? max_out - *cnt : 0;
       float *dst = out + (long long)(*cnt < max_out ? *cnt : max_out - 1) * out_stride;
       // more emissions than room: they all land in the last slot
-      if ((rc = run_head(m, F, ring_walk(o0, 1, m->Ro), head_zero, F == 1 ? n_emit : 0, skip, dst, n_emit <= room ? out_stride : 0,
-                         s)))
+      if ((rc = run_head(m, bt, F, ring_walk(o0, 1, bt.Ro), head_zero, F == 1 ? n_emit : 0, skip, dst,
+                         n_emit <= room ? out_stride : 0, s)))
         return rc;
       *cnt += n_emit;
       emit_last = n_emit > 0 ? 1 : 0;
     } else {
       for (int f = 0; f < F; ++f) {
         float *dst = out + (long long)(*cnt < max_out ? *cnt : max_out - 1) * out_stride;
-        if ((rc = read_block(m, last.out, mod_slot(o0 + f, m->Ro), dst, s))) return rc;
+        if ((rc = read_block(m, bt, bt.blk[c.n_blocks - 1].out, mod_slot(o0 + f, bt.Ro), dst, s))) return rc;
         *cnt += 1;
       }
       emit_last = 1;
     }
   }
   if ((rc = prof_mark(m, -1, -1, s))) return rc;  // closes the last interval of this walk
-  m->last_flags[c.n_blocks] = (emit_last && m->last_flags[c.n_blocks - 1]) ? 1 : 0;
-  if (flush < 0) m->frame += F0;
+  bt.last_flags[c.n_blocks] = (emit_last && bt.last_flags[c.n_blocks - 1]) ? 1 : 0;
+  if (flush < 0) k.frame += F0;
   return COSK_OK;
 }
 
@@ -1577,14 +1546,14 @@ int end_walks(cosk_model *m, int rc, int32_t cnt, cudaStream_t s) {
 
 // F frames of a (N, C, T, V, S) clip through the stack, the first at x (nc_stride = T*V*S): chunks of the time chunk where
 // batched_ok admits them, else frame by frame (cosk_steps, cosk_prime_streams).
-int walk_frames(cosk_model *m, const float *x, long long nc_stride, int F, float *out, long long out_stride, int32_t max_out,
-                int32_t *cnt, cudaStream_t s) {
+int walk_frames(cosk_model *m, Batch &bt, const float *x, long long nc_stride, int F, float *out, long long out_stride,
+                int32_t max_out, int32_t *cnt, cudaStream_t s) {
   const long long frame_elems = (long long)m->cfg.vertices * m->cfg.persons;
-  const bool batched = batched_ok(m);
-  const int chunk = batched ? m->tchunk : 1;
+  const bool batched = batched_ok(m, bt);
+  const int chunk = batched ? bt.tchunk : 1;
   int rc = COSK_OK;
   for (int t0 = 0; t0 < F && !rc; t0 += chunk)
-    rc = walk(m, x + t0 * frame_elems, nc_stride, frame_elems, std::min(chunk, F - t0), !batched, out, out_stride, max_out, cnt, s);
+    rc = walk(m, bt, x + t0 * frame_elems, nc_stride, frame_elems, std::min(chunk, F - t0), !batched, out, out_stride, max_out, cnt, s);
   return rc;
 }
 
@@ -1606,64 +1575,88 @@ std::string gcn_name(const BlockW &b) {
   return std::string(attn[(int)b.route.attn]) + t;
 }
 
-// Allocates the per-stream buffers of `n_streams` streams on a handle without buffers (contents undefined except the
-// scratch, which starts zeroed).
-int alloc_state(cosk_model *m, int64_t n_streams) {
+// The geometry and ring sizes of `n_streams` streams at time chunk `time_chunk` into `b`, which holds no buffers; nothing
+// is allocated.  Refuses a time chunk out of range and a batch whose rings need more than 32-bit rows (`b` left empty).
+int batch_geometry(cosk_model *m, int64_t n_streams, int time_chunk, Batch &b) {
   const cosk_config &c = m->cfg;
-  m->n_streams = n_streams;
+  if (n_streams < 1 || time_chunk < 1 || time_chunk > 4096)
+    return fail(m, COSK_ERR_ARG, "%lld streams at time chunk %d", (long long)n_streams, time_chunk);
+  b.n_streams = n_streams;
+  b.tchunk = time_chunk;
+  b.R = (kRingSlots - 1) + time_chunk;
+  b.Ro = (kOutSlots - 1) + time_chunk;
   const long long skel = n_streams * c.persons;
-  m->n_tokens = skel * c.vertices;
-  m->skel_per_tile = kTileRows / c.vertices;
-  m->tile_tokens = m->skel_per_tile * c.vertices;
-  m->n_tiles = (int)((skel + m->skel_per_tile - 1) / m->skel_per_tile);
+  b.n_tokens = skel * c.vertices;
+  b.skel_per_tile = kTileRows / c.vertices;
+  b.tile_tokens = b.skel_per_tile * c.vertices;
+  const long long n_tiles = (skel + b.skel_per_tile - 1) / b.skel_per_tile;
   // +1 tile: with an odd tile count the second CTA of the last pair walks a phantom tile (loads only)
-  m->t_alloc = round_up((int)((long long)(m->n_tiles + 1) * m->tile_tokens + (kTileRows - m->tile_tokens)), 8);
-  if ((long long)m->R * 2 * m->t_alloc > 0x7fffffffLL) return fail(m, COSK_ERR_ARG, "too many streams (x time chunk) for 32-bit rows");
-  int rc = alloc_act(m, m->xin, m->Ro, c.c_in);
+  b.t_alloc = ((n_tiles + 1) * b.tile_tokens + (kTileRows - b.tile_tokens) + 7) / 8 * 8;
+  if ((long long)b.R * 2 * b.t_alloc > 0x7fffffffLL) {
+    b = Batch();
+    return fail(m, COSK_ERR_ARG, "too many streams (x time chunk) for 32-bit rows");
+  }
+  b.n_tiles = (int)n_tiles;
+  return COSK_OK;
+}
+
+int alloc_buffers(cosk_model *m, Batch &b) {
+  const cosk_config &c = m->cfg;
+  int rc = alloc_act(m, b, b.xin, b.Ro, c.c_in);
   if (rc) return rc;
   for (int i = 0; i < c.n_blocks; ++i) {
-    if ((rc = alloc_act(m, m->blk[i].ring, m->R, c.blocks[i].cout))) return rc;
-    if ((rc = alloc_act(m, m->blk[i].out, m->Ro, c.blocks[i].cout))) return rc;
+    if ((rc = alloc_act(m, b, b.blk[i].ring, b.R, c.blocks[i].cout))) return rc;
+    if ((rc = alloc_act(m, b, b.blk[i].out, b.Ro, c.blocks[i].cout))) return rc;
   }
   if (c.classes > 0) {
     const size_t cl = (size_t)c.blocks[c.n_blocks - 1].cout;
-    CK(cudaMalloc(&m->d_pool_ring, (size_t)c.pool_size * n_streams * cl * sizeof(float)));
-    CK(cudaMalloc(&m->d_pool_sum, (size_t)n_streams * cl * sizeof(double)));
-    m->state_bytes += (int64_t)((size_t)c.pool_size * n_streams * cl * sizeof(float) + (size_t)n_streams * cl * sizeof(double));
+    CK(cudaMalloc(&b.d_pool_ring, (size_t)c.pool_size * b.n_streams * cl * sizeof(float)));
+    CK(cudaMalloc(&b.d_pool_sum, (size_t)b.n_streams * cl * sizeof(double)));
+    b.state_bytes += (int64_t)((size_t)c.pool_size * b.n_streams * cl * sizeof(float) + (size_t)b.n_streams * cl * sizeof(double));
   }
   bool any_adaptive = false;
   int max_nq = 0;
   for (int i = 0; i < c.n_blocks; ++i) {
     any_adaptive |= c.blocks[i].gconv == COSK_GCONV_ADAPTIVE;
     if (c.blocks[i].gconv == COSK_GCONV_ATTENTION) {
+      BlockBufs &buf = b.blk[i];
       max_nq = std::max(max_nq, 2 * (c.blocks[i].cout / 4) + c.blocks[i].cout);
-      if ((rc = alloc_act(m, m->blk[i].sa, 1, c.blocks[i].cout))) return rc;
-      CK(cudaMemset(m->blk[i].sa.ptr, 0, m->blk[i].sa.bytes()));
+      if ((rc = alloc_act(m, b, buf.sa, 1, c.blocks[i].cout))) return rc;
+      CK(cudaMemset(buf.sa.ptr, 0, buf.sa.bytes()));
       const GcnRoute g = m->blk[i].route.gcn;
       if (g != GcnRoute::kSaSimt) {
-        if ((rc = alloc_act(m, m->blk[i].sa_x, 1, c.blocks[i].cin))) return rc;
-        CK(cudaMemset(m->blk[i].sa_x.ptr, 0, m->blk[i].sa_x.bytes()));
+        if ((rc = alloc_act(m, b, buf.sa_x, 1, c.blocks[i].cin))) return rc;
+        CK(cudaMemset(buf.sa_x.ptr, 0, buf.sa_x.bytes()));
         if (g == GcnRoute::kSaTcQkv) {
-          if ((rc = alloc_act(m, m->blk[i].sa_q, 1, kSaQkvCols))) return rc;
-          CK(cudaMemset(m->blk[i].sa_q.ptr, 0, m->blk[i].sa_q.bytes()));
+          if ((rc = alloc_act(m, b, buf.sa_q, 1, kSaQkvCols))) return rc;
+          CK(cudaMemset(buf.sa_q.ptr, 0, buf.sa_q.bytes()));
         }
       }
     }
   }
   if (max_nq) {
-    const size_t bytes = (size_t)m->t_alloc * max_nq * sizeof(float);
-    CK(cudaMalloc(&m->d_qkv, bytes));
-    m->state_bytes += (int64_t)bytes;  // scratch, counted in the footprint
+    const size_t bytes = (size_t)b.t_alloc * max_nq * sizeof(float);
+    CK(cudaMalloc(&b.d_qkv, bytes));
+    b.state_bytes += (int64_t)bytes;  // scratch, counted in the footprint
   }
   if (any_adaptive) {
-    m->dense_vp = round_up(c.vertices, 4);
-    const size_t bytes = (size_t)m->t_alloc * 3 * m->dense_vp * sizeof(float);
-    CK(cudaMalloc(&m->d_dense, bytes));
-    CK(cudaMemset(m->d_dense, 0, bytes));
-    m->state_bytes += (int64_t)bytes;  // scratch, not state, but part of the per-stream footprint
+    b.dense_vp = round_up(c.vertices, 4);
+    const size_t bytes = (size_t)b.t_alloc * 3 * b.dense_vp * sizeof(float);
+    CK(cudaMalloc(&b.d_dense, bytes));
+    CK(cudaMemset(b.d_dense, 0, bytes));
+    b.state_bytes += (int64_t)bytes;  // scratch, not state, but part of the per-stream footprint
   }
-  CK(cudaMalloc(&m->d_idx, (size_t)n_streams * sizeof(long long)));  // index list of the per-stream calls, not counted
+  CK(cudaMalloc(&b.d_idx, (size_t)b.n_streams * sizeof(long long)));  // index list of the per-stream calls, not counted
   return COSK_OK;
+}
+
+// Builds the batch of `n_streams` streams at time chunk `time_chunk` into `b`, which holds no buffers: counters zero,
+// buffer contents undefined except the scratch, which starts zeroed.  Refusals (batch_geometry) come before any
+// allocation; on failure `b` is left empty.
+int alloc_batch(cosk_model *m, int64_t n_streams, int time_chunk, Batch &b) {
+  int rc = batch_geometry(m, n_streams, time_chunk, b);
+  if (!rc && (rc = alloc_buffers(m, b))) free_batch(b);
+  return rc;
 }
 
 }  // namespace
@@ -1701,7 +1694,6 @@ int cosk_create(const cosk_config *cfg, cosk_model **out) {
   cosk_model *m = new cosk_model();
   m->cfg = *cfg;
   m->blk.resize(cfg->n_blocks);
-  m->last_flags.assign(cfg->n_blocks + 1, 0);
   int ndev = 0;
   cudaError_t e = cudaGetDeviceCount(&ndev);
   if (e != cudaSuccess || cfg->device < 0 || cfg->device >= ndev) {
@@ -1757,7 +1749,7 @@ int cosk_create(const cosk_config *cfg, cosk_model **out) {
 void cosk_destroy(cosk_model *m) {
   if (!m) return;
   DeviceGuard guard_(m->cfg.device);
-  free_state(m);
+  free_batch(m->batch);
   for (auto &b : m->blk) {
     dfree(b.d_gcn_w);
     dfree(b.d_gcn_b);
@@ -1837,32 +1829,31 @@ int cosk_load_weights(cosk_model *m, const char *name, const float *host, size_t
 int cosk_set_batch(cosk_model *m, int64_t n_streams) { return cosk_set_batch_ex(m, n_streams, 1); }
 
 int cosk_set_batch_ex(cosk_model *m, int64_t n_streams, int32_t time_chunk) {
-  if (!m || n_streams < 1 || time_chunk < 1 || time_chunk > 4096) return COSK_ERR_ARG;
+  if (!m) return COSK_ERR_ARG;
+  Batch nb;
+  int rc = batch_geometry(m, n_streams, time_chunk, nb);  // a refused call leaves the handle's batch as it was
+  if (rc) return rc;
   DeviceGuard guard_(m->cfg.device);
-  m->tchunk = time_chunk;
-  m->R = (kRingSlots - 1) + time_chunk;
-  m->Ro = (kOutSlots - 1) + time_chunk;
-  if (!m->prepared) {
-    int rc = prepare(m);
-    if (rc) return rc;
+  if (!m->prepared && (rc = prepare(m))) return rc;
+  CK(cudaDeviceSynchronize());
+  free_batch(m->batch);  // before the new one is allocated: the peak is the new state alone
+  rc = alloc_batch(m, n_streams, time_chunk, nb);
+  if (!rc) rc = zero_state(m, nb, 0);
+  if (!rc && cudaDeviceSynchronize() != cudaSuccess) rc = fail(m, COSK_ERR_CUDA, "cosk_set_batch: zeroing the state failed");
+  if (rc) {  // the handle stays without a batch until a cosk_set_batch succeeds
+    free_batch(nb);
+    return rc;
   }
-  CK(cudaDeviceSynchronize());
-  free_state(m);
-  int rc = alloc_state(m, n_streams);
-  if (rc) return rc;
-  rc = zero_state(m, 0);
-  if (rc) return rc;
-  CK(cudaDeviceSynchronize());
+  std::swap(m->batch, nb);
   return COSK_OK;
 }
 
-
 int cosk_reset(cosk_model *m) {
   if (!m) return COSK_ERR_ARG;
-  if (m->n_streams == 0) return fail(m, COSK_ERR_STATE, "cosk_reset before cosk_set_batch");
+  if (m->batch.n_streams == 0) return fail(m, COSK_ERR_STATE, "cosk_reset before cosk_set_batch");
   DeviceGuard guard_(m->cfg.device);
   CK(cudaDeviceSynchronize());
-  int rc = zero_state(m, 0);
+  int rc = zero_state(m, m->batch, 0);
   if (rc) return rc;
   CK(cudaDeviceSynchronize());
   return COSK_OK;
@@ -1872,7 +1863,7 @@ int cosk_reset(cosk_model *m) {
 // leaves the host counters ahead of the device state, and a fired pipeline watchdog (bounded mbarrier wait,
 // ptx.cuh) makes every later result garbage: both refuse further steps until cosk_reset / cosk_set_batch.
 static int step_entry(cosk_model *m, const char *what = "step") {
-  if (m->n_streams == 0) return fail(m, COSK_ERR_STATE, "%s before cosk_set_batch", what);
+  if (m->batch.n_streams == 0) return fail(m, COSK_ERR_STATE, "%s before cosk_set_batch", what);
   if (!m->prepared) return fail(m, COSK_ERR_STATE, "weights changed after cosk_set_batch: call cosk_set_batch again");
   if (m->h_dbg && m->h_dbg[0] != 0) m->failed = true;  // written by the async copy behind an earlier emitting call
   if (m->failed) {
@@ -1890,7 +1881,7 @@ int cosk_step(cosk_model *m, const float *x_dev, int64_t nc_stride, float *out_d
   if (rc) return rc;
   DeviceGuard guard_(m->cfg.device);
   int32_t cnt = 0;
-  rc = walk(m, x_dev, nc_stride, 0, 1, true, out_dev, 0, 1, &cnt, (cudaStream_t)stream);
+  rc = walk(m, m->batch, x_dev, nc_stride, 0, 1, true, out_dev, 0, 1, &cnt, (cudaStream_t)stream);
   if ((rc = end_walks(m, rc, cnt, (cudaStream_t)stream))) return rc;
   if (emitted) *emitted = cnt;
   return COSK_OK;
@@ -1908,8 +1899,9 @@ int cosk_steps_ex(cosk_model *m, const float *x_dev, int32_t T, float *out_dev, 
   if (rc) return rc;
   DeviceGuard guard_(m->cfg.device);
   const cudaStream_t s = (cudaStream_t)stream;
+  Batch &bt = m->batch;
   int32_t cnt = 0;
-  rc = walk_frames(m, x_dev, (long long)T * m->cfg.vertices * m->cfg.persons, T, out_dev, out_stride, max_out, &cnt, s);
+  rc = walk_frames(m, bt, x_dev, (long long)T * m->cfg.vertices * m->cfg.persons, T, out_dev, out_stride, max_out, &cnt, s);
   if (pad_end) {
     // The clip is over: every temporal module flushes its end padding, module by module (first the blocks in order,
     // `padding` zero frames into each temporal conv, then `pool_padding` zero vectors into the pooling window).  What a
@@ -1919,33 +1911,34 @@ int cosk_steps_ex(cosk_model *m, const float *x_dev, int32_t T, float *out_dev, 
     const int stages = m->cfg.n_blocks + 1;
     for (int st = 0; st < stages && !rc; ++st) {
       const int reps = st < m->cfg.n_blocks ? m->cfg.padding : (m->cfg.classes > 0 ? m->cfg.pool_padding : 0);
-      for (int z = 0; z < reps && !rc; ++z) rc = walk(m, nullptr, 0, 0, 1, true, out_dev, out_stride, max_out, &cnt, s, st);
+      for (int z = 0; z < reps && !rc; ++z) rc = walk(m, bt, nullptr, 0, 0, 1, true, out_dev, out_stride, max_out, &cnt, s, st);
     }
   }
   if ((rc = end_walks(m, rc, cnt, s))) return rc;
   // the padded frames are not part of the stream: the sequence ends here and the state starts over
-  if (pad_end && (rc = zero_state(m, s))) return rc;
+  if (pad_end && (rc = zero_state(m, bt, s))) return rc;
   if (n_emitted) *n_emitted = cnt;
   return COSK_OK;
 }
 
-int64_t cosk_state_bytes(const cosk_model *m) { return m ? m->state_bytes : 0; }
+int64_t cosk_state_bytes(const cosk_model *m) { return m ? m->batch.state_bytes : 0; }
 
 int cosk_last_schedule(const cosk_model *m, int32_t *flags, int32_t n) {
   if (!m || !flags || n < m->cfg.n_blocks + 1) return COSK_ERR_ARG;
-  for (int i = 0; i <= m->cfg.n_blocks; ++i) flags[i] = m->last_flags[i];
+  for (int i = 0; i <= m->cfg.n_blocks; ++i) flags[i] = m->batch.last_flags[i];
   return COSK_OK;
 }
 
-int64_t cosk_frame_count(const cosk_model *m) { return m ? m->frame : 0; }
+int64_t cosk_frame_count(const cosk_model *m) { return m ? m->batch.cnt.frame : 0; }
 
 int cosk_read_block(cosk_model *m, int32_t block, float *dst_dev, void *stream) {
   if (!m || !dst_dev || block < 0 || block >= m->cfg.n_blocks) return COSK_ERR_ARG;
-  if (m->n_streams == 0) return fail(m, COSK_ERR_STATE, "cosk_read_block before cosk_set_batch");
-  const BlockW &b = m->blk[block];
-  if (b.n_out == 0) return fail(m, COSK_ERR_STATE, "block %d has not emitted yet", block);
+  const Batch &bt = m->batch;
+  if (bt.n_streams == 0) return fail(m, COSK_ERR_STATE, "cosk_read_block before cosk_set_batch");
+  const long long n_out = bt.cnt.n_out[block];
+  if (n_out == 0) return fail(m, COSK_ERR_STATE, "block %d has not emitted yet", block);
   DeviceGuard guard_(m->cfg.device);
-  return read_block(m, b.out, (int)((b.n_out - 1) % m->Ro), dst_dev, (cudaStream_t)stream);
+  return read_block(m, bt, bt.blk[block].out, (int)((n_out - 1) % bt.Ro), dst_dev, (cudaStream_t)stream);
 }
 
 int64_t cosk_launch_count(const cosk_model *m) { return m ? m->launches : 0; }
@@ -1974,7 +1967,7 @@ int cosk_describe(const cosk_model *m, char *buf, size_t n) {
       o += t;
       continue;
     }
-    if (r.tcn_tc) snprintf(t, sizeof t, "%s<%d>", tcn_on_pair(m, bc.cout) ? "k_tc_tcn2" : "k_tc_tcn", bc.cout);
+    if (r.tcn_tc) snprintf(t, sizeof t, "%s<%d>", tcn_on_pair(m->batch, bc.cout) ? "k_tc_tcn2" : "k_tc_tcn", bc.cout);
     const std::string tc = r.tcn_tc ? t : "k_tcn_simt";
     snprintf(t, sizeof t, "%s{\"gcn\": \"%s\", \"tcn\": \"%s\"}", i ? ", " : "", gcn_name(m->blk[i]).c_str(), tc.c_str());
     o += t;
@@ -2007,8 +2000,8 @@ int cosk_device_error(cosk_model *m, uint32_t *code) {
 
 int cosk_simulate_schedule(const cosk_config *cfg, int32_t T, int32_t *flags) {
   if (!cfg || !flags || T < 0 || cfg->n_blocks < 1 || cfg->n_blocks > COSK_MAX_BLOCKS) return COSK_ERR_ARG;
-  long long n_in[COSK_MAX_BLOCKS] = {0}, pool_n = 0;
-  for (int t = 0; t < T; ++t) schedule_frame(*cfg, n_in, &pool_n, flags + (size_t)t * (cfg->n_blocks + 1));
+  Counters k;
+  for (int t = 0; t < T; ++t) schedule_frame(*cfg, k, flags + (size_t)t * (cfg->n_blocks + 1));
   return COSK_OK;
 }
 
@@ -2021,19 +2014,17 @@ int cosk_schedule_compatible(const cosk_config *cfg, int64_t frame_a, int64_t fr
     period *= cfg->blocks[i].stride;
   }
   if (frame_a == frame_b) return 1;
-  long long in_a[COSK_MAX_BLOCKS], in_b[COSK_MAX_BLOCKS], pool_a, pool_b;
-  counters_at(*cfg, frame_a, in_a, &pool_a);
-  counters_at(*cfg, frame_b, in_b, &pool_b);
+  Counters a = counters_at(*cfg, frame_a), b = counters_at(*cfg, frame_b);
   // Compare the flags frame by frame until both counters are past the warm-up; from there on both schedules repeat with
   // the period (the product of the strides), so one more period decides every later frame.
   int32_t fa[COSK_MAX_BLOCKS + 1], fb[COSK_MAX_BLOCKS + 1];
   long long left = -1;
   while (left != 0) {
-    schedule_frame(*cfg, in_a, &pool_a, fa);
-    schedule_frame(*cfg, in_b, &pool_b, fb);
+    schedule_frame(*cfg, a, fa);
+    schedule_frame(*cfg, b, fb);
     if (memcmp(fa, fb, sizeof(int32_t) * (cfg->n_blocks + 1)) != 0) return 0;
     if (left > 0) --left;
-    else if (past_warmup(*cfg, in_a, pool_a) && past_warmup(*cfg, in_b, pool_b)) left = period;
+    else if (past_warmup(*cfg, a) && past_warmup(*cfg, b)) left = period;
   }
   return 1;
 }
@@ -2073,45 +2064,39 @@ int cosk_profile_read(cosk_model *m, int32_t kind, int32_t block, double *ms, in
   return COSK_OK;
 }
 
-int64_t cosk_stream_bytes(const cosk_model *m) {
-  if (!m) return 0;
-  return state_args(const_cast<cosk_model *>(m)).stream_bytes;
-}
+int64_t cosk_stream_bytes(const cosk_model *m) { return m ? state_args(m, m->batch).stream_bytes : 0; }
 
 int cosk_reset_streams(cosk_model *m, const int64_t *idx, int64_t n, void *stream) {
   if (!m) return COSK_ERR_ARG;
   int rc = step_entry(m, "cosk_reset_streams");
-  if (rc || (rc = check_indices(m, idx, n, 0, m->n_streams, true))) return rc;
+  if (rc || (rc = check_indices(m, idx, n, 0, m->batch.n_streams, true))) return rc;
   DeviceGuard guard_(m->cfg.device);
-  StateArgs a = state_args(m);
-  return launch_stream_state(m, a, kStateZero, nullptr, (cudaStream_t)stream);
+  return launch_stream_state(m, m->batch, kStateZero, nullptr, (cudaStream_t)stream);
 }
 
 int cosk_export_streams(cosk_model *m, const int64_t *idx, int64_t n, void *dst_dev, cosk_stream_meta *meta, void *stream) {
   if (!m || !meta || (n > 0 && !dst_dev)) return COSK_ERR_ARG;
   int rc = step_entry(m, "cosk_export_streams");
-  if (rc || (rc = check_indices(m, idx, n, 0, m->n_streams, true))) return rc;
+  if (rc || (rc = check_indices(m, idx, n, 0, m->batch.n_streams, true))) return rc;
   DeviceGuard guard_(m->cfg.device);
   meta->abi_version = COSK_ABI_VERSION;
   meta->geometry = geometry_of(m->cfg);
-  meta->frame = m->frame;
-  StateArgs a = state_args(m);
-  return launch_stream_state(m, a, kStateGather, dst_dev, (cudaStream_t)stream);
+  meta->frame = m->batch.cnt.frame;
+  return launch_stream_state(m, m->batch, kStateGather, dst_dev, (cudaStream_t)stream);
 }
 
 int cosk_import_streams(cosk_model *m, const int64_t *idx, int64_t n, const void *src_dev, const cosk_stream_meta *meta,
                         void *stream) {
   if (!m || !meta || (n > 0 && !src_dev)) return COSK_ERR_ARG;
   int rc = step_entry(m, "cosk_import_streams");
-  if (rc || (rc = check_indices(m, idx, n, 0, m->n_streams, true))) return rc;
+  if (rc || (rc = check_indices(m, idx, n, 0, m->batch.n_streams, true))) return rc;
   if (meta->abi_version != COSK_ABI_VERSION || meta->geometry != geometry_of(m->cfg))
     return fail(m, COSK_ERR_STATE, "stream payload of another model geometry or library version");
-  if (cosk_schedule_compatible(&m->cfg, meta->frame, m->frame) != 1)
+  if (cosk_schedule_compatible(&m->cfg, meta->frame, m->batch.cnt.frame) != 1)
     return fail(m, COSK_ERR_STATE, "stream payload exported at frame %lld does not fit the schedule at frame %lld",
-                (long long)meta->frame, m->frame);
+                (long long)meta->frame, m->batch.cnt.frame);
   DeviceGuard guard_(m->cfg.device);
-  StateArgs a = state_args(m);
-  return launch_stream_state(m, a, kStateScatter, const_cast<void *>(src_dev), (cudaStream_t)stream);
+  return launch_stream_state(m, m->batch, kStateScatter, const_cast<void *>(src_dev), (cudaStream_t)stream);
 }
 
 int cosk_resize_batch(cosk_model *m, int64_t n_streams, const int64_t *src) {
@@ -2119,95 +2104,85 @@ int cosk_resize_batch(cosk_model *m, int64_t n_streams, const int64_t *src) {
   int rc = step_entry(m, "cosk_resize_batch");
   if (rc) return rc;
   if (n_streams < 1 || !src) return fail(m, COSK_ERR_ARG, "cosk_resize_batch: n_streams %lld", (long long)n_streams);
-  if ((rc = check_indices(m, src, n_streams, -1, m->n_streams, false))) return rc;
+  if ((rc = check_indices(m, src, n_streams, -1, m->batch.n_streams, false))) return rc;
   DeviceGuard guard_(m->cfg.device);
   CK(cudaDeviceSynchronize());  // no step or state call is in flight on the old buffers
-  StateArgs a = state_args(m);
-  StateSet old = detach_state(m);
-  rc = alloc_state(m, n_streams);
-  if (!rc) rc = zero_buffers(m, 0);
+  // The new batch keeps the time chunk, the counters and the last step's flags; it is filled from the old one and
+  // installed only once that has worked.
+  Batch nb;
+  rc = alloc_batch(m, n_streams, m->batch.tchunk, nb);
   if (!rc) {
-    StateArgs b = state_args(m);
-    memcpy(b.from, a.state, sizeof b.from);
-    rc = launch_stream_state(m, b, kStateMove, nullptr, 0);
+    nb.cnt = m->batch.cnt;
+    memcpy(nb.last_flags, m->batch.last_flags, sizeof nb.last_flags);
+    rc = zero_buffers(m, nb, 0);
   }
+  if (!rc) rc = launch_stream_state(m, nb, kStateMove, nullptr, 0, &m->batch);
   if (!rc && cudaDeviceSynchronize() != cudaSuccess) rc = fail(m, COSK_ERR_CUDA, "cosk_resize_batch: state move failed");
-  if (rc) {  // the handle goes back to the old buffers, untouched
-    cudaGetLastError();
-    free_state(m);
-    attach_state(m, old);
-    return rc;
-  }
-  free_set(old);
-  return COSK_OK;
+  if (rc) cudaGetLastError();
+  else std::swap(m->batch, nb);
+  free_batch(nb);  // whichever batch lost
+  return rc;
 }
 
 int cosk_prime_streams(cosk_model *m, const int64_t *idx, int64_t n, const float *x_dev, int32_t T, int32_t time_chunk,
                        void *stream) {
   if (!m) return COSK_ERR_ARG;
+  Batch &bt = m->batch;
   int rc = step_entry(m, "cosk_prime_streams");
-  if (rc || (rc = check_indices(m, idx, n, 0, m->n_streams, true))) return rc;
+  if (rc || (rc = check_indices(m, idx, n, 0, bt.n_streams, true))) return rc;
   if (T < 0 || (n > 0 && T > 0 && !x_dev) || time_chunk < 1 || time_chunk > 4096)
     return fail(m, COSK_ERR_ARG, "cosk_prime_streams: T %d, time_chunk %d", (int)T, (int)time_chunk);
   if (n == 0) return COSK_OK;
   DeviceGuard guard_(m->cfg.device);
   const cudaStream_t s = (cudaStream_t)stream;
-  const int H = (int)std::min<long long>(T, m->frame);  // the handle's streams have not seen further back either
+  const int H = (int)std::min<long long>(T, bt.cnt.frame);  // the handle's streams have not seen further back either
   if (H == 0) {
-    StateArgs a = state_args(m);
-    if ((rc = launch_stream_state(m, a, kStateZero, nullptr, s))) return rc;
+    if ((rc = launch_stream_state(m, bt, kStateZero, nullptr, s))) return rc;
     CK(cudaDeviceSynchronize());
     return COSK_OK;
   }
   const cosk_config &c = m->cfg;
   const std::vector<long long> dst = m->h_idx;
-  const HostSide saved = save_host_side(m);
-  const long long stream_bytes = state_args(m).stream_bytes;
+  const long long stream_bytes = state_args(m, bt).stream_bytes;
   const size_t out_elems = c.classes > 0 ? (size_t)n * c.classes : (size_t)n * c.persons * c.vertices * c.blocks[c.n_blocks - 1].cout;
   void *payload = nullptr;
   float *out = nullptr;
   uint32_t watchdog = 0;
-  // The n streams walk on a scratch set of their own, rings sized for `time_chunk`, from the counters of frame F - H; the
-  // handle's set waits detached and untouched.
-  StateSet own = detach_state(m);
-  m->tchunk = time_chunk;
-  m->R = (kRingSlots - 1) + time_chunk;
-  m->Ro = (kOutSlots - 1) + time_chunk;
-  rc = alloc_state(m, n);
-  if (!rc) rc = zero_buffers(m, s);
+  // The n streams walk on a scratch batch of their own, rings sized for `time_chunk`, from the counters of frame F - H.
+  // The handle's batch is not touched before the scatter, so its time chunk, counters and flags stay as they were.
+  Batch sb;
+  rc = alloc_batch(m, n, time_chunk, sb);
+  if (!rc) rc = zero_buffers(m, sb, s);
   if (!rc && (cudaMalloc(&payload, (size_t)n * stream_bytes) != cudaSuccess || cudaMalloc(&out, out_elems * sizeof(float)) != cudaSuccess))
     rc = fail(m, COSK_ERR_CUDA, "cosk_prime_streams: out of device memory for %lld streams", (long long)n);
   if (!rc) {
-    set_counters_at(m, saved.frame - H);
+    sb.cnt = counters_at(c, bt.cnt.frame - H);
     int32_t cnt = 0;  // emissions all land in the one scratch output row
-    rc = walk_frames(m, x_dev + (long long)(T - H) * c.vertices * c.persons, (long long)T * c.vertices * c.persons, H, out, 0, 1,
-                     &cnt, s);
+    rc = walk_frames(m, sb, x_dev + (long long)(T - H) * c.vertices * c.persons, (long long)T * c.vertices * c.persons, H, out, 0,
+                     1, &cnt, s);
   }
   // The counters are a function of the frame count alone, so the walk ends where the handle stands and the scratch
-  // streams' state fits the handle's schedule.
-  if (!rc && !counters_equal(m, saved)) rc = fail(m, COSK_ERR_STATE, "cosk_prime_streams: walk ended off the handle's counters");
+  // streams' state fits the handle's schedule.  (Counters is all long long: no padding bytes to compare.)
+  if (!rc && memcmp(&sb.cnt, &bt.cnt, sizeof sb.cnt) != 0)
+    rc = fail(m, COSK_ERR_STATE, "cosk_prime_streams: walk ended off the handle's counters");
   if (!rc) {
     m->h_idx.resize((size_t)n);
     for (int64_t q = 0; q < n; ++q) m->h_idx[(size_t)q] = q;
-    StateArgs a = state_args(m);
-    rc = launch_stream_state(m, a, kStateGather, payload, s);
+    rc = launch_stream_state(m, sb, kStateGather, payload, s);
   }
   if (!rc && cudaMemcpyAsync(m->h_dbg, m->d_dbg, sizeof(unsigned int), cudaMemcpyDeviceToHost, s) != cudaSuccess)
     rc = fail(m, COSK_ERR_CUDA, "cudaMemcpyAsync of the watchdog word failed");
   if (!rc && cudaDeviceSynchronize() != cudaSuccess) rc = fail(m, COSK_ERR_CUDA, "cosk_prime_streams: priming walk failed");
   if (!rc) watchdog = m->h_dbg[0];
   if (rc) cudaGetLastError();
-  free_state(m);
-  attach_state(m, own);
-  restore_host_side(m, saved);
+  free_batch(sb);
   if (!rc && watchdog) {
     m->failed = true;  // as after any walk: step_entry reports the code
     rc = fail(m, COSK_ERR_STATE, "device pipeline watchdog fired (code 0x%08x) while priming streams; cosk_reset to continue", watchdog);
   }
   if (!rc) {
     m->h_idx = dst;
-    StateArgs a = state_args(m);
-    rc = launch_stream_state(m, a, kStateScatter, payload, s);
+    rc = launch_stream_state(m, bt, kStateScatter, payload, s);
   }
   if (!rc && cudaDeviceSynchronize() != cudaSuccess) rc = fail(m, COSK_ERR_CUDA, "cosk_prime_streams: scatter failed");
   dfree(payload);

@@ -1,6 +1,6 @@
 // Host half of the per-stream state calls (cosk_reset_streams, cosk_export_streams, cosk_import_streams,
-// cosk_resize_batch, cosk_prime_streams): the payload layout as a StateArgs table, index checks, the one k_stream_state
-// launch per call, and the host-side snapshot a priming walk saves and restores.
+// cosk_resize_batch, cosk_prime_streams): the payload layout of a batch as a StateArgs table, index checks, and the one
+// k_stream_state launch per call on the batch it is handed.
 // Part of cosk.cu (included after its helpers, whose names it uses); the kernel is in stream_state.cuh.  The step route
 // table of the GPU tests covers the step kernels; k_stream_state is checked by tests/test_gpu_streams.py.
 #pragma once
@@ -36,31 +36,30 @@ void add_ring(StateArgs &a, long long &off, void *base, long long plane_bytes, i
   off += (long long)entries * planes * run_bytes;
 }
 
-void add_act_ring(cosk_model *m, StateArgs &a, long long &off, const ActBuf &b, int c, int slots, int entries, long long cnt) {
+void add_act_ring(const cosk_model *m, StateArgs &a, long long &off, const ActBuf &b, int c, int slots, int entries, long long cnt) {
   const int cs = round_up(c, 8);
   const int run = m->cfg.persons * m->cfg.vertices * cs * (int)sizeof(__nv_bfloat16);
   add_ring(a, off, b.ptr, (long long)b.t_alloc * cs * (long long)sizeof(__nv_bfloat16), run, 2, entries, slots, cnt);
 }
 
-// The layout above for the handle's buffers and counters (buffers may be absent: geometry only).
-StateArgs state_args(cosk_model *m) {
+// The layout above for the buffers and counters of a batch (an empty batch: geometry only).
+StateArgs state_args(const cosk_model *m, const Batch &bt) {
   const cosk_config &c = m->cfg;
   StateArgs a;
   memset(&a, 0, sizeof a);
   long long off = 0;
   const int first_res = c.blocks[0].res_kind != COSK_RES_NONE ? kResDelay : 0;
-  add_act_ring(m, a, off, m->xin, c.c_in, m->Ro, first_res, m->blk[0].n_in);
+  add_act_ring(m, a, off, bt.xin, c.c_in, bt.Ro, first_res, bt.cnt.n_in[0]);
   for (int i = 0; i < c.n_blocks; ++i) {
-    const BlockW &b = m->blk[i];
     const bool next_res = i + 1 < c.n_blocks && c.blocks[i + 1].res_kind != COSK_RES_NONE;
-    add_act_ring(m, a, off, b.ring, c.blocks[i].cout, m->R, kTaps - 1, b.n_in);
-    add_act_ring(m, a, off, b.out, c.blocks[i].cout, m->Ro, next_res ? kResDelay : 1, b.n_out);
+    add_act_ring(m, a, off, bt.blk[i].ring, c.blocks[i].cout, bt.R, kTaps - 1, bt.cnt.n_in[i]);
+    add_act_ring(m, a, off, bt.blk[i].out, c.blocks[i].cout, bt.Ro, next_res ? kResDelay : 1, bt.cnt.n_out[i]);
   }
   if (c.classes > 0) {
     const int cl = c.blocks[c.n_blocks - 1].cout;
-    add_ring(a, off, m->d_pool_ring, m->n_streams * cl * (long long)sizeof(float), cl * (int)sizeof(float), 1, c.pool_size,
-             c.pool_size, m->pool_n);
-    add_ring(a, off, m->d_pool_sum, m->n_streams * cl * (long long)sizeof(double), cl * (int)sizeof(double), 1, 1, 1, 1);
+    add_ring(a, off, bt.d_pool_ring, bt.n_streams * cl * (long long)sizeof(float), cl * (int)sizeof(float), 1, c.pool_size,
+             c.pool_size, bt.cnt.pool_n);
+    add_ring(a, off, bt.d_pool_sum, bt.n_streams * cl * (long long)sizeof(double), cl * (int)sizeof(double), 1, 1, 1, 1);
   }
   a.stream_bytes = off;
   return a;
@@ -69,7 +68,7 @@ StateArgs state_args(cosk_model *m) {
 // Host index list -> bounds and distinctness checked copy in m->h_idx.  lo = -1 admits "no source".
 int check_indices(cosk_model *m, const int64_t *idx, int64_t n, long long lo, long long hi, bool distinct) {
   if (n < 0 || (n > 0 && !idx)) return fail(m, COSK_ERR_ARG, "bad index list");
-  if (n > m->n_streams && distinct) return fail(m, COSK_ERR_ARG, "%lld indices for %lld streams", (long long)n, m->n_streams);
+  if (n > hi && distinct) return fail(m, COSK_ERR_ARG, "%lld indices for %lld streams", (long long)n, hi);
   std::vector<char> seen(distinct ? (size_t)hi : 0, 0);
   for (int64_t q = 0; q < n; ++q) {
     if (idx[q] < lo || idx[q] >= hi) return fail(m, COSK_ERR_ARG, "stream index %lld out of range [%lld, %lld)", (long long)idx[q], lo, hi);
@@ -79,17 +78,20 @@ int check_indices(cosk_model *m, const int64_t *idx, int64_t n, long long lo, lo
   return COSK_OK;
 }
 
-// One k_stream_state launch over the m->h_idx streams.  The index upload waits for the previous call's kernel, which
-// reads the same device buffer, so calls on different CUDA streams cannot overwrite each other's indices.
-int launch_stream_state(cosk_model *m, StateArgs &a, int mode, void *payload, cudaStream_t s) {
+// One k_stream_state launch over the m->h_idx streams of batch `bt` (kStateMove: from the batch `from`).  The index upload
+// waits for the previous call's kernel, which may read the same device buffer, so calls on different CUDA streams cannot
+// overwrite each other's indices.
+int launch_stream_state(cosk_model *m, const Batch &bt, int mode, void *payload, cudaStream_t s, const Batch *from = nullptr) {
   const long long k = (long long)m->h_idx.size();
   if (k == 0) return COSK_OK;
   if (!m->ev_idx) CK(cudaEventCreateWithFlags(&m->ev_idx, cudaEventDisableTiming));
   else CK(cudaStreamWaitEvent(s, m->ev_idx, 0));
-  CK(cudaMemcpyAsync(m->d_idx, m->h_idx.data(), (size_t)k * sizeof(long long), cudaMemcpyHostToDevice, s));
+  CK(cudaMemcpyAsync(bt.d_idx, m->h_idx.data(), (size_t)k * sizeof(long long), cudaMemcpyHostToDevice, s));
+  StateArgs a = state_args(m, bt);
+  if (from) memcpy(a.from, state_args(m, *from).state, sizeof a.from);
   a.mode = mode;
   a.k = k;
-  a.idx = m->d_idx;
+  a.idx = bt.d_idx;
   a.payload = static_cast<char *>(payload);
   const long long items = k * a.runs;
   const int grid = (int)std::min<long long>(items, (long long)m->num_sms * 8);
@@ -97,49 +99,6 @@ int launch_stream_state(cosk_model *m, StateArgs &a, int mode, void *payload, cu
   m->launches++;
   CK(cudaEventRecord(m->ev_idx, s));
   return COSK_OK;
-}
-
-// What of the handle's host side a priming walk (cosk_prime_streams) changes: the counters, the last step's flags and the
-// time chunk with the ring sizes it implies.  The walk runs on a scratch set whose rings are sized for its own chunk.
-struct HostSide {
-  long long frame = 0, pool_n = 0;
-  std::vector<long long> n_in, n_out;
-  std::vector<int32_t> last_flags;
-  int tchunk = 1, R = 0, Ro = 0;
-};
-
-HostSide save_host_side(const cosk_model *m) {
-  HostSide h;
-  h.frame = m->frame, h.pool_n = m->pool_n;
-  for (const BlockW &b : m->blk) h.n_in.push_back(b.n_in), h.n_out.push_back(b.n_out);
-  h.last_flags = m->last_flags;
-  h.tchunk = m->tchunk, h.R = m->R, h.Ro = m->Ro;
-  return h;
-}
-
-void restore_host_side(cosk_model *m, const HostSide &h) {
-  m->frame = h.frame, m->pool_n = h.pool_n;
-  for (size_t i = 0; i < m->blk.size(); ++i) m->blk[i].n_in = h.n_in[i], m->blk[i].n_out = h.n_out[i];
-  m->last_flags = h.last_flags;
-  m->tchunk = h.tchunk, m->R = h.R, m->Ro = h.Ro;
-}
-
-// The counters the walks reach after `frames` frames from zero: counters_at, plus each block's emission count.
-void set_counters_at(cosk_model *m, long long frames) {
-  const cosk_config &c = m->cfg;
-  long long n_in[COSK_MAX_BLOCKS];
-  counters_at(c, frames, n_in, &m->pool_n);
-  for (int i = 0; i < c.n_blocks; ++i) {
-    m->blk[i].n_in = n_in[i];
-    m->blk[i].n_out = firing(c.padding, c.blocks[i].stride, 0, n_in[i]).count;
-  }
-  m->frame = frames;
-}
-
-bool counters_equal(const cosk_model *m, const HostSide &h) {
-  for (size_t i = 0; i < m->blk.size(); ++i)
-    if (m->blk[i].n_in != h.n_in[i] || m->blk[i].n_out != h.n_out[i]) return false;
-  return m->frame == h.frame && m->pool_n == h.pool_n;
 }
 
 // Fingerprint of every config field that shapes the payload or the meaning of its entries (FNV-1a).

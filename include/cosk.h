@@ -107,7 +107,10 @@ void cosk_destroy(cosk_model *m);
 int cosk_load_weights(cosk_model *m, const char *name, const float *host, size_t n);
 
 /* Stands behind clean_state_on_shape_change (models/base.py:161-164): (re)allocates all state for
- * `n_streams` concurrent streams and zeroes it. */
+ * `n_streams` concurrent streams and zeroes it.  A refused call (COSK_ERR_ARG: a stream count or time chunk out of
+ * range, or rings past 32-bit rows) leaves the handle as it was.  The old state is freed before the new state is
+ * allocated; if allocating or zeroing it fails the handle has no batch, and every call that needs one returns
+ * COSK_ERR_STATE until a cosk_set_batch succeeds. */
 int cosk_set_batch(cosk_model *m, int64_t n_streams);
 /* The same with a time chunk: cosk_steps then runs the stack module by module over chunks of up to `time_chunk` frames -- one
  * launch per kernel and chunk, its work items (frame, tile) pairs -- the way the library's forward_steps walks a clip

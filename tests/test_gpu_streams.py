@@ -275,6 +275,11 @@ def test_refusals_leave_state_intact(tag):
     fe = fresh._sync(torch.device(DEV))
     assert fe.lib.cosk_reset_streams(fe.h, idx, 1, None) == -3
     assert fe.lib.cosk_resize_batch(fe.h, 1, idx) == -3
+    # a set_batch refused for 32-bit rows leaves the handle's batch as it was (checked before anything is launched on it)
+    ae, held = a._engine, a.state_bytes()
+    rc = ae.lib.cosk_set_batch(ae.h, 1 << 22)
+    assert a.state_bytes() == held
+    assert rc == -1
     allr = _rows(list(range(N)))
     for t in range(F, F + 3 * a.stride):
         oa, fa = _step(a, frames[t % 8])
